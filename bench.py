@@ -10,6 +10,7 @@ data path) => weak scaling; `value` is the whole-job particle-timesteps/s.
   python bench.py                      # 1 GPU, defaults
   torchrun ... bench.py --gpus N ...   # one rank per GPU (the driver launches this)
   python bench.py --impl reference     # the reference's own CPU implementation (oracle/_ref)
+  python bench.py --dump-outputs DIR   # also write the estimates of the last timed step to DIR/*.npy
 
 Prints ONE JSON line (rank 0).
 """
@@ -343,6 +344,18 @@ def timed_events(fn, reps, warm):
     return float(np.median(ts))
 
 
+# the estimates pmmh_flps_sv_corr returns (its diagnostics counters and workspace are not results)
+DUMP_KEYS = ("log_like", "filt", "smo", "gradient", "traj", "hess1", "hess2")
+
+
+def dump_outputs(out, path):
+    """Writes the estimates of one evaluation as float64 `<name>.npy` files under `path` (about 100 KB at
+    T = 1000), so that two builds can be compared output for output on the same seeded inputs."""
+    os.makedirs(path, exist_ok=True)
+    for k in DUMP_KEYS:
+        np.save(os.path.join(path, k + ".npy"), out[k].cpu().numpy().astype(np.float64))
+
+
 def max_over_ranks(seconds, dev, dist):
     import torch
     if dist is None:
@@ -600,6 +613,8 @@ def run_ours(args, rank, world, local_rank):
     e_all1.record()
     sync_all()
     clocks = sampler.stop()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(out, args.dump_outputs)
     total_ms = e_all0.elapsed_time(e_all1)
     kern_ms = float(np.mean([a.elapsed_time(b) for a, b in ev]))
     if dist is not None:
@@ -861,7 +876,14 @@ def main():
     ap.add_argument("--split-steps", type=int, default=1000)
     ap.add_argument("--traffic-bytes", type=float, default=None,
                     help="dram bytes per launch from the committed ncu capture (profiles/)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the estimates of the last timed step (rank 0) to DIR/<name>.npy (float64); "
+                         "GPU path only")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs covers the GPU path only (--impl ours)")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
