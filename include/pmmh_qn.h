@@ -67,7 +67,7 @@ extern "C" {
                                    difference between the reference's sequential cumulative sums and parallel ones
                                    (eps N (4 + 2 sqrt N) child-index units): only these can differ from the reference */
 #define PMMH_DIAG_TRAJ_IDX 5    /* bpf: sampled trajectory index */
-#define PMMH_DIAG_KERNEL 6      /* kernel that produced the outputs: 1 general, 2 exchange, 3 chain, 4 split */
+#define PMMH_DIAG_KERNEL 6      /* kernel that produced the outputs: 1 general, 2 exchange, 3 chain, 4 split (streaming), 5 grid */
 #define PMMH_DIAG_FAST_INFO 7   /* exchange kernel: abandon reason (1 run / 2 chunk overflow) |
                                    step << 8 | longest mailbox run << 32 */
 #define PMMH_DIAG_COUNT 8
@@ -79,20 +79,33 @@ int pmmh_device_info(int* sm_count, int* cc_major, int* cc_minor);
 
 /* ---------------------------------------------------------------- SV particle methods -- */
 
-/* Kernel selection for pmmh_flps_sv_corr (process-wide; default 0).
- *   0  automatic, for log-likelihood + gradient (compute_hessian == 0): the "chain" kernel (one
- *      CTA per problem, everything in shared memory) when n_particles <= 4096 and lag <= 10, the
- *      two-exchange "exchange" kernel for teams of CTAs; the streaming kernels for one problem
- *      with N >= 2^20 particles (faster than the exchange kernel there and without its size
- *      limit of ~1.16 M particles; variant 5 below N = 2^23, variant 4 from there on); the general kernel for everything else and as the
- *      fallback for problems those abandon (degenerate clouds)
+/* Kernel selection for pmmh_flps_sv_corr and pmmh_flps_sv_corr_streamed (per host thread; default 0).
+ *   0  automatic, tried in this order:
+ *      chain kernel (one CTA per problem, everything in shared memory): n_particles <= 4096, lag <= 10,
+ *        ctas_per_problem <= 1 (device-resident u only);
+ *      grid kernel (one persistent launch, one tile of the sorted generation per CTA): one problem,
+ *        ctas_per_problem == 0, N >= 2^14 while a tile of N / #SMs fits one CTA (N <= ~1.06 M);
+ *      streaming kernels: one problem without Hessian or history, ctas_per_problem == 0, N >= 2^20 (no
+ *        size limit; with device-resident u: variant 5 below N = 2^23, variant 4 from there on; host-streamed:
+ *        variant 5, and only where the exchange kernel does not take the size);
+ *      exchange kernel (two exchanges per step between the CTAs of a team): without Hessian, for more than
+ *        one CTA per problem (N > 1024 alone, N > 4096 in a batch, or ctas_per_problem > 1), up to ~1.16 M
+ *        particles;
+ *      general kernel: everything else (the host-streamed entry refuses instead), and after each of the
+ *        kernels above the fallback pass for problems they abandon (degenerate clouds)
  *   1  general kernel only
- *   2  diagnostics: exchange kernel where eligible, without the fallback pass
- *   3  diagnostics: chain kernel where eligible, without the fallback pass
+ *   2  exchange kernel where eligible, without the fallback pass (else the general kernel)
+ *   3  chain kernel where eligible, without the fallback pass (else the general kernel)
  *   4  streaming kernels (sv_split.cu driven on one device: ~11 launches per time step, no
- *      persistent kernel) for one problem with compute_hessian == 0 and no history output
+ *      persistent kernel) for one problem with compute_hessian == 0, no history output and
+ *      ctas_per_problem == 0, without the fallback pass (else the general kernel)
  *   5  the same with path storage: a generation is stored once in birth order (value + parent
  *      row), no records are copied; the lagged ancestors are reached through jump tables
+ *   6  grid kernel for one problem (also with compute_hessian) where a tile fits one CTA, without the
+ *      fallback pass (else the general kernel)
+ * pmmh_flps_sv_corr_streamed has no fallback pass: 0 as above, 2 the exchange kernel, 5 the streaming
+ * kernels from N = 2^20 on, 6 the grid kernel with ctas_per_problem == 0; sizes no kernel takes and the other
+ * algorithms are refused (pmmh_sv_streamed_eligible).
  * Call before pmmh_sv_workspace_bytes: the workspace size depends on it. */
 int pmmh_sv_set_algorithm(int algorithm);
 

@@ -69,184 +69,193 @@ int get_device_info(DeviceInfo* out) {
     return PMMH_OK;
 }
 
-struct SvPlan {
-    int G, n_teams, grid, NB, RING, SQ, SQW;
-    size_t stamp_bytes, sync_bytes, team_stride, total;
-    // exchange kernel (sv_fast.cu); use_fast = 0 when the problem is not eligible
-    int use_fast, NSUB, CP;
-    int use_chain;
-    size_t chain_stride, chain_total;
-    int skip_fast;           // the exchange kernel is eligible but the streaming kernels are preferred
-    int use_split;           // streaming kernels (sv_split.cu), one problem, log-likelihood + gradient
-    int split_path;          // ... with path storage (1) or with records (0)
-    size_t split_total;
-    size_t fast_sync_bytes, fast_team_stride, fast_total, general_total;
-    int use_grid, grid_G;    // grid kernel (sv_grid.cu): one problem, log-likelihood + gradient, one tile per CTA
-    size_t grid_total;
+// The SV smoother's kernels (diag[PMMH_DIAG_KERNEL] in brackets)
+enum class SvKernel {
+    None,            // host-streamed entry: no kernel takes the sizes (the call is refused)
+    General,         // sv_filter.cu, any problem (diag 1)
+    Chain,           // sv_chain.cu, one CTA per problem (diag 3)
+    Grid,            // sv_grid.cu, one problem, one tile per CTA (diag 5)
+    StreamRecords,   // sv_split.cu, one problem, genealogy records (diag 4)
+    StreamPath,      // sv_split.cu, one problem, path storage (diag 4)
+    Exchange,        // sv_fast.cu, teams of CTAs (diag 2)
+};
+// pmmh_flps_sv_corr / pmmh_bpf_sv_corr (u in device memory) or pmmh_flps_sv_corr_streamed (u in host memory)
+enum class SvEntry { Resident, HostStreamed };
+
+struct SvShape {
+    int nobs, n, lag, batch, hess, mode, hist, ctas;
 };
 
-// 0 = automatic (chain kernel for problems that fit one CTA, exchange kernel for teams of CTAs,
-//     general kernel otherwise and as their fallback),
-// 1 = general kernel only, 2 = exchange kernel where eligible WITHOUT the fallback pass (diagnostics),
-// 3 = chain kernel where eligible WITHOUT the fallback pass (diagnostics)
+struct SvChoice {
+    SvKernel kernel;
+    bool fallback;   // the general kernel re-runs the problems `kernel` abandoned (diag status 1)
+    int G;           // general kernel: CTAs per problem (its summation order depends on it); exchange kernel too
+    int grid_G;      // grid kernel: CTAs (tiles)
+    int NSUB, CP;    // exchange kernel
+};
+
+struct SvPlan {
+    SvChoice c;
+    // general kernel
+    int G, n_teams, grid, NB, RING, SQ, SQW;
+    size_t stamp_bytes, sync_bytes, team_stride;
+    // chain / exchange kernel
+    size_t chain_stride, fast_sync_bytes, fast_team_stride;
+    size_t total;   // the chosen kernel's workspace; on the resident entry at least the general kernel's
+};
+
+// pmmh_sv_set_algorithm (0 = automatic; how each value selects the kernel: sv_choose).
 // The selection is per host thread (thread_local): a thread that calls pmmh_sv_set_algorithm changes the
 // sizing and the kernel choice of its own later calls only, so a toggle on one thread cannot land between
 // another thread's workspace query and its run call.
 thread_local int g_sv_algorithm = 0;
-int g_split_min_particles = 1 << 20;   // automatic selection of the streaming kernels from this N on
-int g_split_path_max_particles = 1 << 23;   // ... with path storage below this N, with records from it on
-int g_grid_min_particles = 1 << 14;         // automatic selection of the grid kernel from this N on (while a tile fits one CTA)
-int g_grid_hess_min_particles = 1 << 14;    // ... with the Hessian branch (T = 1000: 51.8 ms against 101.8 ms on the general kernel at 2^14)
+constexpr int kSplitMinParticles = 1 << 20;       // automatic selection of the streaming kernels from this N on
+constexpr int kSplitPathMaxParticles = 1 << 23;   // ... with path storage below this N, with records from it on
+constexpr int kGridMinParticles = 1 << 14;        // automatic selection of the grid kernel from this N on (while a tile fits one CTA)
+constexpr int kGridHessMinParticles = 1 << 14;    // ... with the Hessian branch (T = 1000: 51.8 ms against 101.8 ms on the general kernel at 2^14)
 long long* g_sv_prof = nullptr;   // development: per-CTA phase clocks of the exchange kernel
 constexpr int kMaxDynSmem = 227 * 1024;
 
-int sv_make_plan(int nobs, int n, int lag, int batch, int hess, int mode, int have_hist, int ctas,
-                 SvPlan* p, bool for_host_streamed = false) {
-    if (nobs < 2 || n < 1 || batch < 1) return fail(PMMH_ERR_INVALID, "sizes must be positive");
-    if (mode == pmmh::kSvFlps) {
-        if (lag < 2 || lag >= 64) return fail(PMMH_ERR_INVALID, "lag must be in [2, 63]");
-        if (nobs < lag + 1) return fail(PMMH_ERR_INVALID, "n_obs must be at least lag + 1");
+// Does the exchange kernel take N particles on G CTAs per problem?
+bool exchange_fits(int n, int G, int* nsub, int* cp) {
+    if (!pmmh::sv_fast_eligible(n, G)) return false;
+    *nsub = pmmh::sv_fast_nsub(n, G);
+    *cp = pmmh::sv_fast_pair_cap(n, G);
+    const long long nv = (long long)G * G * (pmmh::kFastThreads / 32) * *cp;
+    return nv < (1ll << 31) && pmmh::sv_fast_smem_bytes(n, G, *nsub) <= kMaxDynSmem &&
+           2 * *nsub + 10 <= pmmh::kMaxAllgatherHost;
+}
+
+// The kernel that evaluates shape `s` under algorithm A on `sm` SMs.  In order:
+//  1. chain: flps, A in {0, 3}, ctas <= 1, N <= 4096, lag <= 10 and its shared memory fits (resident entry
+//     only; where the rule holds but the kernel cannot run, G = 1 keeps the exchange kernel out as well);
+//  2. grid: flps, one problem, A = 6 or automatically (A = 0, ctas = 0) from N = 2^14 on, while a tile of
+//     N / G particles fits one CTA; the host-streamed entry takes it only with ctas = 0;
+//  3. streaming (resident entry): flps without Hessian or history, one problem, ctas = 0, A in {4, 5} or
+//     automatically from N = 2^20 on: there they are as fast as the exchange kernel or faster (174.7 vs
+//     181.0 ms at N = 2^20, T = 1000) and have no size limit (the exchange kernel stops at ~1.16 M
+//     particles; the general kernel is ~4x slower).  Path storage for A = 5 or, automatically, while its
+//     jump tables stay (mostly) L2 resident (7.2e9 vs 6.4e9 particle-steps/s at N = 2^22); records from
+//     N = 2^23 on (6.45e9 vs 6.24e9 at 2^23, 5.8e9 vs 4.9e9 at 2^24: random 4-byte reads from HBM);
+//  4. exchange: flps without Hessian, A = 2 or automatically for teams of CTAs (G > 1: one CTA per problem
+//     has no exchange to save, the general kernel is faster there: 8.8e9 vs 7.0e9 particle-steps/s at
+//     1024 x N = 4096).  The host-streamed entry tries it before the streaming kernels (at N = 2^20: 206 ms
+//     per call against 242 ms, whose strided reads of the particle-major slots cost more than they save)
+//     and takes those (path storage only) for A in {0, 5} from N = 2^20 on;
+//  5. the general kernel on the resident entry; the host-streamed entry has none left and refuses.
+// With A = 0 the general kernel follows a special kernel as the fallback pass; A = 2 .. 6 run theirs alone.
+SvChoice sv_choose(const SvShape& s, int A, SvEntry entry, int sm) {
+    const bool resident = entry == SvEntry::Resident;
+    const bool flps = s.mode == pmmh::kSvFlps;
+    SvChoice c = {};
+    const bool chain_rule = flps && (A == 0 || A == 3) && s.ctas <= 1 && pmmh::sv_chain_eligible(s.n, s.lag);
+    int G;
+    if (s.ctas > 0) G = s.ctas;
+    else if (chain_rule) G = 1;
+    else if (s.batch > 1) G = (s.n + 4095) / 4096;
+    else G = (s.n + 1023) / 1024;
+    if (G < 1) G = 1;
+    if (G > sm) G = sm;
+    c.G = G;
+    c.grid_G = pmmh::sv_grid_ctas(s.n, sm, s.ctas);
+    auto pick = [&](SvKernel k) {
+        c.kernel = k;
+        c.fallback = resident && A == 0 && k != SvKernel::General;
+        return c;
+    };
+    if (resident && chain_rule && pmmh::sv_chain_smem_bytes(s.n) <= kMaxDynSmem) return pick(SvKernel::Chain);
+    const int grid_min = s.hess ? kGridHessMinParticles : kGridMinParticles;
+    if (flps && s.batch == 1 && (resident || s.ctas == 0) &&
+        (A == 6 || (A == 0 && s.ctas == 0 && s.n >= grid_min)) &&
+        pmmh::sv_grid_eligible(s.nobs, s.n, s.lag, c.grid_G))
+        return pick(SvKernel::Grid);
+    const bool stream_wanted = resident ? (A == 4 || A == 5 || (A == 0 && s.n >= kSplitMinParticles))
+                                        : ((A == 0 || A == 5) && s.n >= kSplitMinParticles);
+    const bool stream = flps && !s.hess && s.batch == 1 && !s.hist && s.ctas == 0 && stream_wanted &&
+                        pmmh::sv_split_single_eligible(s.nobs, s.n, s.lag);
+    const bool path = !resident || A == 5 || (A == 0 && s.n < kSplitPathMaxParticles);
+    const SvKernel streaming = path ? SvKernel::StreamPath : SvKernel::StreamRecords;
+    if (resident && stream) return pick(streaming);
+    if (flps && !s.hess && (A == 2 || (A == 0 && G > 1)) && exchange_fits(s.n, G, &c.NSUB, &c.CP))
+        return pick(SvKernel::Exchange);
+    if (stream) return pick(streaming);
+    return pick(resident ? SvKernel::General : SvKernel::None);
+}
+
+int sv_make_plan(SvShape s, SvEntry entry, SvPlan* p) {
+    if (s.nobs < 2 || s.n < 1 || s.batch < 1) return fail(PMMH_ERR_INVALID, "sizes must be positive");
+    if (s.mode == pmmh::kSvFlps) {
+        if (s.lag < 2 || s.lag >= 64) return fail(PMMH_ERR_INVALID, "lag must be in [2, 63]");
+        if (s.nobs < s.lag + 1) return fail(PMMH_ERR_INVALID, "n_obs must be at least lag + 1");
     } else {
-        lag = 2;
+        s.lag = 2;
     }
-    if ((long long)n + nobs >= (1ll << 31)) return fail(PMMH_ERR_INVALID, "n_particles too large");
+    if ((long long)s.n + s.nobs >= (1ll << 31)) return fail(PMMH_ERR_INVALID, "n_particles too large");
     DeviceInfo di;
     int rc = get_device_info(&di);
     if (rc != PMMH_OK) return rc;
     if (di.major < 10) return fail(PMMH_ERR_NO_DEVICE, "an sm_100 (B200) device is required");
     if (!di.coop) return fail(PMMH_ERR_NO_DEVICE, "device lacks cooperative launch");
-    // log-likelihood + gradient of a problem that fits one CTA: the chain kernel (everything in
-    // shared memory, no exchanges)
-    const bool chain_ok = (mode == pmmh::kSvFlps) && pmmh::sv_chain_eligible(n, lag) &&
-                          (g_sv_algorithm == 0 || g_sv_algorithm == 3) && (ctas <= 1);
-    int G;
-    if (ctas > 0) G = ctas;
-    else if (chain_ok) G = 1;
-    else if (batch > 1) G = (n + 4095) / 4096;
-    else G = (n + 1023) / 1024;
-    if (G < 1) G = 1;
-    if (G > di.sm) G = di.sm;
+    memset(p, 0, sizeof(*p));
+    p->c = sv_choose(s, g_sv_algorithm, entry, di.sm);
+    const int G = p->c.G, n = s.n, nobs = s.nobs;
     int n_teams = di.sm / G;
-    if (n_teams > batch) n_teams = batch;
+    if (n_teams > s.batch) n_teams = s.batch;
     if (n_teams < 1) n_teams = 1;
     p->G = G;
     p->n_teams = n_teams;
     p->grid = G * n_teams;
     p->NB = ((n + 31) / 32) * 32;
     if (p->NB < 64) p->NB = 64;
-    p->RING = lag + 1;
-    p->SQ = hess ? (nobs + n - 2) / nobs + 1 : 1;
-    p->SQW = (mode != pmmh::kSvFlps) ? (n + nobs - 1) / nobs : 0;
+    p->RING = s.lag + 1;
+    p->SQ = s.hess ? (nobs + n - 2) / nobs + 1 : 1;
+    p->SQW = (s.mode != pmmh::kSvFlps) ? (n + nobs - 1) / nobs : 0;
     p->stamp_bytes = pmmh::sv_align((size_t)p->grid * sizeof(unsigned));
     p->sync_bytes = p->stamp_bytes +
                     pmmh::sv_align((size_t)n_teams * 2 * G * pmmh::kMaxAllgatherHost * sizeof(double));
-    p->team_stride = pmmh::sv_ws_layout(n, nobs, lag, p->NB, p->RING, hess, mode, p->SQ, p->SQW,
-                                        have_hist, nullptr, nullptr);
-    p->general_total = p->sync_bytes + (size_t)n_teams * p->team_stride;
-    p->total = p->general_total;
-    p->use_chain = 0;
-    p->chain_stride = p->chain_total = 0;
-    if (chain_ok && G == 1 && pmmh::sv_chain_smem_bytes(n) <= kMaxDynSmem) {
-        p->use_chain = 1;
-        p->chain_stride = pmmh::sv_chain_ws_bytes(n, lag, nobs, hess);
-        p->chain_total = (size_t)p->grid * p->chain_stride;
-        if (p->chain_total > p->total) p->total = p->chain_total;
+    p->team_stride = pmmh::sv_ws_layout(n, nobs, s.lag, p->NB, p->RING, s.hess, s.mode, p->SQ, p->SQW,
+                                        s.hist, nullptr, nullptr);
+    // the general kernel (the fallback pass) uses the head of the chosen kernel's workspace
+    if (entry == SvEntry::Resident) p->total = p->sync_bytes + (size_t)n_teams * p->team_stride;
+    size_t kernel_bytes = 0;
+    switch (p->c.kernel) {
+    case SvKernel::Chain:
+        p->chain_stride = pmmh::sv_chain_ws_bytes(n, s.lag, nobs, s.hess);
+        kernel_bytes = (size_t)p->grid * p->chain_stride;
+        break;
+    case SvKernel::Grid:
+        kernel_bytes = pmmh::sv_grid_ws_bytes(nobs, n, s.lag, p->c.grid_G, s.hist, s.hess);
+        break;
+    case SvKernel::StreamRecords: kernel_bytes = pmmh::sv_split_single_ws_bytes(nobs, n, s.lag); break;
+    case SvKernel::StreamPath: kernel_bytes = pmmh::sv_split_path_ws_bytes(nobs, n, s.lag); break;
+    case SvKernel::Exchange:
+        p->fast_sync_bytes = pmmh::sv_fast_sync_bytes(G, n_teams);
+        p->fast_team_stride = pmmh::sv_fast_ws_bytes(n, G, p->c.NSUB, p->c.CP, s.lag, s.hist);
+        kernel_bytes = p->fast_sync_bytes + (size_t)n_teams * p->fast_team_stride;
+        break;
+    default: break;
     }
-    p->use_split = 0;
-    p->split_path = 0;
-    p->split_total = 0;
-    p->use_fast = 0;
-    p->NSUB = 0;
-    p->fast_sync_bytes = p->fast_team_stride = p->fast_total = 0;
-    p->CP = 0;
-    // one CTA per problem (batches of small problems) has no exchange to save: the general kernel
-    // is the faster one there (measured: 8.8e9 vs 7.0e9 particle-steps/s at 1024 x N=4096)
-    const bool want_fast = !p->use_chain && g_sv_algorithm != 4 && g_sv_algorithm != 5 && g_sv_algorithm != 6 && ((g_sv_algorithm == 2) || (g_sv_algorithm == 0 && G > 1));
-    if (mode == pmmh::kSvFlps && !hess && want_fast && pmmh::sv_fast_eligible(n, G)) {
-        const int S = pmmh::sv_fast_nsub(n, G);
-        const int CP = pmmh::sv_fast_pair_cap(n, G);
-        const long long nv = (long long)G * G * (pmmh::kFastThreads / 32) * CP;
-        if (nv < (1ll << 31) && pmmh::sv_fast_smem_bytes(n, G, S) <= kMaxDynSmem &&
-            2 * S + 10 <= pmmh::kMaxAllgatherHost) {
-            p->use_fast = 1;
-            p->NSUB = S;
-            p->CP = CP;
-            p->fast_sync_bytes = pmmh::sv_fast_sync_bytes(G, n_teams);
-            p->fast_team_stride = pmmh::sv_fast_ws_bytes(n, G, S, CP, lag, have_hist);
-            p->fast_total = p->fast_sync_bytes + (size_t)n_teams * p->fast_team_stride;
-            if (p->fast_total > p->total) p->total = p->fast_total;
-        }
-    }
-    // one problem, log-likelihood + gradient: the grid kernel (one persistent launch, one tile of the
-    // sorted generation per CTA) while N / #SMs fits the shared memory of one CTA
-    p->use_grid = 0;
-    p->grid_G = 0;
-    p->grid_total = 0;
-    // (with compute_hessian: the kernel's second instantiation, automatically from g_grid_hess_min_particles on)
-    if (mode == pmmh::kSvFlps && batch == 1 && !p->use_chain &&
-        (g_sv_algorithm == 6 || (g_sv_algorithm == 0 && ctas == 0 && !for_host_streamed &&
-                                 n >= (hess ? g_grid_hess_min_particles : g_grid_min_particles)))) {
-        const int GG = pmmh::sv_grid_ctas(n, di.sm, ctas);
-        if (pmmh::sv_grid_eligible(nobs, n, lag, GG)) {
-            p->use_grid = 1;
-            p->grid_G = GG;
-            p->grid_total = pmmh::sv_grid_ws_bytes(nobs, n, lag, GG, have_hist, hess);
-            // (the general kernel's fallback pass uses the head of the same workspace)
-            if (p->grid_total > p->total) p->total = p->grid_total;
-        }
-    }
-    // one large problem, log-likelihood + gradient, no history dump: the streaming kernels -- on
-    // request (algorithm 4 / 5), or automatically from N = 2^20 on: there they are as fast as the
-    // exchange kernel or faster (174.7 vs 181.0 ms at N = 2^20, T = 1000) and they have no size
-    // limit (the exchange kernel stops at ~1.16 M particles; the general kernel is ~4x slower).
-    // The host-streamed entry point (pmmh_flps_sv_corr_streamed) stays on the exchange kernel.
-    p->skip_fast = 0;
-    if (mode == pmmh::kSvFlps && !hess && batch == 1 && !have_hist && ctas == 0 && !p->use_chain && !p->use_grid &&
-        (g_sv_algorithm == 4 || g_sv_algorithm == 5 ||
-         (g_sv_algorithm == 0 && !for_host_streamed && n >= g_split_min_particles)) &&
-        pmmh::sv_split_single_eligible(nobs, n, lag)) {
-        p->use_split = 1;
-        p->skip_fast = 1;
-        // automatic selection: path storage while its jump tables stay (mostly) L2 resident
-        // (7.2e9 vs 6.4e9 particle-steps/s at N = 2^22), the record variant from N = 2^23 on
-        // (6.45e9 vs 6.24e9 at 2^23, 5.8e9 vs 4.9e9 at 2^24: random 4-byte reads from HBM)
-        p->split_path = (g_sv_algorithm == 5 || (g_sv_algorithm == 0 && n < g_split_path_max_particles)) ? 1 : 0;
-        p->split_total = p->split_path ? pmmh::sv_split_path_ws_bytes(nobs, n, lag)
-                                               : pmmh::sv_split_single_ws_bytes(nobs, n, lag);
-        // the general kernel (fallback pass) reuses the head of the same workspace
-        if (p->split_total > p->total) p->total = p->split_total;
-    }
+    if (kernel_bytes > p->total) p->total = kernel_bytes;
     return PMMH_OK;
 }
 
-int sv_run(int mode, const double* d_obs, long long obs_stride, const double* d_params,
-           const double* d_rvr, const double* d_u, int nobs, int n, int lag, int batch, int hess,
-           double* d_filt, double* d_smo, double* d_ll, double* d_grad, double* d_traj, double* d_h1,
-           double* d_h2, long long* d_diag, double* d_xh, int* d_ah, void* d_ws, size_t ws_bytes,
-           int ctas, void* stream) {
-    if (!d_obs || !d_params || !d_rvr || !d_u || !d_filt || !d_ll || !d_traj || !d_diag || !d_ws)
-        return fail(PMMH_ERR_INVALID, "null pointer argument");
-    if (mode == pmmh::kSvFlps && (!d_smo || !d_grad || !d_h1 || !d_h2))
-        return fail(PMMH_ERR_INVALID, "null output pointer");
-    if ((d_xh == nullptr) != (d_ah == nullptr))
-        return fail(PMMH_ERR_INVALID, "d_x_hist and d_a_hist must be given together");
-    SvPlan p;
-    int rc = sv_make_plan(nobs, n, lag, batch, hess, mode, d_xh != nullptr, ctas, &p);
-    if (rc != PMMH_OK) return rc;
-    if (ws_bytes < p.total) return fail(PMMH_ERR_WORKSPACE, "workspace too small");
-    cudaStream_t st = (cudaStream_t)stream;
+// Arguments of the general, chain and exchange kernels (the ws_* fields are per kernel)
+pmmh::SvArgs sv_args(const SvPlan& p, const SvShape& s, const double* d_obs, long long obs_stride,
+                     const double* d_params, const double* d_rvr, const double* d_u, double* d_filt, double* d_smo,
+                     double* d_ll, double* d_grad, double* d_traj, double* d_h1, double* d_h2, long long* d_diag,
+                     double* d_xh, int* d_ah, void* d_ws) {
     pmmh::SvArgs a;
     memset(&a, 0, sizeof(a));
-    a.N = n;
-    a.NOBS = nobs;
-    a.LAG = (mode == pmmh::kSvFlps) ? lag : 2;
-    a.B = batch;
+    a.N = s.n;
+    a.NOBS = s.nobs;
+    a.LAG = (s.mode == pmmh::kSvFlps) ? s.lag : 2;
+    a.B = s.batch;
     a.G = p.G;
     a.n_teams = p.n_teams;
     a.NB = p.NB;
     a.RING = p.RING;
-    a.mode = mode;
-    a.hess = hess;
+    a.mode = s.mode;
+    a.hess = s.hess;
     a.SQ = p.SQ;
     a.SQW = p.SQW;
     a.obs = d_obs;
@@ -266,17 +275,45 @@ int sv_run(int mode, const double* d_obs, long long obs_stride, const double* d_
     a.Ahist = d_ah;
     a.prof = g_sv_prof;
     a.ws = (char*)d_ws;
-    if (p.use_chain) {
-        // chain kernel first; problems it abandons (diag status 1) are re-run by the general kernel
+    return a;
+}
+
+cudaError_t exchange_launch(const SvPlan& p, pmmh::SvArgs& a, cudaStream_t st) {
+    a.NSUB = p.c.NSUB;
+    a.CP = p.c.CP;
+    a.ws_sync_bytes = p.fast_sync_bytes;
+    a.ws_team_stride = p.fast_team_stride;
+    cudaError_t err = cudaMemsetAsync(a.ws, 0, p.fast_sync_bytes, st);
+    return err != cudaSuccess ? err : pmmh::sv_fast_launch(a, p.grid, st);
+}
+
+int sv_run(int mode, const double* d_obs, long long obs_stride, const double* d_params,
+           const double* d_rvr, const double* d_u, int nobs, int n, int lag, int batch, int hess,
+           double* d_filt, double* d_smo, double* d_ll, double* d_grad, double* d_traj, double* d_h1,
+           double* d_h2, long long* d_diag, double* d_xh, int* d_ah, void* d_ws, size_t ws_bytes,
+           int ctas, void* stream) {
+    if (!d_obs || !d_params || !d_rvr || !d_u || !d_filt || !d_ll || !d_traj || !d_diag || !d_ws)
+        return fail(PMMH_ERR_INVALID, "null pointer argument");
+    if (mode == pmmh::kSvFlps && (!d_smo || !d_grad || !d_h1 || !d_h2))
+        return fail(PMMH_ERR_INVALID, "null output pointer");
+    if ((d_xh == nullptr) != (d_ah == nullptr))
+        return fail(PMMH_ERR_INVALID, "d_x_hist and d_a_hist must be given together");
+    const SvShape s = {nobs, n, lag, batch, hess, mode, d_xh != nullptr, ctas};
+    SvPlan p;
+    int rc = sv_make_plan(s, SvEntry::Resident, &p);
+    if (rc != PMMH_OK) return rc;
+    if (ws_bytes < p.total) return fail(PMMH_ERR_WORKSPACE, "workspace too small");
+    cudaStream_t st = (cudaStream_t)stream;
+    pmmh::SvArgs a = sv_args(p, s, d_obs, obs_stride, d_params, d_rvr, d_u, d_filt, d_smo, d_ll, d_grad, d_traj,
+                             d_h1, d_h2, d_diag, d_xh, d_ah, d_ws);
+    switch (p.c.kernel) {
+    case SvKernel::Chain:
         a.ws_sync_bytes = 0;
         a.ws_team_stride = p.chain_stride;
         PMMH_CUDA(pmmh::sv_chain_launch(a, p.grid, st));
-        if (g_sv_algorithm == 3) return PMMH_OK;   // diagnostics: no fallback pass
-        a.only_failed = 1;
-    }
-    if (p.use_grid) {
-        // grid kernel first; an abandoned evaluation (diag status 1) is re-run by the general kernel
-        rc = pmmh::sv_grid_run(d_obs, d_params, d_rvr, d_u, nobs, n, lag, p.grid_G, d_filt, d_smo, d_ll, d_grad,
+        break;
+    case SvKernel::Grid:
+        rc = pmmh::sv_grid_run(d_obs, d_params, d_rvr, d_u, nobs, n, lag, p.c.grid_G, d_filt, d_smo, d_ll, d_grad,
                                d_traj, d_diag, d_xh, d_ah, d_ws, ws_bytes, g_sv_prof, st, 0, nullptr,
                                hess ? d_h1 : nullptr, hess ? d_h2 : nullptr);
         if (rc != PMMH_OK) return rc;
@@ -284,13 +321,10 @@ int sv_run(int mode, const double* d_obs, long long obs_stride, const double* d_
             PMMH_CUDA(cudaMemsetAsync(d_h1, 0, 16 * sizeof(double), st));
             PMMH_CUDA(cudaMemsetAsync(d_h2, 0, 16 * sizeof(double), st));
         }
-        if (g_sv_algorithm == 6) return PMMH_OK;   // diagnostics: no fallback pass
-        a.only_failed = 1;
-    }
-    if (p.use_split) {
-        // streaming kernels first; an abandoned evaluation (diag status 1) is re-run by the general
-        // kernel in the same stream
-        rc = p.split_path
+        break;
+    case SvKernel::StreamRecords:
+    case SvKernel::StreamPath:
+        rc = p.c.kernel == SvKernel::StreamPath
                  ? pmmh::sv_split_path_run(d_obs, d_params, d_rvr, d_u, nobs, n, lag, d_filt, d_smo, d_ll,
                                            d_grad, d_traj, d_diag, d_ws, ws_bytes, st)
                  : pmmh::sv_split_single_run(d_obs, d_params, d_rvr, d_u, nobs, n, lag, d_filt, d_smo, d_ll,
@@ -298,20 +332,15 @@ int sv_run(int mode, const double* d_obs, long long obs_stride, const double* d_
         if (rc != PMMH_OK) return rc;
         PMMH_CUDA(cudaMemsetAsync(d_h1, 0, 16 * sizeof(double), st));
         PMMH_CUDA(cudaMemsetAsync(d_h2, 0, 16 * sizeof(double), st));
-        if (g_sv_algorithm == 4 || g_sv_algorithm == 5) return PMMH_OK;   // no fallback pass
-        a.only_failed = 1;
+        break;
+    case SvKernel::Exchange:
+        PMMH_CUDA(exchange_launch(p, a, st));
+        break;
+    default: break;
     }
-    if (p.use_fast && !p.skip_fast && !p.use_grid) {
-        // exchange kernel first; problems it abandons (diag status 1) are re-run by the general
-        // kernel in the same stream, reusing the workspace
-        a.NSUB = p.NSUB;
-        a.CP = p.CP;
-        a.ws_sync_bytes = p.fast_sync_bytes;
-        a.ws_team_stride = p.fast_team_stride;
-        PMMH_CUDA(cudaMemsetAsync(d_ws, 0, p.fast_sync_bytes, st));
-        PMMH_CUDA(pmmh::sv_fast_launch(a, p.grid, st));
-        if (g_sv_algorithm == 2) return PMMH_OK;   // diagnostics: no fallback pass
-        a.only_failed = 1;
+    if (p.c.kernel != SvKernel::General) {
+        if (!p.c.fallback) return PMMH_OK;
+        a.only_failed = 1;   // in the same stream, reusing the workspace
     }
     a.ws_sync_bytes = p.sync_bytes;
     a.ws_team_stride = p.team_stride;
@@ -365,9 +394,9 @@ int pmmh_sv_workspace_bytes(int n_obs, int n_particles, int lag, int batch, int 
                             int mode, int have_history, int ctas_per_problem, size_t* bytes) {
     if (!bytes) return fail(PMMH_ERR_INVALID, "bytes is null");
     SvPlan p;
-    int rc = sv_make_plan(n_obs, n_particles, lag, batch, compute_hessian,
-                          mode == 0 ? pmmh::kSvFlps : pmmh::kSvBpfParity, have_history,
-                          ctas_per_problem, &p);
+    int rc = sv_make_plan({n_obs, n_particles, lag, batch, compute_hessian,
+                           mode == 0 ? pmmh::kSvFlps : pmmh::kSvBpfParity, have_history, ctas_per_problem},
+                          SvEntry::Resident, &p);
     if (rc != PMMH_OK) return rc;
     *bytes = p.total;
     return PMMH_OK;
@@ -416,43 +445,27 @@ int pmmh_flps_sv_corr_philox_workspace_bytes(int n_obs, int n_particles, int lag
 
 // ---- host-resident auxiliary variables, copied while the kernel runs ----------------------
 namespace {
-constexpr int kUChunk = 64;   // time steps per copy chunk (512-byte rows for the copy engine)
-struct StreamedState {
-    std::vector<cudaEvent_t> ev_chunk;   // streaming kernels: one event per landed chunk
-    cudaStream_t copy_stream = nullptr;
-    cudaEvent_t ev_start = nullptr, ev_reset = nullptr, ev_done = nullptr;
-};
-thread_local StreamedState g_streamed[64];
+// The copy engine lays the reference's particle-major host array down in slots of time steps: slot c holds
+// steps [c W, (c + 1) W) of every particle as rows of W doubles.
+constexpr int kUSlot = 64;        // exchange and streaming kernels (512-byte rows)
+constexpr int kGridUSlot = 256;   // grid kernel (2 KB rows)
+constexpr int kGridUTaperMin = 48;   // smallest copy of the grid kernel's tapered schedule, in time steps
 
-int streamed_chunks(int n_obs) { return (n_obs + kUChunk - 1) / kUChunk; }
-size_t streamed_data_bytes(int n_obs, int n) {
-    return (size_t)streamed_chunks(n_obs) * (size_t)n * kUChunk * sizeof(double);
+size_t staged_bytes(int n_obs, int n, int slot) {
+    return (size_t)((n_obs + slot - 1) / slot) * (size_t)n * slot * sizeof(double);
 }
-}  // namespace
 
-namespace {
-// grid kernel with host-resident u: chunks of g_grid_u_chunk time steps (2 KB rows for the copy engine)
-int grid_u_chunk() {
-    static int v = 0;
-    if (!v) {
-        const char* e = getenv("PMMH_GRID_U_CHUNK");
-        v = e ? atoi(e) : 256;
-        if (v < 16 || v > 4096 || (v & 3)) v = 256;   // a multiple of 4 (32-byte sectors of the staged rows)
-    }
-    return v;
-}
-// smallest copy of the tapered schedule of the last chunk slot, in time steps (0 = no taper)
-int grid_u_taper_min() {
-    static int v = -1;
-    if (v < 0) {
-        const char* e = getenv("PMMH_GRID_U_TAPER");
-        v = e ? atoi(e) : 48;
-        if (v < 0 || v > 4096) v = 48;
-    }
-    return v;
-}
-// next piece of the copy schedule of the host-streamed grid path (see pmmh_flps_sv_corr_streamed): time steps
-// [t0, t0 + return value); never crosses a slot of `ch` steps, ends on a multiple of 4 steps unless it ends the series
+// Next piece of a copy schedule: time steps [t0, t0 + return value).  It never crosses a slot of `ch` steps
+// and ends on a multiple of 4 steps unless it ends the series (32-byte sectors of the staged rows, ch % 4 == 0).
+// taper_min = 0: whole slots.  Otherwise the pieces get shorter towards the end of the series.  The kernel
+// needs ~0.11 ms per time step, the host link ~0.157 ms (2 KB rows: 53.5 GB/s; 1 KB: 51.7; 512 B: 48.4; and
+// ~8 ns per row whatever its width, i.e. 8.4 ms for any piece of fewer than ~52 steps at N = 2^20).  The kernel
+// can only start a piece when all of it has landed, so after the last copy it still has to work off what it was
+// behind: a piece of p steps that starts with `rem` steps to go delays the end unless
+// 0.157 p <= (0.157 - 0.11) rem + 0.11 p_last, i.e. p <= 0.3 rem + 0.7 p_last.  Hence: whole slots (widest rows)
+// while that holds, then pieces of ~0.3 x what remains, the last one ~taper_min steps.  Measured at T = 1000,
+// N = 2^20: one copy per slot 157.7 ms of copies + 26.3 ms of kernel after the last one; this schedule: see
+// DESIGN 3.
 int grid_u_next_piece(int t0, int n_obs, int ch, int taper_min) {
     const int c = t0 / ch, in = t0 - c * ch;
     const int rem = n_obs - t0;
@@ -468,10 +481,7 @@ int grid_u_next_piece(int t0, int n_obs, int ch, int taper_min) {
     if (wsteps > whole || (taper_min > 0 && whole - wsteps < (whole == rem ? taper_min / 2 : taper_min))) wsteps = whole;
     return wsteps;
 }
-size_t streamed_grid_data_bytes(int n_obs, int n) {
-    const int ch = grid_u_chunk();
-    return (size_t)((n_obs + ch - 1) / ch) * (size_t)n * ch * sizeof(double);
-}
+
 // immutable pinned table tab[i] = i: the copy engine writes &tab[rows landed] to the device flag, so
 // no call ever rewrites a host value that a queued copy may still read
 const int* step_table(int need) {
@@ -489,24 +499,78 @@ const int* step_table(int need) {
     }
     return tab;
 }
-bool streamed_grid_ok(int n_obs, int n, int lag, int ctas, int* G_out) {
-    if (!(g_sv_algorithm == 0 || g_sv_algorithm == 6) || ctas != 0) return false;
-    if (g_sv_algorithm == 0 && n < g_grid_min_particles) return false;
-    DeviceInfo di;
-    if (get_device_info(&di) != PMMH_OK || di.major < 10 || !di.coop) return false;
-    const int GG = pmmh::sv_grid_ctas(n, di.sm, 0);
-    if (!pmmh::sv_grid_eligible(n_obs, n, lag, GG)) return false;
-    if (G_out) *G_out = GG;
-    return true;
+
+// the copy stream and events of the current device and host thread
+struct StreamedState {
+    cudaStream_t copy_stream = nullptr;
+    cudaEvent_t ev_start = nullptr, ev_reset = nullptr, ev_done = nullptr;
+    std::vector<cudaEvent_t> ev_slot;   // signal by event: one per slot
+};
+
+int streamed_state(StreamedState** out) {
+    static thread_local StreamedState states[64];
+    int dev = 0;
+    PMMH_CUDA(cudaGetDevice(&dev));
+    if (dev < 0 || dev >= 64) return fail(PMMH_ERR_NO_DEVICE, "device ordinal out of range");
+    StreamedState& s = states[dev];
+    if (!s.copy_stream) PMMH_CUDA(cudaStreamCreateWithFlags(&s.copy_stream, cudaStreamNonBlocking));
+    for (cudaEvent_t* e : {&s.ev_start, &s.ev_reset, &s.ev_done})
+        if (!*e) PMMH_CUDA(cudaEventCreateWithFlags(e, cudaEventDisableTiming));
+    *out = &s;
+    return PMMH_OK;
+}
+
+// Enqueues the copies of u from the reference's (n_obs, N + 1) host array into the slots of `slot` steps of
+// d_stage, on the copy stream, once everything queued so far on `st` has finished (the previous evaluation may
+// still be reading the staging buffer).  Pieces follow grid_u_next_piece(.., taper_min).  Each piece is
+// signalled either through the device flag d_flag (steps landed so far; `st` then waits until the flag has
+// been reset) or, with d_flag == NULL, by the event of its slot, ss.ev_slot[c].  ss.ev_done follows the last copy.
+int enqueue_u_copies(const double* h_rvs, int n_obs, int n, char* d_stage, int slot, int taper_min, int* d_flag,
+                     StreamedState& ss, cudaStream_t st) {
+    const int* tab = nullptr;
+    if (d_flag) {
+        tab = step_table(n_obs);
+        if (!tab) return fail(PMMH_ERR_CUDA, "pinned step table allocation failed");
+    }
+    while (!d_flag && (int)ss.ev_slot.size() < (n_obs + slot - 1) / slot) {
+        cudaEvent_t e;
+        PMMH_CUDA(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
+        ss.ev_slot.push_back(e);
+    }
+    PMMH_CUDA(cudaEventRecord(ss.ev_start, st));
+    PMMH_CUDA(cudaStreamWaitEvent(ss.copy_stream, ss.ev_start, 0));
+    if (d_flag) {
+        PMMH_CUDA(cudaMemsetAsync(d_flag, 0, sizeof(int), ss.copy_stream));
+        PMMH_CUDA(cudaEventRecord(ss.ev_reset, ss.copy_stream));
+    }
+    for (int t0 = 0; t0 < n_obs;) {
+        const int c = t0 / slot, in = t0 - c * slot;
+        const int w = grid_u_next_piece(t0, n_obs, slot, taper_min);
+        const double* src = h_rvs + (size_t)n_obs + (size_t)t0;   // rvp[i + j * n_obs], cython.py:89-91
+        char* dst = d_stage + ((size_t)c * (size_t)n * slot + (size_t)in) * sizeof(double);
+        PMMH_CUDA(cudaMemcpy2DAsync(dst, (size_t)slot * sizeof(double), src, (size_t)n_obs * sizeof(double),
+                                    (size_t)w * sizeof(double), (size_t)n, cudaMemcpyHostToDevice, ss.copy_stream));
+        if (d_flag)
+            PMMH_CUDA(cudaMemcpyAsync(d_flag, &tab[t0 + w], sizeof(int), cudaMemcpyHostToDevice, ss.copy_stream));
+        else
+            PMMH_CUDA(cudaEventRecord(ss.ev_slot[c], ss.copy_stream));
+        t0 += w;
+    }
+    PMMH_CUDA(cudaEventRecord(ss.ev_done, ss.copy_stream));
+    if (d_flag) PMMH_CUDA(cudaStreamWaitEvent(st, ss.ev_reset, 0));   // the kernel must not start before the flag is reset
+    return PMMH_OK;
+}
+
+int streamed_plan(int n_obs, int n, int lag, int ctas, SvPlan* p) {
+    return sv_make_plan({n_obs, n, lag, 1, 0, pmmh::kSvFlps, 0, ctas}, SvEntry::HostStreamed, p);
 }
 }  // namespace
 
 int pmmh_sv_stream_schedule(int n_obs, int* pieces, int max_pieces) {
     if (n_obs < 1 || (max_pieces > 0 && !pieces)) return -1;
-    const int ch = grid_u_chunk(), taper = grid_u_taper_min();
     int t0 = 0, k = 0;
     while (t0 < n_obs) {
-        const int w = grid_u_next_piece(t0, n_obs, ch, taper);
+        const int w = grid_u_next_piece(t0, n_obs, kGridUSlot, kGridUTaperMin);
         if (k < max_pieces) pieces[k] = w;
         ++k;
         t0 += w;
@@ -516,45 +580,23 @@ int pmmh_sv_stream_schedule(int n_obs, int* pieces, int max_pieces) {
 
 int pmmh_sv_stage_bytes(int n_obs, int n_particles, size_t* bytes) {
     if (!bytes || n_obs < 2 || n_particles < 1) return fail(PMMH_ERR_INVALID, "pmmh_sv_stage_bytes: bad arguments");
-    size_t b = streamed_data_bytes(n_obs, n_particles);
-    const size_t bg = streamed_grid_data_bytes(n_obs, n_particles);
-    if (bg > b) b = bg;
-    *bytes = b + 256;
+    const size_t b = staged_bytes(n_obs, n_particles, kUSlot), bg = staged_bytes(n_obs, n_particles, kGridUSlot);
+    *bytes = (bg > b ? bg : b) + 256;   // + the device flag
     return PMMH_OK;
 }
 
 int pmmh_sv_streamed_workspace_bytes(int n_obs, int n_particles, int lag, int ctas_per_problem, size_t* bytes) {
     if (!bytes) return fail(PMMH_ERR_INVALID, "bytes is null");
     SvPlan p;
-    int rc = sv_make_plan(n_obs, n_particles, lag, 1, 0, pmmh::kSvFlps, 0, ctas_per_problem, &p, true);
+    int rc = streamed_plan(n_obs, n_particles, lag, ctas_per_problem, &p);
     if (rc != PMMH_OK) return rc;
-    size_t b = p.total;
-    int GG = 0;
-    if (streamed_grid_ok(n_obs, n_particles, lag, ctas_per_problem, &GG)) {
-        const size_t g = pmmh::sv_grid_ws_bytes(n_obs, n_particles, lag, GG, 0);
-        if (g > b) b = g;
-    }
-    if (pmmh::sv_split_single_eligible(n_obs, n_particles, lag)) {
-        const size_t sp = pmmh::sv_split_path_ws_bytes(n_obs, n_particles, lag);
-        if (sp > b) b = sp;
-    }
-    *bytes = b;
+    *bytes = p.total;
     return PMMH_OK;
 }
 
-namespace {
-// the streaming kernels take host-resident u as well (and are the preferred kernels from N = 2^20)
-bool streamed_prefers_split(int n_obs, int n, int lag, int ctas) {
-    return (g_sv_algorithm == 0 || g_sv_algorithm == 5) && ctas == 0 && n >= g_split_min_particles &&
-           pmmh::sv_split_single_eligible(n_obs, n, lag);
-}
-}  // namespace
-
 int pmmh_sv_streamed_eligible(int n_obs, int n_particles, int lag, int ctas_per_problem) {
     SvPlan p;
-    if (sv_make_plan(n_obs, n_particles, lag, 1, 0, pmmh::kSvFlps, 0, ctas_per_problem, &p, true) != PMMH_OK) return 0;
-    return (p.use_fast || streamed_prefers_split(n_obs, n_particles, lag, ctas_per_problem) ||
-            streamed_grid_ok(n_obs, n_particles, lag, ctas_per_problem, nullptr)) ? 1 : 0;
+    return streamed_plan(n_obs, n_particles, lag, ctas_per_problem, &p) == PMMH_OK && p.c.kernel != SvKernel::None;
 }
 
 int pmmh_flps_sv_corr_streamed(const double* h_rvs, const double* d_obs, const double* d_params,
@@ -566,217 +608,54 @@ int pmmh_flps_sv_corr_streamed(const double* h_rvs, const double* d_obs, const d
     if (!h_rvs || !d_obs || !d_params || !d_rvr || !d_stage || !d_filt || !d_smo || !d_log_like || !d_gradient ||
         !d_traj || !d_hess1 || !d_hess2 || !d_diag || !d_workspace)
         return fail(PMMH_ERR_INVALID, "pmmh_flps_sv_corr_streamed: null pointer argument");
-    // The grid kernel where it takes the size: the copy engine lays the reference's particle-major host
-    // array down in chunks of 256 time steps (2 KB rows), the kernel reads its column of the chunk with a
-    // stride and polls one flag per time step; the call is bound by the host link, not by the kernel.
-    int GGs = 0;
-    if (streamed_grid_ok(n_obs, n_particles, lag, ctas_per_problem, &GGs)) {
-        const int ch = grid_u_chunk();
-        const size_t gws = pmmh::sv_grid_ws_bytes(n_obs, n_particles, lag, GGs, 0);
-        if (workspace_bytes < gws) return fail(PMMH_ERR_WORKSPACE, "workspace too small (pmmh_sv_streamed_workspace_bytes)");
-        const size_t gdata = streamed_grid_data_bytes(n_obs, n_particles);
-        if (stage_bytes < gdata + 256) return fail(PMMH_ERR_WORKSPACE, "staging buffer too small");
-        if (((uintptr_t)d_stage & 31) != 0) return fail(PMMH_ERR_INVALID, "d_stage must be 32-byte aligned (the kernel reads 32-byte sectors of the staged rows)");
-        int devg = 0;
-        PMMH_CUDA(cudaGetDevice(&devg));
-        if (devg < 0 || devg >= 64) return fail(PMMH_ERR_NO_DEVICE, "device ordinal out of range");
-        StreamedState& sg = g_streamed[devg];
-        if (!sg.copy_stream) {
-            PMMH_CUDA(cudaStreamCreateWithFlags(&sg.copy_stream, cudaStreamNonBlocking));
-            PMMH_CUDA(cudaEventCreateWithFlags(&sg.ev_start, cudaEventDisableTiming));
-            PMMH_CUDA(cudaEventCreateWithFlags(&sg.ev_reset, cudaEventDisableTiming));
-        }
-        if (!sg.ev_done) PMMH_CUDA(cudaEventCreateWithFlags(&sg.ev_done, cudaEventDisableTiming));
-        const int* tab = step_table(n_obs + ch);
-        if (!tab) return fail(PMMH_ERR_CUDA, "pinned step table allocation failed");
-        cudaStream_t stg = (cudaStream_t)stream;
-        char* stageg = (char*)d_stage;
-        int* d_flagg = (int*)(stageg + gdata);
-        // development: PMMH_STREAM_TIMING=1 prints when the copies and the kernel of this call ended (blocks the host)
-        static const bool timing = getenv("PMMH_STREAM_TIMING") != nullptr;
-        cudaEvent_t tv[3] = {nullptr, nullptr, nullptr};
-        if (timing)
-            for (int i = 0; i < 3; ++i) PMMH_CUDA(cudaEventCreate(&tv[i]));
-        PMMH_CUDA(cudaEventRecord(sg.ev_start, stg));
-        PMMH_CUDA(cudaStreamWaitEvent(sg.copy_stream, sg.ev_start, 0));
-        if (timing) PMMH_CUDA(cudaEventRecord(tv[0], sg.copy_stream));
-        PMMH_CUDA(cudaMemsetAsync(d_flagg, 0, sizeof(int), sg.copy_stream));
-        PMMH_CUDA(cudaEventRecord(sg.ev_reset, sg.copy_stream));
-        // Copy schedule.  The kernel needs ~0.11 ms per time step, the host link ~0.157 ms (2 KB rows: 53.5 GB/s; 1 KB:
-        // 51.7; 512 B: 48.4; and ~8 ns per row whatever its width, i.e. 8.4 ms for any piece of fewer than ~52 steps at
-        // N = 2^20).  The kernel can only start a piece when all of it has landed, so after the last copy it still has
-        // to work off what it was behind: a piece of p steps that starts with `rem` steps to go delays the end unless
-        // 0.157 p <= (0.157 - 0.11) rem + 0.11 p_last, i.e. p <= 0.3 rem + 0.7 p_last.  Hence: whole slots (widest rows) while
-        // that holds, then pieces of ~0.3 x what remains, the last one ~52 steps.  Measured at T = 1000, N = 2^20
-        // (PMMH_STREAM_TIMING=1): one copy per slot 157.7 ms of copies + 26.3 ms of kernel after the last one; this
-        // schedule: see DESIGN 3.  PMMH_GRID_U_TAPER=0: one copy per slot.  The staging layout does not change.
-        int t0 = 0;
-        while (t0 < n_obs) {
-            const int c = t0 / ch, in = t0 - c * ch;
-            const int wsteps = grid_u_next_piece(t0, n_obs, ch, grid_u_taper_min());
-            const double* src = h_rvs + (size_t)n_obs + (size_t)t0;   // rvp[i + j * n_obs], cython.py:89-91
-            char* dst = stageg + ((size_t)c * (size_t)n_particles * ch + (size_t)in) * sizeof(double);
-            PMMH_CUDA(cudaMemcpy2DAsync(dst, (size_t)ch * sizeof(double), src, (size_t)n_obs * sizeof(double),
-                                        (size_t)wsteps * sizeof(double), (size_t)n_particles, cudaMemcpyHostToDevice,
-                                        sg.copy_stream));
-            PMMH_CUDA(cudaMemcpyAsync(d_flagg, &tab[t0 + wsteps], sizeof(int), cudaMemcpyHostToDevice, sg.copy_stream));
-            t0 += wsteps;
-        }
-        if (timing) PMMH_CUDA(cudaEventRecord(tv[1], sg.copy_stream));
-        PMMH_CUDA(cudaEventRecord(sg.ev_done, sg.copy_stream));
-        PMMH_CUDA(cudaStreamWaitEvent(stg, sg.ev_reset, 0));   // the kernel must not start before the flag is reset
-        int rcg = pmmh::sv_grid_run(d_obs, d_params, d_rvr, (const double*)d_stage, n_obs, n_particles, lag, GGs, d_filt,
-                                    d_smo, d_log_like, d_gradient, d_traj, d_diag, nullptr, nullptr, d_workspace,
-                                    workspace_bytes, g_sv_prof, stg, ch, d_flagg);
-        if (rcg != PMMH_OK) return rcg;
-        PMMH_CUDA(cudaMemsetAsync(d_hess1, 0, 16 * sizeof(double), stg));
-        PMMH_CUDA(cudaMemsetAsync(d_hess2, 0, 16 * sizeof(double), stg));
-        // an evaluation that is abandoned early leaves copies behind: the caller's stream ends after them
-        PMMH_CUDA(cudaStreamWaitEvent(stg, sg.ev_done, 0));
-        if (timing) {
-            PMMH_CUDA(cudaEventRecord(tv[2], stg));
-            PMMH_CUDA(cudaEventSynchronize(tv[2]));
-            float copies_ms = 0.f, all_ms = 0.f;
-            cudaEventElapsedTime(&copies_ms, tv[0], tv[1]);
-            cudaEventElapsedTime(&all_ms, tv[0], tv[2]);
-            fprintf(stderr, "[pmmh stream timing] copies %.2f ms (%.1f GB/s), kernel ends %.2f ms after the last copy\n",
-                    copies_ms, (double)n_obs * n_particles * 8.0 / (copies_ms * 1e6), all_ms - copies_ms);
-            for (int i = 0; i < 3; ++i) cudaEventDestroy(tv[i]);
-        }
-        return PMMH_OK;
-    }
-    // Host-resident u runs on the exchange kernel where it takes the size (measured at N = 2^20:
-    // 206 ms per call against 242 ms on the streaming kernels, whose strided reads of the
-    // particle-major chunks cost more than they save) and on the streaming kernels beyond it.
-    bool exchange_ok = false;
-    {
-        SvPlan p0;
-        if (sv_make_plan(n_obs, n_particles, lag, 1, 0, pmmh::kSvFlps, 0, ctas_per_problem, &p0, true) == PMMH_OK)
-            exchange_ok = p0.use_fast != 0;
-    }
-    if (!exchange_ok && streamed_prefers_split(n_obs, n_particles, lag, ctas_per_problem)) {
-        // streaming kernels with path storage: the copy engine fills particle-major chunks of 64
-        // time steps; the (host-driven) step loop waits for a chunk's event when it enters it
-        if (workspace_bytes < pmmh::sv_split_path_ws_bytes(n_obs, n_particles, lag))
-            return fail(PMMH_ERR_WORKSPACE, "workspace too small");
-        const size_t data_bytes2 = streamed_data_bytes(n_obs, n_particles);
-        if (stage_bytes < data_bytes2 + 256) return fail(PMMH_ERR_WORKSPACE, "staging buffer too small");
-        int dev2 = 0;
-        PMMH_CUDA(cudaGetDevice(&dev2));
-        if (dev2 < 0 || dev2 >= 64) return fail(PMMH_ERR_NO_DEVICE, "device ordinal out of range");
-        StreamedState& s2 = g_streamed[dev2];
-        const int chunks2 = streamed_chunks(n_obs);
-        if (!s2.copy_stream) {
-            PMMH_CUDA(cudaStreamCreateWithFlags(&s2.copy_stream, cudaStreamNonBlocking));
-            PMMH_CUDA(cudaEventCreateWithFlags(&s2.ev_start, cudaEventDisableTiming));
-            PMMH_CUDA(cudaEventCreateWithFlags(&s2.ev_reset, cudaEventDisableTiming));
-        }
-        while ((int)s2.ev_chunk.size() < chunks2) {
-            cudaEvent_t e;
-            PMMH_CUDA(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
-            s2.ev_chunk.push_back(e);
-        }
-        cudaStream_t st2 = (cudaStream_t)stream;
-        PMMH_CUDA(cudaEventRecord(s2.ev_start, st2));
-        PMMH_CUDA(cudaStreamWaitEvent(s2.copy_stream, s2.ev_start, 0));
-        for (int c = 0; c < chunks2; ++c) {
-            const int t0 = c * kUChunk;
-            const int wsteps = (n_obs - t0 < kUChunk) ? (n_obs - t0) : kUChunk;
-            const double* src = h_rvs + (size_t)n_obs + (size_t)t0;   // rvp[i + j * n_obs], cython.py:89-91
-            char* dst = (char*)d_stage + (size_t)c * (size_t)n_particles * kUChunk * sizeof(double);
-            PMMH_CUDA(cudaMemcpy2DAsync(dst, (size_t)kUChunk * sizeof(double), src, (size_t)n_obs * sizeof(double),
-                                        (size_t)wsteps * sizeof(double), (size_t)n_particles,
-                                        cudaMemcpyHostToDevice, s2.copy_stream));
-            PMMH_CUDA(cudaEventRecord(s2.ev_chunk[c], s2.copy_stream));
-        }
-        PMMH_CUDA(cudaMemsetAsync(d_hess1, 0, 16 * sizeof(double), st2));
-        PMMH_CUDA(cudaMemsetAsync(d_hess2, 0, 16 * sizeof(double), st2));
-        return pmmh::sv_split_path_run(d_obs, d_params, d_rvr, (const double*)d_stage, n_obs, n_particles, lag,
-                                       d_filt, d_smo, d_log_like, d_gradient, d_traj, d_diag, d_workspace,
-                                       workspace_bytes, st2, kUChunk, s2.ev_chunk.data());
-    }
     SvPlan p;
-    int rc = sv_make_plan(n_obs, n_particles, lag, 1, 0, pmmh::kSvFlps, 0, ctas_per_problem, &p, true);
+    int rc = streamed_plan(n_obs, n_particles, lag, ctas_per_problem, &p);
     if (rc != PMMH_OK) return rc;
-    if (!p.use_fast) return fail(PMMH_ERR_INVALID, "pmmh_flps_sv_corr_streamed: exchange kernel not eligible for these sizes");
-    if (workspace_bytes < p.total) return fail(PMMH_ERR_WORKSPACE, "workspace too small");
-    const size_t data_bytes = streamed_data_bytes(n_obs, n_particles);
+    const SvKernel k = p.c.kernel;
+    if (k == SvKernel::None)
+        return fail(PMMH_ERR_INVALID, "pmmh_flps_sv_corr_streamed: no kernel takes these sizes (pmmh_sv_streamed_eligible)");
+    if (workspace_bytes < p.total) return fail(PMMH_ERR_WORKSPACE, "workspace too small (pmmh_sv_streamed_workspace_bytes)");
+    // The grid kernel reads its column of a slot with a stride and polls one flag per time step; the call is
+    // bound by the host link, not by the kernel.  The exchange kernel polls the flag as well; the host-driven
+    // step loop of the streaming kernels waits for a slot's event when it enters it.
+    const int slot = k == SvKernel::Grid ? kGridUSlot : kUSlot;
+    const size_t data_bytes = staged_bytes(n_obs, n_particles, slot);
     if (stage_bytes < data_bytes + 256) return fail(PMMH_ERR_WORKSPACE, "staging buffer too small");
-    int dev = 0;
-    PMMH_CUDA(cudaGetDevice(&dev));
-    if (dev < 0 || dev >= 64) return fail(PMMH_ERR_NO_DEVICE, "device ordinal out of range");
-    StreamedState& ss = g_streamed[dev];
-    const int chunks = streamed_chunks(n_obs);
-    if (!ss.copy_stream) {
-        PMMH_CUDA(cudaStreamCreateWithFlags(&ss.copy_stream, cudaStreamNonBlocking));
-        PMMH_CUDA(cudaEventCreateWithFlags(&ss.ev_start, cudaEventDisableTiming));
-        PMMH_CUDA(cudaEventCreateWithFlags(&ss.ev_reset, cudaEventDisableTiming));
-    }
-    if (!ss.ev_done) PMMH_CUDA(cudaEventCreateWithFlags(&ss.ev_done, cudaEventDisableTiming));
-    const int* tabx = step_table(n_obs + kUChunk);   // immutable pinned table: no host value is ever rewritten
-    if (!tabx) return fail(PMMH_ERR_CUDA, "pinned step table allocation failed");
+    if (k == SvKernel::Grid && ((uintptr_t)d_stage & 31) != 0)
+        return fail(PMMH_ERR_INVALID, "d_stage must be 32-byte aligned (the kernel reads 32-byte sectors of the staged rows)");
+    StreamedState* ss = nullptr;
+    rc = streamed_state(&ss);
+    if (rc != PMMH_OK) return rc;
     cudaStream_t st = (cudaStream_t)stream;
-    char* stage = (char*)d_stage;
-    int* d_flag = (int*)(stage + data_bytes);
-    // the copies may start once everything queued so far on the caller's stream has finished
-    // (the previous evaluation may still be reading the staging buffer)
-    PMMH_CUDA(cudaEventRecord(ss.ev_start, st));
-    PMMH_CUDA(cudaStreamWaitEvent(ss.copy_stream, ss.ev_start, 0));
-    PMMH_CUDA(cudaMemsetAsync(d_flag, 0, sizeof(int), ss.copy_stream));
-    PMMH_CUDA(cudaEventRecord(ss.ev_reset, ss.copy_stream));
-    for (int c = 0; c < chunks; ++c) {
-        const int t0 = c * kUChunk;
-        const int wsteps = (n_obs - t0 < kUChunk) ? (n_obs - t0) : kUChunk;
-        // rows = particles: rvp[i + j * n_obs] with rvp = rvs_flat + n_obs (cython.py:89-91)
-        const double* src = h_rvs + (size_t)n_obs + (size_t)t0;
-        char* dst = stage + (size_t)c * (size_t)n_particles * kUChunk * sizeof(double);
-        PMMH_CUDA(cudaMemcpy2DAsync(dst, (size_t)kUChunk * sizeof(double), src, (size_t)n_obs * sizeof(double),
-                                    (size_t)wsteps * sizeof(double), (size_t)n_particles, cudaMemcpyHostToDevice,
-                                    ss.copy_stream));
-        PMMH_CUDA(cudaMemcpyAsync(d_flag, &tabx[t0 + wsteps], sizeof(int), cudaMemcpyHostToDevice, ss.copy_stream));
+    const double* d_u = (const double*)d_stage;
+    int* d_flag = k == SvKernel::StreamPath ? nullptr : (int*)((char*)d_stage + data_bytes);
+    rc = enqueue_u_copies(h_rvs, n_obs, n_particles, (char*)d_stage, slot, k == SvKernel::Grid ? kGridUTaperMin : 0,
+                          d_flag, *ss, st);
+    if (rc != PMMH_OK) return rc;
+    if (k == SvKernel::Grid) {
+        rc = pmmh::sv_grid_run(d_obs, d_params, d_rvr, d_u, n_obs, n_particles, lag, p.c.grid_G, d_filt, d_smo,
+                               d_log_like, d_gradient, d_traj, d_diag, nullptr, nullptr, d_workspace, workspace_bytes,
+                               g_sv_prof, st, slot, d_flag);
+        if (rc != PMMH_OK) return rc;
+        PMMH_CUDA(cudaMemsetAsync(d_hess1, 0, 16 * sizeof(double), st));
+        PMMH_CUDA(cudaMemsetAsync(d_hess2, 0, 16 * sizeof(double), st));
+    } else if (k == SvKernel::Exchange) {
+        const SvShape s = {n_obs, n_particles, lag, 1, 0, pmmh::kSvFlps, 0, ctas_per_problem};
+        pmmh::SvArgs a = sv_args(p, s, d_obs, 0, d_params, d_rvr, d_u, d_filt, d_smo, d_log_like, d_gradient, d_traj,
+                                 d_hess1, d_hess2, d_diag, nullptr, nullptr, d_workspace);
+        a.u_chunk = slot;
+        a.u_ready = d_flag;
+        PMMH_CUDA(exchange_launch(p, a, st));
+    } else {
+        PMMH_CUDA(cudaMemsetAsync(d_hess1, 0, 16 * sizeof(double), st));
+        PMMH_CUDA(cudaMemsetAsync(d_hess2, 0, 16 * sizeof(double), st));
+        rc = pmmh::sv_split_path_run(d_obs, d_params, d_rvr, d_u, n_obs, n_particles, lag, d_filt, d_smo, d_log_like,
+                                     d_gradient, d_traj, d_diag, d_workspace, workspace_bytes, st, slot,
+                                     ss->ev_slot.data());
+        if (rc != PMMH_OK) return rc;
     }
-    PMMH_CUDA(cudaEventRecord(ss.ev_done, ss.copy_stream));
-    // the kernel must not start before the flag has been reset
-    PMMH_CUDA(cudaStreamWaitEvent(st, ss.ev_reset, 0));
-    pmmh::SvArgs a;
-    memset(&a, 0, sizeof(a));
-    a.N = n_particles;
-    a.NOBS = n_obs;
-    a.LAG = lag;
-    a.B = 1;
-    a.G = p.G;
-    a.n_teams = p.n_teams;
-    a.NB = p.NB;
-    a.RING = p.RING;
-    a.mode = pmmh::kSvFlps;
-    a.hess = 0;
-    a.SQ = p.SQ;
-    a.SQW = p.SQW;
-    a.obs = d_obs;
-    a.obs_stride = 0;
-    a.params = d_params;
-    a.rvr = d_rvr;
-    a.U = (const double*)d_stage;
-    a.u_chunk = kUChunk;
-    a.u_ready = d_flag;
-    a.filt = d_filt;
-    a.smo = d_smo;
-    a.loglike = d_log_like;
-    a.grad = d_gradient;
-    a.traj = d_traj;
-    a.hess1 = d_hess1;
-    a.hess2 = d_hess2;
-    a.diag = d_diag;
-    a.prof = g_sv_prof;
-    a.ws = (char*)d_workspace;
-    a.NSUB = p.NSUB;
-    a.CP = p.CP;
-    a.ws_sync_bytes = p.fast_sync_bytes;
-    a.ws_team_stride = p.fast_team_stride;
-    PMMH_CUDA(cudaMemsetAsync(d_workspace, 0, p.fast_sync_bytes, st));
-    PMMH_CUDA(pmmh::sv_fast_launch(a, p.grid, st));
     // an evaluation that is abandoned early leaves copies behind: the caller's stream ends after them
-    PMMH_CUDA(cudaStreamWaitEvent(st, ss.ev_done, 0));
+    PMMH_CUDA(cudaStreamWaitEvent(st, ss->ev_done, 0));
     return PMMH_OK;
 }
 

@@ -1850,39 +1850,19 @@ int sv_grid_run(const double* d_obs, const double* d_params, const double* d_rvr
     // control block, histograms, reservation counters, tile info: zero
     GRID_CUDA(cudaMemsetAsync(ws + L.ctrl, 0, L.H - L.ctrl, st));
     static thread_local bool attr_set[64] = {false};
-    static int threads = 0;
-    if (!threads) {
-        const char* e = getenv("PMMH_GRID_THREADS");
-        threads = (e && atoi(e) == 512) ? 512 : 1024;
-    }
     int dev = 0;
     GRID_CUDA(cudaGetDevice(&dev));
-    {
-        // the two genealogy record tables live in the persisting part of L2 (their reuse distance is a
-        // whole time step); the limit is a device-wide setting, set once per device and size
-        static size_t persist_set[64] = {0};
-        size_t want = 0;
-        const char* e = getenv("PMMH_GRID_L2_PERSIST_MB");
-        if (e) want = (size_t)atoi(e) << 20;
-        int maxp = 0;
-        GRID_CUDA(cudaDeviceGetAttribute(&maxp, cudaDevAttrMaxPersistingL2CacheSize, dev));
-        if (want > (size_t)maxp) want = (size_t)maxp;
-        if (dev >= 0 && dev < 64 && persist_set[dev] != want + 1) {
-            GRID_CUDA(cudaDeviceSetLimit(cudaLimitPersistingL2CacheSize, want));
-            persist_set[dev] = want + 1;
-        }
-    }
     if (dev >= 0 && dev < 64 && !attr_set[dev]) {
-        GRID_CUDA(cudaFuncSetAttribute(sv_grid_kernel<512, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kDynSmem));
+        // no persisting L2 set-aside for the kernel's evict_last accesses: with one every phase is slower
+        // (DESIGN 4.0), and left unset the evaluation at N = 2^20 is ~6 % slower
+        GRID_CUDA(cudaDeviceSetLimit(cudaLimitPersistingL2CacheSize, 0));
         GRID_CUDA(cudaFuncSetAttribute(sv_grid_kernel<1024, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kDynSmem));
-        GRID_CUDA(cudaFuncSetAttribute(sv_grid_kernel<512, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kDynSmem));
         GRID_CUDA(cudaFuncSetAttribute(sv_grid_kernel<1024, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kDynSmem));
         attr_set[dev] = true;
     }
     void* kargs[] = {(void*)&a};
-    const void* kern = hess ? (threads == 1024 ? (const void*)sv_grid_kernel<1024, true> : (const void*)sv_grid_kernel<512, true>)
-                            : (threads == 1024 ? (const void*)sv_grid_kernel<1024, false> : (const void*)sv_grid_kernel<512, false>);
-    GRID_CUDA(cudaLaunchCooperativeKernel(kern, dim3(G), dim3(threads), kargs, kDynSmem, st));
+    const void* kern = hess ? (const void*)sv_grid_kernel<1024, true> : (const void*)sv_grid_kernel<1024, false>;
+    GRID_CUDA(cudaLaunchCooperativeKernel(kern, dim3(G), dim3(1024), kargs, kDynSmem, st));
     double* sums = (double*)(ws + L.sums);
     double* tailpart = (double*)(ws + L.tailpart);
     double* tail = (double*)(ws + L.tail);

@@ -52,9 +52,10 @@ def device_info():
 
 
 def set_sv_algorithm(algorithm):
-    """0 = automatic (chain / exchange / streaming kernels where eligible), 1 = general kernel only,
-    2 / 3 = exchange / chain kernel without the general-kernel fallback, 4 / 5 = streaming kernels with
-    records / with path storage (pmmh_sv_set_algorithm)."""
+    """0 = automatic (chain / grid / streaming / exchange kernel where eligible, the general kernel
+    otherwise and as their fallback), 1 = general kernel only, 2 / 3 = exchange / chain kernel without
+    the general-kernel fallback, 4 / 5 = streaming kernels with records / with path storage, 6 = grid
+    kernel (pmmh_sv_set_algorithm; the selection table is in include/pmmh_qn.h)."""
     lib = _lib.load()
     _lib.check(lib.pmmh_sv_set_algorithm(int(algorithm)), "pmmh_sv_set_algorithm")
 
@@ -184,7 +185,8 @@ def flps_sv_corr_philox(obs, params, rvr, seed, philox_offset, n_particles, lag=
 
 
 def sv_streamed_eligible(n_obs, n_particles, lag=10, ctas_per_problem=0):
-    """True if pmmh_flps_sv_corr_streamed takes these sizes (the exchange kernel is eligible)."""
+    """True if pmmh_flps_sv_corr_streamed takes these sizes under the current algorithm (a grid,
+    exchange or streaming kernel is selected for them)."""
     return bool(_lib.load().pmmh_sv_streamed_eligible(int(n_obs), int(n_particles), int(lag),
                                                       int(ctas_per_problem)))
 
