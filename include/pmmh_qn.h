@@ -181,10 +181,17 @@ int pmmh_flps_sv_corr_philox(const double* d_obs, const double* d_params, const 
  * (sorted correlated systematic resampling, fixed-lag score terms, tail, quirks Q1 / Q5 / Q6) with the
  * model's propagation, log-weight and score formulas plugged in through the device-function interface
  * of csrc/pf_model.cuh -- the three things python/README.md:73-76 tells a user to change in the Cython
- * smoother for another scalar-state model.  One CTA per problem (chain kernel): 2 <= n_particles <= 4096,
- * 2 <= lag <= 10, any batch.  d_params [batch][4] (unused slots ignored), gradient [4][n_obs] (unused rows 0).
- * PMMH_MODEL_SV_LEVERAGE gives bit-identical results to pmmh_flps_sv_corr at these sizes.  No fallback
- * inside: d_diag[PMMH_DIAG_STATUS] == 1 reports an abandoned problem (log-likelihood NaN). */
+ * smoother for another scalar-state model.  2 <= lag <= 10.  The kernel (d_diag[PMMH_DIAG_KERNEL]):
+ *   3  chain kernel, one CTA per problem: 2 <= n_particles <= 4096, any batch;
+ *   5  grid kernel, one persistent launch over the GPU: batch == 1, n_obs >= 2 lag and a tile of
+ *      n_particles / min(SMs, ceil(n_particles / 2048)) particles fits one CTA (<= 7168: up to 1,060,864
+ *      particles on 148 SMs); d_x_hist / d_a_hist as on pmmh_flps_sv_corr's grid kernel;
+ * other sizes are refused (PMMH_ERR_INVALID; also by pmmh_flps_model_workspace_bytes, which returns the size
+ * with history for the kernel the call runs).  d_params [batch][4] (unused slots ignored), gradient [4][n_obs]
+ * (unused rows 0).  PMMH_MODEL_SV_LEVERAGE gives bit-identical results to pmmh_flps_sv_corr run on the same
+ * kernel: the chain kernel (algorithm 3) up to 4096 particles, the grid kernel (algorithm 6, or 0 from 2^14 on)
+ * above.  No fallback inside: d_diag[PMMH_DIAG_STATUS] == 1 reports an abandoned problem (chain kernel:
+ * log-likelihood NaN). */
 #define PMMH_MODEL_SV_LEVERAGE 0      /* mu, phi, sigma_v, rho   (models/stochastic_volatility.py) */
 #define PMMH_MODEL_LINEAR_GAUSSIAN 1  /* phi, sigma_v, sigma_e: x' = phi x + sigma_v v, y = x + sigma_e e */
 #define PMMH_MODEL_LINEAR_GAUSSIAN_FA 2 /* the same model as a FULLY ADAPTED particle filter: pass the observations shifted by

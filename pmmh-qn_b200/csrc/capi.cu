@@ -659,13 +659,38 @@ int pmmh_flps_sv_corr_streamed(const double* h_rvs, const double* d_obs, const d
     return PMMH_OK;
 }
 
-// ---- model-generic entry point: the chain kernel instantiated for a model of pf_model.cuh ----------
-int pmmh_flps_model_workspace_bytes(int n_obs, int n_particles, int lag, int batch, size_t* bytes) {
-    if (!bytes || n_obs < 2 || batch < 1) return fail(PMMH_ERR_INVALID, "pmmh_flps_model_workspace_bytes: bad arguments");
-    if (!pmmh::sv_chain_eligible(n_particles, lag) || pmmh::sv_chain_smem_bytes(n_particles) > kMaxDynSmem)
-        return fail(PMMH_ERR_INVALID, "pmmh_flps_model_corr: 2 <= n_particles <= 4096 and 2 <= lag <= 10");
+// ---- model-generic entry point: the chain or the grid kernel instantiated for a model of pf_model.cuh ----------
+namespace {
+// The kernel pmmh_flps_model_corr runs: the chain kernel wherever it applies (any batch), else the grid kernel for
+// one problem on sv_grid_ctas(N, SMs, 0) CTAs; anything else is refused.  *G = the grid kernel's CTAs.
+int model_choose(int n_obs, int n, int lag, int batch, SvKernel* k, int* G) {
+    if (n_obs < 2 || batch < 1) return fail(PMMH_ERR_INVALID, "pmmh_flps_model_corr: bad arguments");
     DeviceInfo di;
     int rc = get_device_info(&di);
+    if (rc != PMMH_OK) return rc;
+    *G = pmmh::sv_grid_ctas(n, di.sm, 0);
+    if (pmmh::sv_chain_eligible(n, lag) && pmmh::sv_chain_smem_bytes(n) <= kMaxDynSmem) *k = SvKernel::Chain;
+    else if (batch == 1 && pmmh::sv_grid_eligible(n_obs, n, lag, *G)) *k = SvKernel::Grid;
+    else
+        return fail(PMMH_ERR_INVALID, "pmmh_flps_model_corr: 2 <= lag <= 10 and 2 <= n_particles <= 4096 (any batch), "
+                                      "or batch == 1, n_obs >= 2 lag and n_particles up to 7168 per SM "
+                                      "(1,060,864 on 148 SMs)");
+    return PMMH_OK;
+}
+}  // namespace
+
+int pmmh_flps_model_workspace_bytes(int n_obs, int n_particles, int lag, int batch, size_t* bytes) {
+    if (!bytes) return fail(PMMH_ERR_INVALID, "pmmh_flps_model_workspace_bytes: bad arguments");
+    SvKernel k;
+    int G;
+    int rc = model_choose(n_obs, n_particles, lag, batch, &k, &G);
+    if (rc != PMMH_OK) return rc;
+    if (k == SvKernel::Grid) {
+        *bytes = pmmh::sv_grid_ws_bytes(n_obs, n_particles, lag, G, 1);   // with history (the query has no flag)
+        return PMMH_OK;
+    }
+    DeviceInfo di;
+    rc = get_device_info(&di);
     if (rc != PMMH_OK) return rc;
     const int grid = batch < di.sm ? batch : di.sm;
     *bytes = (size_t)grid * pmmh::sv_chain_ws_bytes(n_particles, lag, n_obs, 0);
@@ -694,6 +719,17 @@ int pmmh_flps_model_corr(int model_id, const double* d_obs, long long obs_stride
     rc = get_device_info(&di);
     if (rc != PMMH_OK) return rc;
     if (di.major < 10) return fail(PMMH_ERR_NO_DEVICE, "an sm_100 (B200) device is required");
+    SvKernel k;
+    int G;
+    rc = model_choose(n_obs, n_particles, lag, batch, &k, &G);
+    if (rc != PMMH_OK) return rc;
+    if (k == SvKernel::Grid) {
+        if (!di.coop) return fail(PMMH_ERR_NO_DEVICE, "device lacks cooperative launch");
+        // (no fallback pass: an abandoned evaluation is reported in d_diag[PMMH_DIAG_STATUS])
+        return pmmh::sv_grid_run(d_obs, d_params, d_rvr, d_u, n_obs, n_particles, lag, G, d_filt, d_smo, d_log_like,
+                                 d_gradient, d_traj, d_diag, d_x_hist, d_a_hist, d_workspace, workspace_bytes, nullptr,
+                                 (cudaStream_t)stream, 0, nullptr, nullptr, nullptr, model_id);
+    }
     pmmh::SvArgs a;
     memset(&a, 0, sizeof(a));
     a.N = n_particles;

@@ -1,5 +1,5 @@
 // pf_model.cuh -- the device-function interface a scalar-state model implements to run on the
-// chain kernel (sv_chain.cu): the three things the reference tells a user to change when porting
+// chain kernel (sv_chain.cu) and the grid kernel (sv_grid.cu): the three things the reference tells a user to change when porting
 // its Cython particle smoother to another model (/root/reference/python/README.md:73-76:
 // "how the propagation and weighting of particles is carried out as well as the gradients of the
 // log joint distribution of states and measurements").  Everything else -- sorted correlated
@@ -13,6 +13,10 @@
 //                                        flps starts all particles at one point, Q1)
 //   M::propagate(c, x_parent, y_prev, u) child value; u = the particle's standard normal
 //                                        (SV: stochastic_volatility.pyx:354-358)
+//   M::prop_mean(c, x_parent, y_prev)    the same split as mean + sd * u: propagate(c, xp, y, u) ==
+//   M::prop_sd(c)                        prop_mean(c, xp, y) + prop_sd(c) * u bit for bit (the grid
+//                                        kernel stores the mean with the parent and predicts the
+//                                        children's value range from its weighted moments)
 //   M::child_range(c, xmin, xmax, y_prev, nsd, lo, hi)
 //                                        an interval holding the children of parents in
 //                                        [xmin, xmax] up to nsd innovation sd (sort-bin range)
@@ -25,6 +29,8 @@
 //                                        over (Q5) (SV: :452-465)
 //   M::score_tail(c, curr, next, y, g)   the same in the tail loop, y = obs[time(next) - 1]
 //                                        wrapped (Q6) (SV: :548-557, another operation order)
+//   M::kScoreIsZero                      constexpr: score_main / score_tail are identically 0 (the
+//                                        grid kernel then skips the calls; the smoother still runs)
 // Unused gradient slots stay 0.  Model ids are part of the C ABI (include/pmmh_qn.h).
 #pragma once
 #include <math.h>
@@ -41,11 +47,18 @@ struct SvLeverageModel {
         const double stdev0 = c.sigmav / sqrt(1.0 - (c.phi * c.phi));
         return c.mu + stdev0 * 0.0;   // :309 (Q1)
     }
+    static constexpr bool kScoreIsZero = false;
     static __device__ __forceinline__ double propagate(const Const& c, double xp, double y1, double u) {
         double mean = c.mu + c.phi * (xp - c.mu);
         mean += c.sr * exp(-0.5 * xp) * y1;
         return mean + c.sd * u;
     }
+    static __device__ __forceinline__ double prop_mean(const Const& c, double xp, double y1) {
+        double mean = c.mu + c.phi * (xp - c.mu);
+        mean += c.sr * exp(-0.5 * xp) * y1;
+        return mean;
+    }
+    static __device__ __forceinline__ double prop_sd(const Const& c) { return c.sd; }
     static __device__ __forceinline__ void child_range(const Const& c, double xmin, double xmax, double y1, double nsd,
                                                        double& lo, double& hi) {
         sv_child_range(c, xmin, xmax, y1, nsd, lo, hi);
@@ -88,9 +101,12 @@ struct LinearGaussianModel {
         c.log_se = log(c.se);
     }
     static __device__ __forceinline__ double initial_state(const Const&) { return 0.0; }
+    static constexpr bool kScoreIsZero = false;
     static __device__ __forceinline__ double propagate(const Const& c, double xp, double, double u) {
         return c.phi * xp + c.sv * u;
     }
+    static __device__ __forceinline__ double prop_mean(const Const& c, double xp, double) { return c.phi * xp; }
+    static __device__ __forceinline__ double prop_sd(const Const& c) { return c.sv; }
     static __device__ __forceinline__ void child_range(const Const& c, double xmin, double xmax, double, double nsd,
                                                        double& lo, double& hi) {
         const double a = c.phi * xmin, b = c.phi * xmax;
@@ -145,10 +161,16 @@ struct LinearGaussianFullyAdapted {
     }
     static __device__ __forceinline__ double initial_state(const Const&) { return 0.0; }
     // x_t | x_{t-1}, y_t ~ N(phi x + k (y_t - phi x), sv^2 se^2 / (sv^2 + se^2))
+    static constexpr bool kScoreIsZero = true;
     static __device__ __forceinline__ double propagate(const Const& c, double xp, double y_now, double u) {
         const double m = c.phi * xp;
         return (m + c.k * (y_now - m)) + c.sdp * u;
     }
+    static __device__ __forceinline__ double prop_mean(const Const& c, double xp, double y_now) {
+        const double m = c.phi * xp;
+        return m + c.k * (y_now - m);
+    }
+    static __device__ __forceinline__ double prop_sd(const Const& c) { return c.sdp; }
     static __device__ __forceinline__ void child_range(const Const& c, double xmin, double xmax, double y_now, double nsd,
                                                        double& lo, double& hi) {
         const double a = c.phi * xmin, b = c.phi * xmax;

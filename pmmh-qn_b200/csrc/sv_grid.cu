@@ -48,6 +48,9 @@
 //     sector of 64-byte record / payload entries; 162 us per step (DESIGN 4.0).
 //   * host-resident u: particle-major slots filled by the copy engine, one 32-byte sector (4 steps) per particle re-laid
 //     time-major every fourth step (DESIGN 3).
+//   * template over the model (pf_model.cuh): SvLeverageModel is everything above; another model runs the generic path
+//     in the same body (XE = (x, propagation mean of the children), payload = (parent value, -, -, value), score terms
+//     M::score_main / M::score_tail), gradient only (DESIGN 4.0).
 //
 // Deviations from the reference's operation order: parallel sums / scans, log(exp(x/2)) = x/2 and
 // 1/exp(x/2)^2 = exp(-x/2)^2 in the log-weight, cumulative weights multiplied by 1/S; any
@@ -61,8 +64,11 @@
 #include <stdlib.h>
 #include <string.h>
 
+#include <type_traits>
+
 #include "../../include/pmmh_qn.h"
 #include "common.cuh"
+#include "pf_model.cuh"
 #include "sv_grid.cuh"
 #include "sv_math.cuh"
 
@@ -148,6 +154,12 @@ struct StepScalars {
 };
 
 // ---- small device helpers ---------------------------------------------------------------------
+// the SV model's constants, which the SV code of the kernel reads; another model has none (zeros, never used)
+__device__ __forceinline__ const SvConst& sv_of(const SvConst& k) { return k; }
+template <class C>
+__device__ __forceinline__ SvConst sv_of(const C&) {
+    return SvConst();
+}
 __device__ __forceinline__ void red_release_add(unsigned* p, unsigned v) {
     asm volatile("red.release.gpu.global.add.u32 [%0], %1;" ::"l"(p), "r"(v) : "memory");
 }
@@ -371,9 +383,14 @@ __device__ __forceinline__ void deferred_alpha_pass(const GridArgs& a, const SvC
 // ---------------------------------------------------------------------------------------------
 // the kernel
 // ---------------------------------------------------------------------------------------------
-// HESS: the Hessian branch of the reference with its quirks Q7 / Q8 (second instantiation)
-template <int GT, bool HESS>
+// HESS: the Hessian branch of the reference with its quirks Q7 / Q8 (second instantiation, SV only).
+// M: the model (pf_model.cuh).  SvLeverageModel runs the SV code with its shared exp(-x/2); any other model
+// runs the generic path: the second double of XE is the propagation mean prop_mean(x, obs[t]) of the
+// children, a payload is (parent value, -, -, own value) and the score terms are M::score_main of the pair.
+template <int GT, bool HESS, class M>
 __global__ void __launch_bounds__(GT, 1) sv_grid_kernel(const GridArgs a) {
+    constexpr bool GEN = !std::is_same<M, SvLeverageModel>::value;
+    static_assert(!(GEN && HESS), "the Hessian branch exists for the SV model only");
     constexpr int KPT = kCap / GT;          // entries per thread (strided assignment)
     constexpr int KCH = KPT | 1;            // longest chunk of the thread-contiguous passes (odd)
     constexpr int BPT = kNF / GT;           // histogram bins per thread
@@ -402,7 +419,7 @@ __global__ void __launch_bounds__(GT, 1) sv_grid_kernel(const GridArgs a) {
     int* s_fhist = (int*)smem;                         // [kNF] histogram of this CTA's children
     unsigned short* s_tileof = (unsigned short*)(smem + 32768);   // [kNF] tile of a histogram bin
 
-    __shared__ SvConst s_k;
+    __shared__ typename M::Const s_k;
     __shared__ StepScalars s_sc;
     __shared__ double s_tot[kMaxTiles], s_off[kMaxTiles + 1];
     __shared__ int s_tstart[kMaxTiles + 1], s_tbin[kMaxTiles + 1], s_tcnt[kMaxTiles], s_tbase[kMaxTiles];
@@ -502,7 +519,7 @@ __global__ void __launch_bounds__(GT, 1) sv_grid_kernel(const GridArgs a) {
     } while (0)
 
     if (tid == 0) {
-        sv_const_init(s_k, a.params);
+        M::init(s_k, a.params);
         s_sc.abort_now = 0;
         for (int i = 0; i < kProf; ++i) s_prof[i] = 0;
     }
@@ -510,16 +527,23 @@ __global__ void __launch_bounds__(GT, 1) sv_grid_kernel(const GridArgs a) {
     __syncthreads();
 
     // ------------------------------------------------------------------------------------------
-    // generation 0 (:306-323, Q1): every particle = mu, uniform weights, identity order
+    // generation 0 (:306-323, Q1): every particle = mu (M::initial_state), uniform weights, identity order
     // ------------------------------------------------------------------------------------------
     const int jb = min(N, c * Wc), je = min(N, jb + Wc), nc = je - jb;   // this CTA's children
     int pstart = jb, n = nc;                                             // this CTA's tile
     double toff;                                                          // cumulative weight in front of this thread's chunk
     {
-        const double mu = s_k.mu;
-        const double e0 = exp(-0.5 * mu);
-        double m0 = s_k.mu + s_k.phi * (mu - s_k.mu);
-        m0 += (s_k.sr * e0) * a.obs[0];
+        double mu, e0, m0;   // value, second double of XE, propagation mean
+        if constexpr (GEN) {
+            mu = M::initial_state(s_k);
+            m0 = M::prop_mean(s_k, mu, a.obs[0]);
+            e0 = m0;
+        } else {
+            mu = s_k.mu;
+            e0 = exp(-0.5 * mu);
+            m0 = s_k.mu + s_k.phi * (mu - s_k.mu);
+            m0 += (s_k.sr * e0) * a.obs[0];
+        }
         for (int q = tid; q < n; q += GT) {
             __stcg(&a.XE[pstart + q], make_double2(mu, e0));
             __stcg(&a.perm[pstart + q], pstart + q);
@@ -698,7 +722,12 @@ __global__ void __launch_bounds__(GT, 1) sv_grid_kernel(const GridArgs a) {
             const double mhat = mom1 / S;
             double var = mom2 / S - mhat * mhat;
             if (!(var > 0.0)) var = 0.0;
-            var = var + s_k.sd * s_k.sd;
+            if constexpr (GEN) {
+                const double psd = M::prop_sd(s_k);
+                var = var + psd * psd;
+            } else {
+                var = var + s_k.sd * s_k.sd;
+            }
             const double shat = sqrt(var);
             s_sc.mhat = mhat;
             s_sc.shat = shat;
@@ -735,7 +764,7 @@ __global__ void __launch_bounds__(GT, 1) sv_grid_kernel(const GridArgs a) {
             const double y1 = a.obs[t - 1];
             const double ylag = a.obs[t >= 2 ? t - 2 : 0];   // Q5: the score terms of step i use obs[i - LAG]; i = t + LAG - 2
             const double mhat = s_sc.mhat, inv_shat = s_sc.inv_shat;
-            const double mu = s_k.mu, phi = s_k.phi, sr = s_k.sr, sd = s_k.sd;
+            const double mu = sv_of(s_k).mu, phi = sv_of(s_k).phi, sr = sv_of(s_k).sr, sd = M::prop_sd(s_k);
             const double* Ut = a.U + (size_t)(t / a.u_cs) * a.u_cstride + (size_t)(t % a.u_cs) * a.u_tstride;
             long long ujs = a.u_jstride;
             if (a.u_flag) {
@@ -800,13 +829,20 @@ __global__ void __launch_bounds__(GT, 1) sv_grid_kernel(const GridArgs a) {
                     const int i = (k0 + u) * GT + tid;
                     xn[k0 + u] = 0.0;
                     if (i < nc) {
-                        double mean = mu + phi * (xe[u].x - mu);     // :355
-                        mean += (sr * xe[u].y) * y1;                  // :356
-                        const double x = mean + sd * uu[u];           // :357-358
+                        double x;
+                        if constexpr (GEN) {
+                            x = xe[u].y + sd * uu[u];                 // M::propagate, the mean stored with the parent
+                        } else {
+                            double mean = mu + phi * (xe[u].x - mu);     // :355
+                            mean += (sr * xe[u].y) * y1;                  // :356
+                            x = mean + sd * uu[u];                        // :357-358
+                        }
                         if (!isfinite(x)) bad = true;
                         xn[k0 + u] = x;
                         atomicAdd(&s_fhist[fine_bin(x, mhat, inv_shat)], 1);
-                        if (!(a.dbg & 2)) {
+                        if constexpr (GEN) {
+                            if (!(a.dbg & 2)) st_stream_f64x4(&Pt[(size_t)(jb + i) * RS], pol_stream, xe[u].x, 0.0, 0.0, x);
+                        } else if (!(a.dbg & 2)) {
                             // residual of the transition parent -> child as the score terms use it (:452-453)
                             double sq = x - mu - phi * (xe[u].x - mu);
                             sq -= sr * xe[u].y * ylag;
@@ -1033,10 +1069,14 @@ __global__ void __launch_bounds__(GT, 1) sv_grid_kernel(const GridArgs a) {
             const double y = a.obs[t];
             const double xmin = mhat + shat * ((double)s_sc.binlo * kBinW - kZ);
             const double xmax = mhat + shat * ((double)(s_sc.binhi + 1) * kBinW - kZ);
-            double xs_ = (y != 0.0) ? 2.0 * log(fabs(y)) : xmin;
-            xs_ = fmin(fmax(xs_, xmin), xmax);
-            const double es_ = exp(-0.5 * xs_);
-            s_sc.shift = (-0.91893853320467267 - 0.5 * xs_) - (0.5 * y * y) * (es_ * es_);
+            if constexpr (GEN) {
+                s_sc.shift = M::logw_max(s_k, xmin, xmax, y);
+            } else {
+                double xs_ = (y != 0.0) ? 2.0 * log(fabs(y)) : xmin;
+                xs_ = fmin(fmax(xs_, xmin), xmax);
+                const double es_ = exp(-0.5 * xs_);
+                s_sc.shift = (-0.91893853320467267 - 0.5 * xs_) - (0.5 * y * y) * (es_ * es_);
+            }
             if (c == 0) a.shiftv[t] = s_sc.shift;
         }
         PROF_MARK(6);   // A2 scan+scatter
@@ -1190,10 +1230,10 @@ __global__ void __launch_bounds__(GT, 1) sv_grid_kernel(const GridArgs a) {
             PROF_MARK(26);   // B: reorder
         }
         {
-            // weights (:427-437): lw = -0.9189 - x/2 - y^2 exp(-x) / 2, sh = exp(lw - shift);
+            // weights (:427-437): lw = -0.9189 - x/2 - y^2 exp(-x) / 2 (M::logw), sh = exp(lw - shift);
             // fixed-lag score terms (:445-470): ancestor pair (time t-L+1, t-L+2) from one half sector
             const double y = a.obs[t], hy2 = 0.5 * y * y, shift = s_sc.shift;
-            const double mu = s_k.mu, phi = s_k.phi, sr = s_k.sr;
+            const double mu = sv_of(s_k).mu, phi = sv_of(s_k).phi, sr = sv_of(s_k).sr;
             bool bad = false;
 #pragma unroll
             for (int kk = 0; kk < KPT; ++kk) {
@@ -1201,8 +1241,9 @@ __global__ void __launch_bounds__(GT, 1) sv_grid_kernel(const GridArgs a) {
                 if (q < n) {
                     const double x = s_xb[q];
                     const int j = s_jb[q];
-                    const double e = exp(-0.5 * x);
-                    const double lw = (-0.91893853320467267 - 0.5 * x) - hy2 * (e * e);
+                    // e: the second double of XE (SV exp(-x/2), else the children's propagation mean)
+                    const double e = GEN ? M::prop_mean(s_k, x, y) : exp(-0.5 * x);
+                    const double lw = GEN ? M::logw(s_k, x, y) : (-0.91893853320467267 - 0.5 * x) - hy2 * (e * e);
                     double sh = exp(lw - shift);
                     if (!isfinite(sh)) {
                         bad = true;
@@ -1224,8 +1265,8 @@ __global__ void __launch_bounds__(GT, 1) sv_grid_kernel(const GridArgs a) {
                         a.Ahist[(size_t)t * N + pstart + q] = __ldcg(&a.parentpos[j]);
                     }
                     acc[0] = fma(sh, x, acc[0]);
-                    double m = mu + phi * (x - mu);
-                    m += (sr * e) * y;
+                    double m = GEN ? e : mu + phi * (x - mu);
+                    if (!GEN) m += (sr * e) * y;
                     const double shm = sh * m;
                     acc[1] += shm;
                     acc[2] = fma(shm, m, acc[2]);
@@ -1310,38 +1351,74 @@ __global__ void __launch_bounds__(GT, 1) sv_grid_kernel(const GridArgs a) {
 #pragma unroll
                 for (int i = 0; i < 4; ++i) hm[i] = 0.0;
             }
+            if constexpr (GEN) {
+                // generic path: sc[0] = sum sh curr (smoother), sc[1 + k] = sum sh g[k] of M::score_main on the pair
+                // (curr, next) = (parent value, own value) of the ancestor; y = obs[t - LAG] (Q5)
+                const double yl = a.obs[t - L];
 #pragma unroll
-            for (int k0 = 0; k0 < KPT; k0 += 4) {
-                double pc[4], psq[4], pey[4];
+                for (int k0 = 0; k0 < KPT; k0 += 4) {
+                    double pc[4], px[4];
 #pragma unroll
-                for (int u = 0; u < 4; ++u) {
-                    const int q = (k0 + u) * GT + tid;
-                    pc[u] = psq[u] = pey[u] = 0.0;
-                    if (q < n) {
-                        const PEntry* pp = &Pg[(size_t)min(max(s_ab[q], 0), N - 1) * RS];
-                        double d3;
-                        asm volatile("ld.global.cg.L2::cache_hint.v4.f64 {%0,%1,%2,%3}, [%4], %5;"
-                                     : "=d"(pc[u]), "=d"(psq[u]), "=d"(pey[u]), "=d"(d3)
-                                     : "l"(pp), "l"(HESS ? pol_keep : pol_pld));
+                    for (int u = 0; u < 4; ++u) {
+                        const int q = (k0 + u) * GT + tid;
+                        pc[u] = px[u] = 0.0;
+                        if (q < n) {
+                            const PEntry* pp = &Pg[(size_t)min(max(s_ab[q], 0), N - 1) * RS];
+                            double d1, d2;
+                            asm volatile("ld.global.cg.L2::cache_hint.v4.f64 {%0,%1,%2,%3}, [%4], %5;"
+                                         : "=d"(pc[u]), "=d"(d1), "=d"(d2), "=d"(px[u])
+                                         : "l"(pp), "l"(pol_pld));
+                        }
+                    }
+#pragma unroll
+                    for (int u = 0; u < 4; ++u) {
+                        const int q = (k0 + u) * GT + tid;
+                        if (q < n) {
+                            const double wd = s_sh[q];
+                            sc[0] = fma(wd, pc[u], sc[0]);
+                            if constexpr (!M::kScoreIsZero) {
+                                double g[4];
+                                M::score_main(s_k, pc[u], px[u], yl, g);
+#pragma unroll
+                                for (int i = 0; i < 4; ++i) sc[1 + i] = fma(wd, g[i], sc[1 + i]);
+                            }
+                        }
                     }
                 }
+            } else {
 #pragma unroll
-                for (int u = 0; u < 4; ++u) {
-                    const int q = (k0 + u) * GT + tid;
-                    if (q < n) {
-                        const double wd = s_sh[q];
-                        const double ws = wd * psq[u];
-                        sc[0] = fma(wd, pc[u], sc[0]);
-                        sc[1] += ws;
-                        sc[2] = fma(ws, pc[u], sc[2]);
-                        sc[3] = fma(ws, psq[u], sc[3]);
-                        sc[4] = fma(ws, pey[u], sc[4]);
-                        if constexpr (HESS) {
-                            const double we = wd * pey[u], wc = wd * pc[u];
-                            hm[0] += we;
-                            hm[1] = fma(wc, pc[u], hm[1]);
-                            hm[2] = fma(wc, pey[u], hm[2]);
-                            hm[3] = fma(we, pey[u], hm[3]);
+                for (int k0 = 0; k0 < KPT; k0 += 4) {
+                    double pc[4], psq[4], pey[4];
+#pragma unroll
+                    for (int u = 0; u < 4; ++u) {
+                        const int q = (k0 + u) * GT + tid;
+                        pc[u] = psq[u] = pey[u] = 0.0;
+                        if (q < n) {
+                            const PEntry* pp = &Pg[(size_t)min(max(s_ab[q], 0), N - 1) * RS];
+                            double d3;
+                            asm volatile("ld.global.cg.L2::cache_hint.v4.f64 {%0,%1,%2,%3}, [%4], %5;"
+                                         : "=d"(pc[u]), "=d"(psq[u]), "=d"(pey[u]), "=d"(d3)
+                                         : "l"(pp), "l"(HESS ? pol_keep : pol_pld));
+                        }
+                    }
+#pragma unroll
+                    for (int u = 0; u < 4; ++u) {
+                        const int q = (k0 + u) * GT + tid;
+                        if (q < n) {
+                            const double wd = s_sh[q];
+                            const double ws = wd * psq[u];
+                            sc[0] = fma(wd, pc[u], sc[0]);
+                            sc[1] += ws;
+                            sc[2] = fma(ws, pc[u], sc[2]);
+                            sc[3] = fma(ws, psq[u], sc[3]);
+                            sc[4] = fma(ws, pey[u], sc[4]);
+                            if constexpr (HESS) {
+                                const double we = wd * pey[u], wc = wd * pc[u];
+                                hm[0] += we;
+                                hm[1] = fma(wc, pc[u], hm[1]);
+                                hm[2] = fma(wc, pey[u], hm[2]);
+                                hm[3] = fma(we, pey[u], hm[3]);
+                            }
                         }
                     }
                 }
@@ -1487,8 +1564,8 @@ __global__ void __launch_bounds__(256) grid_reduce_kernel(const double* __restri
 // with i = NOBS - L + irel, idx = L - 1 - irel; hist_k[p] = value of the ancestor k steps back of
 // the particle at sorted position p of the final generation.
 // HESS: partH[irel][block][0..19] = the hessian1 / hessian2 terms of :564-626 (alpha of the ancestor LAG-2 steps
-// back of the final particle, weights W_i, obs[i - LAG] with wrap-around, Q8)
-template <bool HESS>
+// back of the final particle, weights W_i, obs[i - LAG] with wrap-around, Q8).  M: the model (g = M::score_tail).
+template <bool HESS, class M>
 __global__ void __launch_bounds__(256) grid_tail_kernel(GridArgs a, const double* __restrict__ sums,
                                                         double* __restrict__ part, double* __restrict__ partH,
                                                         int nblk) {
@@ -1496,8 +1573,8 @@ __global__ void __launch_bounds__(256) grid_tail_kernel(GridArgs a, const double
     const int tid = threadIdx.x;
     const int L = a.LAG, N = a.N, T = a.NOBS - 1, RP = a.RP;
     const int irel = blockIdx.y, i = a.NOBS - L + irel, idx = L - 1 - irel;
-    SvConst k;
-    sv_const_init(k, a.params);
+    typename M::Const k;
+    M::init(k, a.params);
     const double y1 = obs_wrap(a.obs, i - 1, a.NOBS);
     const double ST = sums[(size_t)T * 8], Si = sums[(size_t)i * 8];
     const double* shT = a.shring + (size_t)(T % L) * N;
@@ -1528,9 +1605,13 @@ __global__ void __launch_bounds__(256) grid_tail_kernel(GridArgs a, const double
             const double pe_n = pe.x;
             acc[0] += wT * curr;
             const double wi = shi[p] / Si;
-            double sq, g[4];
-            const double ec = exp(-0.5 * curr);
-            sv_score_tail_e(k, curr, ec, pe_n, y1, sq, g);   // the tail uses obs[i - 1] (Q6)
+            double sq, g[4], ec;
+            if constexpr (std::is_same<M, SvLeverageModel>::value) {
+                ec = exp(-0.5 * curr);
+                sv_score_tail_e(k, curr, ec, pe_n, y1, sq, g);   // the tail uses obs[i - 1] (Q6)
+            } else {
+                M::score_tail(k, curr, pe_n, y1, g);
+            }
 #pragma unroll
             for (int q = 0; q < 4; ++q) acc[1 + q] += g[q] * wi;
             if constexpr (HESS) {
@@ -1640,7 +1721,9 @@ __global__ void __launch_bounds__(256) grid_tail_reduce_kernel(const double* __r
 }
 
 // sums[t][0] = sum sh, [1] = sum sh x, [2] = sum sh c, [3] = sum sh sq, [4] = sum sh sq c, [5] = sum sh sq^2,
-// [6] = sum sh sq ey (c = lagged ancestor value, sq / ey as stored in P);  tail[irel][0..4]
+// [6] = sum sh sq ey (c = lagged ancestor value, sq / ey as stored in P);  tail[irel][0..4].
+// GEN (the generic path of a model other than SV): [3..6] = sum sh g[0..3], traj[0] = the initial state.
+template <bool GEN>
 __global__ void grid_finish_kernel(const GridCtrl* __restrict__ ctrl, const double* __restrict__ sums,
                                    const double* __restrict__ shift, const double* __restrict__ xmin,
                                    const double* __restrict__ tail, const double* __restrict__ params,
@@ -1686,20 +1769,24 @@ __global__ void grid_finish_kernel(const GridCtrl* __restrict__ ctrl, const doub
     }
     for (int t = tid; t < nobs; t += gridDim.x * blockDim.x) {
         filt[t] = sums[(size_t)t * 8 + 1] / sums[(size_t)t * 8];
-        traj[t] = (t == 0) ? params[0] : xmin[t];   // Q10/Q11: traj[t] = X_t[0] for t >= 1, X_0 == mu
+        traj[t] = (t == 0 && !GEN) ? params[0] : xmin[t];   // Q10/Q11: traj[t] = X_t[0] for t >= 1, X_0 == mu
         double s = 0.0, g[4] = {0.0, 0.0, 0.0, 0.0};
         const int src = t + L - 1;   // main-loop terms land at tt = i - L + 1 (:445-470)
         if (t >= 1 && src < nobs) {
             const double* sm = sums + (size_t)src * 8;
             const double S = sm[0];
-            SvConst k;
-            sv_const_init(k, params);
             s = sm[2] / S;
-            // weighted means of g[0..3] of :454-465 written in the monomials sq, sq c, sq^2, sq ey
-            g[0] = k.q * k.one_m_phi * sm[3] / S;
-            g[1] = k.q * k.one_m_phi2 * (sm[4] - k.mu * sm[3]) / S;
-            g[2] = (k.q * sm[5] + k.q * k.sr * sm[6] - S) / S;
-            g[3] = (k.rho * S - k.q * k.rho * sm[5] + k.inv_sv * sm[6]) / S;
+            if constexpr (GEN) {
+                for (int q = 0; q < 4; ++q) g[q] = sm[3 + q] / S;
+            } else {
+                SvConst k;
+                sv_const_init(k, params);
+                // weighted means of g[0..3] of :454-465 written in the monomials sq, sq c, sq^2, sq ey
+                g[0] = k.q * k.one_m_phi * sm[3] / S;
+                g[1] = k.q * k.one_m_phi2 * (sm[4] - k.mu * sm[3]) / S;
+                g[2] = (k.q * sm[5] + k.q * k.sr * sm[6] - S) / S;
+                g[3] = (k.rho * S - k.q * k.rho * sm[5] + k.inv_sv * sm[6]) / S;
+            }
         }
         const int irel_s = t - (nobs - L);   // tail: i = nobs-L+irel adds smo[i], gradient[.][i-L+1]
         if (irel_s >= 0 && irel_s < L) s += tail[irel_s * 8];
@@ -1788,10 +1875,14 @@ size_t sv_grid_ws_bytes(int nobs, int n, int lag, int G, int hist, int hess) {
 int sv_grid_run(const double* d_obs, const double* d_params, const double* d_rvr, const double* d_u, int nobs,
                 int n, int lag, int G, double* d_filt, double* d_smo, double* d_ll, double* d_grad, double* d_traj,
                 long long* d_diag, double* d_xh, int* d_ah, void* d_ws, size_t ws_bytes, long long* d_prof,
-                cudaStream_t st, int u_chunk_steps, const int* d_u_flag, double* d_hess1, double* d_hess2) {
+                cudaStream_t st, int u_chunk_steps, const int* d_u_flag, double* d_hess1, double* d_hess2, int model) {
     if (!sv_grid_eligible(nobs, n, lag, G)) return set_error(PMMH_ERR_INVALID, "grid kernel: sizes not eligible");
     const int hist = d_xh != nullptr;
     const int hess = d_hess1 != nullptr && d_hess2 != nullptr;
+    if (model != PMMH_MODEL_SV_LEVERAGE && model != PMMH_MODEL_LINEAR_GAUSSIAN && model != PMMH_MODEL_LINEAR_GAUSSIAN_FA)
+        return set_error(PMMH_ERR_INVALID, "grid kernel: unknown model id");
+    if (hess && model != PMMH_MODEL_SV_LEVERAGE)
+        return set_error(PMMH_ERR_INVALID, "grid kernel: the Hessian branch exists for the SV model only");
     const GridLayout L = grid_layout(nobs, n, lag, G, hist, hess);
     if (ws_bytes < L.total) return set_error(PMMH_ERR_WORKSPACE, "grid kernel: workspace too small");
     char* ws = (char*)d_ws;
@@ -1856,12 +1947,17 @@ int sv_grid_run(const double* d_obs, const double* d_params, const double* d_rvr
         // no persisting L2 set-aside for the kernel's evict_last accesses: with one every phase is slower
         // (DESIGN 4.0), and left unset the evaluation at N = 2^20 is ~6 % slower
         GRID_CUDA(cudaDeviceSetLimit(cudaLimitPersistingL2CacheSize, 0));
-        GRID_CUDA(cudaFuncSetAttribute(sv_grid_kernel<1024, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kDynSmem));
-        GRID_CUDA(cudaFuncSetAttribute(sv_grid_kernel<1024, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kDynSmem));
+        GRID_CUDA(cudaFuncSetAttribute(sv_grid_kernel<1024, false, SvLeverageModel>, cudaFuncAttributeMaxDynamicSharedMemorySize, kDynSmem));
+        GRID_CUDA(cudaFuncSetAttribute(sv_grid_kernel<1024, true, SvLeverageModel>, cudaFuncAttributeMaxDynamicSharedMemorySize, kDynSmem));
+        GRID_CUDA(cudaFuncSetAttribute(sv_grid_kernel<1024, false, LinearGaussianModel>, cudaFuncAttributeMaxDynamicSharedMemorySize, kDynSmem));
+        GRID_CUDA(cudaFuncSetAttribute(sv_grid_kernel<1024, false, LinearGaussianFullyAdapted>, cudaFuncAttributeMaxDynamicSharedMemorySize, kDynSmem));
         attr_set[dev] = true;
     }
     void* kargs[] = {(void*)&a};
-    const void* kern = hess ? (const void*)sv_grid_kernel<1024, true> : (const void*)sv_grid_kernel<1024, false>;
+    const void* kern = hess ? (const void*)sv_grid_kernel<1024, true, SvLeverageModel>
+                            : (const void*)sv_grid_kernel<1024, false, SvLeverageModel>;
+    if (model == PMMH_MODEL_LINEAR_GAUSSIAN) kern = (const void*)sv_grid_kernel<1024, false, LinearGaussianModel>;
+    if (model == PMMH_MODEL_LINEAR_GAUSSIAN_FA) kern = (const void*)sv_grid_kernel<1024, false, LinearGaussianFullyAdapted>;
     GRID_CUDA(cudaLaunchCooperativeKernel(kern, dim3(G), dim3(1024), kargs, kDynSmem, st));
     double* sums = (double*)(ws + L.sums);
     double* tailpart = (double*)(ws + L.tailpart);
@@ -1871,15 +1967,19 @@ int sv_grid_run(const double* d_obs, const double* d_params, const double* d_rvr
         double* sumsH = (double*)(ws + L.sumsH);
         double* tailpartH = (double*)(ws + L.tailpartH);
         grid_reduceH_kernel<<<nobs, 640, 0, st>>>(a.psumH, G, lag, sumsH);
-        grid_tail_kernel<true><<<dim3(L.nblk, lag), 256, 0, st>>>(a, sums, tailpart, tailpartH, L.nblk);
+        grid_tail_kernel<true, SvLeverageModel><<<dim3(L.nblk, lag), 256, 0, st>>>(a, sums, tailpart, tailpartH, L.nblk);
         grid_hess_finish_kernel<<<1, 32, 0, st>>>(a.ctrl, sums, sumsH, tailpartH, d_params, L.nblk, nobs, lag, d_hess1, d_hess2);
+    } else if (model == PMMH_MODEL_LINEAR_GAUSSIAN) {
+        grid_tail_kernel<false, LinearGaussianModel><<<dim3(L.nblk, lag), 256, 0, st>>>(a, sums, tailpart, nullptr, L.nblk);
+    } else if (model == PMMH_MODEL_LINEAR_GAUSSIAN_FA) {
+        grid_tail_kernel<false, LinearGaussianFullyAdapted><<<dim3(L.nblk, lag), 256, 0, st>>>(a, sums, tailpart, nullptr, L.nblk);
     } else {
-        grid_tail_kernel<false><<<dim3(L.nblk, lag), 256, 0, st>>>(a, sums, tailpart, nullptr, L.nblk);
+        grid_tail_kernel<false, SvLeverageModel><<<dim3(L.nblk, lag), 256, 0, st>>>(a, sums, tailpart, nullptr, L.nblk);
     }
     grid_tail_reduce_kernel<<<lag, 256, 0, st>>>(tailpart, L.nblk, tail);
-    grid_finish_kernel<<<(nobs + 255) / 256, 256, 0, st>>>(a.ctrl, sums, a.shiftv, a.xminv, tail, d_params, nobs, lag,
-                                                           (double)n, d_ll, d_filt, d_smo, d_grad, d_traj, d_diag,
-                                                           (long long*)(ws + L.info));
+    auto finish = model == PMMH_MODEL_SV_LEVERAGE ? grid_finish_kernel<false> : grid_finish_kernel<true>;
+    finish<<<(nobs + 255) / 256, 256, 0, st>>>(a.ctrl, sums, a.shiftv, a.xminv, tail, d_params, nobs, lag, (double)n, d_ll,
+                                               d_filt, d_smo, d_grad, d_traj, d_diag, (long long*)(ws + L.info));
     GRID_CUDA(cudaGetLastError());
     return PMMH_OK;
 }

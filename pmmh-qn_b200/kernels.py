@@ -125,8 +125,12 @@ def flps_sv_corr(obs, params, rvr, u, lag=10, compute_hessian=False, store_histo
 
 def flps_model_corr(model_id, obs, params, rvr, u, lag=10, store_history=False, workspace=None):
     """Model-generic fixed-lag smoother (pmmh_flps_model_corr, csrc/pf_model.cuh): log-likelihood +
-    gradient of [B] problems with N <= 4096 particles each, one CTA per problem.  ``model_id``:
-    _lib.MODEL_SV_LEVERAGE or _lib.MODEL_LINEAR_GAUSSIAN; params [B, 4] (unused slots ignored)."""
+    gradient of [B] problems.  2 <= lag <= 10.  Up to 4096 particles: any B, one CTA per problem (chain
+    kernel, diag kernel 3).  Above: B == 1, n_obs >= 2 lag and up to 7168 particles per SM (1,060,864 on
+    148 SMs), one persistent launch over the GPU (grid kernel, diag kernel 5).  Other sizes raise PmmhError.
+    ``model_id``: _lib.MODEL_SV_LEVERAGE (bit-identical to flps_sv_corr on the same kernel),
+    _lib.MODEL_LINEAR_GAUSSIAN or _lib.MODEL_LINEAR_GAUSSIAN_FA; params [B, 4] (unused slots ignored).
+    No fallback pass: diag[:, PMMH_DIAG_STATUS] == 1 reports an abandoned evaluation."""
     lib = _lib.load()
     obs, obs_stride, params, rvr, u, batch, n_obs, n = _sv_common(obs, params, rvr, u)
     dev = u.device
