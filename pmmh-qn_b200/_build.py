@@ -13,7 +13,7 @@ CSRC = os.path.join(HERE, "csrc")
 LIB_DIR = os.path.join(HERE, "lib")
 LIB_PATH = os.path.join(LIB_DIR, "libpmmh_qn_b200.so")
 SOURCES = ["sv_filter.cu", "sv_fast.cu", "sv_chain.cu", "sv_split.cu", "sv_grid.cu", "aux_kernels.cu", "capi.cu"]
-HEADERS = ["common.cuh", "sv_filter.cuh", "sv_math.cuh", "aux_kernels.cuh", "philox.cuh", "sv_split.cuh", "sv_grid.cuh", "pf_model.cuh", os.path.join("..", "..", "include", "pmmh_qn.h")]
+HEADERS = ["common.cuh", "sv_filter.cuh", "sv_math.cuh", "aux_kernels.cuh", "philox.cuh", "sv_split.cuh", "sv_grid.cuh", "sv_call.h", "pf_model.cuh", os.path.join("..", "..", "include", "pmmh_qn.h")]
 
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a",

@@ -69,6 +69,13 @@ int get_device_info(DeviceInfo* out) {
     return PMMH_OK;
 }
 
+// an sm_100 device and, for the kernels that need it, cooperative launch
+int check_device(const DeviceInfo& di, bool coop) {
+    if (di.major < 10) return fail(PMMH_ERR_NO_DEVICE, "an sm_100 (B200) device is required");
+    if (coop && !di.coop) return fail(PMMH_ERR_NO_DEVICE, "device lacks cooperative launch");
+    return PMMH_OK;
+}
+
 // The SV smoother's kernels (diag[PMMH_DIAG_KERNEL] in brackets)
 enum class SvKernel {
     None,            // host-streamed entry: no kernel takes the sizes (the call is refused)
@@ -193,9 +200,8 @@ int sv_make_plan(SvShape s, SvEntry entry, SvPlan* p) {
     if ((long long)s.n + s.nobs >= (1ll << 31)) return fail(PMMH_ERR_INVALID, "n_particles too large");
     DeviceInfo di;
     int rc = get_device_info(&di);
+    if (rc == PMMH_OK) rc = check_device(di, true);
     if (rc != PMMH_OK) return rc;
-    if (di.major < 10) return fail(PMMH_ERR_NO_DEVICE, "an sm_100 (B200) device is required");
-    if (!di.coop) return fail(PMMH_ERR_NO_DEVICE, "device lacks cooperative launch");
     memset(p, 0, sizeof(*p));
     p->c = sv_choose(s, g_sv_algorithm, entry, di.sm);
     const int G = p->c.G, n = s.n, nobs = s.nobs;
@@ -240,10 +246,7 @@ int sv_make_plan(SvShape s, SvEntry entry, SvPlan* p) {
 }
 
 // Arguments of the general, chain and exchange kernels (the ws_* fields are per kernel)
-pmmh::SvArgs sv_args(const SvPlan& p, const SvShape& s, const double* d_obs, long long obs_stride,
-                     const double* d_params, const double* d_rvr, const double* d_u, double* d_filt, double* d_smo,
-                     double* d_ll, double* d_grad, double* d_traj, double* d_h1, double* d_h2, long long* d_diag,
-                     double* d_xh, int* d_ah, void* d_ws) {
+pmmh::SvArgs sv_args(const SvPlan& p, const SvShape& s, const pmmh::SvCall& c) {
     pmmh::SvArgs a;
     memset(&a, 0, sizeof(a));
     a.N = s.n;
@@ -256,25 +259,28 @@ pmmh::SvArgs sv_args(const SvPlan& p, const SvShape& s, const double* d_obs, lon
     a.RING = p.RING;
     a.mode = s.mode;
     a.hess = s.hess;
+    a.model_id = c.model;
     a.SQ = p.SQ;
     a.SQW = p.SQW;
-    a.obs = d_obs;
-    a.obs_stride = obs_stride;
-    a.params = d_params;
-    a.rvr = d_rvr;
-    a.U = d_u;
-    a.filt = d_filt;
-    a.smo = d_smo;
-    a.loglike = d_ll;
-    a.grad = d_grad;
-    a.traj = d_traj;
-    a.hess1 = d_h1;
-    a.hess2 = d_h2;
-    a.diag = d_diag;
-    a.Xhist = d_xh;
-    a.Ahist = d_ah;
-    a.prof = g_sv_prof;
-    a.ws = (char*)d_ws;
+    a.obs = c.obs;
+    a.obs_stride = c.obs_stride;
+    a.params = c.params;
+    a.rvr = c.rvr;
+    a.U = c.u;
+    a.u_chunk = c.slot;
+    a.u_ready = c.u_flag;
+    a.filt = c.filt;
+    a.smo = c.smo;
+    a.loglike = c.ll;
+    a.grad = c.grad;
+    a.traj = c.traj;
+    a.hess1 = c.hess1;
+    a.hess2 = c.hess2;
+    a.diag = c.diag;
+    a.Xhist = c.x_hist;
+    a.Ahist = c.a_hist;
+    a.prof = c.prof;
+    a.ws = (char*)c.ws;
     return a;
 }
 
@@ -285,6 +291,51 @@ cudaError_t exchange_launch(const SvPlan& p, pmmh::SvArgs& a, cudaStream_t st) {
     a.ws_team_stride = p.fast_team_stride;
     cudaError_t err = cudaMemsetAsync(a.ws, 0, p.fast_sync_bytes, st);
     return err != cudaSuccess ? err : pmmh::sv_fast_launch(a, p.grid, st);
+}
+
+// Runs the plan's kernel on call `c`, then the general kernel where it is the plan's kernel or its fallback pass
+// (in the same stream, reusing the workspace).  The grid kernel without its Hessian branch and the streaming
+// kernels write no Hessian: where the entry has Hessian outputs they are zeroed.
+int sv_launch_plan(const SvPlan& p, const SvShape& s, const pmmh::SvCall& c) {
+    pmmh::SvArgs a = sv_args(p, s, c);
+    int rc = PMMH_OK;
+    bool zero_hess = false;
+    switch (p.c.kernel) {
+    case SvKernel::Chain:
+        a.ws_team_stride = p.chain_stride;
+        PMMH_CUDA(pmmh::sv_chain_launch(a, p.grid, c.stream));
+        break;
+    case SvKernel::Grid:
+        rc = pmmh::sv_grid_run(c, s.nobs, s.n, s.lag, p.c.grid_G, s.hess);
+        zero_hess = !s.hess;
+        break;
+    case SvKernel::StreamRecords:
+        rc = pmmh::sv_split_single_run(c, s.nobs, s.n, s.lag);
+        zero_hess = true;
+        break;
+    case SvKernel::StreamPath:
+        rc = pmmh::sv_split_path_run(c, s.nobs, s.n, s.lag);
+        zero_hess = true;
+        break;
+    case SvKernel::Exchange:
+        PMMH_CUDA(exchange_launch(p, a, c.stream));
+        break;
+    default: break;
+    }
+    if (rc != PMMH_OK) return rc;
+    if (zero_hess && c.hess1) {
+        PMMH_CUDA(cudaMemsetAsync(c.hess1, 0, 16 * sizeof(double), c.stream));
+        PMMH_CUDA(cudaMemsetAsync(c.hess2, 0, 16 * sizeof(double), c.stream));
+    }
+    if (p.c.kernel != SvKernel::General) {
+        if (!p.c.fallback) return PMMH_OK;
+        a.only_failed = 1;
+    }
+    a.ws_sync_bytes = p.sync_bytes;
+    a.ws_team_stride = p.team_stride;
+    PMMH_CUDA(cudaMemsetAsync(c.ws, 0, p.stamp_bytes, c.stream));
+    PMMH_CUDA(pmmh::sv_launch(a, p.grid, c.stream));
+    return PMMH_OK;
 }
 
 int sv_run(int mode, const double* d_obs, long long obs_stride, const double* d_params,
@@ -303,50 +354,12 @@ int sv_run(int mode, const double* d_obs, long long obs_stride, const double* d_
     int rc = sv_make_plan(s, SvEntry::Resident, &p);
     if (rc != PMMH_OK) return rc;
     if (ws_bytes < p.total) return fail(PMMH_ERR_WORKSPACE, "workspace too small");
-    cudaStream_t st = (cudaStream_t)stream;
-    pmmh::SvArgs a = sv_args(p, s, d_obs, obs_stride, d_params, d_rvr, d_u, d_filt, d_smo, d_ll, d_grad, d_traj,
-                             d_h1, d_h2, d_diag, d_xh, d_ah, d_ws);
-    switch (p.c.kernel) {
-    case SvKernel::Chain:
-        a.ws_sync_bytes = 0;
-        a.ws_team_stride = p.chain_stride;
-        PMMH_CUDA(pmmh::sv_chain_launch(a, p.grid, st));
-        break;
-    case SvKernel::Grid:
-        rc = pmmh::sv_grid_run(d_obs, d_params, d_rvr, d_u, nobs, n, lag, p.c.grid_G, d_filt, d_smo, d_ll, d_grad,
-                               d_traj, d_diag, d_xh, d_ah, d_ws, ws_bytes, g_sv_prof, st, 0, nullptr,
-                               hess ? d_h1 : nullptr, hess ? d_h2 : nullptr);
-        if (rc != PMMH_OK) return rc;
-        if (!hess) {
-            PMMH_CUDA(cudaMemsetAsync(d_h1, 0, 16 * sizeof(double), st));
-            PMMH_CUDA(cudaMemsetAsync(d_h2, 0, 16 * sizeof(double), st));
-        }
-        break;
-    case SvKernel::StreamRecords:
-    case SvKernel::StreamPath:
-        rc = p.c.kernel == SvKernel::StreamPath
-                 ? pmmh::sv_split_path_run(d_obs, d_params, d_rvr, d_u, nobs, n, lag, d_filt, d_smo, d_ll,
-                                           d_grad, d_traj, d_diag, d_ws, ws_bytes, st)
-                 : pmmh::sv_split_single_run(d_obs, d_params, d_rvr, d_u, nobs, n, lag, d_filt, d_smo, d_ll,
-                                             d_grad, d_traj, d_diag, d_ws, ws_bytes, st);
-        if (rc != PMMH_OK) return rc;
-        PMMH_CUDA(cudaMemsetAsync(d_h1, 0, 16 * sizeof(double), st));
-        PMMH_CUDA(cudaMemsetAsync(d_h2, 0, 16 * sizeof(double), st));
-        break;
-    case SvKernel::Exchange:
-        PMMH_CUDA(exchange_launch(p, a, st));
-        break;
-    default: break;
-    }
-    if (p.c.kernel != SvKernel::General) {
-        if (!p.c.fallback) return PMMH_OK;
-        a.only_failed = 1;   // in the same stream, reusing the workspace
-    }
-    a.ws_sync_bytes = p.sync_bytes;
-    a.ws_team_stride = p.team_stride;
-    PMMH_CUDA(cudaMemsetAsync(d_ws, 0, p.stamp_bytes, st));
-    PMMH_CUDA(pmmh::sv_launch(a, p.grid, st));
-    return PMMH_OK;
+    pmmh::SvCall c = {};
+    c.obs = d_obs; c.obs_stride = obs_stride; c.params = d_params; c.rvr = d_rvr; c.u = d_u;
+    c.filt = d_filt; c.smo = d_smo; c.ll = d_ll; c.grad = d_grad; c.traj = d_traj; c.hess1 = d_h1; c.hess2 = d_h2;
+    c.diag = d_diag; c.x_hist = d_xh; c.a_hist = d_ah; c.prof = g_sv_prof;
+    c.ws = d_ws; c.ws_bytes = ws_bytes; c.stream = (cudaStream_t)stream;
+    return sv_launch_plan(p, s, c);
 }
 
 struct DevBuf {
@@ -425,15 +438,21 @@ int pmmh_flps_sv_corr_philox(const double* d_obs, const double* d_params, const 
         return fail(PMMH_ERR_INVALID, "pmmh_flps_sv_corr_philox: null pointer argument");
     DeviceInfo di;
     int rc = get_device_info(&di);
+    if (rc == PMMH_OK) rc = check_device(di, false);
     if (rc != PMMH_OK) return rc;
-    if (di.major < 10) return fail(PMMH_ERR_NO_DEVICE, "an sm_100 (B200) device is required");
     if (!pmmh::sv_split_single_eligible(n_obs, n_particles, lag))
         return fail(PMMH_ERR_INVALID, "pmmh_flps_sv_corr_philox: needs lag in [2, 63] and n_obs >= 2 * lag");
     if (workspace_bytes < pmmh::sv_split_path_ws_bytes(n_obs, n_particles, lag))
         return fail(PMMH_ERR_WORKSPACE, "workspace too small");
-    return pmmh::sv_split_path_run(d_obs, d_params, d_rvr, nullptr, n_obs, n_particles, lag, d_filt, d_smo,
-                                   d_log_like, d_gradient, d_traj, d_diag, d_workspace, workspace_bytes,
-                                   (cudaStream_t)stream, 0, nullptr, seed, philox_offset);
+    SvPlan p = {};
+    p.c.kernel = SvKernel::StreamPath;
+    const SvShape s = {n_obs, n_particles, lag, 1, 0, pmmh::kSvFlps, 0, 0};
+    pmmh::SvCall c = {};
+    c.obs = d_obs; c.params = d_params; c.rvr = d_rvr; c.seed = seed; c.philox_offset = philox_offset;
+    c.filt = d_filt; c.smo = d_smo; c.ll = d_log_like; c.grad = d_gradient; c.traj = d_traj; c.diag = d_diag;
+    c.prof = g_sv_prof;
+    c.ws = d_workspace; c.ws_bytes = workspace_bytes; c.stream = (cudaStream_t)stream;
+    return sv_launch_plan(p, s, c);
 }
 
 int pmmh_flps_sv_corr_philox_workspace_bytes(int n_obs, int n_particles, int lag, size_t* bytes) {
@@ -561,9 +580,7 @@ int enqueue_u_copies(const double* h_rvs, int n_obs, int n, char* d_stage, int s
     return PMMH_OK;
 }
 
-int streamed_plan(int n_obs, int n, int lag, int ctas, SvPlan* p) {
-    return sv_make_plan({n_obs, n, lag, 1, 0, pmmh::kSvFlps, 0, ctas}, SvEntry::HostStreamed, p);
-}
+SvShape streamed_shape(int n_obs, int n, int lag, int ctas) { return {n_obs, n, lag, 1, 0, pmmh::kSvFlps, 0, ctas}; }
 }  // namespace
 
 int pmmh_sv_stream_schedule(int n_obs, int* pieces, int max_pieces) {
@@ -588,7 +605,7 @@ int pmmh_sv_stage_bytes(int n_obs, int n_particles, size_t* bytes) {
 int pmmh_sv_streamed_workspace_bytes(int n_obs, int n_particles, int lag, int ctas_per_problem, size_t* bytes) {
     if (!bytes) return fail(PMMH_ERR_INVALID, "bytes is null");
     SvPlan p;
-    int rc = streamed_plan(n_obs, n_particles, lag, ctas_per_problem, &p);
+    int rc = sv_make_plan(streamed_shape(n_obs, n_particles, lag, ctas_per_problem), SvEntry::HostStreamed, &p);
     if (rc != PMMH_OK) return rc;
     *bytes = p.total;
     return PMMH_OK;
@@ -596,7 +613,8 @@ int pmmh_sv_streamed_workspace_bytes(int n_obs, int n_particles, int lag, int ct
 
 int pmmh_sv_streamed_eligible(int n_obs, int n_particles, int lag, int ctas_per_problem) {
     SvPlan p;
-    return streamed_plan(n_obs, n_particles, lag, ctas_per_problem, &p) == PMMH_OK && p.c.kernel != SvKernel::None;
+    return sv_make_plan(streamed_shape(n_obs, n_particles, lag, ctas_per_problem), SvEntry::HostStreamed, &p) == PMMH_OK &&
+           p.c.kernel != SvKernel::None;
 }
 
 int pmmh_flps_sv_corr_streamed(const double* h_rvs, const double* d_obs, const double* d_params,
@@ -608,8 +626,9 @@ int pmmh_flps_sv_corr_streamed(const double* h_rvs, const double* d_obs, const d
     if (!h_rvs || !d_obs || !d_params || !d_rvr || !d_stage || !d_filt || !d_smo || !d_log_like || !d_gradient ||
         !d_traj || !d_hess1 || !d_hess2 || !d_diag || !d_workspace)
         return fail(PMMH_ERR_INVALID, "pmmh_flps_sv_corr_streamed: null pointer argument");
+    const SvShape s = streamed_shape(n_obs, n_particles, lag, ctas_per_problem);
     SvPlan p;
-    int rc = streamed_plan(n_obs, n_particles, lag, ctas_per_problem, &p);
+    int rc = sv_make_plan(s, SvEntry::HostStreamed, &p);
     if (rc != PMMH_OK) return rc;
     const SvKernel k = p.c.kernel;
     if (k == SvKernel::None)
@@ -632,28 +651,14 @@ int pmmh_flps_sv_corr_streamed(const double* h_rvs, const double* d_obs, const d
     rc = enqueue_u_copies(h_rvs, n_obs, n_particles, (char*)d_stage, slot, k == SvKernel::Grid ? kGridUTaperMin : 0,
                           d_flag, *ss, st);
     if (rc != PMMH_OK) return rc;
-    if (k == SvKernel::Grid) {
-        rc = pmmh::sv_grid_run(d_obs, d_params, d_rvr, d_u, n_obs, n_particles, lag, p.c.grid_G, d_filt, d_smo,
-                               d_log_like, d_gradient, d_traj, d_diag, nullptr, nullptr, d_workspace, workspace_bytes,
-                               g_sv_prof, st, slot, d_flag);
-        if (rc != PMMH_OK) return rc;
-        PMMH_CUDA(cudaMemsetAsync(d_hess1, 0, 16 * sizeof(double), st));
-        PMMH_CUDA(cudaMemsetAsync(d_hess2, 0, 16 * sizeof(double), st));
-    } else if (k == SvKernel::Exchange) {
-        const SvShape s = {n_obs, n_particles, lag, 1, 0, pmmh::kSvFlps, 0, ctas_per_problem};
-        pmmh::SvArgs a = sv_args(p, s, d_obs, 0, d_params, d_rvr, d_u, d_filt, d_smo, d_log_like, d_gradient, d_traj,
-                                 d_hess1, d_hess2, d_diag, nullptr, nullptr, d_workspace);
-        a.u_chunk = slot;
-        a.u_ready = d_flag;
-        PMMH_CUDA(exchange_launch(p, a, st));
-    } else {
-        PMMH_CUDA(cudaMemsetAsync(d_hess1, 0, 16 * sizeof(double), st));
-        PMMH_CUDA(cudaMemsetAsync(d_hess2, 0, 16 * sizeof(double), st));
-        rc = pmmh::sv_split_path_run(d_obs, d_params, d_rvr, d_u, n_obs, n_particles, lag, d_filt, d_smo, d_log_like,
-                                     d_gradient, d_traj, d_diag, d_workspace, workspace_bytes, st, slot,
-                                     ss->ev_slot.data());
-        if (rc != PMMH_OK) return rc;
-    }
+    pmmh::SvCall c = {};
+    c.obs = d_obs; c.params = d_params; c.rvr = d_rvr;
+    c.u = d_u; c.slot = slot; c.u_flag = d_flag; c.slot_ready = ss->ev_slot.data();
+    c.filt = d_filt; c.smo = d_smo; c.ll = d_log_like; c.grad = d_gradient; c.traj = d_traj;
+    c.hess1 = d_hess1; c.hess2 = d_hess2; c.diag = d_diag; c.prof = g_sv_prof;
+    c.ws = d_workspace; c.ws_bytes = workspace_bytes; c.stream = st;
+    rc = sv_launch_plan(p, s, c);
+    if (rc != PMMH_OK) return rc;
     // an evaluation that is abandoned early leaves copies behind: the caller's stream ends after them
     PMMH_CUDA(cudaStreamWaitEvent(st, ss->ev_done, 0));
     return PMMH_OK;
@@ -661,39 +666,42 @@ int pmmh_flps_sv_corr_streamed(const double* h_rvs, const double* d_obs, const d
 
 // ---- model-generic entry point: the chain or the grid kernel instantiated for a model of pf_model.cuh ----------
 namespace {
-// The kernel pmmh_flps_model_corr runs: the chain kernel wherever it applies (any batch), else the grid kernel for
-// one problem on sv_grid_ctas(N, SMs, 0) CTAs; anything else is refused.  *G = the grid kernel's CTAs.
-int model_choose(int n_obs, int n, int lag, int batch, SvKernel* k, int* G) {
+// The plan pmmh_flps_model_corr runs: the chain kernel wherever it applies (any batch), else the grid kernel for one
+// problem on sv_grid_ctas(N, SMs, 0) CTAs; anything else is refused.  The workspace is the chosen kernel's alone (there
+// is no fallback pass), with history on the grid kernel (the query has no flag).
+int model_choose(int n_obs, int n, int lag, int batch, DeviceInfo* di, SvPlan* p) {
     if (n_obs < 2 || batch < 1) return fail(PMMH_ERR_INVALID, "pmmh_flps_model_corr: bad arguments");
-    DeviceInfo di;
-    int rc = get_device_info(&di);
+    int rc = get_device_info(di);
     if (rc != PMMH_OK) return rc;
-    *G = pmmh::sv_grid_ctas(n, di.sm, 0);
-    if (pmmh::sv_chain_eligible(n, lag) && pmmh::sv_chain_smem_bytes(n) <= kMaxDynSmem) *k = SvKernel::Chain;
-    else if (batch == 1 && pmmh::sv_grid_eligible(n_obs, n, lag, *G)) *k = SvKernel::Grid;
-    else
+    memset(p, 0, sizeof(*p));
+    p->c.grid_G = pmmh::sv_grid_ctas(n, di->sm, 0);
+    // G, n_teams and grid are the chain kernel's launch shape (one CTA per problem, at most one problem per SM at a
+    // time); the grid plan carries them unused (sv_grid_run reads grid_G only)
+    p->G = 1;
+    p->n_teams = p->grid = batch < di->sm ? batch : di->sm;
+    if (pmmh::sv_chain_eligible(n, lag) && pmmh::sv_chain_smem_bytes(n) <= kMaxDynSmem) {
+        p->c.kernel = SvKernel::Chain;
+        p->chain_stride = pmmh::sv_chain_ws_bytes(n, lag, n_obs, 0);
+        p->total = (size_t)p->grid * p->chain_stride;
+    } else if (batch == 1 && pmmh::sv_grid_eligible(n_obs, n, lag, p->c.grid_G)) {
+        p->c.kernel = SvKernel::Grid;
+        p->total = pmmh::sv_grid_ws_bytes(n_obs, n, lag, p->c.grid_G, 1);
+    } else {
         return fail(PMMH_ERR_INVALID, "pmmh_flps_model_corr: 2 <= lag <= 10 and 2 <= n_particles <= 4096 (any batch), "
                                       "or batch == 1, n_obs >= 2 lag and n_particles up to 7168 per SM "
                                       "(1,060,864 on 148 SMs)");
+    }
     return PMMH_OK;
 }
 }  // namespace
 
 int pmmh_flps_model_workspace_bytes(int n_obs, int n_particles, int lag, int batch, size_t* bytes) {
     if (!bytes) return fail(PMMH_ERR_INVALID, "pmmh_flps_model_workspace_bytes: bad arguments");
-    SvKernel k;
-    int G;
-    int rc = model_choose(n_obs, n_particles, lag, batch, &k, &G);
-    if (rc != PMMH_OK) return rc;
-    if (k == SvKernel::Grid) {
-        *bytes = pmmh::sv_grid_ws_bytes(n_obs, n_particles, lag, G, 1);   // with history (the query has no flag)
-        return PMMH_OK;
-    }
     DeviceInfo di;
-    rc = get_device_info(&di);
+    SvPlan p;
+    int rc = model_choose(n_obs, n_particles, lag, batch, &di, &p);
     if (rc != PMMH_OK) return rc;
-    const int grid = batch < di.sm ? batch : di.sm;
-    *bytes = (size_t)grid * pmmh::sv_chain_ws_bytes(n_particles, lag, n_obs, 0);
+    *bytes = p.total;
     return PMMH_OK;
 }
 
@@ -711,56 +719,21 @@ int pmmh_flps_model_corr(int model_id, const double* d_obs, long long obs_stride
     if ((d_x_hist == nullptr) != (d_a_hist == nullptr))
         return fail(PMMH_ERR_INVALID, "d_x_hist and d_a_hist must be given together");
     if (n_obs < lag + 1) return fail(PMMH_ERR_INVALID, "n_obs must be at least lag + 1");
-    size_t need = 0;
-    int rc = pmmh_flps_model_workspace_bytes(n_obs, n_particles, lag, batch, &need);
-    if (rc != PMMH_OK) return rc;
-    if (workspace_bytes < need) return fail(PMMH_ERR_WORKSPACE, "workspace too small");
     DeviceInfo di;
-    rc = get_device_info(&di);
+    SvPlan p;
+    int rc = model_choose(n_obs, n_particles, lag, batch, &di, &p);
     if (rc != PMMH_OK) return rc;
-    if (di.major < 10) return fail(PMMH_ERR_NO_DEVICE, "an sm_100 (B200) device is required");
-    SvKernel k;
-    int G;
-    rc = model_choose(n_obs, n_particles, lag, batch, &k, &G);
+    if (workspace_bytes < p.total) return fail(PMMH_ERR_WORKSPACE, "workspace too small");
+    rc = check_device(di, p.c.kernel == SvKernel::Grid);
     if (rc != PMMH_OK) return rc;
-    if (k == SvKernel::Grid) {
-        if (!di.coop) return fail(PMMH_ERR_NO_DEVICE, "device lacks cooperative launch");
-        // (no fallback pass: an abandoned evaluation is reported in d_diag[PMMH_DIAG_STATUS])
-        return pmmh::sv_grid_run(d_obs, d_params, d_rvr, d_u, n_obs, n_particles, lag, G, d_filt, d_smo, d_log_like,
-                                 d_gradient, d_traj, d_diag, d_x_hist, d_a_hist, d_workspace, workspace_bytes, nullptr,
-                                 (cudaStream_t)stream, 0, nullptr, nullptr, nullptr, model_id);
-    }
-    pmmh::SvArgs a;
-    memset(&a, 0, sizeof(a));
-    a.N = n_particles;
-    a.NOBS = n_obs;
-    a.LAG = lag;
-    a.B = batch;
-    a.G = 1;
-    a.n_teams = batch < di.sm ? batch : di.sm;
-    a.mode = pmmh::kSvFlps;
-    a.model_id = model_id;
-    a.obs = d_obs;
-    a.obs_stride = obs_stride;
-    a.params = d_params;
-    a.rvr = d_rvr;
-    a.U = d_u;
-    a.filt = d_filt;
-    a.smo = d_smo;
-    a.loglike = d_log_like;
-    a.grad = d_gradient;
-    a.traj = d_traj;
-    a.hess1 = nullptr;
-    a.hess2 = nullptr;
-    a.diag = d_diag;
-    a.Xhist = d_x_hist;
-    a.Ahist = d_a_hist;
-    a.prof = nullptr;
-    a.ws = (char*)d_workspace;
-    a.ws_sync_bytes = 0;
-    a.ws_team_stride = pmmh::sv_chain_ws_bytes(n_particles, lag, n_obs, 0);
-    PMMH_CUDA(pmmh::sv_chain_launch(a, a.n_teams, (cudaStream_t)stream));
-    return PMMH_OK;
+    // (no fallback pass: an abandoned evaluation is reported in d_diag[PMMH_DIAG_STATUS])
+    const SvShape s = {n_obs, n_particles, lag, batch, 0, pmmh::kSvFlps, d_x_hist != nullptr, 0};
+    pmmh::SvCall c = {};
+    c.obs = d_obs; c.obs_stride = obs_stride; c.params = d_params; c.rvr = d_rvr; c.u = d_u;
+    c.filt = d_filt; c.smo = d_smo; c.ll = d_log_like; c.grad = d_gradient; c.traj = d_traj; c.diag = d_diag;
+    c.x_hist = d_x_hist; c.a_hist = d_a_hist; c.model = model_id; c.prof = g_sv_prof;
+    c.ws = d_workspace; c.ws_bytes = workspace_bytes; c.stream = (cudaStream_t)stream;
+    return sv_launch_plan(p, s, c);
 }
 
 int pmmh_bpf_sv_corr(const double* d_obs, long long obs_stride, const double* d_params,

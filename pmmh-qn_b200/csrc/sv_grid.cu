@@ -1872,20 +1872,18 @@ size_t sv_grid_ws_bytes(int nobs, int n, int lag, int G, int hist, int hess) {
     return grid_layout(nobs, n, lag, G, hist, hess).total;
 }
 
-int sv_grid_run(const double* d_obs, const double* d_params, const double* d_rvr, const double* d_u, int nobs,
-                int n, int lag, int G, double* d_filt, double* d_smo, double* d_ll, double* d_grad, double* d_traj,
-                long long* d_diag, double* d_xh, int* d_ah, void* d_ws, size_t ws_bytes, long long* d_prof,
-                cudaStream_t st, int u_chunk_steps, const int* d_u_flag, double* d_hess1, double* d_hess2, int model) {
+int sv_grid_run(const SvCall& c, int nobs, int n, int lag, int G, int hess) {
     if (!sv_grid_eligible(nobs, n, lag, G)) return set_error(PMMH_ERR_INVALID, "grid kernel: sizes not eligible");
-    const int hist = d_xh != nullptr;
-    const int hess = d_hess1 != nullptr && d_hess2 != nullptr;
+    const int hist = c.x_hist != nullptr;
+    const int model = c.model;
     if (model != PMMH_MODEL_SV_LEVERAGE && model != PMMH_MODEL_LINEAR_GAUSSIAN && model != PMMH_MODEL_LINEAR_GAUSSIAN_FA)
         return set_error(PMMH_ERR_INVALID, "grid kernel: unknown model id");
     if (hess && model != PMMH_MODEL_SV_LEVERAGE)
         return set_error(PMMH_ERR_INVALID, "grid kernel: the Hessian branch exists for the SV model only");
     const GridLayout L = grid_layout(nobs, n, lag, G, hist, hess);
-    if (ws_bytes < L.total) return set_error(PMMH_ERR_WORKSPACE, "grid kernel: workspace too small");
-    char* ws = (char*)d_ws;
+    if (c.ws_bytes < L.total) return set_error(PMMH_ERR_WORKSPACE, "grid kernel: workspace too small");
+    char* ws = (char*)c.ws;
+    const cudaStream_t st = c.stream;
     GridArgs a;
     memset(&a, 0, sizeof(a));
     a.N = n;
@@ -1895,16 +1893,16 @@ int sv_grid_run(const double* d_obs, const double* d_params, const double* d_rvr
     a.Wc = (n + G - 1) / G;
     a.RP = L.RP;
     a.hist = hist;
-    a.obs = d_obs;
-    a.params = d_params;
-    a.rvr = d_rvr;
-    a.U = d_u;
-    if (u_chunk_steps > 0) {   // particle-major chunks of u_chunk_steps time steps (host-streamed)
-        a.u_cs = u_chunk_steps;
-        a.u_cstride = (long long)n * u_chunk_steps;
+    a.obs = c.obs;
+    a.params = c.params;
+    a.rvr = c.rvr;
+    a.U = c.u;
+    if (c.slot > 0) {   // particle-major slots of c.slot time steps (host-streamed)
+        a.u_cs = c.slot;
+        a.u_cstride = (long long)n * c.slot;
         a.u_tstride = 1;
-        a.u_jstride = u_chunk_steps;
-        a.u_flag = d_u_flag;
+        a.u_jstride = c.slot;
+        a.u_flag = c.u_flag;
         a.ustash = (double*)(ws + L.ustash);
     } else {
         a.u_cs = 1 << 30;
@@ -1931,9 +1929,9 @@ int sv_grid_run(const double* d_obs, const double* d_params, const double* d_rvr
     a.psumH = (double*)(ws + L.psumH);
     a.SQ = L.SQ;
     a.RS = hess ? 2 : 1;
-    a.Xhist = d_xh;
-    a.Ahist = d_ah;
-    a.prof = d_prof;
+    a.Xhist = c.x_hist;
+    a.Ahist = c.a_hist;
+    a.prof = c.prof;
     {
         const char* e = getenv("PMMH_GRID_DEBUG");
         a.dbg = e ? atoi(e) : 0;
@@ -1968,7 +1966,7 @@ int sv_grid_run(const double* d_obs, const double* d_params, const double* d_rvr
         double* tailpartH = (double*)(ws + L.tailpartH);
         grid_reduceH_kernel<<<nobs, 640, 0, st>>>(a.psumH, G, lag, sumsH);
         grid_tail_kernel<true, SvLeverageModel><<<dim3(L.nblk, lag), 256, 0, st>>>(a, sums, tailpart, tailpartH, L.nblk);
-        grid_hess_finish_kernel<<<1, 32, 0, st>>>(a.ctrl, sums, sumsH, tailpartH, d_params, L.nblk, nobs, lag, d_hess1, d_hess2);
+        grid_hess_finish_kernel<<<1, 32, 0, st>>>(a.ctrl, sums, sumsH, tailpartH, c.params, L.nblk, nobs, lag, c.hess1, c.hess2);
     } else if (model == PMMH_MODEL_LINEAR_GAUSSIAN) {
         grid_tail_kernel<false, LinearGaussianModel><<<dim3(L.nblk, lag), 256, 0, st>>>(a, sums, tailpart, nullptr, L.nblk);
     } else if (model == PMMH_MODEL_LINEAR_GAUSSIAN_FA) {
@@ -1978,16 +1976,9 @@ int sv_grid_run(const double* d_obs, const double* d_params, const double* d_rvr
     }
     grid_tail_reduce_kernel<<<lag, 256, 0, st>>>(tailpart, L.nblk, tail);
     auto finish = model == PMMH_MODEL_SV_LEVERAGE ? grid_finish_kernel<false> : grid_finish_kernel<true>;
-    finish<<<(nobs + 255) / 256, 256, 0, st>>>(a.ctrl, sums, a.shiftv, a.xminv, tail, d_params, nobs, lag, (double)n, d_ll,
-                                               d_filt, d_smo, d_grad, d_traj, d_diag, (long long*)(ws + L.info));
+    finish<<<(nobs + 255) / 256, 256, 0, st>>>(a.ctrl, sums, a.shiftv, a.xminv, tail, c.params, nobs, lag, (double)n, c.ll,
+                                               c.filt, c.smo, c.grad, c.traj, c.diag, (long long*)(ws + L.info));
     GRID_CUDA(cudaGetLastError());
-    return PMMH_OK;
-}
-
-// soft ties / raw status of the last evaluation that used this workspace (after synchronisation)
-int sv_grid_read_info(const void* d_ws, int nobs, int n, int lag, int G, int hist, long long* h_info) {
-    const GridLayout L = grid_layout(nobs, n, lag, G, hist, 0);   // (the Hessian buffers sit behind `info`)
-    GRID_CUDA(cudaMemcpy(h_info, (const char*)d_ws + L.info, 2 * sizeof(long long), cudaMemcpyDeviceToHost));
     return PMMH_OK;
 }
 

@@ -42,13 +42,11 @@
 #include <stdlib.h>
 #include <string.h>
 
-#include <algorithm>
-#include <vector>
-
 #include "../../include/pmmh_qn.h"
 #include "common.cuh"
 #include "philox.cuh"
 #include "sv_math.cuh"
+#include "sv_split.cuh"
 
 namespace pmmh {
 
@@ -1199,321 +1197,6 @@ bool sv_split_single_eligible(int nobs, int n, int lag) {
 using namespace pmmh;
 
 extern "C" {
-int pmmh_svsplit_init(void*, size_t, long long, int, int, int, int, long long, long long, int, const double*,
-                      double*, int*, double*, void*);
-int pmmh_svsplit_weights(void*, size_t, long long, long long, int, int, int, int, const double*, const double*,
-                         const double*, const int*, const double*, double*, double*, double*, void*);
-int pmmh_svsplit_children(void*, size_t, long long, long long, int, int, const double*, const double*,
-                          const double*, const double*, unsigned long long, unsigned long long, const double*,
-                          const double*, int*, double*, double*, void*);
-static int children_impl(void*, size_t, long long, long long, int, int, const double*, const double*,
-                         const double*, const double*, unsigned long long, unsigned long long, const double*,
-                         const double*, int*, double*, double*, void*, double*, const int*, int*, int, int);
-static int weights_impl(void*, size_t, long long, long long, int, int, int, int, const double*, const double*,
-                        const double*, const int*, const double*, double*, double*, double*, void*, int);
-int pmmh_svsplit_plan(void*, size_t, long long, long long, int, const int*, int*, void*);
-int pmmh_svsplit_pack(void*, size_t, long long, long long, const int*, const double*, double*, double*, void*);
-int pmmh_svsplit_sort(void*, size_t, long long, long long, int, int, int, const double*, const double*, int,
-                      double*, int*, void*);
-int pmmh_svsplit_normalise(const double*, int, const double*, double*, void*);
-int pmmh_svsplit_tail(void*, size_t, long long, long long, int, int, int, const double*, const double*,
-                      const int*, const double*, const double*, const double*, long long, double*, void*);
-int pmmh_svsplit_finish(const double*, const double*, const double*, const double*, const double*, int,
-                        const double*, int, int, long long, double*, double*, double*, double*, double*,
-                        void*);
-}
-
-namespace pmmh {
-
-// The whole evaluation on ONE device (world = 1): the same phases, no exchange, no host
-// synchronisation -- T x 11 kernel launches on `st`.  Returns a PMMH_* status.
-int sv_split_single_run(const double* d_obs, const double* d_params, const double* d_rvr, const double* d_u,
-                        int nobs, int n, int lag, double* d_filt, double* d_smo, double* d_ll,
-                        double* d_grad, double* d_traj, long long* d_diag, void* d_ws, size_t ws_bytes,
-                        cudaStream_t st) {
-    if (!sv_split_single_eligible(nobs, n, lag)) return set_error(PMMH_ERR_INVALID, "split kernels: sizes not eligible");
-    const SingleLayout S = make_single_layout(nobs, n, lag);
-    if (ws_bytes < S.total) return set_error(PMMH_ERR_WORKSPACE, "split kernels: workspace too small");
-    char* ws = (char*)d_ws;
-    void* sws = ws + S.split;
-    const size_t sb = S.split_bytes;
-    double* xs = (double*)(ws + S.xs);
-    int* perm = (int*)(ws + S.perm);
-    double* xs_next = (double*)(ws + S.xs2);
-    int* perm_next = (int*)(ws + S.perm2);
-    double* rec = (double*)(ws + S.recA);
-    double* rec_next = (double*)(ws + S.recB);
-    double* sums = (double*)(ws + S.sums);
-    double* shift = (double*)(ws + S.shift);
-    double* xmin = (double*)(ws + S.xmin);
-    double* gather = (double*)(ws + S.gather);
-    int* hist = (int*)(ws + S.hist);
-    double* keep = (double*)(ws + S.keep);
-    double* tail = (double*)(ws + S.tail);
-    const Layout L = make_layout(n, n);
-    const int nf_bound = (int)(n / kFine + kBins);
-    int rc;
-    // pack (record traffic, DRAM bound) and the sort (latency / L2 bound) both depend only on
-    // the plan: they run side by side on two streams
-    static thread_local cudaStream_t side[64] = {nullptr};
-    static thread_local cudaEvent_t ev_fork[64] = {nullptr}, ev_join[64] = {nullptr};
-    int dev = 0;
-    SPLIT_CUDA(cudaGetDevice(&dev));
-    if (dev < 0 || dev >= 64) return set_error(PMMH_ERR_NO_DEVICE, "device ordinal out of range");
-    if (!side[dev]) {
-        SPLIT_CUDA(cudaStreamCreateWithFlags(&side[dev], cudaStreamNonBlocking));
-        SPLIT_CUDA(cudaEventCreateWithFlags(&ev_fork[dev], cudaEventDisableTiming));
-        SPLIT_CUDA(cudaEventCreateWithFlags(&ev_join[dev], cudaEventDisableTiming));
-    }
-    SPLIT_CUDA(cudaMemsetAsync(sums, 0, (size_t)nobs * 8 * 8, st));
-    if ((rc = pmmh_svsplit_init(sws, sb, n, nobs, 1, 0, lag, n, n, n, d_params, xs, perm, rec, st))) return rc;
-    if ((rc = pmmh_svsplit_weights(sws, sb, n, n, 0, n, lag, nobs, d_obs, d_params, xs, perm, rec, sums, gather,
-                                   nullptr, st)))
-        return rc;
-    for (int t = 1; t < nobs; ++t) {
-        if ((rc = pmmh_svsplit_children(sws, sb, n, n, t, n, d_obs, d_params, d_rvr, d_u, 0, 0, gather, xs, hist,
-                                        shift, xmin, st)))
-            return rc;
-        if ((rc = pmmh_svsplit_plan(sws, sb, n, n, 1, hist, nullptr, st))) return rc;
-        SPLIT_CUDA(cudaEventRecord(ev_fork[dev], st));
-        SPLIT_CUDA(cudaStreamWaitEvent(side[dev], ev_fork[dev], 0));
-        if ((rc = pmmh_svsplit_pack(sws, sb, n, n, perm, rec, rec_next, nullptr, side[dev]))) return rc;
-        SPLIT_CUDA(cudaEventRecord(ev_join[dev], side[dev]));
-        double* tmp = rec;
-        rec = rec_next;
-        rec_next = tmp;
-        // the sort reads the dense child values and writes xs / perm of the NEW generation: pack
-        // still reads perm of the OLD one, so the new order goes to the alternate buffers
-        if ((rc = pmmh_svsplit_sort(sws, sb, n, n, n, nf_bound, lag, rec, nullptr, 1, xs_next, perm_next, st))) return rc;
-        SPLIT_CUDA(cudaStreamWaitEvent(st, ev_join[dev], 0));
-        { double* tx = xs; xs = xs_next; xs_next = tx; int* tp = perm; perm = perm_next; perm_next = tp; }
-        double* kp = (t >= nobs - lag) ? keep + (size_t)(t % lag) * n : nullptr;
-        if ((rc = pmmh_svsplit_weights(sws, sb, n, n, t, n, lag, nobs, d_obs, d_params, xs, perm, rec, sums,
-                                       gather, kp, st)))
-            return rc;
-    }
-    // tail: normalised weights of the last `lag` generations, in place (same global positions)
-    for (int irel = 0; irel < lag; ++irel) {
-        const int i = nobs - lag + irel;
-        double* kp = keep + (size_t)(i % lag) * n;
-        if ((rc = pmmh_svsplit_normalise(kp, n, sums + (size_t)i * 8, kp, st))) return rc;
-    }
-    // the tail kernel indexes lagged weights as [irel][p]: slot of generation nobs-lag+irel is
-    // (nobs - lag + irel) % lag = a rotation of irel; pass the rotated base per call through a view
-    // by copying nothing: rotation r0 = (nobs - lag) % lag, so slot(irel) = (r0 + irel) % lag.
-    // The kernel takes one base + stride, so rotate into rec_next (free now) when r0 != 0.
-    const int r0 = (nobs - lag) % lag;
-    double* wl = keep;
-    if (r0 != 0) {
-        wl = rec_next;
-        for (int irel = 0; irel < lag; ++irel)
-            SPLIT_CUDA(cudaMemcpyAsync(wl + (size_t)irel * n, keep + (size_t)((r0 + irel) % lag) * n,
-                                       (size_t)n * 8, cudaMemcpyDeviceToDevice, st));
-    }
-    if ((rc = pmmh_svsplit_tail(sws, sb, n, n, n, lag, nobs, d_obs, d_params, perm, rec,
-                                wl + (size_t)(lag - 1) * n, wl, n, tail, st)))
-        return rc;
-    if ((rc = pmmh_svsplit_finish(sums, shift, xmin, tail, gather, 1, d_params, nobs, lag, n, d_ll, d_filt, d_smo,
-                                  d_grad, d_traj, st)))
-        return rc;
-    split_diag_kernel<<<1, 32, 0, st>>>((const SplitState*)((char*)sws + L.state), d_diag);
-    SPLIT_CUDA(cudaGetLastError());
-    return PMMH_OK;
-}
-
-// ---- path storage on one device (algorithm 5) ------------------------------------------------
-namespace {
-struct PathLayout {
-    size_t split, xs, perm, X, J, sums, shift, xmin, gather, hist, keep, tail, rec, total, split_bytes;
-    int R, Q;
-};
-
-PathLayout make_path_layout(int nobs, long long n, int lag) {
-    PathLayout P;
-    P.R = lag + 1;
-    P.Q = 0;
-    while ((2 << P.Q) <= lag - 2) ++P.Q;      // largest q with 2^q <= lag - 2 (0 when lag <= 3)
-    size_t o = 0;
-    P.split_bytes = make_layout(n, n).total;
-    P.split = o;   o += al(P.split_bytes);
-    P.xs = o;      o += al((size_t)n * 8);
-    P.perm = o;    o += al((size_t)n * 4);
-    P.X = o;       o += al((size_t)P.R * n * 8);
-    P.J = o;       o += al((size_t)(P.Q + 1) * P.R * n * 4);
-    P.sums = o;    o += al((size_t)nobs * 8 * 8);
-    P.shift = o;   o += al((size_t)nobs * 8);
-    P.xmin = o;    o += al((size_t)nobs * 8);
-    P.gather = o;  o += al(4 * 8);
-    P.hist = o;    o += al((size_t)kBins * 4);
-    P.keep = o;    o += al((size_t)n * lag * 8);
-    P.tail = o;    o += al((size_t)lag * 8 * 8);
-    P.rec = o;     o += al((size_t)n * lag * 8);
-    P.total = o;
-    return P;
-}
-}  // namespace
-
-size_t sv_split_path_ws_bytes(int nobs, int n, int lag) { return make_path_layout(nobs, n, lag).total; }
-
-int sv_split_path_run(const double* d_obs, const double* d_params, const double* d_rvr, const double* d_u,
-                      int nobs, int n, int lag, double* d_filt, double* d_smo, double* d_ll, double* d_grad,
-                      double* d_traj, long long* d_diag, void* d_ws, size_t ws_bytes, cudaStream_t st,
-                      int u_pm_chunk, const cudaEvent_t* chunk_ready, unsigned long long seed,
-                      unsigned long long philox_offset) {
-    if (!sv_split_single_eligible(nobs, n, lag)) return set_error(PMMH_ERR_INVALID, "split kernels: sizes not eligible");
-    const PathLayout P = make_path_layout(nobs, n, lag);
-    if (ws_bytes < P.total) return set_error(PMMH_ERR_WORKSPACE, "split kernels: workspace too small");
-    char* ws = (char*)d_ws;
-    void* sws = ws + P.split;
-    const size_t sb = P.split_bytes;
-    const int R = P.R, Q = P.Q;
-    double* xs = (double*)(ws + P.xs);
-    int* perm = (int*)(ws + P.perm);
-    double* X = (double*)(ws + P.X);
-    int* J = (int*)(ws + P.J);
-    double* sums = (double*)(ws + P.sums);
-    double* shift = (double*)(ws + P.shift);
-    double* xmin = (double*)(ws + P.xmin);
-    double* gather = (double*)(ws + P.gather);
-    int* hist = (int*)(ws + P.hist);
-    double* keep = (double*)(ws + P.keep);
-    double* tail = (double*)(ws + P.tail);
-    double* rec = (double*)(ws + P.rec);
-    const Layout L = make_layout(n, n);
-    SplitState* state = (SplitState*)((char*)sws + L.state);
-    const int nf_bound = (int)(n / kFine + kBins);
-    int rc;
-    static thread_local cudaStream_t side[64] = {nullptr};
-    static thread_local cudaEvent_t ev_fork[64] = {nullptr}, ev_join[64][2] = {{nullptr, nullptr}};
-    int dev = 0;
-    SPLIT_CUDA(cudaGetDevice(&dev));
-    if (dev < 0 || dev >= 64) return set_error(PMMH_ERR_NO_DEVICE, "device ordinal out of range");
-    if (!side[dev]) {
-        SPLIT_CUDA(cudaStreamCreateWithFlags(&side[dev], cudaStreamNonBlocking));
-        SPLIT_CUDA(cudaEventCreateWithFlags(&ev_fork[dev], cudaEventDisableTiming));
-        SPLIT_CUDA(cudaEventCreateWithFlags(&ev_join[dev][0], cudaEventDisableTiming));
-        SPLIT_CUDA(cudaEventCreateWithFlags(&ev_join[dev][1], cudaEventDisableTiming));
-    }
-    const size_t gstride = al((size_t)kLineageGrid * 8 * 8);
-    SPLIT_CUDA(cudaMemsetAsync(sums, 0, (size_t)nobs * 8 * 8, st));
-    // generation 0: xs = mu, perm = identity, X[0] = mu (the LR = 1 "records" of init are X[0])
-    if ((rc = pmmh_svsplit_init(sws, sb, n, nobs, 1, 0, 0, n, n, n, d_params, xs, perm, X, st))) return rc;
-    if ((rc = weights_impl(sws, sb, n, n, 0, n, lag, nobs, d_obs, d_params, xs, perm, nullptr, sums, gather,
-                           nullptr, st, 1)))
-        return rc;
-    // development: PMMH_SPLIT_TIMING=1 prints the average time of every phase of a step (events on
-    // the main stream; the lineage kernel runs beside the sort on the second stream)
-    static int timing = -1;
-    if (timing < 0) {
-        const char* e = getenv("PMMH_SPLIT_TIMING");
-        timing = e ? atoi(e) : 0;
-    }
-    const int kEv = 5;
-    std::vector<cudaEvent_t> evs;
-    int t_first = 0, t_last = 0;
-    if (timing) {
-        t_first = nobs / 2;
-        t_last = std::min(nobs - 1, t_first + 100);
-        evs.resize((size_t)(t_last - t_first) * kEv);
-        for (auto& e : evs) cudaEventCreate(&e);
-    }
-#define PMMH_MARK(slot)                                                                      \
-    do {                                                                                     \
-        if (timing && t >= t_first && t < t_last) cudaEventRecord(evs[(size_t)(t - t_first) * kEv + (slot)], st); \
-    } while (0)
-    for (int t = 1; t < nobs; ++t) {
-        double* Xt = X + (size_t)(t % R) * n;
-        int* J1t = J + (size_t)(t % R) * n;
-        PMMH_MARK(0);
-        // host-streamed u: d_u holds particle-major chunks of u_pm_chunk time steps that the copy
-        // engine is still filling; wait for the chunk of this step when it is entered
-        const double* ut = d_u;
-        if (u_pm_chunk) {
-            if (t == 1 || t % u_pm_chunk == 0) SPLIT_CUDA(cudaStreamWaitEvent(st, chunk_ready[t / u_pm_chunk], 0));
-            ut = d_u + (size_t)(t / u_pm_chunk) * (size_t)n * (size_t)u_pm_chunk;
-        }
-        if ((rc = children_impl(sws, sb, n, n, t, n, d_obs, d_params, d_rvr, ut, seed, philox_offset, gather, xs, hist, shift,
-                                xmin, st, Xt, perm, J1t, 1, u_pm_chunk)))
-            return rc;
-        PMMH_MARK(1);
-        // jump tables + fixed-lag sums (birth order) on the second stream.  They depend only on the
-        // children and feed only outputs, so they get a whole step of slack: the weights phase of
-        // step t picks up the sums of generation t - 1 (its ring slots stay untouched until t + lag)
-        SPLIT_CUDA(cudaEventRecord(ev_fork[dev], st));
-        SPLIT_CUDA(cudaStreamWaitEvent(side[dev], ev_fork[dev], 0));
-        split_lineage_kernel<<<kLineageGrid, 256, 0, side[dev]>>>(
-            state, t, n, lag, R, Q, X, J, d_obs, d_params, shift,
-            (double*)((char*)sws + L.gpart + (size_t)(t & 1) * gstride));
-        SPLIT_CUDA(cudaEventRecord(ev_join[dev][t & 1], side[dev]));
-        if ((rc = pmmh_svsplit_sort(sws, sb, n, n, n, nf_bound, 0, Xt, Xt, 0, xs, perm, st))) return rc;
-        PMMH_MARK(2);
-        if (t > 1) SPLIT_CUDA(cudaStreamWaitEvent(st, ev_join[dev][(t - 1) & 1], 0));
-        PMMH_MARK(3);
-        double* kp = (t >= nobs - lag) ? keep + (size_t)(t % lag) * n : nullptr;
-        if ((rc = weights_impl(sws, sb, n, n, t, n, lag, nobs, d_obs, d_params, xs, perm, nullptr, sums, gather,
-                               kp, st, 1)))
-            return rc;
-        PMMH_MARK(4);
-    }
-#undef PMMH_MARK
-    if (timing) {
-        SPLIT_CUDA(cudaStreamSynchronize(st));
-        double acc[kEv] = {0, 0, 0, 0, 0};
-        const int cnt = t_last - t_first;
-        for (int q = 0; q < cnt; ++q) {
-            for (int k = 0; k + 1 < kEv; ++k) {
-                float ms = 0.f;
-                cudaEventElapsedTime(&ms, evs[(size_t)q * kEv + k], evs[(size_t)q * kEv + k + 1]);
-                acc[k] += ms;
-            }
-            if (q + 1 < cnt) {
-                float ms = 0.f;
-                cudaEventElapsedTime(&ms, evs[(size_t)q * kEv + kEv - 1], evs[(size_t)(q + 1) * kEv]);
-                acc[kEv - 1] += ms;
-            }
-        }
-        fprintf(stderr, "[pmmh split] us per step: children(+plan) %.1f | sort %.1f | wait for lineage %.1f | "
-                        "weights+finalize %.1f | gap to next step %.1f\n",
-                acc[0] / cnt * 1e3, acc[1] / cnt * 1e3, acc[2] / cnt * 1e3, acc[3] / cnt * 1e3,
-                acc[4] / std::max(1, cnt - 1) * 1e3);
-        for (auto& e : evs) cudaEventDestroy(e);
-    }
-    for (int irel = 0; irel < lag; ++irel) {
-        const int i = nobs - lag + irel;
-        double* kp = keep + (size_t)(i % lag) * n;
-        if ((rc = pmmh_svsplit_normalise(kp, n, sums + (size_t)i * 8, kp, st))) return rc;
-    }
-    // sums of the last generation's lineage kernel
-    SPLIT_CUDA(cudaStreamWaitEvent(st, ev_join[dev][(nobs - 1) & 1], 0));
-    if (nobs - 1 >= lag)
-        split_lineage_reduce_kernel<<<1, 256, 0, st>>>(
-            (const double*)((char*)sws + L.gpart + (size_t)((nobs - 1) & 1) * gstride),
-            sums + (size_t)(nobs - 1) * 8);
-    // the tail reads records of the final generation: built once from the stored paths
-    split_build_records_kernel<<<grid_for(n, 256), 256, 0, st>>>(nobs - 1, n, lag, R, X, J, rec);
-    const int r0 = (nobs - lag) % lag;
-    double* wl = keep;
-    if (r0 != 0) {
-        // rotate the kept weights into [irel][p] order; X is free now and large enough (R > lag rows)
-        wl = X;
-        for (int irel = 0; irel < lag; ++irel)
-            SPLIT_CUDA(cudaMemcpyAsync(wl + (size_t)irel * n, keep + (size_t)((r0 + irel) % lag) * n,
-                                       (size_t)n * 8, cudaMemcpyDeviceToDevice, st));
-    }
-    if ((rc = pmmh_svsplit_tail(sws, sb, n, n, n, lag, nobs, d_obs, d_params, perm, rec,
-                                wl + (size_t)(lag - 1) * n, wl, n, tail, st)))
-        return rc;
-    if ((rc = pmmh_svsplit_finish(sums, shift, xmin, tail, gather, 1, d_params, nobs, lag, n, d_ll, d_filt, d_smo,
-                                  d_grad, d_traj, st)))
-        return rc;
-    split_diag_kernel<<<1, 32, 0, st>>>(state, d_diag);
-    SPLIT_CUDA(cudaGetLastError());
-    return PMMH_OK;
-}
-
-}  // namespace pmmh
-
-extern "C" {
 
 int pmmh_svsplit_workspace_bytes(long long cap_particles, long long cap_children, size_t* bytes) {
     if (cap_particles < 1 || cap_children < 1 || cap_particles >= (1ll << 31) - 4096 ||
@@ -1796,3 +1479,240 @@ int pmmh_svsplit_diag(void* d_ws, size_t ws_bytes, long long cap_particles, long
 }
 
 }  // extern "C"
+
+namespace pmmh {
+
+namespace {
+// The second stream of the current device and host thread, beside the caller's: a fork event and two join events
+// (the records driver joins through join[0], the path driver alternates between both)
+struct SideStream {
+    cudaStream_t s = nullptr;
+    cudaEvent_t fork = nullptr, join[2] = {nullptr, nullptr};
+};
+
+int side_stream(SideStream** out) {
+    static thread_local SideStream sides[64];
+    int dev = 0;
+    SPLIT_CUDA(cudaGetDevice(&dev));
+    if (dev < 0 || dev >= 64) return set_error(PMMH_ERR_NO_DEVICE, "device ordinal out of range");
+    SideStream& side = sides[dev];
+    if (!side.s) {
+        SPLIT_CUDA(cudaStreamCreateWithFlags(&side.s, cudaStreamNonBlocking));
+        for (cudaEvent_t* e : {&side.fork, &side.join[0], &side.join[1]})
+            SPLIT_CUDA(cudaEventCreateWithFlags(e, cudaEventDisableTiming));
+    }
+    *out = &side;
+    return PMMH_OK;
+}
+
+// The end of a one-device evaluation (layout WsLayout: SingleLayout or PathLayout): the weights kept for the last
+// `lag` generations are normalised in place; then before_tail() enqueues what else the tail needs; then the tail,
+// finish and diag kernels.  The tail kernel takes the lagged weights as one base and stride, [irel][p]: generation
+// nobs - lag + irel sits in slot (r0 + irel) % lag, r0 = (nobs - lag) % lag, so unless r0 == 0 they are rotated into
+// `scratch` (lag x n doubles, free by then).
+template <class WsLayout, class BeforeTail>
+int split_end(const SvCall& c, int nobs, int n, int lag, const WsLayout& S, const int* perm, const double* rec,
+              double* scratch, BeforeTail before_tail) {
+    char* ws = (char*)c.ws;
+    void* sws = ws + S.split;
+    double* sums = (double*)(ws + S.sums);
+    double* keep = (double*)(ws + S.keep);
+    double* tail = (double*)(ws + S.tail);
+    int rc;
+    for (int irel = 0; irel < lag; ++irel) {
+        const int i = nobs - lag + irel;
+        double* kp = keep + (size_t)(i % lag) * n;
+        if ((rc = pmmh_svsplit_normalise(kp, n, sums + (size_t)i * 8, kp, c.stream))) return rc;
+    }
+    rc = before_tail();
+    if (rc != PMMH_OK) return rc;
+    const int r0 = (nobs - lag) % lag;
+    double* wl = keep;
+    if (r0 != 0) {
+        wl = scratch;
+        for (int irel = 0; irel < lag; ++irel)
+            SPLIT_CUDA(cudaMemcpyAsync(wl + (size_t)irel * n, keep + (size_t)((r0 + irel) % lag) * n,
+                                       (size_t)n * 8, cudaMemcpyDeviceToDevice, c.stream));
+    }
+    if ((rc = pmmh_svsplit_tail(sws, S.split_bytes, n, n, n, lag, nobs, c.obs, c.params, perm, rec,
+                                wl + (size_t)(lag - 1) * n, wl, n, tail, c.stream)))
+        return rc;
+    if ((rc = pmmh_svsplit_finish(sums, (double*)(ws + S.shift), (double*)(ws + S.xmin), tail,
+                                  (double*)(ws + S.gather), 1, c.params, nobs, lag, n, c.ll, c.filt, c.smo, c.grad,
+                                  c.traj, c.stream)))
+        return rc;
+    split_diag_kernel<<<1, 32, 0, c.stream>>>((const SplitState*)((char*)sws + make_layout(n, n).state), c.diag);
+    SPLIT_CUDA(cudaGetLastError());
+    return PMMH_OK;
+}
+
+// ---- path storage on one device (algorithm 5) ------------------------------------------------
+struct PathLayout {
+    size_t split, xs, perm, X, J, sums, shift, xmin, gather, hist, keep, tail, rec, total, split_bytes;
+    int R, Q;
+};
+
+PathLayout make_path_layout(int nobs, long long n, int lag) {
+    PathLayout P;
+    P.R = lag + 1;
+    P.Q = 0;
+    while ((2 << P.Q) <= lag - 2) ++P.Q;      // largest q with 2^q <= lag - 2 (0 when lag <= 3)
+    size_t o = 0;
+    P.split_bytes = make_layout(n, n).total;
+    P.split = o;   o += al(P.split_bytes);
+    P.xs = o;      o += al((size_t)n * 8);
+    P.perm = o;    o += al((size_t)n * 4);
+    P.X = o;       o += al((size_t)P.R * n * 8);
+    P.J = o;       o += al((size_t)(P.Q + 1) * P.R * n * 4);
+    P.sums = o;    o += al((size_t)nobs * 8 * 8);
+    P.shift = o;   o += al((size_t)nobs * 8);
+    P.xmin = o;    o += al((size_t)nobs * 8);
+    P.gather = o;  o += al(4 * 8);
+    P.hist = o;    o += al((size_t)kBins * 4);
+    P.keep = o;    o += al((size_t)n * lag * 8);
+    P.tail = o;    o += al((size_t)lag * 8 * 8);
+    P.rec = o;     o += al((size_t)n * lag * 8);
+    P.total = o;
+    return P;
+}
+}  // namespace
+
+size_t sv_split_path_ws_bytes(int nobs, int n, int lag) { return make_path_layout(nobs, n, lag).total; }
+
+// The whole evaluation on ONE device (world = 1): the same phases, no exchange, no host
+// synchronisation -- T x 11 kernel launches on c.stream.  Returns a PMMH_* status.
+int sv_split_single_run(const SvCall& c, int nobs, int n, int lag) {
+    if (!sv_split_single_eligible(nobs, n, lag)) return set_error(PMMH_ERR_INVALID, "split kernels: sizes not eligible");
+    const SingleLayout S = make_single_layout(nobs, n, lag);
+    if (c.ws_bytes < S.total) return set_error(PMMH_ERR_WORKSPACE, "split kernels: workspace too small");
+    const double *d_obs = c.obs, *d_params = c.params, *d_rvr = c.rvr, *d_u = c.u;
+    const cudaStream_t st = c.stream;
+    char* ws = (char*)c.ws;
+    void* sws = ws + S.split;
+    const size_t sb = S.split_bytes;
+    double* xs = (double*)(ws + S.xs);
+    int* perm = (int*)(ws + S.perm);
+    double* xs_next = (double*)(ws + S.xs2);
+    int* perm_next = (int*)(ws + S.perm2);
+    double* rec = (double*)(ws + S.recA);
+    double* rec_next = (double*)(ws + S.recB);
+    double* sums = (double*)(ws + S.sums);
+    double* shift = (double*)(ws + S.shift);
+    double* xmin = (double*)(ws + S.xmin);
+    double* gather = (double*)(ws + S.gather);
+    int* hist = (int*)(ws + S.hist);
+    double* keep = (double*)(ws + S.keep);
+    const int nf_bound = (int)(n / kFine + kBins);
+    int rc;
+    // pack (record traffic, DRAM bound) and the sort (latency / L2 bound) both depend only on
+    // the plan: they run side by side on two streams
+    SideStream* side = nullptr;
+    if ((rc = side_stream(&side))) return rc;
+    SPLIT_CUDA(cudaMemsetAsync(sums, 0, (size_t)nobs * 8 * 8, st));
+    if ((rc = pmmh_svsplit_init(sws, sb, n, nobs, 1, 0, lag, n, n, n, d_params, xs, perm, rec, st))) return rc;
+    if ((rc = pmmh_svsplit_weights(sws, sb, n, n, 0, n, lag, nobs, d_obs, d_params, xs, perm, rec, sums, gather,
+                                   nullptr, st)))
+        return rc;
+    for (int t = 1; t < nobs; ++t) {
+        if ((rc = pmmh_svsplit_children(sws, sb, n, n, t, n, d_obs, d_params, d_rvr, d_u, 0, 0, gather, xs, hist,
+                                        shift, xmin, st)))
+            return rc;
+        if ((rc = pmmh_svsplit_plan(sws, sb, n, n, 1, hist, nullptr, st))) return rc;
+        SPLIT_CUDA(cudaEventRecord(side->fork, st));
+        SPLIT_CUDA(cudaStreamWaitEvent(side->s, side->fork, 0));
+        if ((rc = pmmh_svsplit_pack(sws, sb, n, n, perm, rec, rec_next, nullptr, side->s))) return rc;
+        SPLIT_CUDA(cudaEventRecord(side->join[0], side->s));
+        double* tmp = rec;
+        rec = rec_next;
+        rec_next = tmp;
+        // the sort reads the dense child values and writes xs / perm of the NEW generation: pack
+        // still reads perm of the OLD one, so the new order goes to the alternate buffers
+        if ((rc = pmmh_svsplit_sort(sws, sb, n, n, n, nf_bound, lag, rec, nullptr, 1, xs_next, perm_next, st))) return rc;
+        SPLIT_CUDA(cudaStreamWaitEvent(st, side->join[0], 0));
+        { double* tx = xs; xs = xs_next; xs_next = tx; int* tp = perm; perm = perm_next; perm_next = tp; }
+        double* kp = (t >= nobs - lag) ? keep + (size_t)(t % lag) * n : nullptr;
+        if ((rc = pmmh_svsplit_weights(sws, sb, n, n, t, n, lag, nobs, d_obs, d_params, xs, perm, rec, sums,
+                                       gather, kp, st)))
+            return rc;
+    }
+    // the alternate record buffer is free now
+    return split_end(c, nobs, n, lag, S, perm, rec, rec_next, [] { return (int)PMMH_OK; });
+}
+
+int sv_split_path_run(const SvCall& c, int nobs, int n, int lag) {
+    if (!sv_split_single_eligible(nobs, n, lag)) return set_error(PMMH_ERR_INVALID, "split kernels: sizes not eligible");
+    const PathLayout P = make_path_layout(nobs, n, lag);
+    if (c.ws_bytes < P.total) return set_error(PMMH_ERR_WORKSPACE, "split kernels: workspace too small");
+    const double *d_obs = c.obs, *d_params = c.params, *d_rvr = c.rvr, *d_u = c.u;
+    const int u_pm_chunk = c.slot;
+    const cudaStream_t st = c.stream;
+    char* ws = (char*)c.ws;
+    void* sws = ws + P.split;
+    const size_t sb = P.split_bytes;
+    const int R = P.R, Q = P.Q;
+    double* xs = (double*)(ws + P.xs);
+    int* perm = (int*)(ws + P.perm);
+    double* X = (double*)(ws + P.X);
+    int* J = (int*)(ws + P.J);
+    double* sums = (double*)(ws + P.sums);
+    double* shift = (double*)(ws + P.shift);
+    double* xmin = (double*)(ws + P.xmin);
+    double* gather = (double*)(ws + P.gather);
+    int* hist = (int*)(ws + P.hist);
+    double* keep = (double*)(ws + P.keep);
+    double* rec = (double*)(ws + P.rec);
+    const Layout L = make_layout(n, n);
+    SplitState* state = (SplitState*)((char*)sws + L.state);
+    const int nf_bound = (int)(n / kFine + kBins);
+    int rc;
+    SideStream* side = nullptr;
+    if ((rc = side_stream(&side))) return rc;
+    const size_t gstride = al((size_t)kLineageGrid * 8 * 8);
+    SPLIT_CUDA(cudaMemsetAsync(sums, 0, (size_t)nobs * 8 * 8, st));
+    // generation 0: xs = mu, perm = identity, X[0] = mu (the LR = 1 "records" of init are X[0])
+    if ((rc = pmmh_svsplit_init(sws, sb, n, nobs, 1, 0, 0, n, n, n, d_params, xs, perm, X, st))) return rc;
+    if ((rc = weights_impl(sws, sb, n, n, 0, n, lag, nobs, d_obs, d_params, xs, perm, nullptr, sums, gather,
+                           nullptr, st, 1)))
+        return rc;
+    for (int t = 1; t < nobs; ++t) {
+        double* Xt = X + (size_t)(t % R) * n;
+        int* J1t = J + (size_t)(t % R) * n;
+        // host-streamed u: d_u holds particle-major chunks of u_pm_chunk time steps that the copy
+        // engine is still filling; wait for the chunk of this step when it is entered
+        const double* ut = d_u;
+        if (u_pm_chunk) {
+            if (t == 1 || t % u_pm_chunk == 0) SPLIT_CUDA(cudaStreamWaitEvent(st, c.slot_ready[t / u_pm_chunk], 0));
+            ut = d_u + (size_t)(t / u_pm_chunk) * (size_t)n * (size_t)u_pm_chunk;
+        }
+        if ((rc = children_impl(sws, sb, n, n, t, n, d_obs, d_params, d_rvr, ut, c.seed, c.philox_offset, gather, xs, hist, shift,
+                                xmin, st, Xt, perm, J1t, 1, u_pm_chunk)))
+            return rc;
+        // jump tables + fixed-lag sums (birth order) on the second stream.  They depend only on the
+        // children and feed only outputs, so they get a whole step of slack: the weights phase of
+        // step t picks up the sums of generation t - 1 (its ring slots stay untouched until t + lag)
+        SPLIT_CUDA(cudaEventRecord(side->fork, st));
+        SPLIT_CUDA(cudaStreamWaitEvent(side->s, side->fork, 0));
+        split_lineage_kernel<<<kLineageGrid, 256, 0, side->s>>>(
+            state, t, n, lag, R, Q, X, J, d_obs, d_params, shift,
+            (double*)((char*)sws + L.gpart + (size_t)(t & 1) * gstride));
+        SPLIT_CUDA(cudaEventRecord(side->join[t & 1], side->s));
+        if ((rc = pmmh_svsplit_sort(sws, sb, n, n, n, nf_bound, 0, Xt, Xt, 0, xs, perm, st))) return rc;
+        if (t > 1) SPLIT_CUDA(cudaStreamWaitEvent(st, side->join[(t - 1) & 1], 0));
+        double* kp = (t >= nobs - lag) ? keep + (size_t)(t % lag) * n : nullptr;
+        if ((rc = weights_impl(sws, sb, n, n, t, n, lag, nobs, d_obs, d_params, xs, perm, nullptr, sums, gather,
+                               kp, st, 1)))
+            return rc;
+    }
+    // the tail waits for the sums of the last generation's lineage kernel and reads records of the final
+    // generation, built once from the stored paths; X is free by then and large enough (R > lag rows)
+    return split_end(c, nobs, n, lag, P, perm, rec, X, [&]() -> int {
+        SPLIT_CUDA(cudaStreamWaitEvent(st, side->join[(nobs - 1) & 1], 0));
+        if (nobs - 1 >= lag)
+            split_lineage_reduce_kernel<<<1, 256, 0, st>>>(
+                (const double*)((char*)sws + L.gpart + (size_t)((nobs - 1) & 1) * gstride),
+                sums + (size_t)(nobs - 1) * 8);
+        split_build_records_kernel<<<grid_for(n, 256), 256, 0, st>>>(nobs - 1, n, lag, R, X, J, rec);
+        return PMMH_OK;
+    });
+}
+}  // namespace pmmh

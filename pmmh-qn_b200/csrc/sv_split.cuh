@@ -3,18 +3,14 @@
 #include <cuda_runtime.h>
 #include <stddef.h>
 
+#include "sv_call.h"
+
 namespace pmmh {
 size_t sv_split_single_ws_bytes(int nobs, int n, int lag);
 bool sv_split_single_eligible(int nobs, int n, int lag);
-int sv_split_single_run(const double* d_obs, const double* d_params, const double* d_rvr, const double* d_u,
-                        int nobs, int n, int lag, double* d_filt, double* d_smo, double* d_ll,
-                        double* d_grad, double* d_traj, long long* d_diag, void* d_ws, size_t ws_bytes,
-                        cudaStream_t st);
-// path storage variant (algorithm 5): generations stored once in birth order, jump tables
+int sv_split_single_run(const SvCall& c, int nobs, int n, int lag);
+// path storage variant (algorithm 5): generations stored once in birth order, jump tables.  Also reads u as
+// particle-major slots signalled by c.slot_ready, or, with c.u == NULL, as the Philox stream (c.seed, c.philox_offset)
 size_t sv_split_path_ws_bytes(int nobs, int n, int lag);
-int sv_split_path_run(const double* d_obs, const double* d_params, const double* d_rvr, const double* d_u,
-                      int nobs, int n, int lag, double* d_filt, double* d_smo, double* d_ll, double* d_grad,
-                      double* d_traj, long long* d_diag, void* d_ws, size_t ws_bytes, cudaStream_t st,
-                      int u_pm_chunk = 0, const cudaEvent_t* chunk_ready = nullptr,
-                      unsigned long long seed = 0, unsigned long long philox_offset = 0);   // d_u == NULL: Philox stream
+int sv_split_path_run(const SvCall& c, int nobs, int n, int lag);
 }  // namespace pmmh

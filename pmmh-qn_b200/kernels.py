@@ -88,6 +88,28 @@ def _sv_common(obs, params, rvr, u):
     return obs, obs_stride, params, rvr, u, batch, n_obs, n
 
 
+def _sv_outputs(dev, batch, n_obs, n=0, smoother=True, hessian=False, history=False):
+    """Output tensors of the smoother / filter entries: filt, (smo), log_like, (gradient), traj, (hess1, hess2),
+    diag and, with history, X / A [B, n_obs, N]."""
+    def f64(*shape):
+        return torch.empty(shape, dtype=_F64, device=dev)
+    out = {"filt": f64(batch, n_obs)}
+    if smoother:
+        out["smo"] = f64(batch, n_obs)
+    out["log_like"] = f64(batch)
+    if smoother:
+        out["gradient"] = f64(batch, 4, n_obs)
+    out["traj"] = f64(batch, n_obs)
+    if hessian:
+        out["hess1"] = f64(batch, 4, 4)
+        out["hess2"] = f64(batch, 4, 4)
+    out["diag"] = torch.zeros((batch, _lib.DIAG_COUNT), dtype=torch.int64, device=dev)
+    if history:
+        out["X"] = f64(batch, n_obs, n)
+        out["A"] = torch.empty((batch, n_obs, n), dtype=torch.int32, device=dev)
+    return out
+
+
 def flps_sv_corr(obs, params, rvr, u, lag=10, compute_hessian=False, store_history=False,
                  ctas_per_problem=0, workspace=None):
     """Fixed-lag particle smoother (pmmh_flps_sv_corr).  u is time-major [B, n_obs, N].
@@ -96,22 +118,8 @@ def flps_sv_corr(obs, params, rvr, u, lag=10, compute_hessian=False, store_histo
     obs, obs_stride, params, rvr, u, batch, n_obs, n = _sv_common(obs, params, rvr, u)
     dev = u.device
     hess = int(bool(compute_hessian))
-    out = {
-        "filt": torch.empty((batch, n_obs), dtype=_F64, device=dev),
-        "smo": torch.empty((batch, n_obs), dtype=_F64, device=dev),
-        "log_like": torch.empty((batch,), dtype=_F64, device=dev),
-        "gradient": torch.empty((batch, 4, n_obs), dtype=_F64, device=dev),
-        "traj": torch.empty((batch, n_obs), dtype=_F64, device=dev),
-        "hess1": torch.empty((batch, 4, 4), dtype=_F64, device=dev),
-        "hess2": torch.empty((batch, 4, 4), dtype=_F64, device=dev),
-        "diag": torch.zeros((batch, _lib.DIAG_COUNT), dtype=torch.int64, device=dev),
-    }
-    xh = ah = None
-    if store_history:
-        xh = torch.empty((batch, n_obs, n), dtype=_F64, device=dev)
-        ah = torch.empty((batch, n_obs, n), dtype=torch.int32, device=dev)
-        out["X"] = xh
-        out["A"] = ah
+    out = _sv_outputs(dev, batch, n_obs, n, hessian=True, history=store_history)
+    xh, ah = out.get("X"), out.get("A")
     nbytes = sv_workspace_bytes(n_obs, n, lag, batch, hess, 0, store_history, ctas_per_problem)
     ws = (workspace or Workspace()).get(nbytes, dev)
     _lib.check(lib.pmmh_flps_sv_corr(
@@ -134,20 +142,8 @@ def flps_model_corr(model_id, obs, params, rvr, u, lag=10, store_history=False, 
     lib = _lib.load()
     obs, obs_stride, params, rvr, u, batch, n_obs, n = _sv_common(obs, params, rvr, u)
     dev = u.device
-    out = {
-        "filt": torch.empty((batch, n_obs), dtype=_F64, device=dev),
-        "smo": torch.empty((batch, n_obs), dtype=_F64, device=dev),
-        "log_like": torch.empty((batch,), dtype=_F64, device=dev),
-        "gradient": torch.empty((batch, 4, n_obs), dtype=_F64, device=dev),
-        "traj": torch.empty((batch, n_obs), dtype=_F64, device=dev),
-        "diag": torch.zeros((batch, _lib.DIAG_COUNT), dtype=torch.int64, device=dev),
-    }
-    xh = ah = None
-    if store_history:
-        xh = torch.empty((batch, n_obs, n), dtype=_F64, device=dev)
-        ah = torch.empty((batch, n_obs, n), dtype=torch.int32, device=dev)
-        out["X"] = xh
-        out["A"] = ah
+    out = _sv_outputs(dev, batch, n_obs, n, history=store_history)
+    xh, ah = out.get("X"), out.get("A")
     wb = ctypes.c_size_t()
     _lib.check(lib.pmmh_flps_model_workspace_bytes(n_obs, n, lag, batch, ctypes.byref(wb)),
                "pmmh_flps_model_workspace_bytes")
@@ -167,14 +163,7 @@ def flps_sv_corr_philox(obs, params, rvr, seed, philox_offset, n_particles, lag=
     _need_cuda(obs, params, rvr)
     dev = obs.device
     n_obs = obs.shape[0]
-    out = {
-        "filt": torch.empty((1, n_obs), dtype=_F64, device=dev),
-        "smo": torch.empty((1, n_obs), dtype=_F64, device=dev),
-        "log_like": torch.empty((1,), dtype=_F64, device=dev),
-        "gradient": torch.empty((1, 4, n_obs), dtype=_F64, device=dev),
-        "traj": torch.empty((1, n_obs), dtype=_F64, device=dev),
-        "diag": torch.zeros((1, _lib.DIAG_COUNT), dtype=torch.int64, device=dev),
-    }
+    out = _sv_outputs(dev, 1, n_obs)
     nb = ctypes.c_size_t()
     _lib.check(lib.pmmh_flps_sv_corr_philox_workspace_bytes(n_obs, int(n_particles), int(lag), ctypes.byref(nb)),
                "pmmh_flps_sv_corr_philox_workspace_bytes")
@@ -208,16 +197,7 @@ def flps_sv_corr_streamed(rvs_host, obs, params, rvr, n_obs, n_particles, lag=10
     dev = obs.device
     params = params.reshape(1, 4)
     rvr = rvr.reshape(1, n_obs)
-    out = {
-        "filt": torch.empty((1, n_obs), dtype=_F64, device=dev),
-        "smo": torch.empty((1, n_obs), dtype=_F64, device=dev),
-        "log_like": torch.empty((1,), dtype=_F64, device=dev),
-        "gradient": torch.empty((1, 4, n_obs), dtype=_F64, device=dev),
-        "traj": torch.empty((1, n_obs), dtype=_F64, device=dev),
-        "hess1": torch.empty((1, 4, 4), dtype=_F64, device=dev),
-        "hess2": torch.empty((1, 4, 4), dtype=_F64, device=dev),
-        "diag": torch.zeros((1, _lib.DIAG_COUNT), dtype=torch.int64, device=dev),
-    }
+    out = _sv_outputs(dev, 1, n_obs, hessian=True)
     wb = ctypes.c_size_t()
     _lib.check(lib.pmmh_sv_streamed_workspace_bytes(n_obs, n_particles, lag, ctas_per_problem, ctypes.byref(wb)),
                "pmmh_sv_streamed_workspace_bytes")
@@ -241,18 +221,8 @@ def bpf_sv_corr(obs, params, rvr, u, read_mode=_lib.BPF_PARITY, store_history=Fa
     lib = _lib.load()
     obs, obs_stride, params, rvr, u, batch, n_obs, n = _sv_common(obs, params, rvr, u)
     dev = u.device
-    out = {
-        "filt": torch.empty((batch, n_obs), dtype=_F64, device=dev),
-        "log_like": torch.empty((batch,), dtype=_F64, device=dev),
-        "traj": torch.empty((batch, n_obs), dtype=_F64, device=dev),
-        "diag": torch.zeros((batch, _lib.DIAG_COUNT), dtype=torch.int64, device=dev),
-    }
-    xh = ah = None
-    if store_history:
-        xh = torch.empty((batch, n_obs, n), dtype=_F64, device=dev)
-        ah = torch.empty((batch, n_obs, n), dtype=torch.int32, device=dev)
-        out["X"] = xh
-        out["A"] = ah
+    out = _sv_outputs(dev, batch, n_obs, n, smoother=False, history=store_history)
+    xh, ah = out.get("X"), out.get("A")
     nbytes = sv_workspace_bytes(n_obs, n, 2, batch, 0, 1, store_history, ctas_per_problem)
     ws = (workspace or Workspace()).get(nbytes, dev)
     _lib.check(lib.pmmh_bpf_sv_corr(
