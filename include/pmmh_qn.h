@@ -203,6 +203,25 @@ int pmmh_flps_model_corr(int model_id, const double* d_obs, long long obs_stride
                          long long* d_diag, double* d_x_hist, int* d_a_hist, void* d_workspace,
                          size_t workspace_bytes, void* stream);
 
+/* Model-generic particle filter: the log-likelihood without the fixed-lag smoother.  The filter half of
+ * pmmh_flps_model_corr, unchanged (Q1 initial state, sorted correlated systematic resampling, the model's
+ * propagation and log-weight, Q10 / Q11 trajectory); no genealogy, score terms or tail, and no lag.  On every
+ * shape both entries take, d_log_like, d_filt, d_traj, d_diag and the history d_x_hist / d_a_hist are
+ * bit-identical to pmmh_flps_model_corr's for any lag.  The kernel (d_diag[PMMH_DIAG_KERNEL]):
+ *   3  chain kernel: n_obs >= 2, 2 <= n_particles <= 4096, any batch (no workspace: 0 bytes, d_workspace may be NULL);
+ *   5  grid kernel: n_obs >= 2, batch == 1 and a tile of n_particles / min(SMs, ceil(n_particles / 2048))
+ *      particles fits one CTA (<= 7168: up to 1,060,864 particles on 148 SMs), on the same tiles as
+ *      pmmh_flps_model_corr; its workspace has no genealogy records or payloads;
+ * other sizes are refused (PMMH_ERR_INVALID; also by pmmh_filter_model_workspace_bytes, which returns the size
+ * with history for the kernel the call runs).  No fallback inside: d_diag[PMMH_DIAG_STATUS] == 1 reports an
+ * abandoned problem. */
+int pmmh_filter_model_workspace_bytes(int n_obs, int n_particles, int batch, size_t* bytes);
+int pmmh_filter_model_corr(int model_id, const double* d_obs, long long obs_stride, const double* d_params,
+                           const double* d_rvr, const double* d_u, int n_obs, int n_particles, int batch,
+                           double* d_filt, double* d_log_like, double* d_traj, long long* d_diag,
+                           double* d_x_hist, int* d_a_hist, void* d_workspace, size_t workspace_bytes,
+                           void* stream);
+
 /* Bootstrap particle filter (filter only).  read_mode: PMMH_BPF_PARITY / PMMH_BPF_INTENDED. */
 int pmmh_bpf_sv_corr(const double* d_obs, long long obs_stride, const double* d_params,
                      const double* d_rvr, const double* d_u, int n_obs, int n_particles, int batch,

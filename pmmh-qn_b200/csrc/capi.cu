@@ -226,7 +226,7 @@ int sv_make_plan(SvShape s, SvEntry entry, SvPlan* p) {
     size_t kernel_bytes = 0;
     switch (p->c.kernel) {
     case SvKernel::Chain:
-        p->chain_stride = pmmh::sv_chain_ws_bytes(n, s.lag, nobs, s.hess);
+        p->chain_stride = pmmh::sv_chain_ws_bytes(n, s.lag, nobs, s.hess, 0);
         kernel_bytes = (size_t)p->grid * p->chain_stride;
         break;
     case SvKernel::Grid:
@@ -303,7 +303,7 @@ int sv_launch_plan(const SvPlan& p, const SvShape& s, const pmmh::SvCall& c) {
     switch (p.c.kernel) {
     case SvKernel::Chain:
         a.ws_team_stride = p.chain_stride;
-        PMMH_CUDA(pmmh::sv_chain_launch(a, p.grid, c.stream));
+        PMMH_CUDA(pmmh::sv_chain_launch(a, p.grid, c.filter, c.stream));
         break;
     case SvKernel::Grid:
         rc = pmmh::sv_grid_run(c, s.nobs, s.n, s.lag, p.c.grid_G, s.hess);
@@ -664,13 +664,15 @@ int pmmh_flps_sv_corr_streamed(const double* h_rvs, const double* d_obs, const d
     return PMMH_OK;
 }
 
-// ---- model-generic entry point: the chain or the grid kernel instantiated for a model of pf_model.cuh ----------
+// ---- model-generic entry points: the chain or the grid kernel instantiated for a model of pf_model.cuh ----------
 namespace {
-// The plan pmmh_flps_model_corr runs: the chain kernel wherever it applies (any batch), else the grid kernel for one
-// problem on sv_grid_ctas(N, SMs, 0) CTAs; anything else is refused.  The workspace is the chosen kernel's alone (there
-// is no fallback pass), with history on the grid kernel (the query has no flag).
-int model_choose(int n_obs, int n, int lag, int batch, DeviceInfo* di, SvPlan* p) {
-    if (n_obs < 2 || batch < 1) return fail(PMMH_ERR_INVALID, "pmmh_flps_model_corr: bad arguments");
+// The plan pmmh_flps_model_corr (filter = 0) or pmmh_filter_model_corr (filter = 1, lag 2: no lag condition) runs:
+// the chain kernel wherever it applies (any batch), else the grid kernel for one problem on sv_grid_ctas(N, SMs, 0)
+// CTAs; anything else is refused.  The workspace is the chosen kernel's alone (there is no fallback pass), with
+// history on the grid kernel (the query has no flag).
+int model_choose(int n_obs, int n, int lag, int batch, int filter, DeviceInfo* di, SvPlan* p) {
+    if (n_obs < 2 || batch < 1)
+        return fail(PMMH_ERR_INVALID, filter ? "pmmh_filter_model_corr: bad arguments" : "pmmh_flps_model_corr: bad arguments");
     int rc = get_device_info(di);
     if (rc != PMMH_OK) return rc;
     memset(p, 0, sizeof(*p));
@@ -681,11 +683,15 @@ int model_choose(int n_obs, int n, int lag, int batch, DeviceInfo* di, SvPlan* p
     p->n_teams = p->grid = batch < di->sm ? batch : di->sm;
     if (pmmh::sv_chain_eligible(n, lag) && pmmh::sv_chain_smem_bytes(n) <= kMaxDynSmem) {
         p->c.kernel = SvKernel::Chain;
-        p->chain_stride = pmmh::sv_chain_ws_bytes(n, lag, n_obs, 0);
+        p->chain_stride = pmmh::sv_chain_ws_bytes(n, lag, n_obs, 0, filter);
         p->total = (size_t)p->grid * p->chain_stride;
-    } else if (batch == 1 && pmmh::sv_grid_eligible(n_obs, n, lag, p->c.grid_G)) {
+    } else if (batch == 1 && (filter ? pmmh::sv_grid_filter_eligible(n_obs, n, p->c.grid_G)
+                                     : pmmh::sv_grid_eligible(n_obs, n, lag, p->c.grid_G))) {
         p->c.kernel = SvKernel::Grid;
-        p->total = pmmh::sv_grid_ws_bytes(n_obs, n, lag, p->c.grid_G, 1);
+        p->total = pmmh::sv_grid_ws_bytes(n_obs, n, lag, p->c.grid_G, 1, 0, filter);
+    } else if (filter) {
+        return fail(PMMH_ERR_INVALID, "pmmh_filter_model_corr: n_obs >= 2 and 2 <= n_particles <= 4096 (any batch), "
+                                      "or batch == 1 and n_particles up to 7168 per SM (1,060,864 on 148 SMs)");
     } else {
         return fail(PMMH_ERR_INVALID, "pmmh_flps_model_corr: 2 <= lag <= 10 and 2 <= n_particles <= 4096 (any batch), "
                                       "or batch == 1, n_obs >= 2 lag and n_particles up to 7168 per SM "
@@ -699,7 +705,7 @@ int pmmh_flps_model_workspace_bytes(int n_obs, int n_particles, int lag, int bat
     if (!bytes) return fail(PMMH_ERR_INVALID, "pmmh_flps_model_workspace_bytes: bad arguments");
     DeviceInfo di;
     SvPlan p;
-    int rc = model_choose(n_obs, n_particles, lag, batch, &di, &p);
+    int rc = model_choose(n_obs, n_particles, lag, batch, 0, &di, &p);
     if (rc != PMMH_OK) return rc;
     *bytes = p.total;
     return PMMH_OK;
@@ -721,7 +727,7 @@ int pmmh_flps_model_corr(int model_id, const double* d_obs, long long obs_stride
     if (n_obs < lag + 1) return fail(PMMH_ERR_INVALID, "n_obs must be at least lag + 1");
     DeviceInfo di;
     SvPlan p;
-    int rc = model_choose(n_obs, n_particles, lag, batch, &di, &p);
+    int rc = model_choose(n_obs, n_particles, lag, batch, 0, &di, &p);
     if (rc != PMMH_OK) return rc;
     if (workspace_bytes < p.total) return fail(PMMH_ERR_WORKSPACE, "workspace too small");
     rc = check_device(di, p.c.kernel == SvKernel::Grid);
@@ -732,6 +738,45 @@ int pmmh_flps_model_corr(int model_id, const double* d_obs, long long obs_stride
     c.obs = d_obs; c.obs_stride = obs_stride; c.params = d_params; c.rvr = d_rvr; c.u = d_u;
     c.filt = d_filt; c.smo = d_smo; c.ll = d_log_like; c.grad = d_gradient; c.traj = d_traj; c.diag = d_diag;
     c.x_hist = d_x_hist; c.a_hist = d_a_hist; c.model = model_id; c.prof = g_sv_prof;
+    c.ws = d_workspace; c.ws_bytes = workspace_bytes; c.stream = (cudaStream_t)stream;
+    return sv_launch_plan(p, s, c);
+}
+
+int pmmh_filter_model_workspace_bytes(int n_obs, int n_particles, int batch, size_t* bytes) {
+    if (!bytes) return fail(PMMH_ERR_INVALID, "pmmh_filter_model_workspace_bytes: bad arguments");
+    DeviceInfo di;
+    SvPlan p;
+    int rc = model_choose(n_obs, n_particles, 2, batch, 1, &di, &p);
+    if (rc != PMMH_OK) return rc;
+    *bytes = p.total;
+    return PMMH_OK;
+}
+
+int pmmh_filter_model_corr(int model_id, const double* d_obs, long long obs_stride, const double* d_params,
+                           const double* d_rvr, const double* d_u, int n_obs, int n_particles, int batch,
+                           double* d_filt, double* d_log_like, double* d_traj, long long* d_diag,
+                           double* d_x_hist, int* d_a_hist, void* d_workspace, size_t workspace_bytes,
+                           void* stream) {
+    if (!d_obs || !d_params || !d_rvr || !d_u || !d_filt || !d_log_like || !d_traj || !d_diag)
+        return fail(PMMH_ERR_INVALID, "pmmh_filter_model_corr: null pointer argument");
+    if (model_id != PMMH_MODEL_SV_LEVERAGE && model_id != PMMH_MODEL_LINEAR_GAUSSIAN &&
+        model_id != PMMH_MODEL_LINEAR_GAUSSIAN_FA)
+        return fail(PMMH_ERR_INVALID, "pmmh_filter_model_corr: unknown model id");
+    if ((d_x_hist == nullptr) != (d_a_hist == nullptr))
+        return fail(PMMH_ERR_INVALID, "d_x_hist and d_a_hist must be given together");
+    DeviceInfo di;
+    SvPlan p;
+    int rc = model_choose(n_obs, n_particles, 2, batch, 1, &di, &p);
+    if (rc != PMMH_OK) return rc;
+    if (workspace_bytes < p.total) return fail(PMMH_ERR_WORKSPACE, "workspace too small");
+    if (p.total && !d_workspace) return fail(PMMH_ERR_INVALID, "pmmh_filter_model_corr: null workspace");
+    rc = check_device(di, p.c.kernel == SvKernel::Grid);
+    if (rc != PMMH_OK) return rc;
+    const SvShape s = {n_obs, n_particles, 2, batch, 0, pmmh::kSvFlps, d_x_hist != nullptr, 0};
+    pmmh::SvCall c = {};
+    c.obs = d_obs; c.obs_stride = obs_stride; c.params = d_params; c.rvr = d_rvr; c.u = d_u;
+    c.filt = d_filt; c.ll = d_log_like; c.traj = d_traj; c.diag = d_diag;
+    c.x_hist = d_x_hist; c.a_hist = d_a_hist; c.model = model_id; c.filter = 1; c.prof = g_sv_prof;
     c.ws = d_workspace; c.ws_bytes = workspace_bytes; c.stream = (cudaStream_t)stream;
     return sv_launch_plan(p, s, c);
 }

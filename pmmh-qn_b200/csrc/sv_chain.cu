@@ -32,6 +32,9 @@
 // against 1.50 s on the general kernel (0.27 s without the Hessian).
 // A degenerate cloud (a sort bin with more than 1024 keys) abandons the problem with status 1;
 // the host re-runs the general kernel for it.
+// SMO = false is the particle filter alone (pmmh_filter_model_corr): the same resampling, sort, weights and
+// sums, without the carried ancestor positions, the (value, parent value) ring, the fixed-lag terms and the
+// tail; it needs no workspace.
 #include <math.h>
 
 #include "common.cuh"
@@ -141,8 +144,10 @@ __device__ __forceinline__ double4 chain_ld_d4(const double4* p) {
 
 // M = the model (pf_model.cuh): propagation, log-weight, score terms
 // HESS (SvLeverageModel only): the Hessian branch of the reference with its quirks Q7 / Q8
-template <class M, bool HESS>
+// SMO: the fixed-lag smoother (smo, gradient); false: the filter alone (log-likelihood, filt, traj, diag, history)
+template <class M, bool HESS, bool SMO>
 __global__ void __launch_bounds__(kCT, 1) sv_chain_kernel(SvArgs a) {
+    static_assert(SMO || !HESS, "the Hessian branch needs the smoother");
     long long prof_t = clock64();
     extern __shared__ __align__(16) unsigned char dsm_raw[];
     const int N = a.N, NOBS = a.NOBS, LAG = a.LAG;
@@ -169,7 +174,7 @@ __global__ void __launch_bounds__(kCT, 1) sv_chain_kernel(SvArgs a) {
     char* wsbase = a.ws + (size_t)blockIdx.x * a.ws_team_stride;
     ChainWs w;
     const int SQ = HESS ? a.SQ : 1;
-    chain_ws_carve(N, LAG, NOBS, SQ, HESS ? 1 : 0, wsbase, &w);
+    if constexpr (SMO) chain_ws_carve(N, LAG, NOBS, SQ, HESS ? 1 : 0, wsbase, &w);
 #define XPG(t) (w.xp + (size_t)((t) % RXP) * N)
 #define B1G(t) (w.b1 + (size_t)((t) - (NOBS - LAG)) * N)
 #define SHG(t) (w.sh + (size_t)((t) - (NOBS - LAG)) * N)
@@ -199,9 +204,11 @@ __global__ void __launch_bounds__(kCT, 1) sv_chain_kernel(SvArgs a) {
             s_x[p] = x0;
             s_cum[p] = (double)(p + 1);
             s_hist[p] = 0;
-            s_b[p] = s_b[NP + p] = s_b[2 * NP + p] = s_b[3 * NP + p] = 0;
-            for (int q = 0; q < kB4Ring; ++q) s_B4[q * (size_t)NP + p] = 0;
-            XPG(0)[p] = make_double2(x0, x0);
+            if constexpr (SMO) {
+                s_b[p] = s_b[NP + p] = s_b[2 * NP + p] = s_b[3 * NP + p] = 0;
+                for (int q = 0; q < kB4Ring; ++q) s_B4[q * (size_t)NP + p] = 0;
+                XPG(0)[p] = make_double2(x0, x0);
+            }
             if (HESS) {
                 ALG(0)[p] = make_double4(0.0, 0.0, 0.0, 0.0);
                 if (p < SQ) w.xlow[p] = x0;
@@ -211,7 +218,7 @@ __global__ void __launch_bounds__(kCT, 1) sv_chain_kernel(SvArgs a) {
                 Ah[p] = p;
             }
         }
-        for (int t = tid; t < NOBS; t += kCT) {
+        for (int t = tid; SMO && t < NOBS; t += kCT) {
             o_smo[t] = 0.0;
             o_grad[t] = 0.0;
             o_grad[NOBS + t] = 0.0;
@@ -388,10 +395,12 @@ __global__ void __launch_bounds__(kCT, 1) sv_chain_kernel(SvArgs a) {
                     pos[m] = start + rank;
                     xs[m] = key;
                     anc[m] = pay;
-                    xpar[m] = s_x[pay];
-                    ib1[m] = s_b[pay];
-                    ib2[m] = s_b[NP + pay];
-                    ib3[m] = s_b[2 * NP + pay];
+                    if constexpr (SMO) {
+                        xpar[m] = s_x[pay];
+                        ib1[m] = s_b[pay];
+                        ib2[m] = s_b[NP + pay];
+                        ib3[m] = s_b[2 * NP + pay];
+                    }
                 }
             }
             __syncthreads();   // every read of the parent generation is done
@@ -406,15 +415,17 @@ __global__ void __launch_bounds__(kCT, 1) sv_chain_kernel(SvArgs a) {
                     const int p = pos[m];
                     if (p >= 0) {
                         s_x[p] = xs[m];
-                        s_b[p] = (unsigned short)anc[m];
-                        s_b[NP + p] = (unsigned short)ib1[m];
-                        s_b[2 * NP + p] = (unsigned short)ib2[m];
-                        s_b[3 * NP + p] = (unsigned short)ib3[m];
-                        b4n[p] = (unsigned short)ib3[m];
+                        if constexpr (SMO) {
+                            s_b[p] = (unsigned short)anc[m];
+                            s_b[NP + p] = (unsigned short)ib1[m];
+                            s_b[2 * NP + p] = (unsigned short)ib2[m];
+                            s_b[3 * NP + p] = (unsigned short)ib3[m];
+                            b4n[p] = (unsigned short)ib3[m];
+                        }
                         double sh = exp(M::logw(c, xs[m], yi) - shift);
                         if (!isfinite(sh)) sh = 0.0;
                         s_cum[p] = sh;
-                        xpn[p] = make_double2(xs[m], xpar[m]);
+                        if constexpr (SMO) xpn[p] = make_double2(xs[m], xpar[m]);
                         if constexpr (HESS) {
                             // alpha recursion (:361-390).  Q7: particles[i - 1 + ancestors[j]] read through the flat
                             // layout = sorted value `sl` of time tq, or the unsorted new value `sl`, or 0
@@ -440,7 +451,7 @@ __global__ void __launch_bounds__(kCT, 1) sv_chain_kernel(SvArgs a) {
                             ALG(inext)[p] = make_double4(a0 + pa.x, a1 + pa.y, a2 + pa.z, a3 + pa.w);
                             if (p < SQ) w.xlow[(size_t)inext * SQ + p] = xs[m];
                         }
-                        if (keep_tail) {
+                        if (SMO && keep_tail) {
                             B1G(inext)[p] = anc[m];
                             SHG(inext)[p] = sh;
                         }
@@ -455,8 +466,10 @@ __global__ void __launch_bounds__(kCT, 1) sv_chain_kernel(SvArgs a) {
             __syncthreads();
             CPROF(3);   // new generation: weights, tables
             // =========== position order: cumulative weights, sums, fixed-lag terms (:445-470)
-            constexpr int NACC = 6;
-            double acc[NACC] = {0.0, 0.0, 0.0, 0.0, 0.0, 0.0};
+            constexpr int NACC = SMO ? 6 : 1;   // sh x; sh x_lagged, sh g[0..3]
+            double acc[NACC];
+#pragma unroll
+            for (int q = 0; q < NACC; ++q) acc[q] = 0.0;
             double S_i;
             {
                 double v[kP], tsum = 0.0;
@@ -467,12 +480,12 @@ __global__ void __launch_bounds__(kCT, 1) sv_chain_kernel(SvArgs a) {
                     tsum += v[q];
                 }
                 double run = chain_scan_d(tsum, s_w, &S_i);
-                const bool lagged = inext >= LAG;
+                const bool lagged = SMO && inext >= LAG;
                 const double yl = lagged ? obs[inext - LAG] : 0.0;   // Q5
                 const int hop0 = (K >= 1) ? ((K - 1) & 3) : 0;
                 const int nh = (K >= 1) ? ((K - 1) >> 2) : 0;        // 0 or 1 (LAG <= 10)
                 const int g1 = inext - (hop0 + 1);
-                const double2* xpk = XPG(inext - K);
+                const double2* xpk = SMO ? XPG(inext - K) : nullptr;
                 int idl[kP];
 #pragma unroll
                 for (int q = 0; q < kP; ++q) {
@@ -498,7 +511,7 @@ __global__ void __launch_bounds__(kCT, 1) sv_chain_kernel(SvArgs a) {
                         s_cum[p] = run;
                         const double sx = v[q] * s_x[p];
                         if (isfinite(sx)) acc[0] += sx;
-                        if (lagged) {
+                        if constexpr (SMO) if (lagged) {
                             double g[4];
                             if constexpr (HESS) {
                                 double sq;
@@ -531,7 +544,7 @@ __global__ void __launch_bounds__(kCT, 1) sv_chain_kernel(SvArgs a) {
                 s_S[inext % kMaxLagC] = S_i;
                 o_filt[inext] = acc[0] / S_i;
                 o_traj[inext] = s_x[0];   // Q11: traj[i] = X_i[0]
-                if (inext >= LAG) {
+                if constexpr (SMO) if (inext >= LAG) {
                     const int tt = inext - LAG + 1;
                     o_smo[tt] = acc[1] / S_i;
                     o_grad[tt] = acc[2] / S_i;
@@ -546,7 +559,7 @@ __global__ void __launch_bounds__(kCT, 1) sv_chain_kernel(SvArgs a) {
         }   // time loop
 
         // ---------------- tail (:540-562, Q6)
-        if (status == 0) {
+        if (SMO && status == 0) {
             const int T = NOBS - 1;
             const double S_T = s_S[T % kMaxLagC];
             const double* shT = SHG(T);
@@ -655,7 +668,8 @@ __global__ void __launch_bounds__(kCT, 1) sv_chain_kernel(SvArgs a) {
 
 int sv_chain_eligible(int N, int LAG) { return N >= 2 && N <= kChainMaxN && LAG >= 2 && LAG <= 10; }
 
-size_t sv_chain_ws_bytes(int N, int LAG, int NOBS, int hess) {
+size_t sv_chain_ws_bytes(int N, int LAG, int NOBS, int hess, int filter) {
+    if (filter) return 0;
     const int SQ = hess ? (NOBS + N - 2) / NOBS + 1 : 1;
     return chain_ws_carve(N, LAG, NOBS, SQ, hess, nullptr, nullptr);
 }
@@ -665,20 +679,27 @@ int sv_chain_smem_bytes(int N) {
     return (int)(NP * 8 * 3 + (NP + 2) * 4 + NP * 2 * (4 + kB4Ring + 1) + 64);
 }
 
-template <class M, bool HESS>
+template <class M, bool HESS, bool SMO>
 static cudaError_t chain_launch_one(const SvArgs& a, int grid, int smem, cudaStream_t stream) {
-    cudaError_t err = cudaFuncSetAttribute(sv_chain_kernel<M, HESS>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
+    cudaError_t err = cudaFuncSetAttribute(sv_chain_kernel<M, HESS, SMO>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
     if (err != cudaSuccess) return err;
-    sv_chain_kernel<M, HESS><<<grid, kCT, smem, stream>>>(a);
+    sv_chain_kernel<M, HESS, SMO><<<grid, kCT, smem, stream>>>(a);
     return cudaGetLastError();
 }
 
-cudaError_t sv_chain_launch(const SvArgs& a, int grid, cudaStream_t stream) {
+cudaError_t sv_chain_launch(const SvArgs& a, int grid, int filter, cudaStream_t stream) {
     const int smem = sv_chain_smem_bytes(a.N);
-    if (a.model_id == 0) return a.hess ? chain_launch_one<SvLeverageModel, true>(a, grid, smem, stream)
-                                       : chain_launch_one<SvLeverageModel, false>(a, grid, smem, stream);
-    if (a.model_id == 1 && !a.hess) return chain_launch_one<LinearGaussianModel, false>(a, grid, smem, stream);
-    if (a.model_id == 2 && !a.hess) return chain_launch_one<LinearGaussianFullyAdapted, false>(a, grid, smem, stream);
+    if (filter) {
+        if (a.hess) return cudaErrorInvalidValue;
+        if (a.model_id == 0) return chain_launch_one<SvLeverageModel, false, false>(a, grid, smem, stream);
+        if (a.model_id == 1) return chain_launch_one<LinearGaussianModel, false, false>(a, grid, smem, stream);
+        if (a.model_id == 2) return chain_launch_one<LinearGaussianFullyAdapted, false, false>(a, grid, smem, stream);
+        return cudaErrorInvalidValue;
+    }
+    if (a.model_id == 0) return a.hess ? chain_launch_one<SvLeverageModel, true, true>(a, grid, smem, stream)
+                                       : chain_launch_one<SvLeverageModel, false, true>(a, grid, smem, stream);
+    if (a.model_id == 1 && !a.hess) return chain_launch_one<LinearGaussianModel, false, true>(a, grid, smem, stream);
+    if (a.model_id == 2 && !a.hess) return chain_launch_one<LinearGaussianFullyAdapted, false, true>(a, grid, smem, stream);
     return cudaErrorInvalidValue;
 }
 

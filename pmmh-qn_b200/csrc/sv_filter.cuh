@@ -123,11 +123,12 @@ __host__ __device__ inline size_t sv_ws_layout(int N, int NOBS, int LAG, int NB,
 cudaError_t sv_launch(const SvArgs& a, int grid, cudaStream_t stream);
 int sv_dynamic_smem_bytes(int G);
 
-// chain kernel (sv_chain.cu): one CTA per problem, N <= kChainMaxN
+// chain kernel (sv_chain.cu): one CTA per problem, N <= kChainMaxN; filter = 1: the particle filter alone
+// (no fixed-lag smoother, no workspace)
 int sv_chain_eligible(int N, int LAG);
-size_t sv_chain_ws_bytes(int N, int LAG, int NOBS, int hess);
+size_t sv_chain_ws_bytes(int N, int LAG, int NOBS, int hess, int filter);
 int sv_chain_smem_bytes(int N);
-cudaError_t sv_chain_launch(const SvArgs& a, int grid, cudaStream_t stream);
+cudaError_t sv_chain_launch(const SvArgs& a, int grid, int filter, cudaStream_t stream);
 
 // exchange kernel (sv_fast.cu)
 int sv_fast_nsub(int N, int G);

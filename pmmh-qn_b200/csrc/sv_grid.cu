@@ -51,6 +51,9 @@
 //   * template over the model (pf_model.cuh): SvLeverageModel is everything above; another model runs the generic path
 //     in the same body (XE = (x, propagation mean of the children), payload = (parent value, -, -, value), score terms
 //     M::score_main / M::score_tail), gradient only (DESIGN 4.0).
+//   * SMO = false: the particle filter alone (pmmh_filter_model_corr) -- no payloads, no genealogy records, no score
+//     terms, no tail; the workspace has no R / P tables and no weight ring.  The birth rows stay: the in-bin ranking
+//     breaks ties on them.
 //
 // Deviations from the reference's operation order: parallel sums / scans, log(exp(x/2)) = x/2 and
 // 1/exp(x/2)^2 = exp(-x/2)^2 in the log-weight, cumulative weights multiplied by 1/S; any
@@ -387,10 +390,12 @@ __device__ __forceinline__ void deferred_alpha_pass(const GridArgs& a, const SvC
 // M: the model (pf_model.cuh).  SvLeverageModel runs the SV code with its shared exp(-x/2); any other model
 // runs the generic path: the second double of XE is the propagation mean prop_mean(x, obs[t]) of the
 // children, a payload is (parent value, -, -, own value) and the score terms are M::score_main of the pair.
-template <int GT, bool HESS, class M>
+// SMO: the fixed-lag smoother; false: the filter alone, whose outputs are bit-identical to the smoother's.
+template <int GT, bool HESS, class M, bool SMO>
 __global__ void __launch_bounds__(GT, 1) sv_grid_kernel(const GridArgs a) {
     constexpr bool GEN = !std::is_same<M, SvLeverageModel>::value;
     static_assert(!(GEN && HESS), "the Hessian branch exists for the SV model only");
+    static_assert(SMO || !HESS, "the Hessian branch needs the smoother");
     constexpr int KPT = kCap / GT;          // entries per thread (strided assignment)
     constexpr int KCH = KPT | 1;            // longest chunk of the thread-contiguous passes (odd)
     constexpr int BPT = kNF / GT;           // histogram bins per thread
@@ -548,7 +553,7 @@ __global__ void __launch_bounds__(GT, 1) sv_grid_kernel(const GridArgs a) {
             __stcg(&a.XE[pstart + q], make_double2(mu, e0));
             __stcg(&a.perm[pstart + q], pstart + q);
             s_sh[q] = 1.0;
-            st_rec(&a.R[(size_t)(pstart + q) * RS], pol_keep, 0, 0, 0, 0, 0, 0, 0, 0);
+            if constexpr (SMO) st_rec(&a.R[(size_t)(pstart + q) * RS], pol_keep, 0, 0, 0, 0, 0, 0, 0, 0);
             if constexpr (HESS) {
                 st_rec(&a.R[(size_t)(pstart + q) * RS + 1], pol_keep, 0, 0, 0, 0, 0, 0, 0, 0);   // alpha = 0
                 if (pstart + q < a.SQ) a.xlow[(size_t)(pstart + q) * NOBS] = mu;
@@ -840,13 +845,15 @@ __global__ void __launch_bounds__(GT, 1) sv_grid_kernel(const GridArgs a) {
                         if (!isfinite(x)) bad = true;
                         xn[k0 + u] = x;
                         atomicAdd(&s_fhist[fine_bin(x, mhat, inv_shat)], 1);
-                        if constexpr (GEN) {
-                            if (!(a.dbg & 2)) st_stream_f64x4(&Pt[(size_t)(jb + i) * RS], pol_stream, xe[u].x, 0.0, 0.0, x);
-                        } else if (!(a.dbg & 2)) {
-                            // residual of the transition parent -> child as the score terms use it (:452-453)
-                            double sq = x - mu - phi * (xe[u].x - mu);
-                            sq -= sr * xe[u].y * ylag;
-                            st_stream_f64x4(&Pt[(size_t)(jb + i) * RS], pol_stream, xe[u].x, sq, xe[u].y * ylag, x);
+                        if constexpr (SMO) {
+                            if constexpr (GEN) {
+                                if (!(a.dbg & 2)) st_stream_f64x4(&Pt[(size_t)(jb + i) * RS], pol_stream, xe[u].x, 0.0, 0.0, x);
+                            } else if (!(a.dbg & 2)) {
+                                // residual of the transition parent -> child as the score terms use it (:452-453)
+                                double sq = x - mu - phi * (xe[u].x - mu);
+                                sq -= sr * xe[u].y * ylag;
+                                st_stream_f64x4(&Pt[(size_t)(jb + i) * RS], pol_stream, xe[u].x, sq, xe[u].y * ylag, x);
+                            }
                         }
                     }
                 }
@@ -868,7 +875,7 @@ __global__ void __launch_bounds__(GT, 1) sv_grid_kernel(const GridArgs a) {
         }
         PROF_MARK(3);   // A1 children+hist
         GRID_ARRIVE();   // ---- barrier 1: global histogram complete
-        if (!(a.dbg & 1)) {
+        if (SMO && !(a.dbg & 1)) {
             // genealogy records (only feed outputs): child = (parent row, parent's ancestors 1..7)
             const REntry* Rp = a.R + (size_t)((t - 1) & 1) * N * RS;
             REntry* Rc = a.R + (size_t)(t & 1) * N * RS;
@@ -1047,7 +1054,7 @@ __global__ void __launch_bounds__(GT, 1) sv_grid_kernel(const GridArgs a) {
                 if (i < nc) {
                     const int pos = s_tbase[kr[kk] >> 16] + (kr[kk] & 0xffff);
                     const long long xb = __double_as_longlong(xn[kk]);
-                    const int4 ent = make_int4((int)(xb & 0xffffffffll), (int)(xb >> 32), jb + i, bp[kk]);
+                    const int4 ent = make_int4((int)(xb & 0xffffffffll), (int)(xb >> 32), jb + i, SMO ? bp[kk] : 0);
                     if (pos >= 0 && pos < N) st_hint_b128(&mail[pos], pol_keep, ent);
                 }
             }
@@ -1092,7 +1099,7 @@ __global__ void __launch_bounds__(GT, 1) sv_grid_kernel(const GridArgs a) {
                 const double* Un = a.U + (size_t)(t + 1) * N;
                 prefetch_range(Un + jb, Un + je, lane, 32);
             }
-            if (t >= L && (a.dbg & 8)) {   // (measured: the bulk prefetch of the lagged generation costs more than it saves)
+            if (SMO && t >= L && (a.dbg & 8)) {   // (measured: the bulk prefetch of the lagged generation costs more than it saves)
                 const PEntry* Pg = a.P + (size_t)((t - (L - 2)) % RP) * N;
                 prefetch_range(Pg + jb, Pg + je, lane, 32);
             }
@@ -1175,7 +1182,7 @@ __global__ void __launch_bounds__(GT, 1) sv_grid_kernel(const GridArgs a) {
                     const int pos = min(s_sub[sub_bin(bx[kk], lo, scale)] + (int)((unsigned)bae[kk] >> 21), kCap - 1);
                     s_xb[pos] = bx[kk];
                     s_jb[pos] = bj[kk];
-                    s_ab[pos] = bae[kk] & 0x1fffff;
+                    if constexpr (SMO) s_ab[pos] = bae[kk] & 0x1fffff;
                 }
             }
             __syncthreads();
@@ -1197,7 +1204,7 @@ __global__ void __launch_bounds__(GT, 1) sv_grid_kernel(const GridArgs a) {
                     const int j = s_jb[q];
                     bx[kk] = x;
                     bj[kk] = j;
-                    ba[kk] = s_ab[q];
+                    if constexpr (SMO) ba[kk] = s_ab[q];
                     const int kb = sub_bin(x, lo, scale);
                     const int b0 = s_sub[kb];
                     const int b1 = (kb + 1 < kNSB) ? s_sub[kb + 1] : n;
@@ -1223,7 +1230,7 @@ __global__ void __launch_bounds__(GT, 1) sv_grid_kernel(const GridArgs a) {
                 if (q < n && np[kk] != q) {
                     s_xb[np[kk]] = bx[kk];
                     s_jb[np[kk]] = bj[kk];
-                    s_ab[np[kk]] = ba[kk];
+                    if constexpr (SMO) s_ab[np[kk]] = ba[kk];
                 }
             }
             __syncthreads();
@@ -1318,13 +1325,13 @@ __global__ void __launch_bounds__(GT, 1) sv_grid_kernel(const GridArgs a) {
                     __stcg((double2*)&a.tinfo[c * 4 + 2], make_double2(v[1], v[2]));
                     ps[1] = v[0];
                     ps[7] = 0.0;
-                    if (t < L || (a.dbg & 4)) {   // later steps: the score terms below write ps[2..6]
+                    if (!SMO || t < L || (a.dbg & 4)) {   // later steps: the score terms below write ps[2..6]
 #pragma unroll
                         for (int i = 2; i < 7; ++i) ps[i] = 0.0;
                     }
                 }
             }
-            if (t >= NOBS - L) {
+            if (SMO && t >= NOBS - L) {
 #pragma unroll
                 for (int kk = 0; kk < KPT; ++kk) {
                     const int q = kk * GT + tid;
@@ -1334,7 +1341,7 @@ __global__ void __launch_bounds__(GT, 1) sv_grid_kernel(const GridArgs a) {
         }
         PROF_MARK(11);   // B scan+publish
         GRID_ARRIVE();   // ---- barrier 3: tile totals published
-        if (t >= L && !(a.dbg & 4)) {
+        if (SMO && t >= L && !(a.dbg & 4)) {
             // fixed-lag score terms (:445-470): weight x monomials of the payload of the ancestor
             // LAG-2 generations back (one random sector each), fixed summation order
             const PEntry* Pg = a.P + (size_t)((t - (L - 2)) % RP) * N * RS;
@@ -1723,7 +1730,8 @@ __global__ void __launch_bounds__(256) grid_tail_reduce_kernel(const double* __r
 // sums[t][0] = sum sh, [1] = sum sh x, [2] = sum sh c, [3] = sum sh sq, [4] = sum sh sq c, [5] = sum sh sq^2,
 // [6] = sum sh sq ey (c = lagged ancestor value, sq / ey as stored in P);  tail[irel][0..4].
 // GEN (the generic path of a model other than SV): [3..6] = sum sh g[0..3], traj[0] = the initial state.
-template <bool GEN>
+// SMO = false (the filter alone): no smo / grad, tail unused.
+template <bool GEN, bool SMO>
 __global__ void grid_finish_kernel(const GridCtrl* __restrict__ ctrl, const double* __restrict__ sums,
                                    const double* __restrict__ shift, const double* __restrict__ xmin,
                                    const double* __restrict__ tail, const double* __restrict__ params,
@@ -1770,6 +1778,7 @@ __global__ void grid_finish_kernel(const GridCtrl* __restrict__ ctrl, const doub
     for (int t = tid; t < nobs; t += gridDim.x * blockDim.x) {
         filt[t] = sums[(size_t)t * 8 + 1] / sums[(size_t)t * 8];
         traj[t] = (t == 0 && !GEN) ? params[0] : xmin[t];   // Q10/Q11: traj[t] = X_t[0] for t >= 1, X_0 == mu
+        if constexpr (!SMO) continue;
         double s = 0.0, g[4] = {0.0, 0.0, 0.0, 0.0};
         const int src = t + L - 1;   // main-loop terms land at tt = i - L + 1 (:445-470)
         if (t >= 1 && src < nobs) {
@@ -1806,7 +1815,8 @@ struct GridLayout {
 
 size_t al256(size_t x) { return (x + 255) & ~(size_t)255; }
 
-GridLayout grid_layout(int nobs, int n, int lag, int G, int hist, int hess) {
+// filter: the filter alone -- no genealogy records (R), payloads (P), weight ring or tail sums
+GridLayout grid_layout(int nobs, int n, int lag, int G, int hist, int hess, int filter) {
     GridLayout L = GridLayout();
     // ring depth of the payloads: step t writes generation t and gathers from generation t-(lag-2)
     L.RP = lag < 2 ? 2 : lag;
@@ -1821,16 +1831,17 @@ GridLayout grid_layout(int nobs, int n, int lag, int G, int hist, int hess) {
     L.XE = o;        o += al256(N * 16);
     L.perm = o;      o += al256(N * 4);
     const size_t RS = hess ? 2 : 1;   // Hessian branch: 64-byte entries (record | alpha, payload | alpha)
-    L.R = o;         o += al256(2 * N * 32 * RS);
-    L.P = o;         o += al256((size_t)L.RP * N * 32 * RS);
+    const size_t smo = filter ? 0 : 1;
+    L.R = o;         o += al256(smo * 2 * N * 32 * RS);
+    L.P = o;         o += al256(smo * L.RP * N * 32 * RS);
     L.psum = o;      o += al256((size_t)nobs * G * 8 * 8);
     L.shiftv = o;    o += al256((size_t)nobs * 8);
     L.xminv = o;     o += al256((size_t)nobs * 8);
-    L.shring = o;    o += al256((size_t)lag * N * 8);
+    L.shring = o;    o += al256(smo * lag * N * 8);
     L.parentpos = o; o += al256(hist ? N * 4 : 256);
     L.sums = o;      o += al256((size_t)nobs * 8 * 8);
-    L.tailpart = o;  o += al256((size_t)lag * L.nblk * 8 * 8);
-    L.tail = o;      o += al256((size_t)lag * 8 * 8);
+    L.tailpart = o;  o += al256(smo * lag * L.nblk * 8 * 8);
+    L.tail = o;      o += al256(smo * lag * 8 * 8);
     L.info = o;      o += al256(8 * 8);
     L.ustash = o;    o += al256(4 * N * 8);   // host-streamed u: four time steps, time-major
     // Hessian branch: the first SQ sorted values of every generation (Q7: particles[i - 1 + ancestor] read through
@@ -1861,26 +1872,33 @@ int sv_grid_ctas(int n, int sm_count, int ctas) {
 }
 
 // a tile holds N/G particles +- one histogram bin; 12 % head room below the shared-memory capacity
-bool sv_grid_eligible(int nobs, int n, int lag, int G) {
-    if (G < 1 || G > kMaxTiles) return false;
-    if (lag < 2 || lag > 10 || nobs < 2 * lag || n < 32 || n > (1 << 21)) return false;
+static bool grid_tile_fits(int n, int G) {
+    if (G < 1 || G > kMaxTiles || n < 32 || n > (1 << 21)) return false;
     const int Wc = (n + G - 1) / G;
     return Wc <= kCap - kCap / 8;
 }
 
-size_t sv_grid_ws_bytes(int nobs, int n, int lag, int G, int hist, int hess) {
-    return grid_layout(nobs, n, lag, G, hist, hess).total;
+bool sv_grid_eligible(int nobs, int n, int lag, int G) {
+    return lag >= 2 && lag <= 10 && nobs >= 2 * lag && grid_tile_fits(n, G);
+}
+
+bool sv_grid_filter_eligible(int nobs, int n, int G) { return nobs >= 2 && grid_tile_fits(n, G); }
+
+size_t sv_grid_ws_bytes(int nobs, int n, int lag, int G, int hist, int hess, int filter) {
+    return grid_layout(nobs, n, lag, G, hist, hess, filter).total;
 }
 
 int sv_grid_run(const SvCall& c, int nobs, int n, int lag, int G, int hess) {
-    if (!sv_grid_eligible(nobs, n, lag, G)) return set_error(PMMH_ERR_INVALID, "grid kernel: sizes not eligible");
+    const int filter = c.filter;
+    if (filter ? (hess || !sv_grid_filter_eligible(nobs, n, G)) : !sv_grid_eligible(nobs, n, lag, G))
+        return set_error(PMMH_ERR_INVALID, "grid kernel: sizes not eligible");
     const int hist = c.x_hist != nullptr;
     const int model = c.model;
     if (model != PMMH_MODEL_SV_LEVERAGE && model != PMMH_MODEL_LINEAR_GAUSSIAN && model != PMMH_MODEL_LINEAR_GAUSSIAN_FA)
         return set_error(PMMH_ERR_INVALID, "grid kernel: unknown model id");
     if (hess && model != PMMH_MODEL_SV_LEVERAGE)
         return set_error(PMMH_ERR_INVALID, "grid kernel: the Hessian branch exists for the SV model only");
-    const GridLayout L = grid_layout(nobs, n, lag, G, hist, hess);
+    const GridLayout L = grid_layout(nobs, n, lag, G, hist, hess, filter);
     if (c.ws_bytes < L.total) return set_error(PMMH_ERR_WORKSPACE, "grid kernel: workspace too small");
     char* ws = (char*)c.ws;
     const cudaStream_t st = c.stream;
@@ -1945,22 +1963,41 @@ int sv_grid_run(const SvCall& c, int nobs, int n, int lag, int G, int hess) {
         // no persisting L2 set-aside for the kernel's evict_last accesses: with one every phase is slower
         // (DESIGN 4.0), and left unset the evaluation at N = 2^20 is ~6 % slower
         GRID_CUDA(cudaDeviceSetLimit(cudaLimitPersistingL2CacheSize, 0));
-        GRID_CUDA(cudaFuncSetAttribute(sv_grid_kernel<1024, false, SvLeverageModel>, cudaFuncAttributeMaxDynamicSharedMemorySize, kDynSmem));
-        GRID_CUDA(cudaFuncSetAttribute(sv_grid_kernel<1024, true, SvLeverageModel>, cudaFuncAttributeMaxDynamicSharedMemorySize, kDynSmem));
-        GRID_CUDA(cudaFuncSetAttribute(sv_grid_kernel<1024, false, LinearGaussianModel>, cudaFuncAttributeMaxDynamicSharedMemorySize, kDynSmem));
-        GRID_CUDA(cudaFuncSetAttribute(sv_grid_kernel<1024, false, LinearGaussianFullyAdapted>, cudaFuncAttributeMaxDynamicSharedMemorySize, kDynSmem));
+        const void* kernels[] = {(const void*)sv_grid_kernel<1024, false, SvLeverageModel, true>,
+                                 (const void*)sv_grid_kernel<1024, true, SvLeverageModel, true>,
+                                 (const void*)sv_grid_kernel<1024, false, LinearGaussianModel, true>,
+                                 (const void*)sv_grid_kernel<1024, false, LinearGaussianFullyAdapted, true>,
+                                 (const void*)sv_grid_kernel<1024, false, SvLeverageModel, false>,
+                                 (const void*)sv_grid_kernel<1024, false, LinearGaussianModel, false>,
+                                 (const void*)sv_grid_kernel<1024, false, LinearGaussianFullyAdapted, false>};
+        for (const void* k : kernels)
+            GRID_CUDA(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, kDynSmem));
         attr_set[dev] = true;
     }
     void* kargs[] = {(void*)&a};
-    const void* kern = hess ? (const void*)sv_grid_kernel<1024, true, SvLeverageModel>
-                            : (const void*)sv_grid_kernel<1024, false, SvLeverageModel>;
-    if (model == PMMH_MODEL_LINEAR_GAUSSIAN) kern = (const void*)sv_grid_kernel<1024, false, LinearGaussianModel>;
-    if (model == PMMH_MODEL_LINEAR_GAUSSIAN_FA) kern = (const void*)sv_grid_kernel<1024, false, LinearGaussianFullyAdapted>;
+    const void* kern;
+    if (filter) {
+        kern = (const void*)sv_grid_kernel<1024, false, SvLeverageModel, false>;
+        if (model == PMMH_MODEL_LINEAR_GAUSSIAN) kern = (const void*)sv_grid_kernel<1024, false, LinearGaussianModel, false>;
+        if (model == PMMH_MODEL_LINEAR_GAUSSIAN_FA) kern = (const void*)sv_grid_kernel<1024, false, LinearGaussianFullyAdapted, false>;
+    } else {
+        kern = hess ? (const void*)sv_grid_kernel<1024, true, SvLeverageModel, true>
+                    : (const void*)sv_grid_kernel<1024, false, SvLeverageModel, true>;
+        if (model == PMMH_MODEL_LINEAR_GAUSSIAN) kern = (const void*)sv_grid_kernel<1024, false, LinearGaussianModel, true>;
+        if (model == PMMH_MODEL_LINEAR_GAUSSIAN_FA) kern = (const void*)sv_grid_kernel<1024, false, LinearGaussianFullyAdapted, true>;
+    }
     GRID_CUDA(cudaLaunchCooperativeKernel(kern, dim3(G), dim3(1024), kargs, kDynSmem, st));
     double* sums = (double*)(ws + L.sums);
     double* tailpart = (double*)(ws + L.tailpart);
     double* tail = (double*)(ws + L.tail);
     grid_reduce_kernel<<<nobs, 256, 0, st>>>(a.psum, G, sums);
+    if (filter) {
+        auto finish = model == PMMH_MODEL_SV_LEVERAGE ? grid_finish_kernel<false, false> : grid_finish_kernel<true, false>;
+        finish<<<(nobs + 255) / 256, 256, 0, st>>>(a.ctrl, sums, a.shiftv, a.xminv, nullptr, c.params, nobs, lag, (double)n,
+                                                   c.ll, c.filt, nullptr, nullptr, c.traj, c.diag, (long long*)(ws + L.info));
+        GRID_CUDA(cudaGetLastError());
+        return PMMH_OK;
+    }
     if (hess) {
         double* sumsH = (double*)(ws + L.sumsH);
         double* tailpartH = (double*)(ws + L.tailpartH);
@@ -1975,7 +2012,7 @@ int sv_grid_run(const SvCall& c, int nobs, int n, int lag, int G, int hess) {
         grid_tail_kernel<false, SvLeverageModel><<<dim3(L.nblk, lag), 256, 0, st>>>(a, sums, tailpart, nullptr, L.nblk);
     }
     grid_tail_reduce_kernel<<<lag, 256, 0, st>>>(tailpart, L.nblk, tail);
-    auto finish = model == PMMH_MODEL_SV_LEVERAGE ? grid_finish_kernel<false> : grid_finish_kernel<true>;
+    auto finish = model == PMMH_MODEL_SV_LEVERAGE ? grid_finish_kernel<false, true> : grid_finish_kernel<true, true>;
     finish<<<(nobs + 255) / 256, 256, 0, st>>>(a.ctrl, sums, a.shiftv, a.xminv, tail, c.params, nobs, lag, (double)n, c.ll,
                                                c.filt, c.smo, c.grad, c.traj, c.diag, (long long*)(ws + L.info));
     GRID_CUDA(cudaGetLastError());

@@ -9,7 +9,10 @@
 namespace pmmh {
 int sv_grid_ctas(int n, int sm_count, int ctas);
 bool sv_grid_eligible(int nobs, int n, int lag, int G);
-size_t sv_grid_ws_bytes(int nobs, int n, int lag, int G, int hist, int hess = 0);
-// c.model selects the instantiation (PMMH_MODEL_*, pf_model.cuh); hess: the Hessian branch (SV only)
+// the filter alone (no lag): n_obs >= 2 and a tile fits one CTA
+bool sv_grid_filter_eligible(int nobs, int n, int G);
+size_t sv_grid_ws_bytes(int nobs, int n, int lag, int G, int hist, int hess = 0, int filter = 0);
+// c.model selects the instantiation (PMMH_MODEL_*, pf_model.cuh); hess: the Hessian branch (SV only); c.filter: the
+// filter alone (lag unused)
 int sv_grid_run(const SvCall& c, int nobs, int n, int lag, int G, int hess);
 }  // namespace pmmh

@@ -156,6 +156,30 @@ def flps_model_corr(model_id, obs, params, rvr, u, lag=10, store_history=False, 
     return out
 
 
+def filter_model_corr(model_id, obs, params, rvr, u, store_history=False, workspace=None):
+    """Model-generic particle filter (pmmh_filter_model_corr): log-likelihood, filtered means, trajectory and
+    diag of [B] problems without the fixed-lag smoother -- bit-identical to those outputs of flps_model_corr
+    for any lag.  Up to 4096 particles: any B (chain kernel, diag kernel 3).  Above: B == 1 and up to 7168
+    particles per SM (grid kernel, diag kernel 5).  n_obs >= 2; other sizes raise PmmhError.  ``model_id`` and
+    params as for flps_model_corr.  No fallback pass: diag[:, PMMH_DIAG_STATUS] == 1 reports an abandoned
+    evaluation."""
+    lib = _lib.load()
+    obs, obs_stride, params, rvr, u, batch, n_obs, n = _sv_common(obs, params, rvr, u)
+    dev = u.device
+    out = _sv_outputs(dev, batch, n_obs, n, smoother=False, history=store_history)
+    xh, ah = out.get("X"), out.get("A")
+    wb = ctypes.c_size_t()
+    _lib.check(lib.pmmh_filter_model_workspace_bytes(n_obs, n, batch, ctypes.byref(wb)),
+               "pmmh_filter_model_workspace_bytes")
+    ws = (workspace or Workspace()).get(wb.value, dev)
+    _lib.check(lib.pmmh_filter_model_corr(
+        int(model_id), _ptr(obs), obs_stride, _ptr(params), _ptr(rvr), _ptr(u), n_obs, n, batch,
+        _ptr(out["filt"]), _ptr(out["log_like"]), _ptr(out["traj"]), _ptr(out["diag"]), _ptr(xh), _ptr(ah),
+        _ptr(ws), ws.numel(), _stream()), "pmmh_filter_model_corr")
+    out["_workspace"] = ws
+    return out
+
+
 def flps_sv_corr_philox(obs, params, rvr, seed, philox_offset, n_particles, lag=10, workspace=None):
     """Log-likelihood + gradient of one problem whose auxiliary variables are a Philox stream
     (pmmh_flps_sv_corr_philox): any N on one device without ever storing u."""
