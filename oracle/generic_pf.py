@@ -7,9 +7,11 @@ point pmmh_flps_model_corr (csrc/pf_model.cuh); nothing under pmmh-qn_b200/ impo
 Pinning: with the SV callbacks below it must reproduce oracle_flps_sv_corr (oracle/pmmh_oracle.c, itself
 bit-exact against the compiled reference) -- tests/test_oracle_vs_golden.py checks ancestors and sorted
 generations exactly and the estimates to 1e-12 (NumPy's pairwise sums order the additions differently).
-For the linear Gaussian model there is no reference implementation: parity of that instantiation is
-pinned to this restatement only ("parity unpinned" with respect to the reference), plus the exact Kalman
-likelihood as a statistical check.
+For the linear Gaussian model (bootstrap filter, model id 1, and fully adapted filter, model id 2) there is no
+reference implementation: the device instantiations are pinned to the restatements below (ancestors exact), which
+are unpinned with respect to the reference.  The fully adapted restatement is itself checked against closed forms
+(tests/test_oracle_vs_golden.py): its proposal against the precision-weighted conditional moments, its
+likelihood estimate against the exact Kalman likelihood (statistically).
 """
 import numpy as np
 
@@ -82,6 +84,44 @@ class LinearGaussian(object):
         return np.stack([g0, g1, g2, np.zeros_like(g0)])
 
     score_tail = score_main
+
+
+class LinearGaussianFullyAdapted(object):
+    """The linear Gaussian model run as a fully adapted filter (csrc/pf_model.cuh, model id 2), operation for
+    operation: proposal p(x_t | x_{t-1}, y_t), weight p(y_{t+1} | x_t).  flps_generic runs it on the observations
+    shifted by one (obs[1:]); log_p_y1 adds the first observation's term.  No score terms (gradient rows 0)."""
+    n_params = 3
+
+    def __init__(self, params):
+        self.phi, self.sv, self.se = [float(p) for p in params[:3]]
+        s2 = self.sv * self.sv + self.se * self.se
+        self.k = (self.sv * self.sv) / s2
+        self.sdp = np.sqrt((self.sv * self.sv) * (self.se * self.se) / s2)
+        self.inv_s2 = 1.0 / s2
+        self.log_s = 0.5 * np.log(s2)
+
+    def initial_state(self):
+        return 0.0
+
+    def propagate(self, xp, y_now, u):
+        m = self.phi * xp
+        return (m + self.k * (y_now - m)) + self.sdp * u
+
+    def logw(self, x, y_next):
+        r = y_next - self.phi * x
+        return (-0.91893853320467267 - self.log_s) - (0.5 * (r * r)) * self.inv_s2
+
+    def score_main(self, curr, nxt, y):
+        return np.zeros((4,) + np.shape(curr))
+
+    score_tail = score_main
+
+
+def log_p_y1(obs, sv, se):
+    """log p(y_1 | x_0 = 0) = log N(obs[1]; 0, sv^2 + se^2): the term the fully adapted filter's estimate of
+    log p(y_2 .. y_T | y_1) lacks (x_0 = 0, so phi does not enter)."""
+    s2 = sv * sv + se * se
+    return -0.5 * np.log(2.0 * np.pi * s2) - 0.5 * float(obs[1]) ** 2 / s2
 
 
 def systematic_corr(w, rnd):

@@ -142,9 +142,11 @@ struct LinearGaussianModel {
 // drawn from p(x_t | x_{t-1}, y_t) and weighted with the predictive density p(y_{t+1} | x_t), both in closed form
 // for this model.  The kernel's algorithm is untouched: the caller hands over the observations shifted by one
 // (obs'[t] = obs[t + 1]), so `propagate` sees y_t where the SV model sees y_{t-1} (leverage) and `logw` sees
-// y_{t+1}.  The reference has no fully adapted filter (SURVEY 8a note): parity is unpinned, the check is the exact
-// Kalman likelihood.  Outputs: log-likelihood of y_2 .. y_T given y_1 (the caller adds log p(y_1)), and
-// E[x_t | y_1 .. y_{t+1}] in `filt`; the score terms are not defined for this variant (gradient rows 0).
+// y_{t+1}.  The reference has no fully adapted filter (SURVEY 8a note), so parity is unpinned with respect to it; the
+// kernels are pinned to the NumPy restatement oracle/generic_pf.py LinearGaussianFullyAdapted (ancestors exact),
+// which is checked against the conditional moments and the exact Kalman likelihood.  Outputs: log-likelihood of
+// y_2 .. y_T given y_1 (the caller adds log p(y_1)), and E[x_t | y_1 .. y_{t+1}] in `filt`; the score terms are not
+// defined for this variant (gradient rows 0).
 struct LinearGaussianFullyAdapted {
     struct Const {
         double phi, sv, se, k, sdp, inv_s2, log_s;   // gain, proposal sd, predictive variance

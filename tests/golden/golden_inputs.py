@@ -113,7 +113,8 @@ def logit_u(m, seed):
     return np.random.RandomState(seed).normal(size=m)
 
 
-LG_PARAM_SETS = [(0.8, 0.5, 0.3, 0.0), (0.95, 0.2, 1.0, 0.0), (-0.5, 1.0, 0.5, 0.0)]
+# phi = 0: the propagation mean is 0 for every parent, so the predicted child range collapses to +- nsd sd
+LG_PARAM_SETS = [(0.8, 0.5, 0.3, 0.0), (0.95, 0.2, 1.0, 0.0), (-0.5, 1.0, 0.5, 0.0), (0.0, 0.7, 0.5, 0.0)]
 
 
 def lg_obs(nobs, params=(0.8, 0.5, 0.3, 0.0), seed=4711):

@@ -4,7 +4,7 @@
 - On every shape the smoother entry also takes, log_like / filt / traj / diag (and the history X / A) are
   bit-identical to pmmh_flps_model_corr at lag 2 and at lag 10, for the three model ids.
 - Series too short for the smoother (n_obs = 2, 3, 5) against the C oracle (SV), oracle/generic_pf.py (linear
-  Gaussian) and a one-step NumPy filter built from the generic_pf model callbacks.
+  Gaussian, bootstrap and fully adapted) and a one-step NumPy filter built from the generic_pf model callbacks.
 - Refusals with their codes (the workspace query refuses the same shapes), workspace sizes, bit reproducibility.
 """
 import ctypes
@@ -134,15 +134,16 @@ def _one_step(model, obs, rvr, u1, n):
 
 @pytest.mark.parametrize("n", [256, 8192])
 @pytest.mark.parametrize("nobs", [2, 3, 5])
-@pytest.mark.parametrize("model_id", [0, 1])
+@pytest.mark.parametrize("model_id", MODELS)
 def test_short_series_against_the_oracles(cuda_dev, model_id, nobs, n):
     import generic_pf as gp
     import oracle
     from pmmh_qn_b200 import kernels as K
     if model_id == 0:
         obs, params, rvr, rvp = gi.sv_inputs(n, nobs, 3)
-    else:
-        obs, params, rvr, rvp = gi.lg_inputs(n, nobs, 3)
+    else:   # model 2 runs on the series as given (they stand for shifted observations), phi < 0
+        obs, params, rvr, rvp = gi.lg_inputs(n, nobs, 3 if model_id == 1 else 2)
+    callbacks = {0: gp.SvLeverage, 1: gp.LinearGaussian, 2: gp.LinearGaussianFullyAdapted}[model_id]
     obs_d, par_d, rvr_d, u_d = _dev(cuda_dev, obs, params, rvr[:nobs], to_time_major(rvp, n, nobs))
     out = K.filter_model_corr(model_id, obs_d, par_d, rvr_d, u_d)
     res = {k: v[0].cpu().numpy() for k, v in out.items() if not k.startswith("_")}
@@ -150,13 +151,12 @@ def test_short_series_against_the_oracles(cuda_dev, model_id, nobs, n):
     assert int(res["diag"][DIAG_STATUS]) == 0, res["diag"]
     ll = float(res["log_like"])
     if nobs == 2:
-        model = gp.SvLeverage(params) if model_id == 0 else gp.LinearGaussian(params)
-        rll, rfilt, rtraj = _one_step(model, obs, rvr, to_time_major(rvp, n, nobs)[1], n)
+        rll, rfilt, rtraj = _one_step(callbacks(params), obs, rvr, to_time_major(rvp, n, nobs)[1], n)
     else:
         if model_id == 0:
             ref = oracle.flps_sv_corr(obs, params, rvr, rvp, n, lag=2)
         else:
-            ref = gp.flps_generic(gp.LinearGaussian(params), obs, rvr, rvp, n, lag=2)
+            ref = gp.flps_generic(callbacks(params), obs, rvr, rvp, n, lag=2)
         rll, rfilt, rtraj = ref["log_like"], ref["filt"], ref["traj"]
     assert abs(ll - rll) <= 1e-10 * abs(rll), (ll, rll)
     assert relerr(res["filt"], rfilt) <= 1e-10

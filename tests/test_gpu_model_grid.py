@@ -1,7 +1,8 @@
 """pmmh_flps_model_corr beyond the chain kernel: one problem with more than 4096 particles runs on the grid kernel
 (csrc/sv_grid.cu) instantiated for the model (diag[PMMH_DIAG_KERNEL] == 5).
 
-- Linear Gaussian bootstrap filter against the NumPy restatement (oracle/generic_pf.py) from N = 5000 to 2^16:
+- Linear Gaussian bootstrap filter against the NumPy restatement (oracle/generic_pf.py) from N = 4097 to 2^16, for
+  phi > 0, phi < 0 and phi = 0 (golden_inputs.LG_PARAM_SETS by seed):
   ancestors exact, X 1e-12, log-likelihood / filt / smo 1e-10, gradient 1e-9 * ||g||_inf (the SV tolerances).
 - N = 2^20, T = 300: the same oracle with the tolerances DESIGN section 2 states at this N, and the Kalman filter.
 - The fully adapted filter at N = 2^20 against the Kalman filter and the bootstrap filter.
@@ -53,7 +54,8 @@ def _model_ws_bytes(n_obs, n, lag, batch):
 
 @pytest.mark.parametrize("n,nobs,lag,seed", [(5000, 300, 10, 0), (4097, 150, 2, 1), (1 << 14, 120, 4, 1),
                                              (20000, 80, 10, 0), (20000, 60, 2, 1), (65536, 40, 10, 1),
-                                             (65536, 50, 4, 0)])
+                                             (65536, 50, 4, 0), (5003, 80, 10, 2), (20000, 60, 2, 2),
+                                             (65536, 40, 4, 2), (4097, 100, 10, 3), (20000, 60, 2, 3)])
 def test_linear_gaussian_on_the_grid_kernel_vs_generic_oracle(cuda_dev, n, nobs, lag, seed):
     import generic_pf as gp
     from pmmh_qn_b200 import _lib, kernels as K
@@ -117,8 +119,7 @@ def test_fully_adapted_filter_at_2_20(cuda_dev):
     phi, sv, se = params[:3]
     obs = gi.lg_obs(nobs, params)
     exact = gp.kalman_loglike(obs, phi, sv, se)
-    s2 = sv * sv + se * se
-    ll_y1 = -0.5 * np.log(2.0 * np.pi * s2) - 0.5 * obs[1] ** 2 / s2          # log p(y_1 | x_0 = 0)
+    ll_y1 = gp.log_p_y1(obs, sv, se)
     obs_d, obs_s, par_d = _dev(cuda_dev, obs, obs[1:], params)                 # obs'[t] = obs[t + 1]
     fa, boot = [], []
     for r in range(B):

@@ -40,7 +40,7 @@ def test_sv_through_the_generic_entry_is_bit_identical(cuda_dev):
 
 
 @pytest.mark.parametrize("n,nobs,lag,seed", [(500, 150, 10, 0), (4096, 200, 10, 1), (1000, 100, 4, 2), (75, 361, 10, 0),
-                                             (333, 90, 2, 1)])
+                                             (333, 90, 2, 1), (1000, 100, 4, 3), (64, 60, 10, 3)])
 def test_linear_gaussian_vs_generic_oracle(cuda_dev, n, nobs, lag, seed):
     import torch
     import generic_pf as gp
@@ -95,8 +95,7 @@ def test_fully_adapted_filter_against_the_kalman_filter(cuda_dev):
     phi, sv, se = params[:3]
     obs = gi.lg_obs(nobs, params)
     exact = gp.kalman_loglike(obs, phi, sv, se)
-    s2 = sv * sv + se * se
-    ll_y1 = -0.5 * np.log(2.0 * np.pi * s2) - 0.5 * obs[1] ** 2 / s2          # log p(y_1 | x_0 = 0)
+    ll_y1 = gp.log_p_y1(obs, sv, se)
     rs = np.random.RandomState(12)
     u = rs.normal(size=(B, nobs, n))
     rvr = rs.uniform(size=(B, nobs))

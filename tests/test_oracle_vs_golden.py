@@ -135,3 +135,34 @@ def test_generic_numpy_restatement_reproduces_the_c_oracle():
             assert np.max(np.abs(got[k] - ref[k])) <= 1e-12 * np.max(np.abs(ref[k])), k
         assert abs(got["log_like"] - ref["log_like"]) <= 1e-12 * abs(ref["log_like"])
         assert np.max(np.abs(got["traj"][1:] - ref["traj"][1:])) <= 1e-12 * np.max(np.abs(ref["traj"]))
+
+
+@pytest.mark.parametrize("params", gi.LG_PARAM_SETS)
+def test_fully_adapted_proposal_is_the_conditional_law(params):
+    """generic_pf.LinearGaussianFullyAdapted (the checker of model id 2): propagate(xp, y, 0) and sdp^2 are the
+    mean and variance of x_t given x_{t-1} = xp and y_t = y, written in precision-weighted form."""
+    import generic_pf as gp
+    phi, sv, se = params[:3]
+    m = gp.LinearGaussianFullyAdapted(params)
+    rs = np.random.RandomState(5)
+    xp, y = 3.0 * rs.normal(size=1000), 3.0 * rs.normal(size=1000)
+    prec = 1.0 / sv ** 2 + 1.0 / se ** 2
+    mean = (phi * xp / sv ** 2 + y / se ** 2) / prec
+    assert np.max(np.abs(m.propagate(xp, y, 0.0) - mean)) <= 1e-14 * np.max(np.abs(mean))
+    assert abs(m.sdp ** 2 - 1.0 / prec) <= 1e-14 / prec
+
+
+@pytest.mark.parametrize("params", gi.LG_PARAM_SETS)
+def test_fully_adapted_restatement_against_the_kalman_filter(params):
+    """log p(y_1) + flps_generic's estimate of log p(y_2 .. y_T | y_1) with the fully adapted callbacks on obs[1:] is
+    the exact Kalman log-likelihood up to Monte Carlo error (N = 20000, T = 100: errors up to 0.06 were seen over
+    3 seeds per set); its gradient rows are 0."""
+    import generic_pf as gp
+    phi, sv, se = params[:3]
+    n, nobs = 20000, 101
+    obs = gi.lg_obs(nobs, params)
+    rvr, rvp = gi.split_particle(gi.sv_rvs(n, nobs - 1, 200), nobs - 1)
+    r = gp.flps_generic(gp.LinearGaussianFullyAdapted(params), obs[1:], rvr, rvp, n, 10)
+    exact = gp.kalman_loglike(obs, phi, sv, se)
+    assert abs(r["log_like"] + gp.log_p_y1(obs, sv, se) - exact) < 0.25, (r["log_like"], exact)
+    assert np.all(r["gradient"] == 0.0)
