@@ -222,6 +222,44 @@ int pmmh_filter_model_corr(int model_id, const double* d_obs, long long obs_stri
                            double* d_x_hist, int* d_a_hist, void* d_workspace, size_t workspace_bytes,
                            void* stream);
 
+/* Batches on the grid kernel: `batch` problems of one shape, each on its own team of G = ceil(n_particles / 2048)
+ * CTAs (capped at the SM count: the one-problem grid run's G, hence its tiles and its summation order), so that
+ * every output of problem b -- d_log_like, d_filt, d_smo, d_gradient, d_traj, d_hess1 / d_hess2, d_diag and the
+ * history -- is bit-identical to the grid kernel run on that problem alone (pmmh_flps_model_corr /
+ * pmmh_filter_model_corr with batch 1, and for PMMH_MODEL_SV_LEVERAGE pmmh_flps_sv_corr at algorithm 6).  The
+ * problems run in waves of nteams = min(batch, floor(SMs / G)) teams, one cooperative launch per wave, followed by
+ * the reduction and output kernels of each problem (per problem: 2 launches for the filter, 4 for the smoother, 6
+ * with the Hessian).  Each team has its own workspace slice, barrier and status word: a problem whose particle
+ * cloud degenerates is abandoned alone (d_diag[b][PMMH_DIAG_STATUS] == 1; there is no fallback pass), the others
+ * finish.  d_diag[b][PMMH_DIAG_KERNEL] == 5.
+ *   Layouts: those of pmmh_flps_model_corr / pmmh_filter_model_corr -- d_obs [n_obs] (obs_stride 0) or
+ * [batch][obs_stride], d_params [batch][4], d_rvr [batch][n_obs], d_u [batch][n_obs][n_particles]; outputs per
+ * problem d_filt, d_smo, d_traj [n_obs], d_log_like [1], d_gradient [4][n_obs], d_hess1 / d_hess2 [4][4],
+ * d_diag [PMMH_DIAG_COUNT]; optional d_x_hist / d_a_hist [batch][n_obs][n_particles], given together.
+ *   Shapes: any batch >= 1 with a tile of n_particles / G particles that fits one CTA (up to 7168 particles per
+ * CTA); the smoother needs 2 <= lag <= 10 and n_obs >= 2 lag, the filter n_obs >= 2.  compute_hessian == 1 (the
+ * SV model's Hessian branch; d_hess1 / d_hess2 required) is taken for PMMH_MODEL_SV_LEVERAGE only; with 0 the
+ * Hessian outputs may be NULL and are not written.  Anything else is refused with PMMH_ERR_INVALID, by the
+ * workspace queries too; a workspace below the query's size gives PMMH_ERR_WORKSPACE.
+ *   Workspace: min(batch, nteams) slices of the one-problem grid workspace with history (per slice:
+ * pmmh_flps_model_workspace_bytes / pmmh_filter_model_workspace_bytes at batch 1 and the same sizes; the Hessian
+ * slice is larger).
+ *   Speed (B200, T = 1000, lag 10; profiles/r6_grid_batch_T1000.jsonl): see INTEGRATION.md. */
+int pmmh_flps_model_batch_workspace_bytes(int n_obs, int n_particles, int lag, int batch, int compute_hessian,
+                                          size_t* bytes);
+int pmmh_flps_model_batch_corr(int model_id, const double* d_obs, long long obs_stride, const double* d_params,
+                               const double* d_rvr, const double* d_u, int n_obs, int n_particles, int lag, int batch,
+                               int compute_hessian, double* d_filt, double* d_smo, double* d_log_like,
+                               double* d_gradient, double* d_traj, double* d_hess1, double* d_hess2, long long* d_diag,
+                               double* d_x_hist, int* d_a_hist, void* d_workspace, size_t workspace_bytes,
+                               void* stream);
+int pmmh_filter_model_batch_workspace_bytes(int n_obs, int n_particles, int batch, size_t* bytes);
+int pmmh_filter_model_batch_corr(int model_id, const double* d_obs, long long obs_stride, const double* d_params,
+                                 const double* d_rvr, const double* d_u, int n_obs, int n_particles, int batch,
+                                 double* d_filt, double* d_log_like, double* d_traj, long long* d_diag,
+                                 double* d_x_hist, int* d_a_hist, void* d_workspace, size_t workspace_bytes,
+                                 void* stream);
+
 /* Bootstrap particle filter (filter only).  read_mode: PMMH_BPF_PARITY / PMMH_BPF_INTENDED. */
 int pmmh_bpf_sv_corr(const double* d_obs, long long obs_stride, const double* d_params,
                      const double* d_rvr, const double* d_u, int n_obs, int n_particles, int batch,

@@ -40,6 +40,13 @@ SIGNATURES = {
     "pmmh_filter_model_workspace_bytes": (c_int, [c_int, c_int, c_int, ctypes.POINTER(c_size)]),
     "pmmh_filter_model_corr": (c_int, [c_int, c_vp, c_ll, c_vp, c_vp, c_vp, c_int, c_int, c_int,
                                        c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_size, c_vp]),
+    "pmmh_flps_model_batch_workspace_bytes": (c_int, [c_int, c_int, c_int, c_int, c_int, ctypes.POINTER(c_size)]),
+    "pmmh_flps_model_batch_corr": (c_int, [c_int, c_vp, c_ll, c_vp, c_vp, c_vp, c_int, c_int, c_int, c_int, c_int,
+                                           c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_size,
+                                           c_vp]),
+    "pmmh_filter_model_batch_workspace_bytes": (c_int, [c_int, c_int, c_int, ctypes.POINTER(c_size)]),
+    "pmmh_filter_model_batch_corr": (c_int, [c_int, c_vp, c_ll, c_vp, c_vp, c_vp, c_int, c_int, c_int,
+                                             c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_size, c_vp]),
     "pmmh_sv_stage_bytes": (c_int, [c_int, c_int, ctypes.POINTER(c_size)]),
     "pmmh_sv_stream_schedule": (c_int, [c_int, c_vp, c_int]),
     "pmmh_sv_streamed_workspace_bytes": (c_int, [c_int, c_int, c_int, c_int, ctypes.POINTER(c_size)]),

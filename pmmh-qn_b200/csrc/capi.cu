@@ -781,6 +781,105 @@ int pmmh_filter_model_corr(int model_id, const double* d_obs, long long obs_stri
     return sv_launch_plan(p, s, c);
 }
 
+// ---- batches on the grid kernel: one team of sv_grid_ctas(N, SMs, 0) CTAs per problem ------------------------------
+namespace {
+// shapes the batch entries take (filter: no lag), team count and workspace; `who` names the entry in errors
+int grid_batch_plan(const char* who, int model_id, int n_obs, int n, int lag, int batch, int hess, int filter,
+                    DeviceInfo* di, int* G, int* nteams, size_t* bytes) {
+    if (model_id != PMMH_MODEL_SV_LEVERAGE && model_id != PMMH_MODEL_LINEAR_GAUSSIAN &&
+        model_id != PMMH_MODEL_LINEAR_GAUSSIAN_FA)
+        return fail(PMMH_ERR_INVALID, who);
+    if (hess && (filter || model_id != PMMH_MODEL_SV_LEVERAGE)) return fail(PMMH_ERR_INVALID, who);
+    if (batch < 1 || n_obs < 2 || (hess != 0 && hess != 1)) return fail(PMMH_ERR_INVALID, who);
+    int rc = get_device_info(di);
+    if (rc != PMMH_OK) return rc;
+    *G = pmmh::sv_grid_ctas(n, di->sm, 0);
+    if (filter ? !pmmh::sv_grid_filter_eligible(n_obs, n, *G) : !pmmh::sv_grid_eligible(n_obs, n, lag, *G))
+        return fail(PMMH_ERR_INVALID, who);
+    *nteams = pmmh::sv_grid_teams(batch, di->sm, *G);
+    *bytes = (size_t)*nteams * pmmh::sv_grid_team_ws_bytes(n_obs, n, lag, *G, hess, filter);
+    return PMMH_OK;
+}
+constexpr const char* kFlpsBatchShapes =
+    "pmmh_flps_model_batch_corr: batch >= 1, 2 <= lag <= 10, n_obs >= 2 lag, a tile of n_particles / "
+    "ceil(n_particles / 2048) particles fits one CTA, a known model id, compute_hessian only for the SV model";
+constexpr const char* kFilterBatchShapes =
+    "pmmh_filter_model_batch_corr: batch >= 1, n_obs >= 2, a tile of n_particles / ceil(n_particles / 2048) "
+    "particles fits one CTA and a known model id";
+}  // namespace
+
+int pmmh_flps_model_batch_workspace_bytes(int n_obs, int n_particles, int lag, int batch, int compute_hessian,
+                                          size_t* bytes) {
+    if (!bytes) return fail(PMMH_ERR_INVALID, "pmmh_flps_model_batch_workspace_bytes: bytes is null");
+    DeviceInfo di;
+    int G, nteams;
+    // the model is not an argument: any model takes the shape, the Hessian only the SV model
+    return grid_batch_plan(kFlpsBatchShapes, PMMH_MODEL_SV_LEVERAGE, n_obs, n_particles, lag, batch, compute_hessian, 0,
+                           &di, &G, &nteams, bytes);
+}
+
+int pmmh_flps_model_batch_corr(int model_id, const double* d_obs, long long obs_stride, const double* d_params,
+                               const double* d_rvr, const double* d_u, int n_obs, int n_particles, int lag, int batch,
+                               int compute_hessian, double* d_filt, double* d_smo, double* d_log_like,
+                               double* d_gradient, double* d_traj, double* d_hess1, double* d_hess2, long long* d_diag,
+                               double* d_x_hist, int* d_a_hist, void* d_workspace, size_t workspace_bytes,
+                               void* stream) {
+    if (!d_obs || !d_params || !d_rvr || !d_u || !d_filt || !d_smo || !d_log_like || !d_gradient || !d_traj ||
+        !d_diag || !d_workspace || (compute_hessian && (!d_hess1 || !d_hess2)))
+        return fail(PMMH_ERR_INVALID, "pmmh_flps_model_batch_corr: null pointer argument");
+    if ((d_x_hist == nullptr) != (d_a_hist == nullptr))
+        return fail(PMMH_ERR_INVALID, "d_x_hist and d_a_hist must be given together");
+    DeviceInfo di;
+    int G, nteams;
+    size_t bytes;
+    int rc = grid_batch_plan(kFlpsBatchShapes, model_id, n_obs, n_particles, lag, batch, compute_hessian, 0, &di, &G,
+                             &nteams, &bytes);
+    if (rc != PMMH_OK) return rc;
+    if (workspace_bytes < bytes) return fail(PMMH_ERR_WORKSPACE, "pmmh_flps_model_batch_corr: workspace too small");
+    rc = check_device(di, true);
+    if (rc != PMMH_OK) return rc;
+    pmmh::SvCall c = {};
+    c.obs = d_obs; c.obs_stride = obs_stride; c.params = d_params; c.rvr = d_rvr; c.u = d_u;
+    c.filt = d_filt; c.smo = d_smo; c.ll = d_log_like; c.grad = d_gradient; c.traj = d_traj; c.diag = d_diag;
+    if (compute_hessian) { c.hess1 = d_hess1; c.hess2 = d_hess2; }
+    c.x_hist = d_x_hist; c.a_hist = d_a_hist; c.model = model_id;
+    c.ws = d_workspace; c.ws_bytes = workspace_bytes; c.stream = (cudaStream_t)stream;
+    return pmmh::sv_grid_batch_run(c, batch, n_obs, n_particles, lag, G, nteams, compute_hessian);
+}
+
+int pmmh_filter_model_batch_workspace_bytes(int n_obs, int n_particles, int batch, size_t* bytes) {
+    if (!bytes) return fail(PMMH_ERR_INVALID, "pmmh_filter_model_batch_workspace_bytes: bytes is null");
+    DeviceInfo di;
+    int G, nteams;
+    return grid_batch_plan(kFilterBatchShapes, PMMH_MODEL_SV_LEVERAGE, n_obs, n_particles, 2, batch, 0, 1, &di, &G,
+                           &nteams, bytes);
+}
+
+int pmmh_filter_model_batch_corr(int model_id, const double* d_obs, long long obs_stride, const double* d_params,
+                                 const double* d_rvr, const double* d_u, int n_obs, int n_particles, int batch,
+                                 double* d_filt, double* d_log_like, double* d_traj, long long* d_diag,
+                                 double* d_x_hist, int* d_a_hist, void* d_workspace, size_t workspace_bytes,
+                                 void* stream) {
+    if (!d_obs || !d_params || !d_rvr || !d_u || !d_filt || !d_log_like || !d_traj || !d_diag || !d_workspace)
+        return fail(PMMH_ERR_INVALID, "pmmh_filter_model_batch_corr: null pointer argument");
+    if ((d_x_hist == nullptr) != (d_a_hist == nullptr))
+        return fail(PMMH_ERR_INVALID, "d_x_hist and d_a_hist must be given together");
+    DeviceInfo di;
+    int G, nteams;
+    size_t bytes;
+    int rc = grid_batch_plan(kFilterBatchShapes, model_id, n_obs, n_particles, 2, batch, 0, 1, &di, &G, &nteams, &bytes);
+    if (rc != PMMH_OK) return rc;
+    if (workspace_bytes < bytes) return fail(PMMH_ERR_WORKSPACE, "pmmh_filter_model_batch_corr: workspace too small");
+    rc = check_device(di, true);
+    if (rc != PMMH_OK) return rc;
+    pmmh::SvCall c = {};
+    c.obs = d_obs; c.obs_stride = obs_stride; c.params = d_params; c.rvr = d_rvr; c.u = d_u;
+    c.filt = d_filt; c.ll = d_log_like; c.traj = d_traj; c.diag = d_diag;
+    c.x_hist = d_x_hist; c.a_hist = d_a_hist; c.model = model_id; c.filter = 1;
+    c.ws = d_workspace; c.ws_bytes = workspace_bytes; c.stream = (cudaStream_t)stream;
+    return pmmh::sv_grid_batch_run(c, batch, n_obs, n_particles, 2, G, nteams, 0);
+}
+
 int pmmh_bpf_sv_corr(const double* d_obs, long long obs_stride, const double* d_params,
                      const double* d_rvr, const double* d_u, int n_obs, int n_particles, int batch,
                      int read_mode, double* d_filt, double* d_log_like, double* d_traj,

@@ -51,6 +51,11 @@
 //   * template over the model (pf_model.cuh): SvLeverageModel is everything above; another model runs the generic path
 //     in the same body (XE = (x, propagation mean of the children), payload = (parent value, -, -, value), score terms
 //     M::score_main / M::score_tail), gradient only (DESIGN 4.0).
+//   * TEAM = true (pmmh_flps_model_batch_corr / pmmh_filter_model_batch_corr): a batch of problems, one team of G CTAs
+//     per problem -- CTA b runs tile b % G of problem b / G on that team's own slice of the workspace (the one-problem
+//     layout: own barrier counter, abandon bit and status word), so every problem is bit-identical to its one-problem
+//     run and an abandoned problem stops its team only; waves of floor(SMs / G) teams, one cooperative launch each.
+//     TEAM = false compiles to the same SASS as before the team kernels existed (tools/sass_diff.py).
 //   * SMO = false: the particle filter alone (pmmh_filter_model_corr) -- no payloads, no genealogy records, no score
 //     terms, no tail; the workspace has no R / P tables and no weight ring.  The birth rows stay: the in-bin ranking
 //     breaks ties on them.
@@ -383,6 +388,48 @@ __device__ __forceinline__ void deferred_alpha_pass(const GridArgs& a, const SvC
     }
 }
 
+// Teams: CTA b runs tile b % G of problem (team) b / G.  a_in addresses team 0; team k's workspace slice starts
+// ws_stride bytes after team k-1's (the one-problem layout, so every team has its own barrier counter, abandon bit
+// and status word), its inputs and history one problem further on (obs by obs_stride doubles)
+struct GridTeam {
+    long long ws_stride;
+    long long obs_stride;
+};
+template <class T>
+__device__ __forceinline__ T* team_ptr(T* p, long long bytes) {
+    return (T*)((char*)p + bytes);
+}
+__device__ __forceinline__ GridArgs team_args(const GridArgs& a0, const GridTeam& tm) {
+    const int team = blockIdx.x / a0.G;
+    const long long w = tm.ws_stride * team, nu = (long long)a0.NOBS * a0.N * team;
+    GridArgs a = a0;
+    a.obs += tm.obs_stride * team;
+    a.params += 4 * team;
+    a.rvr += (long long)a0.NOBS * team;
+    a.U += nu;
+    a.ctrl = team_ptr(a0.ctrl, w);
+    a.ghist = team_ptr(a0.ghist, w);
+    a.tilecnt = team_ptr(a0.tilecnt, w);
+    a.tinfo = team_ptr(a0.tinfo, w);
+    a.H = team_ptr(a0.H, w);
+    a.XE = team_ptr(a0.XE, w);
+    a.perm = team_ptr(a0.perm, w);
+    a.R = team_ptr(a0.R, w);
+    a.P = team_ptr(a0.P, w);
+    a.psum = team_ptr(a0.psum, w);
+    a.xlow = team_ptr(a0.xlow, w);
+    a.psumH = team_ptr(a0.psumH, w);
+    a.shiftv = team_ptr(a0.shiftv, w);
+    a.xminv = team_ptr(a0.xminv, w);
+    a.shring = team_ptr(a0.shring, w);
+    a.parentpos = team_ptr(a0.parentpos, w);
+    if (a0.hist) {
+        a.Xhist += nu;
+        a.Ahist += nu;
+    }
+    return a;
+}
+
 // ---------------------------------------------------------------------------------------------
 // the kernel
 // ---------------------------------------------------------------------------------------------
@@ -391,8 +438,12 @@ __device__ __forceinline__ void deferred_alpha_pass(const GridArgs& a, const SvC
 // runs the generic path: the second double of XE is the propagation mean prop_mean(x, obs[t]) of the
 // children, a payload is (parent value, -, -, own value) and the score terms are M::score_main of the pair.
 // SMO: the fixed-lag smoother; false: the filter alone, whose outputs are bit-identical to the smoother's.
-template <int GT, bool HESS, class M, bool SMO>
-__global__ void __launch_bounds__(GT, 1) sv_grid_kernel(const GridArgs a) {
+// TEAM: teams of a_in.G CTAs, one per problem (GridTeam below); false: one problem on a_in.G CTAs.
+template <int GT, bool HESS, class M, bool SMO, bool TEAM>
+__global__ void __launch_bounds__(GT, 1) sv_grid_kernel(const GridArgs a_in, const GridTeam tm) {
+    GridArgs a_team;
+    if constexpr (TEAM) a_team = team_args(a_in, tm);
+    const GridArgs& a = TEAM ? a_team : a_in;   // this CTA's problem
     constexpr bool GEN = !std::is_same<M, SvLeverageModel>::value;
     static_assert(!(GEN && HESS), "the Hessian branch exists for the SV model only");
     static_assert(SMO || !HESS, "the Hessian branch needs the smoother");
@@ -435,7 +486,7 @@ __global__ void __launch_bounds__(GT, 1) sv_grid_kernel(const GridArgs a) {
     __shared__ int s_ndef;   // Hessian branch: length of the list of deferred alpha terms
 
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-    const int c = blockIdx.x, G = a.G, N = a.N, NOBS = a.NOBS, L = a.LAG, Wc = a.Wc, RP = a.RP;
+    const int c = TEAM ? (int)(blockIdx.x % (unsigned)a.G) : blockIdx.x, G = a.G, N = a.N, NOBS = a.NOBS, L = a.LAG, Wc = a.Wc, RP = a.RP;
     GridCtrl* ctrl = a.ctrl;
     const double dn = (double)N, inv_n = 1.0 / dn;
     const bool pow2 = (N & (N - 1)) == 0;
@@ -1861,47 +1912,55 @@ GridLayout grid_layout(int nobs, int n, int lag, int G, int hist, int hess, int 
         if (e__ != cudaSuccess) return pmmh::set_cuda_error(e__, #call); \
     } while (0)
 
-}  // namespace
-
-int sv_grid_ctas(int n, int sm_count, int ctas) {
-    int G = ctas > 0 ? ctas : (n + 2047) / 2048;
-    if (G > sm_count) G = sm_count;
-    if (G > kMaxTiles) G = kMaxTiles;
-    if (G < 1) G = 1;
-    return G;
+template <bool HESS, class M, bool SMO>
+const void* grid_kernel_of(bool team) {
+    return team ? (const void*)sv_grid_kernel<1024, HESS, M, SMO, true> : (const void*)sv_grid_kernel<1024, HESS, M, SMO, false>;
+}
+// the persistent kernel of (model, hess, filter): one problem, or teams of CTAs
+const void* grid_kernel_for(int model, int hess, int filter, bool team) {
+    if (filter) {
+        if (model == PMMH_MODEL_LINEAR_GAUSSIAN) return grid_kernel_of<false, LinearGaussianModel, false>(team);
+        if (model == PMMH_MODEL_LINEAR_GAUSSIAN_FA) return grid_kernel_of<false, LinearGaussianFullyAdapted, false>(team);
+        return grid_kernel_of<false, SvLeverageModel, false>(team);
+    }
+    if (model == PMMH_MODEL_LINEAR_GAUSSIAN) return grid_kernel_of<false, LinearGaussianModel, true>(team);
+    if (model == PMMH_MODEL_LINEAR_GAUSSIAN_FA) return grid_kernel_of<false, LinearGaussianFullyAdapted, true>(team);
+    return hess ? grid_kernel_of<true, SvLeverageModel, true>(team) : grid_kernel_of<false, SvLeverageModel, true>(team);
 }
 
-// a tile holds N/G particles +- one histogram bin; 12 % head room below the shared-memory capacity
-static bool grid_tile_fits(int n, int G) {
-    if (G < 1 || G > kMaxTiles || n < 32 || n > (1 << 21)) return false;
-    const int Wc = (n + G - 1) / G;
-    return Wc <= kCap - kCap / 8;
-}
-
-bool sv_grid_eligible(int nobs, int n, int lag, int G) {
-    return lag >= 2 && lag <= 10 && nobs >= 2 * lag && grid_tile_fits(n, G);
-}
-
-bool sv_grid_filter_eligible(int nobs, int n, int G) { return nobs >= 2 && grid_tile_fits(n, G); }
-
-size_t sv_grid_ws_bytes(int nobs, int n, int lag, int G, int hist, int hess, int filter) {
-    return grid_layout(nobs, n, lag, G, hist, hess, filter).total;
-}
-
-int sv_grid_run(const SvCall& c, int nobs, int n, int lag, int G, int hess) {
-    const int filter = c.filter;
-    if (filter ? (hess || !sv_grid_filter_eligible(nobs, n, G)) : !sv_grid_eligible(nobs, n, lag, G))
+int grid_check(const SvCall& c, int nobs, int n, int lag, int G, int hess) {
+    if (c.filter ? (hess || !sv_grid_filter_eligible(nobs, n, G)) : !sv_grid_eligible(nobs, n, lag, G))
         return set_error(PMMH_ERR_INVALID, "grid kernel: sizes not eligible");
-    const int hist = c.x_hist != nullptr;
     const int model = c.model;
     if (model != PMMH_MODEL_SV_LEVERAGE && model != PMMH_MODEL_LINEAR_GAUSSIAN && model != PMMH_MODEL_LINEAR_GAUSSIAN_FA)
         return set_error(PMMH_ERR_INVALID, "grid kernel: unknown model id");
     if (hess && model != PMMH_MODEL_SV_LEVERAGE)
         return set_error(PMMH_ERR_INVALID, "grid kernel: the Hessian branch exists for the SV model only");
-    const GridLayout L = grid_layout(nobs, n, lag, G, hist, hess, filter);
-    if (c.ws_bytes < L.total) return set_error(PMMH_ERR_WORKSPACE, "grid kernel: workspace too small");
-    char* ws = (char*)c.ws;
-    const cudaStream_t st = c.stream;
+    return PMMH_OK;
+}
+
+// dynamic shared memory of every persistent kernel, once per device and host thread
+int grid_set_attributes() {
+    static thread_local bool attr_set[64] = {false};
+    int dev = 0;
+    GRID_CUDA(cudaGetDevice(&dev));
+    if (dev >= 0 && dev < 64 && !attr_set[dev]) {
+        // no persisting L2 set-aside for the kernel's evict_last accesses: with one every phase is slower
+        // (DESIGN 4.0), and left unset the evaluation at N = 2^20 is ~6 % slower
+        GRID_CUDA(cudaDeviceSetLimit(cudaLimitPersistingL2CacheSize, 0));
+        for (int team = 0; team < 2; ++team)
+            for (int model = 0; model < 3; ++model)
+                for (int v = 0; v < 3; ++v)   // smoother, smoother with Hessian (SV only), filter
+                    if (v != 1 || model == PMMH_MODEL_SV_LEVERAGE)
+                        GRID_CUDA(cudaFuncSetAttribute(grid_kernel_for(model, v == 1, v == 2, team != 0),
+                                                       cudaFuncAttributeMaxDynamicSharedMemorySize, kDynSmem));
+        attr_set[dev] = true;
+    }
+    return PMMH_OK;
+}
+
+// arguments of the problem `c` describes, its workspace slice (layout L) at ws
+GridArgs grid_args(const SvCall& c, const GridLayout& L, char* ws, int nobs, int n, int lag, int G, int hess) {
     GridArgs a;
     memset(&a, 0, sizeof(a));
     a.N = n;
@@ -1910,7 +1969,7 @@ int sv_grid_run(const SvCall& c, int nobs, int n, int lag, int G, int hess) {
     a.G = G;
     a.Wc = (n + G - 1) / G;
     a.RP = L.RP;
-    a.hist = hist;
+    a.hist = c.x_hist != nullptr;
     a.obs = c.obs;
     a.params = c.params;
     a.rvr = c.rvr;
@@ -1954,44 +2013,20 @@ int sv_grid_run(const SvCall& c, int nobs, int n, int lag, int G, int hess) {
         const char* e = getenv("PMMH_GRID_DEBUG");
         a.dbg = e ? atoi(e) : 0;
     }
-    // control block, histograms, reservation counters, tile info: zero
-    GRID_CUDA(cudaMemsetAsync(ws + L.ctrl, 0, L.H - L.ctrl, st));
-    static thread_local bool attr_set[64] = {false};
-    int dev = 0;
-    GRID_CUDA(cudaGetDevice(&dev));
-    if (dev >= 0 && dev < 64 && !attr_set[dev]) {
-        // no persisting L2 set-aside for the kernel's evict_last accesses: with one every phase is slower
-        // (DESIGN 4.0), and left unset the evaluation at N = 2^20 is ~6 % slower
-        GRID_CUDA(cudaDeviceSetLimit(cudaLimitPersistingL2CacheSize, 0));
-        const void* kernels[] = {(const void*)sv_grid_kernel<1024, false, SvLeverageModel, true>,
-                                 (const void*)sv_grid_kernel<1024, true, SvLeverageModel, true>,
-                                 (const void*)sv_grid_kernel<1024, false, LinearGaussianModel, true>,
-                                 (const void*)sv_grid_kernel<1024, false, LinearGaussianFullyAdapted, true>,
-                                 (const void*)sv_grid_kernel<1024, false, SvLeverageModel, false>,
-                                 (const void*)sv_grid_kernel<1024, false, LinearGaussianModel, false>,
-                                 (const void*)sv_grid_kernel<1024, false, LinearGaussianFullyAdapted, false>};
-        for (const void* k : kernels)
-            GRID_CUDA(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, kDynSmem));
-        attr_set[dev] = true;
-    }
-    void* kargs[] = {(void*)&a};
-    const void* kern;
-    if (filter) {
-        kern = (const void*)sv_grid_kernel<1024, false, SvLeverageModel, false>;
-        if (model == PMMH_MODEL_LINEAR_GAUSSIAN) kern = (const void*)sv_grid_kernel<1024, false, LinearGaussianModel, false>;
-        if (model == PMMH_MODEL_LINEAR_GAUSSIAN_FA) kern = (const void*)sv_grid_kernel<1024, false, LinearGaussianFullyAdapted, false>;
-    } else {
-        kern = hess ? (const void*)sv_grid_kernel<1024, true, SvLeverageModel, true>
-                    : (const void*)sv_grid_kernel<1024, false, SvLeverageModel, true>;
-        if (model == PMMH_MODEL_LINEAR_GAUSSIAN) kern = (const void*)sv_grid_kernel<1024, false, LinearGaussianModel, true>;
-        if (model == PMMH_MODEL_LINEAR_GAUSSIAN_FA) kern = (const void*)sv_grid_kernel<1024, false, LinearGaussianFullyAdapted, true>;
-    }
-    GRID_CUDA(cudaLaunchCooperativeKernel(kern, dim3(G), dim3(1024), kargs, kDynSmem, st));
+    return a;
+}
+
+// the kernels after the persistent one (reductions, tail, output assembly) for the problem `c` / `a` describe:
+// 2 launches (filter), 4 (smoother), 6 (smoother with the Hessian branch)
+int grid_after(const SvCall& c, const GridArgs& a, const GridLayout& L, char* ws, int nobs, int n, int lag, int G,
+               int hess) {
+    const cudaStream_t st = c.stream;
+    const int model = c.model;
     double* sums = (double*)(ws + L.sums);
     double* tailpart = (double*)(ws + L.tailpart);
     double* tail = (double*)(ws + L.tail);
     grid_reduce_kernel<<<nobs, 256, 0, st>>>(a.psum, G, sums);
-    if (filter) {
+    if (c.filter) {
         auto finish = model == PMMH_MODEL_SV_LEVERAGE ? grid_finish_kernel<false, false> : grid_finish_kernel<true, false>;
         finish<<<(nobs + 255) / 256, 256, 0, st>>>(a.ctrl, sums, a.shiftv, a.xminv, nullptr, c.params, nobs, lag, (double)n,
                                                    c.ll, c.filt, nullptr, nullptr, c.traj, c.diag, (long long*)(ws + L.info));
@@ -2016,6 +2051,116 @@ int sv_grid_run(const SvCall& c, int nobs, int n, int lag, int G, int hess) {
     finish<<<(nobs + 255) / 256, 256, 0, st>>>(a.ctrl, sums, a.shiftv, a.xminv, tail, c.params, nobs, lag, (double)n, c.ll,
                                                c.filt, c.smo, c.grad, c.traj, c.diag, (long long*)(ws + L.info));
     GRID_CUDA(cudaGetLastError());
+    return PMMH_OK;
+}
+
+// problem b of a batch call: its inputs, outputs and history
+SvCall grid_problem(const SvCall& c, int b, int nobs, int n) {
+    SvCall p = c;
+    const size_t bn = (size_t)b * nobs;
+    p.obs = c.obs + b * c.obs_stride;
+    p.params = c.params + 4 * (size_t)b;
+    p.rvr = c.rvr + bn;
+    p.u = c.u + bn * n;
+    p.filt = c.filt + bn;
+    if (c.smo) p.smo = c.smo + bn;
+    p.ll = c.ll + b;
+    if (c.grad) p.grad = c.grad + 4 * bn;
+    p.traj = c.traj + bn;
+    if (c.hess1) p.hess1 = c.hess1 + 16 * (size_t)b;
+    if (c.hess2) p.hess2 = c.hess2 + 16 * (size_t)b;
+    p.diag = c.diag + (size_t)b * PMMH_DIAG_COUNT;
+    if (c.x_hist) p.x_hist = c.x_hist + bn * n;
+    if (c.a_hist) p.a_hist = c.a_hist + bn * n;
+    return p;
+}
+
+}  // namespace
+
+int sv_grid_ctas(int n, int sm_count, int ctas) {
+    int G = ctas > 0 ? ctas : (n + 2047) / 2048;
+    if (G > sm_count) G = sm_count;
+    if (G > kMaxTiles) G = kMaxTiles;
+    if (G < 1) G = 1;
+    return G;
+}
+
+// a tile holds N/G particles +- one histogram bin; 12 % head room below the shared-memory capacity
+static bool grid_tile_fits(int n, int G) {
+    if (G < 1 || G > kMaxTiles || n < 32 || n > (1 << 21)) return false;
+    const int Wc = (n + G - 1) / G;
+    return Wc <= kCap - kCap / 8;
+}
+
+bool sv_grid_eligible(int nobs, int n, int lag, int G) {
+    return lag >= 2 && lag <= 10 && nobs >= 2 * lag && grid_tile_fits(n, G);
+}
+
+bool sv_grid_filter_eligible(int nobs, int n, int G) { return nobs >= 2 && grid_tile_fits(n, G); }
+
+size_t sv_grid_ws_bytes(int nobs, int n, int lag, int G, int hist, int hess, int filter) {
+    return grid_layout(nobs, n, lag, G, hist, hess, filter).total;
+}
+
+int sv_grid_teams(int batch, int sm_count, int G) {
+    int t = G > 0 ? sm_count / G : 0;
+    if (t > batch) t = batch;
+    return t < 1 ? 1 : t;
+}
+
+int sv_grid_run(const SvCall& c, int nobs, int n, int lag, int G, int hess) {
+    int rc = grid_check(c, nobs, n, lag, G, hess);
+    if (rc != PMMH_OK) return rc;
+    const GridLayout L = grid_layout(nobs, n, lag, G, c.x_hist != nullptr, hess, c.filter);
+    if (c.ws_bytes < L.total) return set_error(PMMH_ERR_WORKSPACE, "grid kernel: workspace too small");
+    char* ws = (char*)c.ws;
+    const cudaStream_t st = c.stream;
+    GridArgs a = grid_args(c, L, ws, nobs, n, lag, G, hess);
+    // control block, histograms, reservation counters, tile info: zero
+    GRID_CUDA(cudaMemsetAsync(ws + L.ctrl, 0, L.H - L.ctrl, st));
+    rc = grid_set_attributes();
+    if (rc != PMMH_OK) return rc;
+    GridTeam tm = {0, 0};   // (unused)
+    void* kargs[] = {(void*)&a, (void*)&tm};
+    GRID_CUDA(cudaLaunchCooperativeKernel(grid_kernel_for(c.model, hess, c.filter, false), dim3(G), dim3(1024), kargs,
+                                          kDynSmem, st));
+    return grid_after(c, a, L, ws, nobs, n, lag, G, hess);
+}
+
+size_t sv_grid_team_ws_bytes(int nobs, int n, int lag, int G, int hess, int filter) {
+    return grid_layout(nobs, n, lag, G, 1, hess, filter).total;
+}
+
+int sv_grid_batch_run(const SvCall& c, int batch, int nobs, int n, int lag, int G, int nteams, int hess) {
+    int rc = grid_check(c, nobs, n, lag, G, hess);
+    if (rc != PMMH_OK) return rc;
+    if (batch < 1 || nteams < 1) return set_error(PMMH_ERR_INVALID, "grid kernel: bad team count");
+    if (c.slot > 0 || c.prof) return set_error(PMMH_ERR_INVALID, "grid kernel: teams take device-resident u only");
+    const GridLayout L = grid_layout(nobs, n, lag, G, 1, hess, c.filter);
+    const int slices = batch < nteams ? batch : nteams;
+    if (c.ws_bytes < (size_t)slices * L.total) return set_error(PMMH_ERR_WORKSPACE, "grid kernel: workspace too small");
+    char* ws = (char*)c.ws;
+    const cudaStream_t st = c.stream;
+    rc = grid_set_attributes();
+    if (rc != PMMH_OK) return rc;
+    const void* kern = grid_kernel_for(c.model, hess, c.filter, true);
+    for (int b0 = 0; b0 < batch; b0 += nteams) {
+        const int nw = batch - b0 < nteams ? batch - b0 : nteams;   // problems (teams) of this wave
+        for (int k = 0; k < nw; ++k)
+            GRID_CUDA(cudaMemsetAsync(ws + (size_t)k * L.total + L.ctrl, 0, L.H - L.ctrl, st));
+        GridArgs a = grid_args(grid_problem(c, b0, nobs, n), L, ws, nobs, n, lag, G, hess);
+        GridTeam tm;
+        tm.ws_stride = (long long)L.total;
+        tm.obs_stride = c.obs_stride;
+        void* kargs[] = {(void*)&a, (void*)&tm};
+        GRID_CUDA(cudaLaunchCooperativeKernel(kern, dim3(nw * G), dim3(1024), kargs, kDynSmem, st));
+        for (int k = 0; k < nw; ++k) {
+            char* wk = ws + (size_t)k * L.total;
+            const SvCall pc = grid_problem(c, b0 + k, nobs, n);
+            rc = grid_after(pc, grid_args(pc, L, wk, nobs, n, lag, G, hess), L, wk, nobs, n, lag, G, hess);
+            if (rc != PMMH_OK) return rc;
+        }
+    }
     return PMMH_OK;
 }
 

@@ -180,6 +180,68 @@ def filter_model_corr(model_id, obs, params, rvr, u, store_history=False, worksp
     return out
 
 
+def flps_model_batch_workspace_bytes(n_obs, n_particles, lag, batch, compute_hessian=0):
+    lib = _lib.load()
+    wb = ctypes.c_size_t()
+    _lib.check(lib.pmmh_flps_model_batch_workspace_bytes(n_obs, n_particles, lag, batch, int(bool(compute_hessian)),
+                                                         ctypes.byref(wb)), "pmmh_flps_model_batch_workspace_bytes")
+    return wb.value
+
+
+def filter_model_batch_workspace_bytes(n_obs, n_particles, batch):
+    lib = _lib.load()
+    wb = ctypes.c_size_t()
+    _lib.check(lib.pmmh_filter_model_batch_workspace_bytes(n_obs, n_particles, batch, ctypes.byref(wb)),
+               "pmmh_filter_model_batch_workspace_bytes")
+    return wb.value
+
+
+def flps_model_batch_corr(model_id, obs, params, rvr, u, lag=10, compute_hessian=0, store_history=False,
+                          workspace=None):
+    """Batch of [B] problems on the grid kernel, one team of CTAs per problem (pmmh_flps_model_batch_corr): the
+    outputs of problem b are bit-identical to flps_model_corr on that problem alone with B == 1 (and, for
+    _lib.MODEL_SV_LEVERAGE, to flps_sv_corr on the grid kernel, also with the Hessian).  Any B on every shape the
+    one-problem grid run takes (above 4096 particles: n_obs >= 2 lag, up to 7168 particles per CTA of
+    ceil(N / 2048)); compute_hessian for the SV model only.  Returns the dict of flps_model_corr, plus hess1 /
+    hess2 [B, 4, 4] with compute_hessian.  No fallback pass: diag[:, PMMH_DIAG_STATUS] == 1 reports an abandoned
+    problem, the others are unaffected."""
+    lib = _lib.load()
+    obs, obs_stride, params, rvr, u, batch, n_obs, n = _sv_common(obs, params, rvr, u)
+    dev = u.device
+    hess = int(bool(compute_hessian))
+    out = _sv_outputs(dev, batch, n_obs, n, hessian=bool(hess), history=store_history)
+    xh, ah = out.get("X"), out.get("A")
+    nbytes = flps_model_batch_workspace_bytes(n_obs, n, lag, batch, hess)
+    ws = (workspace or Workspace()).get(nbytes, dev)
+    _lib.check(lib.pmmh_flps_model_batch_corr(
+        int(model_id), _ptr(obs), obs_stride, _ptr(params), _ptr(rvr), _ptr(u), n_obs, n, lag, batch, hess,
+        _ptr(out["filt"]), _ptr(out["smo"]), _ptr(out["log_like"]), _ptr(out["gradient"]), _ptr(out["traj"]),
+        _ptr(out.get("hess1")), _ptr(out.get("hess2")), _ptr(out["diag"]), _ptr(xh), _ptr(ah), _ptr(ws), ws.numel(),
+        _stream()), "pmmh_flps_model_batch_corr")
+    out["_workspace"] = ws
+    return out
+
+
+def filter_model_batch_corr(model_id, obs, params, rvr, u, store_history=False, workspace=None):
+    """Batch of [B] particle filters on the grid kernel, one team of CTAs per problem
+    (pmmh_filter_model_batch_corr): the outputs of problem b are bit-identical to filter_model_corr on that problem
+    alone (and to those outputs of flps_model_batch_corr).  Any B where a tile of the one-problem grid run fits one
+    CTA, n_obs >= 2.  Returns the dict of filter_model_corr."""
+    lib = _lib.load()
+    obs, obs_stride, params, rvr, u, batch, n_obs, n = _sv_common(obs, params, rvr, u)
+    dev = u.device
+    out = _sv_outputs(dev, batch, n_obs, n, smoother=False, history=store_history)
+    xh, ah = out.get("X"), out.get("A")
+    nbytes = filter_model_batch_workspace_bytes(n_obs, n, batch)
+    ws = (workspace or Workspace()).get(nbytes, dev)
+    _lib.check(lib.pmmh_filter_model_batch_corr(
+        int(model_id), _ptr(obs), obs_stride, _ptr(params), _ptr(rvr), _ptr(u), n_obs, n, batch,
+        _ptr(out["filt"]), _ptr(out["log_like"]), _ptr(out["traj"]), _ptr(out["diag"]), _ptr(xh), _ptr(ah),
+        _ptr(ws), ws.numel(), _stream()), "pmmh_filter_model_batch_corr")
+    out["_workspace"] = ws
+    return out
+
+
 def flps_sv_corr_philox(obs, params, rvr, seed, philox_offset, n_particles, lag=10, workspace=None):
     """Log-likelihood + gradient of one problem whose auxiliary variables are a Philox stream
     (pmmh_flps_sv_corr_philox): any N on one device without ever storing u."""
