@@ -306,7 +306,7 @@ int sv_launch_plan(const SvPlan& p, const SvShape& s, const pmmh::SvCall& c) {
         PMMH_CUDA(pmmh::sv_chain_launch(a, p.grid, c.filter, c.stream));
         break;
     case SvKernel::Grid:
-        rc = pmmh::sv_grid_run(c, s.nobs, s.n, s.lag, p.c.grid_G, s.hess);
+        rc = pmmh::sv_grid_run(c, 1, s.nobs, s.n, s.lag, p.c.grid_G, 1, s.hess);
         zero_hess = !s.hess;
         break;
     case SvKernel::StreamRecords:
@@ -797,7 +797,7 @@ int grid_batch_plan(const char* who, int model_id, int n_obs, int n, int lag, in
     if (filter ? !pmmh::sv_grid_filter_eligible(n_obs, n, *G) : !pmmh::sv_grid_eligible(n_obs, n, lag, *G))
         return fail(PMMH_ERR_INVALID, who);
     *nteams = pmmh::sv_grid_teams(batch, di->sm, *G);
-    *bytes = (size_t)*nteams * pmmh::sv_grid_team_ws_bytes(n_obs, n, lag, *G, hess, filter);
+    *bytes = (size_t)*nteams * pmmh::sv_grid_ws_bytes(n_obs, n, lag, *G, 1, hess, filter);
     return PMMH_OK;
 }
 constexpr const char* kFlpsBatchShapes =
@@ -844,7 +844,7 @@ int pmmh_flps_model_batch_corr(int model_id, const double* d_obs, long long obs_
     if (compute_hessian) { c.hess1 = d_hess1; c.hess2 = d_hess2; }
     c.x_hist = d_x_hist; c.a_hist = d_a_hist; c.model = model_id;
     c.ws = d_workspace; c.ws_bytes = workspace_bytes; c.stream = (cudaStream_t)stream;
-    return pmmh::sv_grid_batch_run(c, batch, n_obs, n_particles, lag, G, nteams, compute_hessian);
+    return pmmh::sv_grid_run(c, batch, n_obs, n_particles, lag, G, nteams, compute_hessian);
 }
 
 int pmmh_filter_model_batch_workspace_bytes(int n_obs, int n_particles, int batch, size_t* bytes) {
@@ -877,7 +877,7 @@ int pmmh_filter_model_batch_corr(int model_id, const double* d_obs, long long ob
     c.filt = d_filt; c.ll = d_log_like; c.traj = d_traj; c.diag = d_diag;
     c.x_hist = d_x_hist; c.a_hist = d_a_hist; c.model = model_id; c.filter = 1;
     c.ws = d_workspace; c.ws_bytes = workspace_bytes; c.stream = (cudaStream_t)stream;
-    return pmmh::sv_grid_batch_run(c, batch, n_obs, n_particles, 2, G, nteams, 0);
+    return pmmh::sv_grid_run(c, batch, n_obs, n_particles, 2, G, nteams, 0);
 }
 
 int pmmh_bpf_sv_corr(const double* d_obs, long long obs_stride, const double* d_params,

@@ -55,7 +55,7 @@
 //     per problem -- CTA b runs tile b % G of problem b / G on that team's own slice of the workspace (the one-problem
 //     layout: own barrier counter, abandon bit and status word), so every problem is bit-identical to its one-problem
 //     run and an abandoned problem stops its team only; waves of floor(SMs / G) teams, one cooperative launch each.
-//     TEAM = false compiles to the same SASS as before the team kernels existed (tools/sass_diff.py).
+//     A wave of one problem (and a one-problem call, a batch of one) runs TEAM = false.
 //   * SMO = false: the particle filter alone (pmmh_filter_model_corr) -- no payloads, no genealogy records, no score
 //     terms, no tail; the workspace has no R / P tables and no weight ring.  The birth rows stay: the in-bin ranking
 //     breaks ties on them.
@@ -69,7 +69,6 @@
 #include <cuda_runtime.h>
 #include <math.h>
 #include <stdint.h>
-#include <stdlib.h>
 #include <string.h>
 
 #include <type_traits>
@@ -89,7 +88,6 @@ namespace {
 
 constexpr int kCap = 8192;         // entries of one tile (shared-memory capacity)
 constexpr int kNF = 8192;          // bins of the global value histogram
-constexpr int kNCopy = 1;          // striped copies of the global histogram (CTA c adds into copy c % kNCopy)
 constexpr int kNSB = 4096;         // sub-bins of the in-tile counting sort
 constexpr int kMaxSub = 1024;      // a sub-bin larger than this abandons the evaluation
 constexpr int kMaxTiles = 160;     // >= SM count
@@ -121,7 +119,9 @@ struct GridCtrl {
 
 struct GridArgs {
     int N, NOBS, LAG, G, Wc, RP, hist;
-    int dbg;   // development (timing only, results wrong): 1 skip R records, 2 skip P store, 4 skip score gather, 8 bulk prefetch of the lagged generation, 64 no L2 eviction hints
+    // always 0 (grid_args).  The kernel's tests of it are dead, but deleting them changes register allocation and
+    // measured slower (B200, 1000 W: 94.1 -> 96.9 ms per evaluation at N = 2^20, T = 1000, lag 10)
+    int dbg;
     const double *obs, *params, *rvr, *U;
     // U[t][j] = U[(t / u_cs) * u_cstride + (t % u_cs) * u_tstride + j * u_jstride]: time-major resident array
     // (u_cs = 2^30, u_tstride = N, u_jstride = 1) or particle-major chunks of u_cs time steps as the copy
@@ -131,7 +131,7 @@ struct GridArgs {
     const int* u_flag;   // host-streamed u: number of time rows that have landed (written by the copy engine)
     double* ustash;      // [4][N] host-streamed u: the four time steps of one 32-byte sector per particle, time-major
     GridCtrl* ctrl;
-    int* ghist;        // [2][kNCopy][kNF]
+    int* ghist;        // [2][kNF]
     int* tilecnt;      // [2][kMaxTiles * kCntStride]
     double* tinfo;     // [kMaxTiles][4]  tot, n, sum sh m, sum sh m^2
     int* H;            // [N] ancestor (sorted position) of every child
@@ -197,11 +197,8 @@ __device__ __forceinline__ unsigned long long policy_evict_last() {
     asm volatile("createpolicy.fractional.L2::evict_last.b64 %0, 1.0;" : "=l"(pol));
     return pol;
 }
-__device__ __forceinline__ void prefetch_l2(const void* p) {
-    asm volatile("prefetch.global.L2 [%0];" ::"l"(p));
-}
-// 32-byte genealogy records: one 256-bit access, kept in the persisting part of L2 (evict_last; the
-// host sets cudaLimitPersistingL2CacheSize to the size of the two record tables)
+// 32-byte genealogy records: one 256-bit access with an L2 eviction hint (no persisting L2 set-aside: see
+// grid_set_attributes)
 __device__ __forceinline__ void ld_rec(const REntry* p, unsigned long long pol, int (&r)[8]) {
     asm volatile("ld.global.cg.L2::cache_hint.v8.s32 {%0,%1,%2,%3,%4,%5,%6,%7}, [%8], %9;"
                  : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7])
@@ -213,25 +210,18 @@ __device__ __forceinline__ void st_rec(REntry* p, unsigned long long pol, int a0
                  "r"(a1), "r"(a2), "r"(a3), "r"(a4), "r"(a5), "r"(a6), "r"(a7), "l"(pol)
                  : "memory");
 }
-// streaming 16-byte store that should leave L2 first (written once, read lag - 2 steps later)
-__device__ __forceinline__ void st_stream_f64x2(void* p, unsigned long long pol, double a, double b) {
-    asm volatile("st.global.cs.L2::cache_hint.v2.f64 [%0], {%1,%2}, %3;" ::"l"(p), "d"(a), "d"(b), "l"(pol)
-                 : "memory");
-}
+// streaming 32-byte store that should leave L2 first (written once, read lag - 2 steps later)
 __device__ __forceinline__ void st_stream_f64x4(void* p, unsigned long long pol, double a, double b, double c, double d) {
     asm volatile("st.global.cs.L2::cache_hint.v4.f64 [%0], {%1,%2,%3,%4}, %5;" ::"l"(p), "d"(a), "d"(b), "d"(c), "d"(d),
                  "l"(pol)
                  : "memory");
-}
-__device__ __forceinline__ void st_stream_f64(double* p, unsigned long long pol, double a) {
-    asm volatile("st.global.cs.L2::cache_hint.f64 [%0], %1, %2;" ::"l"(p), "d"(a), "l"(pol) : "memory");
 }
 __device__ __forceinline__ double ld_stream_hint_f64(const double* p, unsigned long long pol) {
     double v;
     asm volatile("ld.global.nc.L1::no_allocate.L2::cache_hint.f64 %0, [%1], %2;" : "=d"(v) : "l"(p), "l"(pol));
     return v;
 }
-// L2 residency plan (dbg & 64 switches it off): what the next phase or the next step reads again -- the
+// L2 residency plan: what the next phase or the next step reads again -- the
 // sorted (x, e) pairs / the mailbox that aliases them, perm, H, the genealogy records being written -- is
 // stored evict_last (56 MB at N = 2^20); what is dead after its read -- the previous record table, the
 // mailbox entries, H, u -- and what is not read for 8 steps -- the payloads -- goes evict_first
@@ -453,13 +443,7 @@ __global__ void __launch_bounds__(GT, 1) sv_grid_kernel(const GridArgs a_in, con
     constexpr int SPT = kNSB / GT;          // sub-bins per thread
     constexpr int NW = GT / 32;
     constexpr int CH = KPT >= 16 ? 8 : 4;   // independent loads in flight per thread in the gather loops
-#ifndef PMMH_GRID_HESS_RB
-#define PMMH_GRID_HESS_RB 2
-#endif
-#ifndef PMMH_GRID_HESS_SB
-#define PMMH_GRID_HESS_SB 1
-#endif
-    constexpr int RB = HESS ? (KPT >= 16 ? 2 * PMMH_GRID_HESS_RB : PMMH_GRID_HESS_RB) : (KPT >= 16 ? 4 : 2);   // genealogy records in flight per thread
+    constexpr int RB = KPT >= 16 ? 4 : 2;   // genealogy records in flight per thread
     constexpr int RS = HESS ? 2 : 1;        // 32-byte sectors per entry of R and P
     static_assert(SPT % 4 == 0 && BPT % 4 == 0, "vector loads of the counters");
     extern __shared__ __align__(16) unsigned char smem[];
@@ -505,40 +489,15 @@ __global__ void __launch_bounds__(GT, 1) sv_grid_kernel(const GridArgs a_in, con
 
 // The arrive is bar.sync + red.release.gpu by one thread, the wait ld.acquire.gpu by one thread + bar.sync: release /
 // acquire at gpu scope are cumulative over what bar.sync ordered before / after them, so no separate __threadfence is
-// needed (measured: 99.5 -> 96.8 ms per evaluation; -DPMMH_GRID_FENCE puts the fences back)
-#ifdef PMMH_GRID_FENCE
-#define GRID_FENCE() __threadfence()
-#else
-#define GRID_FENCE()
-#endif
-#ifdef PMMH_GRID_BACKOFF
-#define GRID_BACKOFF() __nanosleep(PMMH_GRID_BACKOFF)
-#else
-#define GRID_BACKOFF()
-#endif
+// needed (measured: 99.5 -> 96.8 ms per evaluation)
 // Abandoning: the reason goes to ctrl->status (first one wins), and bit 31 of the barrier counter is set, so that the
 // load every CTA polls the barrier with also tells it to stop -- at its next wait, whichever barrier that is (nothing
 // after the time loop needs the grid); a second load of the status word after every barrier costs an L2 round trip
-#ifdef PMMH_GRID_STATUS_LOAD
-#define GRID_FLAG(reason) atomicCAS(&ctrl->status, 0, (int)((epoch + 1u) | ((unsigned)(reason) << 24)))
-#else
 #define GRID_FLAG(reason)                                                                        \
     do {                                                                                         \
         atomicCAS(&ctrl->status, 0, (int)((epoch + 1u) | ((unsigned)(reason) << 24)));           \
         atomicOr(&ctrl->bar, 0x80000000u);                                                       \
     } while (0)
-#endif
-#ifdef PMMH_GRID_STATUS_LOAD
-#define GRID_POLL(tgt)                                                                \
-    do {                                                                              \
-        while (ld_acquire_u32(&ctrl->bar) < (tgt)) {                                  \
-            GRID_BACKOFF();                                                           \
-        }                                                                             \
-        GRID_FENCE();                                                                 \
-        const int stv = *(volatile int*)&ctrl->status;                                \
-        s_sc.abort_now = (stv != 0 && (unsigned)(stv & 0xffffff) <= epoch) ? 1 : 0;   \
-    } while (0)
-#else
 #define GRID_POLL(tgt)                                                                \
     do {                                                                              \
         unsigned v__;                                                                 \
@@ -547,15 +506,11 @@ __global__ void __launch_bounds__(GT, 1) sv_grid_kernel(const GridArgs a_in, con
         } while ((v__ & 0x7fffffffu) < (tgt) && !(v__ & 0x80000000u));                \
         s_sc.abort_now = (int)(v__ >> 31);                                            \
     } while (0)
-#endif
-#define GRID_ARRIVE()                                \
-    do {                                             \
-        __syncthreads();                             \
-        if (tid == 0) {                              \
-            GRID_FENCE();                            \
-            red_release_add(&ctrl->bar, 1u);         \
-        }                                            \
-        ++epoch;                                     \
+#define GRID_ARRIVE()                                    \
+    do {                                                 \
+        __syncthreads();                                 \
+        if (tid == 0) red_release_add(&ctrl->bar, 1u);   \
+        ++epoch;                                         \
     } while (0)
 #define GRID_WAIT()                                                                   \
     do {                                                                              \
@@ -916,7 +871,7 @@ __global__ void __launch_bounds__(GT, 1) sv_grid_kernel(const GridArgs a_in, con
         if (HESS && tid == 0) s_ndef = 0;
         __syncthreads();
         {
-            int* gh = a.ghist + ((size_t)par * kNCopy + (c % kNCopy)) * kNF;
+            int* gh = a.ghist + (size_t)par * kNF;
 #pragma unroll
             for (int kk = 0; kk < BPT; ++kk) {
                 const int b = kk * GT + tid;
@@ -989,10 +944,9 @@ __global__ void __launch_bounds__(GT, 1) sv_grid_kernel(const GridArgs a_in, con
         }
         {
             // housekeeping for the next step
-            constexpr int kZero = kNCopy * kNF;
-            const int zper = (kZero + G - 1) / G;
-            int* ghn = a.ghist + (size_t)(par ^ 1) * kZero;
-            for (int b = c * zper + tid; b < min(kZero, (c + 1) * zper); b += GT) __stcg(&ghn[b], 0);
+            const int zper = (kNF + G - 1) / G;
+            int* ghn = a.ghist + (size_t)(par ^ 1) * kNF;
+            for (int b = c * zper + tid; b < min(kNF, (c + 1) * zper); b += GT) __stcg(&ghn[b], 0);
             if (tid == 0) __stcg(&a.tilecnt[((par ^ 1) * kMaxTiles + c) * kCntStride], 0);
         }
         PROF_MARK(4);   // A1 records
@@ -1015,23 +969,20 @@ __global__ void __launch_bounds__(GT, 1) sv_grid_kernel(const GridArgs a_in, con
         // entries ordered by tile in shared memory, copied to the mailboxes in runs
         // --------------------------------------------------------------------------------------
         {
-            const int* gh = a.ghist + (size_t)par * kNCopy * kNF;
+            const int* gh = a.ghist + (size_t)par * kNF;
             int cnt[BPT];
 #pragma unroll
             for (int i = 0; i < BPT; ++i) cnt[i] = 0;
-            int prevcnt = 0;
 #pragma unroll
-            for (int cp = 0; cp < kNCopy; ++cp) {
-#pragma unroll
-                for (int i = 0; i < BPT; i += 4) {
-                    const int4 v = __ldcg((const int4*)(gh + cp * kNF + BPT * tid + i));
-                    cnt[i] += v.x;
-                    cnt[i + 1] += v.y;
-                    cnt[i + 2] += v.z;
-                    cnt[i + 3] += v.w;
-                }
-                if (tid > 0) prevcnt += __ldcg(gh + cp * kNF + BPT * tid - 1);
+            for (int i = 0; i < BPT; i += 4) {
+                const int4 v = __ldcg((const int4*)(gh + BPT * tid + i));
+                cnt[i] += v.x;
+                cnt[i + 1] += v.y;
+                cnt[i + 2] += v.z;
+                cnt[i + 3] += v.w;
             }
+            int prevcnt = 0;
+            if (tid > 0) prevcnt += __ldcg(gh + BPT * tid - 1);
             int loc = 0, mxb = 0;
 #pragma unroll
             for (int i = 0; i < BPT; ++i) {
@@ -1497,7 +1448,7 @@ __global__ void __launch_bounds__(GT, 1) sv_grid_kernel(const GridArgs a_in, con
                 }
             }
             if constexpr (HESS) {
-                constexpr int SB = PMMH_GRID_HESS_SB;   // 64-byte entries in flight per thread
+                constexpr int SB = 1;   // 64-byte entries in flight per thread
                 double h2[10];
 #pragma unroll
                 for (int i = 0; i < 10; ++i) h2[i] = 0.0;
@@ -1599,8 +1550,6 @@ __global__ void __launch_bounds__(GT, 1) sv_grid_kernel(const GridArgs a_in, con
         for (int i = 0; i < kProf; ++i) a.prof[(size_t)c * kProf + i] += s_prof[i];
 #undef GRID_FLAG
 #undef GRID_POLL
-#undef GRID_FENCE
-#undef GRID_BACKOFF
 #undef GRID_ARRIVE
 #undef GRID_WAIT
 #undef PROF_MARK
@@ -1875,7 +1824,7 @@ GridLayout grid_layout(int nobs, int n, int lag, int G, int hist, int hess, int 
     size_t o = 0;
     const size_t N = (size_t)n;
     L.ctrl = o;      o += al256(sizeof(GridCtrl));
-    L.ghist = o;     o += al256((size_t)2 * kNCopy * kNF * 4);
+    L.ghist = o;     o += al256((size_t)2 * kNF * 4);
     L.tilecnt = o;   o += al256((size_t)2 * kMaxTiles * kCntStride * 4);
     L.tinfo = o;     o += al256((size_t)kMaxTiles * 4 * 8);
     L.H = o;         o += al256(N * 4);
@@ -2009,10 +1958,6 @@ GridArgs grid_args(const SvCall& c, const GridLayout& L, char* ws, int nobs, int
     a.Xhist = c.x_hist;
     a.Ahist = c.a_hist;
     a.prof = c.prof;
-    {
-        const char* e = getenv("PMMH_GRID_DEBUG");
-        a.dbg = e ? atoi(e) : 0;
-    }
     return a;
 }
 
@@ -2108,52 +2053,31 @@ int sv_grid_teams(int batch, int sm_count, int G) {
     return t < 1 ? 1 : t;
 }
 
-int sv_grid_run(const SvCall& c, int nobs, int n, int lag, int G, int hess) {
-    int rc = grid_check(c, nobs, n, lag, G, hess);
-    if (rc != PMMH_OK) return rc;
-    const GridLayout L = grid_layout(nobs, n, lag, G, c.x_hist != nullptr, hess, c.filter);
-    if (c.ws_bytes < L.total) return set_error(PMMH_ERR_WORKSPACE, "grid kernel: workspace too small");
-    char* ws = (char*)c.ws;
-    const cudaStream_t st = c.stream;
-    GridArgs a = grid_args(c, L, ws, nobs, n, lag, G, hess);
-    // control block, histograms, reservation counters, tile info: zero
-    GRID_CUDA(cudaMemsetAsync(ws + L.ctrl, 0, L.H - L.ctrl, st));
-    rc = grid_set_attributes();
-    if (rc != PMMH_OK) return rc;
-    GridTeam tm = {0, 0};   // (unused)
-    void* kargs[] = {(void*)&a, (void*)&tm};
-    GRID_CUDA(cudaLaunchCooperativeKernel(grid_kernel_for(c.model, hess, c.filter, false), dim3(G), dim3(1024), kargs,
-                                          kDynSmem, st));
-    return grid_after(c, a, L, ws, nobs, n, lag, G, hess);
-}
-
-size_t sv_grid_team_ws_bytes(int nobs, int n, int lag, int G, int hess, int filter) {
-    return grid_layout(nobs, n, lag, G, 1, hess, filter).total;
-}
-
-int sv_grid_batch_run(const SvCall& c, int batch, int nobs, int n, int lag, int G, int nteams, int hess) {
+int sv_grid_run(const SvCall& c, int batch, int nobs, int n, int lag, int G, int nteams, int hess) {
     int rc = grid_check(c, nobs, n, lag, G, hess);
     if (rc != PMMH_OK) return rc;
     if (batch < 1 || nteams < 1) return set_error(PMMH_ERR_INVALID, "grid kernel: bad team count");
-    if (c.slot > 0 || c.prof) return set_error(PMMH_ERR_INVALID, "grid kernel: teams take device-resident u only");
-    const GridLayout L = grid_layout(nobs, n, lag, G, 1, hess, c.filter);
+    if (batch > 1 && (c.slot > 0 || c.prof)) return set_error(PMMH_ERR_INVALID, "grid kernel: teams take device-resident u only");
+    const GridLayout L = grid_layout(nobs, n, lag, G, c.x_hist != nullptr, hess, c.filter);
     const int slices = batch < nteams ? batch : nteams;
     if (c.ws_bytes < (size_t)slices * L.total) return set_error(PMMH_ERR_WORKSPACE, "grid kernel: workspace too small");
     char* ws = (char*)c.ws;
     const cudaStream_t st = c.stream;
     rc = grid_set_attributes();
     if (rc != PMMH_OK) return rc;
-    const void* kern = grid_kernel_for(c.model, hess, c.filter, true);
+    GridTeam tm;
+    tm.ws_stride = (long long)L.total;
+    tm.obs_stride = c.obs_stride;
     for (int b0 = 0; b0 < batch; b0 += nteams) {
         const int nw = batch - b0 < nteams ? batch - b0 : nteams;   // problems (teams) of this wave
+        // control block, histograms, reservation counters, tile info of every team: zero
         for (int k = 0; k < nw; ++k)
             GRID_CUDA(cudaMemsetAsync(ws + (size_t)k * L.total + L.ctrl, 0, L.H - L.ctrl, st));
         GridArgs a = grid_args(grid_problem(c, b0, nobs, n), L, ws, nobs, n, lag, G, hess);
-        GridTeam tm;
-        tm.ws_stride = (long long)L.total;
-        tm.obs_stride = c.obs_stride;
         void* kargs[] = {(void*)&a, (void*)&tm};
-        GRID_CUDA(cudaLaunchCooperativeKernel(kern, dim3(nw * G), dim3(1024), kargs, kDynSmem, st));
+        // a wave of one problem runs the one-problem instantiation
+        GRID_CUDA(cudaLaunchCooperativeKernel(grid_kernel_for(c.model, hess, c.filter, nw > 1), dim3(nw * G), dim3(1024),
+                                              kargs, kDynSmem, st));
         for (int k = 0; k < nw; ++k) {
             char* wk = ws + (size_t)k * L.total;
             const SvCall pc = grid_problem(c, b0 + k, nobs, n);

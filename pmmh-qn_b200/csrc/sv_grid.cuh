@@ -12,14 +12,12 @@ bool sv_grid_eligible(int nobs, int n, int lag, int G);
 // the filter alone (no lag): n_obs >= 2 and a tile fits one CTA
 bool sv_grid_filter_eligible(int nobs, int n, int G);
 size_t sv_grid_ws_bytes(int nobs, int n, int lag, int G, int hist, int hess = 0, int filter = 0);
-// c.model selects the instantiation (PMMH_MODEL_*, pf_model.cuh); hess: the Hessian branch (SV only); c.filter: the
-// filter alone (lag unused)
-int sv_grid_run(const SvCall& c, int nobs, int n, int lag, int G, int hess);
-// Teams: `batch` problems of the same shape, each on its own G CTAs (the one-problem tiles, so every problem's outputs
-// are bit-identical to its sv_grid_run), in waves of nteams = sv_grid_teams(batch, SMs, G) problems: one cooperative
-// launch of (problems in the wave) x G CTAs per wave.  The workspace is min(batch, nteams) slices of
-// sv_grid_team_ws_bytes (the one-problem layout with history).  Device-resident u only.
+// `batch` problems of one shape (problem b's inputs and outputs one problem further on), each on its own G CTAs, in
+// waves of nteams = sv_grid_teams(batch, SMs, G) problems: one cooperative launch of (problems in the wave) x G CTAs per
+// wave.  Every problem's outputs are bit-identical to its run alone (batch = nteams = 1).  The workspace is
+// min(batch, nteams) slices of sv_grid_ws_bytes (hist: c.x_hist given).  c.model selects the instantiation (PMMH_MODEL_*, pf_model.cuh); hess:
+// the Hessian branch (SV only); c.filter: the filter alone (lag unused).  Host-streamed u (c.slot > 0) and the phase
+// clocks (c.prof) take batch = 1 only.
 int sv_grid_teams(int batch, int sm_count, int G);
-size_t sv_grid_team_ws_bytes(int nobs, int n, int lag, int G, int hess, int filter);
-int sv_grid_batch_run(const SvCall& c, int batch, int nobs, int n, int lag, int G, int nteams, int hess);
+int sv_grid_run(const SvCall& c, int batch, int nobs, int n, int lag, int G, int nteams, int hess);
 }  // namespace pmmh
