@@ -178,10 +178,15 @@ int pmmh_flps_sv_corr_philox(const double* d_obs, const double* d_params, const 
                              size_t workspace_bytes, void* stream);
 
 /* Model-generic fixed-lag smoother (log-likelihood + gradient): the same algorithm as pmmh_flps_sv_corr
- * (sorted correlated systematic resampling, fixed-lag score terms, tail, quirks Q1 / Q5 / Q6) with the
+ * (sorted correlated systematic resampling, fixed-lag score terms, tail, quirk Q1) with the
  * model's propagation, log-weight and score formulas plugged in through the device-function interface
  * of csrc/pf_model.cuh -- the three things python/README.md:73-76 tells a user to change in the Cython
- * smoother for another scalar-state model.  2 <= lag <= 10.  The kernel (d_diag[PMMH_DIAG_KERNEL]):
+ * smoother for another scalar-state model.  2 <= lag <= 10.  The reference's pairing quirks Q5 / Q6 apply to
+ * PMMH_MODEL_SV_LEVERAGE only (parity).  Models 1 and 2 pair the fixed-lag terms exactly: gradient[k][s] holds the
+ * expectation of d/dtheta_k [log p(x_s | x_{s-1}) + log p(y_s | x_s)] (y_s = obs[s]) under the weights of generation
+ * min(s + lag - 2, n_obs - 1), gradient[k][0] = 0, and the sum over s estimates the score of the log-likelihood;
+ * smo[t] is the mean of x_t under the weights of generation min(t + lag - 1, n_obs - 1).  For model 1 these are
+ * E[. | y_1 .. y_c] of that generation c; model 2's weights condition on one more observation.  The kernel (d_diag[PMMH_DIAG_KERNEL]):
  *   3  chain kernel, one CTA per problem: 2 <= n_particles <= 4096, any batch;
  *   5  grid kernel, one persistent launch over the GPU: batch == 1, n_obs >= 2 lag and a tile of
  *      n_particles / min(SMs, ceil(n_particles / 2048)) particles fits one CTA (<= 7168: up to 1,060,864

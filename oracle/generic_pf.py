@@ -8,8 +8,10 @@ Pinning: with the SV callbacks below it must reproduce oracle_flps_sv_corr (orac
 bit-exact against the compiled reference) -- tests/test_oracle_vs_golden.py checks ancestors and sorted
 generations exactly and the estimates to 1e-12 (NumPy's pairwise sums order the additions differently).
 For the linear Gaussian model (bootstrap filter, model id 1, and fully adapted filter, model id 2) there is no
-reference implementation: the device instantiations are pinned to the restatements below (ancestors exact), which
-are unpinned with respect to the reference.  The fully adapted restatement is itself checked against closed forms
+reference implementation, so there is no parity to keep: the fixed-lag terms pair the states exactly (no Q5 / Q6,
+see flps_generic).  The device instantiations are pinned to the restatements below (ancestors exact), and the
+restatements are pinned statistically to the exact fixed-lag Kalman quantities of oracle/kalman.py
+(tests/test_kalman_reference.py).  The fully adapted restatement is itself checked against closed forms
 (tests/test_oracle_vs_golden.py): its proposal against the precision-weighted conditional moments, its
 likelihood estimate against the exact Kalman likelihood (statistically).
 """
@@ -19,6 +21,7 @@ import numpy as np
 class SvLeverage(object):
     """stochastic_volatility.pyx:306-323 (Q1), :354-358, :427-437, :452-465, :548-557"""
     n_params = 4
+    reference_indexing = True          # the reference's pairing of the fixed-lag terms (Q5 / Q6)
 
     def __init__(self, params):
         self.mu, self.phi, self.sv, self.rho = [float(p) for p in params]
@@ -61,6 +64,7 @@ class SvLeverage(object):
 class LinearGaussian(object):
     """x' = phi x + sigma_v v, y = x + sigma_e e; params (phi, sigma_v, sigma_e, unused) -- csrc/pf_model.cuh"""
     n_params = 3
+    reference_indexing = False         # exact pairing (flps_generic)
 
     def __init__(self, params):
         self.phi, self.sv, self.se = [float(p) for p in params[:3]]
@@ -76,8 +80,9 @@ class LinearGaussian(object):
         return (-0.91893853320467267 - np.log(self.se)) - (0.5 * (r * r)) / (self.se * self.se)
 
     def score_main(self, curr, nxt, y):
+        """d/d(phi, sigma_v, sigma_e) of log N(nxt; phi curr, sigma_v^2) + log N(y; nxt, sigma_e^2), y = obs[time(nxt)]"""
         r = nxt - self.phi * curr
-        ry = y - curr
+        ry = y - nxt
         g0 = (r * curr) / (self.sv * self.sv)
         g1 = ((r * r) / (self.sv * self.sv) - 1.0) / self.sv
         g2 = ((ry * ry) / (self.se * self.se) - 1.0) / self.se
@@ -91,6 +96,7 @@ class LinearGaussianFullyAdapted(object):
     operation: proposal p(x_t | x_{t-1}, y_t), weight p(y_{t+1} | x_t).  flps_generic runs it on the observations
     shifted by one (obs[1:]); log_p_y1 adds the first observation's term.  No score terms (gradient rows 0)."""
     n_params = 3
+    reference_indexing = False
 
     def __init__(self, params):
         self.phi, self.sv, self.se = [float(p) for p in params[:3]]
@@ -135,9 +141,16 @@ def systematic_corr(w, rnd):
 
 
 def flps_generic(model, obs, rvr, rvp, n_particles, lag=10, dumps=False):
-    """Returns filt, smo, log_like, gradient [4][NOBS], traj (+ X, A, W when dumps)."""
+    """Returns filt, smo, log_like, gradient [4][NOBS], traj (+ X, A, W when dumps).
+
+    model.reference_indexing True (SV): the reference's pairing, quirks Q5 / Q6.  False (the linear Gaussian models):
+    the pair (x_t, x_{t+1}), t = 0 .. NOBS-2, adds score(x_t, x_{t+1}, obs[t+1]) once, into gradient slot t+1 (slot 0
+    stays 0), weighted by the generation at which it is read: W_{t+L-1} in the main loop, W_{NOBS-1} in the tail;
+    smo[t] = E[x_t] under the same weights, every slot once (the tail starts one step after the last main-loop slot).
+    """
     obs = np.asarray(obs, dtype=np.float64)
     nobs, n, L = obs.shape[0], int(n_particles), int(lag)
+    ref = model.reference_indexing
     U = np.asarray(rvp, dtype=np.float64).reshape(n, nobs)        # rvp[i + j * NOBS]
     X = np.zeros((nobs, n))
     W = np.zeros((nobs, n))
@@ -169,20 +182,32 @@ def flps_generic(model, obs, rvr, rvp, n_particles, lag=10, dumps=False):
         W[i] = sh / nf
         filt[i] = np.sum(W[i] * X[i])
         traj[i] = X[i][0]                                          # Q11
-        if i >= L:
+        if ref and i >= L:
             tt = i - L + 1
             curr, nxt = ph[L - 1], ph[L - 2]
             smo[tt] += np.sum(W[i] * curr)
             grad[:, tt] += np.sum(model.score_main(curr, nxt, obs[i - L]) * W[i], axis=1)   # Q5
+        elif not ref and i >= L - 1:
+            tt = i - L + 1                                         # pair (tt, tt + 1), tt = 0 included
+            curr, nxt = ph[L - 1], ph[L - 2]
+            smo[tt] += np.sum(W[i] * curr)
+            grad[:, tt + 1] += np.sum(model.score_main(curr, nxt, obs[tt + 1]) * W[i], axis=1)
         log_like += mx + np.log(nf) - np.log(float(n))
-    for i in range(nobs - L, nobs):                                # tail, :540-562 (Q6)
-        idx = nobs - i - 1
-        curr = ph[idx]
-        smo[i] += np.sum(W[nobs - 1] * curr)
-        if idx - 1 >= 0:
-            nxt = ph[idx - 1]
-            y1 = obs[i - 1] if i - 1 >= 0 else obs[i - 1 + nobs]
-            grad[:, i - L + 1] += np.sum(model.score_tail(curr, nxt, y1) * W[i], axis=1)
+    if ref:
+        for i in range(nobs - L, nobs):                            # tail, :540-562 (Q6)
+            idx = nobs - i - 1
+            curr = ph[idx]
+            smo[i] += np.sum(W[nobs - 1] * curr)
+            if idx - 1 >= 0:
+                nxt = ph[idx - 1]
+                y1 = obs[i - 1] if i - 1 >= 0 else obs[i - 1 + nobs]
+                grad[:, i - L + 1] += np.sum(model.score_tail(curr, nxt, y1) * W[i], axis=1)
+    else:
+        for t in range(nobs - L + 1, nobs):                        # tail: final weights, one step after the main loop
+            k = nobs - 1 - t
+            smo[t] += np.sum(W[nobs - 1] * ph[k])
+            if k >= 1:
+                grad[:, t + 1] += np.sum(model.score_tail(ph[k], ph[k - 1], obs[t + 1]) * W[nobs - 1], axis=1)
     out = dict(filt=filt, smo=smo, log_like=float(log_like), gradient=grad, traj=traj)
     if dumps:
         out.update(X=X, A=A, W=W)

@@ -3,8 +3,9 @@
 // its Cython particle smoother to another model (/root/reference/python/README.md:73-76:
 // "how the propagation and weighting of particles is carried out as well as the gradients of the
 // log joint distribution of states and measurements").  Everything else -- sorted correlated
-// systematic resampling, the counting sort, cumulative weights, fixed-lag bookkeeping, the tail,
-// the reference's indexing quirks Q5 / Q6 -- is model independent and lives in the kernel.
+// systematic resampling, the counting sort, cumulative weights, fixed-lag bookkeeping, the tail --
+// is model independent and lives in the kernel; kReferenceIndexing picks how the kernel pairs the
+// fixed-lag score terms.
 //
 // A model M provides (all __device__, fp64, no contraction):
 //   struct M::Const                      constants derived from the parameter vector (<= 4 doubles)
@@ -24,13 +25,22 @@
 //                                        (SV: :427-437)
 //   M::logw_max(c, lo, hi, y)            an upper bound of logw on [lo, hi] that is attained or
 //                                        nearly so (the shift of the weights; any value cancels)
-//   M::score_main(c, curr, next, y, g)   the 4 score terms of the pair (curr, next) in the main
-//                                        loop; y = obs[time(curr) - 1] as the reference hands it
-//                                        over (Q5) (SV: :452-465)
-//   M::score_tail(c, curr, next, y, g)   the same in the tail loop, y = obs[time(next) - 1]
-//                                        wrapped (Q6) (SV: :548-557, another operation order)
+//   M::score_main(c, curr, next, y, g)   the 4 score terms of the pair (curr, next) in the main loop
+//   M::score_tail(c, curr, next, y, g)   the same in the tail loop
 //   M::kScoreIsZero                      constexpr: score_main / score_tail are identically 0 (the
 //                                        grid kernel then skips the calls; the smoother still runs)
+//   M::kReferenceIndexing                constexpr: how the fixed-lag terms are paired (below)
+//
+// kReferenceIndexing = true (the SV model, parity with the reference): the reference's quirks Q5 / Q6.  The main loop
+// at step i >= LAG adds the pair (x_tt, x_tt+1), tt = i - LAG + 1, with y = obs[tt - 1] (score_main, Q5) into slot tt;
+// the tail i = NOBS-LAG .. NOBS-1 adds smo[i] under the final weights and the pair (x_i, x_i+1) with y = obs[i - 1]
+// wrapped (score_tail, Q6, :548-557, another operation order) under the weights of generation i into slot i - LAG + 1.
+// kReferenceIndexing = false (models of no reference: the exact pairing): the pair (x_t, x_t+1), t = 0 .. NOBS-2,
+// contributes d/dtheta log p(x_t+1 | x_t) + d/dtheta log p(y_t+1 | x_t+1) once, with y = obs[t + 1], weighted by the
+// generation at which it is read: W_{t+LAG-1} in the main loop (steps i >= LAG - 1; the pair t = 0 has curr =
+// initial_state for every particle, Q1), W_{NOBS-1} in the tail (t = NOBS-LAG+1 .. NOBS-2).  Gradient slot s holds
+// step s's contribution (the pair (x_s-1, x_s)); slot 0 is 0.  smo[t] = the weighted mean of x_t under the same
+// weights, every slot written once: the tail starts one step after the last main-loop slot.
 // Unused gradient slots stay 0.  Model ids are part of the C ABI (include/pmmh_qn.h).
 #pragma once
 #include <math.h>
@@ -48,6 +58,7 @@ struct SvLeverageModel {
         return c.mu + stdev0 * 0.0;   // :309 (Q1)
     }
     static constexpr bool kScoreIsZero = false;
+    static constexpr bool kReferenceIndexing = true;
     static __device__ __forceinline__ double propagate(const Const& c, double xp, double y1, double u) {
         double mean = c.mu + c.phi * (xp - c.mu);
         mean += c.sr * exp(-0.5 * xp) * y1;
@@ -102,6 +113,7 @@ struct LinearGaussianModel {
     }
     static __device__ __forceinline__ double initial_state(const Const&) { return 0.0; }
     static constexpr bool kScoreIsZero = false;
+    static constexpr bool kReferenceIndexing = false;
     static __device__ __forceinline__ double propagate(const Const& c, double xp, double, double u) {
         return c.phi * xp + c.sv * u;
     }
@@ -124,10 +136,10 @@ struct LinearGaussianModel {
         if (!isfinite(xs)) xs = 0.0;
         return logw(c, xs, y);
     }
-    // d/d(phi, sigma_v, sigma_e) of log N(next; phi curr, sigma_v^2) + log N(y; curr, sigma_e^2)
+    // d/d(phi, sigma_v, sigma_e) of log N(next; phi curr, sigma_v^2) + log N(y; next, sigma_e^2), y = obs[time(next)]
     static __device__ __forceinline__ void score_main(const Const& c, double curr, double next, double y, double g[4]) {
         const double r = next - c.phi * curr;
-        const double ry = y - curr;
+        const double ry = y - next;
         g[0] = (r * curr) * c.inv_sv2;
         g[1] = ((r * r) * c.inv_sv2 - 1.0) / c.sv;
         g[2] = ((ry * ry) * c.inv_se2 - 1.0) / c.se;
@@ -164,6 +176,7 @@ struct LinearGaussianFullyAdapted {
     static __device__ __forceinline__ double initial_state(const Const&) { return 0.0; }
     // x_t | x_{t-1}, y_t ~ N(phi x + k (y_t - phi x), sv^2 se^2 / (sv^2 + se^2))
     static constexpr bool kScoreIsZero = true;
+    static constexpr bool kReferenceIndexing = false;   // smo: x_t under W_{t+LAG-1}, i.e. given y_1 .. y_{t+LAG}
     static __device__ __forceinline__ double propagate(const Const& c, double xp, double y_now, double u) {
         const double m = c.phi * xp;
         return (m + c.k * (y_now - m)) + c.sdp * u;

@@ -22,7 +22,8 @@
 //     comes from a ring in global memory (L2 resident: 64 KB per generation and problem).
 // The tail (:540-562, Q6) chases one-step ancestors through global rings of the last LAG
 // generations.  Quirks reproduced: Q1, Q3 (as in the other kernels: cumulative weights are
-// normalised at look-up), Q5, Q6, Q11.  Sums over particles are fixed-order tree sums.
+// normalised at look-up), Q5 and Q6 for the SV model (M::kReferenceIndexing; the other models pair the fixed-lag terms
+// exactly, pf_model.cuh), Q11.  Sums over particles are fixed-order tree sums.
 // Hessian branch: the cumulative alpha of a particle (4 doubles) lives in a global ring by sorted
 // position next to the (value, parent value) ring; the child adds its own term to its parent's
 // (one 32-byte gather), the score phase gathers the lagged ancestor's; Q7's flat-layout read needs
@@ -480,8 +481,11 @@ __global__ void __launch_bounds__(kCT, 1) sv_chain_kernel(SvArgs a) {
                     tsum += v[q];
                 }
                 double run = chain_scan_d(tsum, s_w, &S_i);
-                const bool lagged = SMO && inext >= LAG;
-                const double yl = lagged ? obs[inext - LAG] : 0.0;   // Q5
+                // pairing of the fixed-lag terms (pf_model.cuh): the reference's (Q5 / Q6) or the exact one, whose main
+                // loop starts one step earlier (the pair (x_0, x_1) at step LAG - 1) and whose tail starts one step later
+                const bool lagged = SMO && inext >= (M::kReferenceIndexing ? LAG : LAG - 1);
+                // the pair (x_tt, x_tt+1), tt = inext - LAG + 1: y = obs[tt - 1] (Q5) or obs[tt + 1]
+                const double yl = lagged ? obs[M::kReferenceIndexing ? inext - LAG : inext - LAG + 2] : 0.0;
                 const int hop0 = (K >= 1) ? ((K - 1) & 3) : 0;
                 const int nh = (K >= 1) ? ((K - 1) >> 2) : 0;        // 0 or 1 (LAG <= 10)
                 const int g1 = inext - (hop0 + 1);
@@ -544,13 +548,14 @@ __global__ void __launch_bounds__(kCT, 1) sv_chain_kernel(SvArgs a) {
                 s_S[inext % kMaxLagC] = S_i;
                 o_filt[inext] = acc[0] / S_i;
                 o_traj[inext] = s_x[0];   // Q11: traj[i] = X_i[0]
-                if constexpr (SMO) if (inext >= LAG) {
+                if constexpr (SMO) if (inext >= (M::kReferenceIndexing ? LAG : LAG - 1)) {
                     const int tt = inext - LAG + 1;
+                    const int gs = M::kReferenceIndexing ? tt : tt + 1;   // gradient slot: tt (Q5) or the pair's second step
                     o_smo[tt] = acc[1] / S_i;
-                    o_grad[tt] = acc[2] / S_i;
-                    o_grad[NOBS + tt] = acc[3] / S_i;
-                    o_grad[2 * NOBS + tt] = acc[4] / S_i;
-                    o_grad[3 * NOBS + tt] = acc[5] / S_i;
+                    o_grad[gs] = acc[2] / S_i;
+                    o_grad[NOBS + gs] = acc[3] / S_i;
+                    o_grad[2 * NOBS + gs] = acc[4] / S_i;
+                    o_grad[3 * NOBS + gs] = acc[5] / S_i;
                 }
             }
             S_prev = S_i;
@@ -558,12 +563,12 @@ __global__ void __launch_bounds__(kCT, 1) sv_chain_kernel(SvArgs a) {
             CPROF(4);   // cumulative weights, sums, fixed-lag terms, outputs
         }   // time loop
 
-        // ---------------- tail (:540-562, Q6)
+        // ---------------- tail (:540-562, Q6; exact pairing: slots NOBS-LAG+1 .. NOBS-1, pairs under the final weights)
         if (SMO && status == 0) {
             const int T = NOBS - 1;
             const double S_T = s_S[T % kMaxLagC];
             const double* shT = SHG(T);
-            for (int k = 0; k < LAG; ++k) {
+            for (int k = 0; k < (M::kReferenceIndexing ? LAG : LAG - 1); ++k) {
                 const int ip = T - k;
                 constexpr int NT = 5;
                 double tacc[NT];
@@ -571,7 +576,7 @@ __global__ void __launch_bounds__(kCT, 1) sv_chain_kernel(SvArgs a) {
                 for (int q = 0; q < NT; ++q) tacc[q] = 0.0;
                 const double ylag = obs_wrap(obs, ip - LAG, NOBS);
                 const double S_ip = s_S[ip % kMaxLagC];
-                const double y1 = obs_wrap(obs, ip - 1, NOBS);
+                const double y1 = M::kReferenceIndexing ? obs_wrap(obs, ip - 1, NOBS) : (k >= 1 ? obs[ip + 1] : 0.0);
                 const double* shI = SHG(ip);
                 for (int j = tid; j < N; j += kCT) {
                     int b = j, bprev = j;
@@ -586,9 +591,14 @@ __global__ void __launch_bounds__(kCT, 1) sv_chain_kernel(SvArgs a) {
                     if (k >= 1) {
                         const double next = __ldcg(&XPG(ip + 1)[bprev]).x;
                         double g[4];
-                        double si = __ldcg(&shI[j]);
-                        if (!isfinite(si)) si = 0.0;
-                        const double wi = si / S_ip;
+                        double wi;
+                        if constexpr (M::kReferenceIndexing) {
+                            double si = __ldcg(&shI[j]);
+                            if (!isfinite(si)) si = 0.0;
+                            wi = si / S_ip;
+                        } else {
+                            wi = sT / S_T;
+                        }
                         if constexpr (HESS) {
                             double sq;
                             sv_score_tail(c, curr, next, y1, sq, g);
@@ -610,7 +620,7 @@ __global__ void __launch_bounds__(kCT, 1) sv_chain_kernel(SvArgs a) {
                 if (tid == 0) {
                     o_smo[ip] += tacc[0];
                     if (k >= 1) {
-                        const int tt = ip - LAG + 1;
+                        const int tt = M::kReferenceIndexing ? ip - LAG + 1 : ip + 1;
                         if (tt >= 0) {
                             o_grad[tt] += tacc[1];
                             o_grad[NOBS + tt] += tacc[2];

@@ -435,6 +435,9 @@ __global__ void __launch_bounds__(GT, 1) sv_grid_kernel(const GridArgs a_in, con
     if constexpr (TEAM) a_team = team_args(a_in, tm);
     const GridArgs& a = TEAM ? a_team : a_in;   // this CTA's problem
     constexpr bool GEN = !std::is_same<M, SvLeverageModel>::value;
+    // first step with fixed-lag terms: the reference's pairing (Q5) starts at LAG, the exact one (pf_model.cuh) one step
+    // earlier with the pair (x_0, x_1)
+    constexpr int LAG0 = M::kReferenceIndexing ? 0 : 1;
     static_assert(!(GEN && HESS), "the Hessian branch exists for the SV model only");
     static_assert(SMO || !HESS, "the Hessian branch needs the smoother");
     constexpr int KPT = kCap / GT;          // entries per thread (strided assignment)
@@ -1327,7 +1330,7 @@ __global__ void __launch_bounds__(GT, 1) sv_grid_kernel(const GridArgs a_in, con
                     __stcg((double2*)&a.tinfo[c * 4 + 2], make_double2(v[1], v[2]));
                     ps[1] = v[0];
                     ps[7] = 0.0;
-                    if (!SMO || t < L || (a.dbg & 4)) {   // later steps: the score terms below write ps[2..6]
+                    if (!SMO || t < L - LAG0 || (a.dbg & 4)) {   // later steps: the score terms below write ps[2..6]
 #pragma unroll
                         for (int i = 2; i < 7; ++i) ps[i] = 0.0;
                     }
@@ -1343,7 +1346,7 @@ __global__ void __launch_bounds__(GT, 1) sv_grid_kernel(const GridArgs a_in, con
         }
         PROF_MARK(11);   // B scan+publish
         GRID_ARRIVE();   // ---- barrier 3: tile totals published
-        if (SMO && t >= L && !(a.dbg & 4)) {
+        if (SMO && t >= L - LAG0 && !(a.dbg & 4)) {
             // fixed-lag score terms (:445-470): weight x monomials of the payload of the ancestor
             // LAG-2 generations back (one random sector each), fixed summation order
             const PEntry* Pg = a.P + (size_t)((t - (L - 2)) % RP) * N * RS;
@@ -1362,8 +1365,9 @@ __global__ void __launch_bounds__(GT, 1) sv_grid_kernel(const GridArgs a_in, con
             }
             if constexpr (GEN) {
                 // generic path: sc[0] = sum sh curr (smoother), sc[1 + k] = sum sh g[k] of M::score_main on the pair
-                // (curr, next) = (parent value, own value) of the ancestor; y = obs[t - LAG] (Q5)
-                const double yl = a.obs[t - L];
+                // (curr, next) = (parent value, own value) of the ancestor = (x_tt, x_tt+1), tt = t - LAG + 1;
+                // y = obs[t - LAG] (Q5) or obs[tt + 1]
+                const double yl = a.obs[M::kReferenceIndexing ? t - L : t - L + 2];
 #pragma unroll
                 for (int k0 = 0; k0 < KPT; k0 += 4) {
                     double pc[4], px[4];
@@ -1569,7 +1573,8 @@ __global__ void __launch_bounds__(256) grid_reduce_kernel(const double* __restri
 
 // part[irel][block][0] = sum_p W_T[p] hist_idx[p];  [1..4] = sum_p W_i[p] g(hist_idx, hist_idx-1)
 // with i = NOBS - L + irel, idx = L - 1 - irel; hist_k[p] = value of the ancestor k steps back of
-// the particle at sorted position p of the final generation.
+// the particle at sorted position p of the final generation.  Exact pairing (pf_model.cuh, !M::kReferenceIndexing):
+// irel = 0 is 0 (the main loop has that slot), the pair is weighted by W_T and takes y = obs[i + 1].
 // HESS: partH[irel][block][0..19] = the hessian1 / hessian2 terms of :564-626 (alpha of the ancestor LAG-2 steps
 // back of the final particle, weights W_i, obs[i - LAG] with wrap-around, Q8).  M: the model (g = M::score_tail).
 template <bool HESS, class M>
@@ -1582,7 +1587,8 @@ __global__ void __launch_bounds__(256) grid_tail_kernel(GridArgs a, const double
     const int irel = blockIdx.y, i = a.NOBS - L + irel, idx = L - 1 - irel;
     typename M::Const k;
     M::init(k, a.params);
-    const double y1 = obs_wrap(a.obs, i - 1, a.NOBS);
+    constexpr bool REF = M::kReferenceIndexing;
+    const double y1 = REF ? obs_wrap(a.obs, i - 1, a.NOBS) : a.obs[min(i + 1, T)];
     const double ST = sums[(size_t)T * 8], Si = sums[(size_t)i * 8];
     const double* shT = a.shring + (size_t)(T % L) * N;
     const double* shi = a.shring + (size_t)(i % L) * N;
@@ -1595,7 +1601,7 @@ __global__ void __launch_bounds__(256) grid_tail_kernel(GridArgs a, const double
         for (int q = 0; q < 20; ++q) hacc[q] = 0.0;
     }
     const double ylagH = obs_wrap(a.obs, i - L, a.NOBS);
-    const bool live = a.ctrl->status == 0;   // an abandoned evaluation leaves stale rows behind
+    const bool live = a.ctrl->status == 0 && (REF || irel >= 1);   // an abandoned evaluation leaves stale rows behind
     for (int p = blockIdx.x * 256 + tid; live && p < N; p += nblk * 256) {
         const int b = min(max(a.perm[p], 0), N - 1);
         const double wT = shT[p] / ST;
@@ -1611,7 +1617,7 @@ __global__ void __launch_bounds__(256) grid_tail_kernel(GridArgs a, const double
             curr = pe.c;
             const double pe_n = pe.x;
             acc[0] += wT * curr;
-            const double wi = shi[p] / Si;
+            const double wi = REF ? shi[p] / Si : wT;
             double sq, g[4], ec;
             if constexpr (std::is_same<M, SvLeverageModel>::value) {
                 ec = exp(-0.5 * curr);
@@ -1729,8 +1735,12 @@ __global__ void __launch_bounds__(256) grid_tail_reduce_kernel(const double* __r
 
 // sums[t][0] = sum sh, [1] = sum sh x, [2] = sum sh c, [3] = sum sh sq, [4] = sum sh sq c, [5] = sum sh sq^2,
 // [6] = sum sh sq ey (c = lagged ancestor value, sq / ey as stored in P);  tail[irel][0..4].
-// GEN (the generic path of a model other than SV): [3..6] = sum sh g[0..3], traj[0] = the initial state.
+// GEN (the generic path of a model other than SV): [3..6] = sum sh g[0..3], traj[0] = the initial state, exact pairing of
+// the fixed-lag terms (pf_model.cuh; models 1 and 2 have kReferenceIndexing = false).
 // SMO = false (the filter alone): no smo / grad, tail unused.
+static_assert(SvLeverageModel::kReferenceIndexing && !LinearGaussianModel::kReferenceIndexing &&
+                  !LinearGaussianFullyAdapted::kReferenceIndexing,
+              "grid_finish_kernel pairs the fixed-lag terms as the reference does for SV (GEN = false), exactly otherwise");
 template <bool GEN, bool SMO>
 __global__ void grid_finish_kernel(const GridCtrl* __restrict__ ctrl, const double* __restrict__ sums,
                                    const double* __restrict__ shift, const double* __restrict__ xmin,
@@ -1780,14 +1790,26 @@ __global__ void grid_finish_kernel(const GridCtrl* __restrict__ ctrl, const doub
         traj[t] = (t == 0 && !GEN) ? params[0] : xmin[t];   // Q10/Q11: traj[t] = X_t[0] for t >= 1, X_0 == mu
         if constexpr (!SMO) continue;
         double s = 0.0, g[4] = {0.0, 0.0, 0.0, 0.0};
-        const int src = t + L - 1;   // main-loop terms land at tt = i - L + 1 (:445-470)
-        if (t >= 1 && src < nobs) {
-            const double* sm = sums + (size_t)src * 8;
-            const double S = sm[0];
-            s = sm[2] / S;
-            if constexpr (GEN) {
-                for (int q = 0; q < 4; ++q) g[q] = sm[3 + q] / S;
-            } else {
+        if constexpr (GEN) {
+            // exact pairing (pf_model.cuh): smo[t] from step t + L - 1 (t >= 0), gradient slot t = the pair (x_t-1, x_t)
+            // from step t + L - 2; the tail (irel >= 1) adds smo[nobs-L+irel] and gradient[.][nobs-L+irel+1]
+            const int ss = t + L - 1, sg = t + L - 2;
+            if (ss < nobs) s = sums[(size_t)ss * 8 + 2] / sums[(size_t)ss * 8];
+            if (t >= 1 && sg < nobs) {
+                const double* sm = sums + (size_t)sg * 8;
+                for (int q = 0; q < 4; ++q) g[q] = sm[3 + q] / sm[0];
+            }
+            const int irel_s = t - (nobs - L);
+            if (irel_s >= 1 && irel_s < L) s += tail[irel_s * 8];
+            const int irel_g = t - 1 - (nobs - L);
+            if (irel_g >= 1 && irel_g < L - 1)
+                for (int q = 0; q < 4; ++q) g[q] += tail[irel_g * 8 + 1 + q];
+        } else {
+            const int src = t + L - 1;   // main-loop terms land at tt = i - L + 1 (:445-470)
+            if (t >= 1 && src < nobs) {
+                const double* sm = sums + (size_t)src * 8;
+                const double S = sm[0];
+                s = sm[2] / S;
                 SvConst k;
                 sv_const_init(k, params);
                 // weighted means of g[0..3] of :454-465 written in the monomials sq, sq c, sq^2, sq ey
@@ -1796,12 +1818,12 @@ __global__ void grid_finish_kernel(const GridCtrl* __restrict__ ctrl, const doub
                 g[2] = (k.q * sm[5] + k.q * k.sr * sm[6] - S) / S;
                 g[3] = (k.rho * S - k.q * k.rho * sm[5] + k.inv_sv * sm[6]) / S;
             }
+            const int irel_s = t - (nobs - L);   // tail: i = nobs-L+irel adds smo[i], gradient[.][i-L+1]
+            if (irel_s >= 0 && irel_s < L) s += tail[irel_s * 8];
+            const int irel_g = t + L - 1 - (nobs - L);
+            if (irel_g >= 0 && irel_g < L - 1)
+                for (int q = 0; q < 4; ++q) g[q] += tail[irel_g * 8 + 1 + q];
         }
-        const int irel_s = t - (nobs - L);   // tail: i = nobs-L+irel adds smo[i], gradient[.][i-L+1]
-        if (irel_s >= 0 && irel_s < L) s += tail[irel_s * 8];
-        const int irel_g = t + L - 1 - (nobs - L);
-        if (irel_g >= 0 && irel_g < L - 1)
-            for (int q = 0; q < 4; ++q) g[q] += tail[irel_g * 8 + 1 + q];
         smo[t] = s;
         for (int q = 0; q < 4; ++q) grad[(size_t)q * nobs + t] = g[q];
     }
