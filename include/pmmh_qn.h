@@ -182,7 +182,8 @@ int pmmh_flps_sv_corr_philox(const double* d_obs, const double* d_params, const 
  * model's propagation, log-weight and score formulas plugged in through the device-function interface
  * of csrc/pf_model.cuh -- the three things python/README.md:73-76 tells a user to change in the Cython
  * smoother for another scalar-state model.  2 <= lag <= 10.  The reference's pairing quirks Q5 / Q6 apply to
- * PMMH_MODEL_SV_LEVERAGE only (parity).  Models 1 and 2 pair the fixed-lag terms exactly: gradient[k][s] holds the
+ * PMMH_MODEL_SV_LEVERAGE only (parity).  Model 4 pairs them predictively (PMMH_MODEL_LINEAR_GAUSSIAN_FA_GRAD
+ * below).  Models 1 and 2 pair the fixed-lag terms exactly: gradient[k][s] holds the
  * expectation of d/dtheta_k [log p(x_s | x_{s-1}) + log p(y_s | x_s)] (y_s = obs[s]) under the weights of generation
  * min(s + lag - 2, n_obs - 1), gradient[k][0] = 0, and the sum over s estimates the score of the log-likelihood;
  * smo[t] is the mean of x_t under the weights of generation min(t + lag - 1, n_obs - 1).  For model 1 these are
@@ -201,6 +202,17 @@ int pmmh_flps_sv_corr_philox(const double* d_obs, const double* d_params, const 
 #define PMMH_MODEL_LINEAR_GAUSSIAN 1  /* phi, sigma_v, sigma_e: x' = phi x + sigma_v v, y = x + sigma_e e */
 #define PMMH_MODEL_LINEAR_GAUSSIAN_FA 2 /* the same model as a FULLY ADAPTED particle filter: pass the observations shifted by
                                          one (obs'[t] = obs[t + 1], n_obs - 1 entries); log-likelihood of y_2..y_T given y_1 */
+/* PMMH_MODEL_LINEAR_GAUSSIAN_FA_GRAD: model 2's fully adapted filter with a fixed-lag gradient.  Same inputs as model 2
+ * (the shifted series obs' = obs[1:], x_0 = 0, y_t = obs[t]); d_filt, d_smo, d_log_like, d_traj, d_diag and the history
+ * are bit-identical to model 2's.  Gradient rows 0..2 are d/d(phi, sigma_v, sigma_e), row 3 is 0, and slot k holds the
+ * contribution of obs'[k] = y_{k+1}: for k <= n_obs - 2 the expectation of
+ * d/dtheta [log p(x_{k+1} | x_k) + log p(obs'[k] | x_{k+1})] under the weights of generation c(k) = min(k + lag - 1,
+ * n_obs - 1), and for k = n_obs - 1 that of d/dtheta log N(obs'[n_obs - 1]; phi x_{n_obs - 1}, sigma_v^2 + sigma_e^2)
+ * under the final weights.  The slots sum to an estimate of the score of the FULL log-likelihood log p(y_1 .. y_T), so the
+ * gradient needs no correction, while d_log_like still lacks log p(y_1) as for model 2.  pmmh_flps_model_corr and
+ * pmmh_flps_model_batch_corr take it on the sizes of model 2 (compute_hessian == 1 is refused); the filter entries run
+ * model 2's filter for it. */
+#define PMMH_MODEL_LINEAR_GAUSSIAN_FA_GRAD 4   /* id 3 is unassigned: every entry refuses it as an unknown id */
 int pmmh_flps_model_workspace_bytes(int n_obs, int n_particles, int lag, int batch, size_t* bytes);
 int pmmh_flps_model_corr(int model_id, const double* d_obs, long long obs_stride, const double* d_params,
                          const double* d_rvr, const double* d_u, int n_obs, int n_particles, int lag, int batch,

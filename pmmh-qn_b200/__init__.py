@@ -17,6 +17,7 @@ _LAZY = {
     "ParticleMethodsCUDA": ("state.particle_methods.cuda", "ParticleMethodsCUDA"),
     "ImportanceSamplingCUDA": ("state.importance_sampling.cuda", "ImportanceSamplingCUDA"),
     "DirectComputationCUDA": ("state.direct.cuda", "DirectComputationCUDA"),
+    "LinearGaussianParticleMethodsCUDA": ("state.particle_methods.linear_gaussian", "LinearGaussianParticleMethodsCUDA"),
     "DeviceRVS": ("parameter.rvs", "DeviceRVS"),
     "propose_rvs": ("parameter.rvs", "propose_rvs"),
     "CorrelatedRVSState": ("parameter.rvs", "CorrelatedRVSState"),

@@ -20,7 +20,7 @@ c_dbl = ctypes.c_double
 DIAG_NEAR_TIES, DIAG_MAX_BIN, DIAG_STATUS, DIAG_KEY_TIES, DIAG_WAVEFRONT, DIAG_TRAJ_IDX, DIAG_KERNEL = range(7)
 DIAG_SOFT_TIES = 4   # flps on the grid kernel (same slot as the bpf wave-front depth)
 DIAG_COUNT = 8
-MODEL_SV_LEVERAGE, MODEL_LINEAR_GAUSSIAN, MODEL_LINEAR_GAUSSIAN_FA = 0, 1, 2
+MODEL_SV_LEVERAGE, MODEL_LINEAR_GAUSSIAN, MODEL_LINEAR_GAUSSIAN_FA, MODEL_LINEAR_GAUSSIAN_FA_GRAD = 0, 1, 2, 4
 BPF_PARITY, BPF_INTENDED = 0, 1
 
 # name -> (restype, argtypes); mirrors include/pmmh_qn.h one to one

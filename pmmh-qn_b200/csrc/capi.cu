@@ -666,6 +666,10 @@ int pmmh_flps_sv_corr_streamed(const double* h_rvs, const double* d_obs, const d
 
 // ---- model-generic entry points: the chain or the grid kernel instantiated for a model of pf_model.cuh ----------
 namespace {
+// the model whose filter instantiation a filter entry runs: model 4 adds a gradient to model 2, so its filter is model 2's
+int filter_model(int model_id) {
+    return model_id == PMMH_MODEL_LINEAR_GAUSSIAN_FA_GRAD ? PMMH_MODEL_LINEAR_GAUSSIAN_FA : model_id;
+}
 // The plan pmmh_flps_model_corr (filter = 0) or pmmh_filter_model_corr (filter = 1, lag 2: no lag condition) runs:
 // the chain kernel wherever it applies (any batch), else the grid kernel for one problem on sv_grid_ctas(N, SMs, 0)
 // CTAs; anything else is refused.  The workspace is the chosen kernel's alone (there is no fallback pass), with
@@ -720,7 +724,7 @@ int pmmh_flps_model_corr(int model_id, const double* d_obs, long long obs_stride
         !d_diag || !d_workspace)
         return fail(PMMH_ERR_INVALID, "pmmh_flps_model_corr: null pointer argument");
     if (model_id != PMMH_MODEL_SV_LEVERAGE && model_id != PMMH_MODEL_LINEAR_GAUSSIAN &&
-        model_id != PMMH_MODEL_LINEAR_GAUSSIAN_FA)
+        model_id != PMMH_MODEL_LINEAR_GAUSSIAN_FA && model_id != PMMH_MODEL_LINEAR_GAUSSIAN_FA_GRAD)
         return fail(PMMH_ERR_INVALID, "pmmh_flps_model_corr: unknown model id");
     if ((d_x_hist == nullptr) != (d_a_hist == nullptr))
         return fail(PMMH_ERR_INVALID, "d_x_hist and d_a_hist must be given together");
@@ -760,7 +764,7 @@ int pmmh_filter_model_corr(int model_id, const double* d_obs, long long obs_stri
     if (!d_obs || !d_params || !d_rvr || !d_u || !d_filt || !d_log_like || !d_traj || !d_diag)
         return fail(PMMH_ERR_INVALID, "pmmh_filter_model_corr: null pointer argument");
     if (model_id != PMMH_MODEL_SV_LEVERAGE && model_id != PMMH_MODEL_LINEAR_GAUSSIAN &&
-        model_id != PMMH_MODEL_LINEAR_GAUSSIAN_FA)
+        model_id != PMMH_MODEL_LINEAR_GAUSSIAN_FA && model_id != PMMH_MODEL_LINEAR_GAUSSIAN_FA_GRAD)
         return fail(PMMH_ERR_INVALID, "pmmh_filter_model_corr: unknown model id");
     if ((d_x_hist == nullptr) != (d_a_hist == nullptr))
         return fail(PMMH_ERR_INVALID, "d_x_hist and d_a_hist must be given together");
@@ -776,7 +780,7 @@ int pmmh_filter_model_corr(int model_id, const double* d_obs, long long obs_stri
     pmmh::SvCall c = {};
     c.obs = d_obs; c.obs_stride = obs_stride; c.params = d_params; c.rvr = d_rvr; c.u = d_u;
     c.filt = d_filt; c.ll = d_log_like; c.traj = d_traj; c.diag = d_diag;
-    c.x_hist = d_x_hist; c.a_hist = d_a_hist; c.model = model_id; c.filter = 1; c.prof = g_sv_prof;
+    c.x_hist = d_x_hist; c.a_hist = d_a_hist; c.model = filter_model(model_id); c.filter = 1; c.prof = g_sv_prof;
     c.ws = d_workspace; c.ws_bytes = workspace_bytes; c.stream = (cudaStream_t)stream;
     return sv_launch_plan(p, s, c);
 }
@@ -787,7 +791,7 @@ namespace {
 int grid_batch_plan(const char* who, int model_id, int n_obs, int n, int lag, int batch, int hess, int filter,
                     DeviceInfo* di, int* G, int* nteams, size_t* bytes) {
     if (model_id != PMMH_MODEL_SV_LEVERAGE && model_id != PMMH_MODEL_LINEAR_GAUSSIAN &&
-        model_id != PMMH_MODEL_LINEAR_GAUSSIAN_FA)
+        model_id != PMMH_MODEL_LINEAR_GAUSSIAN_FA && model_id != PMMH_MODEL_LINEAR_GAUSSIAN_FA_GRAD)
         return fail(PMMH_ERR_INVALID, who);
     if (hess && (filter || model_id != PMMH_MODEL_SV_LEVERAGE)) return fail(PMMH_ERR_INVALID, who);
     if (batch < 1 || n_obs < 2 || (hess != 0 && hess != 1)) return fail(PMMH_ERR_INVALID, who);
@@ -875,7 +879,7 @@ int pmmh_filter_model_batch_corr(int model_id, const double* d_obs, long long ob
     pmmh::SvCall c = {};
     c.obs = d_obs; c.obs_stride = obs_stride; c.params = d_params; c.rvr = d_rvr; c.u = d_u;
     c.filt = d_filt; c.ll = d_log_like; c.traj = d_traj; c.diag = d_diag;
-    c.x_hist = d_x_hist; c.a_hist = d_a_hist; c.model = model_id; c.filter = 1;
+    c.x_hist = d_x_hist; c.a_hist = d_a_hist; c.model = filter_model(model_id); c.filter = 1;
     c.ws = d_workspace; c.ws_bytes = workspace_bytes; c.stream = (cudaStream_t)stream;
     return pmmh::sv_grid_run(c, batch, n_obs, n_particles, 2, G, nteams, 0);
 }

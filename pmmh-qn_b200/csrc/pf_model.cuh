@@ -30,6 +30,8 @@
 //   M::kScoreIsZero                      constexpr: score_main / score_tail are identically 0 (the
 //                                        grid kernel then skips the calls; the smoother still runs)
 //   M::kReferenceIndexing                constexpr: how the fixed-lag terms are paired (below)
+//   M::kPredictiveScore                  constexpr: the exact pairing shifted for a fully adapted filter (below)
+//   M::score_last(c, x, y_next, g)       (kPredictiveScore only) the final generation's term
 //
 // kReferenceIndexing = true (the SV model, parity with the reference): the reference's quirks Q5 / Q6.  The main loop
 // at step i >= LAG adds the pair (x_tt, x_tt+1), tt = i - LAG + 1, with y = obs[tt - 1] (score_main, Q5) into slot tt;
@@ -41,6 +43,11 @@
 // initial_state for every particle, Q1), W_{NOBS-1} in the tail (t = NOBS-LAG+1 .. NOBS-2).  Gradient slot s holds
 // step s's contribution (the pair (x_s-1, x_s)); slot 0 is 0.  smo[t] = the weighted mean of x_t under the same
 // weights, every slot written once: the tail starts one step after the last main-loop slot.
+// kPredictiveScore = true (exact pairing on the shifted series of a fully adapted filter, model 4): the same pairs, read
+// under the same weights, but the pair (x_t, x_t+1) takes y = obs[t] (= y_t+1 of the unshifted series) and goes into
+// slot t; the final generation adds score_last(x_NOBS-1, obs[NOBS-1]) under W_{NOBS-1} into slot NOBS-1 (the pair
+// (x_NOBS-1, x_NOBS) with x_NOBS integrated out).  Slot t then holds the contribution of obs[t], and the slots sum
+// to an estimate of the score of the whole series.
 // Unused gradient slots stay 0.  Model ids are part of the C ABI (include/pmmh_qn.h).
 #pragma once
 #include <math.h>
@@ -59,6 +66,7 @@ struct SvLeverageModel {
     }
     static constexpr bool kScoreIsZero = false;
     static constexpr bool kReferenceIndexing = true;
+    static constexpr bool kPredictiveScore = false;
     static __device__ __forceinline__ double propagate(const Const& c, double xp, double y1, double u) {
         double mean = c.mu + c.phi * (xp - c.mu);
         mean += c.sr * exp(-0.5 * xp) * y1;
@@ -114,6 +122,7 @@ struct LinearGaussianModel {
     static __device__ __forceinline__ double initial_state(const Const&) { return 0.0; }
     static constexpr bool kScoreIsZero = false;
     static constexpr bool kReferenceIndexing = false;
+    static constexpr bool kPredictiveScore = false;
     static __device__ __forceinline__ double propagate(const Const& c, double xp, double, double u) {
         return c.phi * xp + c.sv * u;
     }
@@ -177,6 +186,7 @@ struct LinearGaussianFullyAdapted {
     // x_t | x_{t-1}, y_t ~ N(phi x + k (y_t - phi x), sv^2 se^2 / (sv^2 + se^2))
     static constexpr bool kScoreIsZero = true;
     static constexpr bool kReferenceIndexing = false;   // smo: x_t under W_{t+LAG-1}, i.e. given y_1 .. y_{t+LAG}
+    static constexpr bool kPredictiveScore = false;
     static __device__ __forceinline__ double propagate(const Const& c, double xp, double y_now, double u) {
         const double m = c.phi * xp;
         return (m + c.k * (y_now - m)) + c.sdp * u;
@@ -211,6 +221,49 @@ struct LinearGaussianFullyAdapted {
     }
     static __device__ __forceinline__ void score_tail(const Const&, double, double, double, double g[4]) {
         g[0] = g[1] = g[2] = g[3] = 0.0;
+    }
+};
+
+// ---- 4: model 2's fully adapted filter with a fixed-lag gradient.  Propagation, weights, shift and child range are
+// model 2's (inherited), so every output model 2 has -- filt, smo, log-likelihood, traj, diag, history -- is
+// bit-identical to it.  The gradient pairs the terms predictively (kPredictiveScore above): slot t holds the
+// contribution of obs'[t] = y_t+1, and the slots sum to an estimate of the score of log p(y_1 .. y_T), the first
+// observation's term included (the log-likelihood still lacks log p(y_1)).  Checked against the restatement
+// oracle/generic_pf.py LinearGaussianFullyAdaptedGrad and the exact fixed-lag Kalman targets of oracle/kalman.py.
+struct LinearGaussianFullyAdaptedGrad : LinearGaussianFullyAdapted {
+    struct Const : LinearGaussianFullyAdapted::Const {
+        double inv_sv2, inv_sv, inv_se2, inv_se;
+    };
+    static __device__ __forceinline__ void init(Const& c, const double* par) {
+        LinearGaussianFullyAdapted::init(c, par);
+        c.inv_sv2 = 1.0 / (c.sv * c.sv);
+        c.inv_sv = 1.0 / c.sv;
+        c.inv_se2 = 1.0 / (c.se * c.se);
+        c.inv_se = 1.0 / c.se;
+    }
+    static constexpr bool kScoreIsZero = false;
+    static constexpr bool kPredictiveScore = true;
+    // d/d(phi, sigma_v, sigma_e) of log N(next; phi curr, sigma_v^2) + log N(y; next, sigma_e^2), y = obs'[time(curr)]
+    static __device__ __forceinline__ void score_main(const Const& c, double curr, double next, double y, double g[4]) {
+        const double r = next - c.phi * curr;
+        const double ry = y - next;
+        g[0] = (r * curr) * c.inv_sv2;
+        g[1] = ((r * r) * c.inv_sv2 - 1.0) * c.inv_sv;
+        g[2] = ((ry * ry) * c.inv_se2 - 1.0) * c.inv_se;
+        g[3] = 0.0;
+    }
+    static __device__ __forceinline__ void score_tail(const Const& c, double curr, double next, double y, double g[4]) {
+        score_main(c, curr, next, y, g);
+    }
+    // d/d(phi, sigma_v, sigma_e) of log N(y_next; phi x, sigma_v^2 + sigma_e^2): the last pair with its second state
+    // integrated out (the conditional score of that state has mean 0)
+    static __device__ __forceinline__ void score_last(const Const& c, double x, double y_next, double g[4]) {
+        const double r = y_next - c.phi * x;
+        const double a = (r * r) * c.inv_s2 - 1.0;
+        g[0] = (r * x) * c.inv_s2;
+        g[1] = (a * c.sv) * c.inv_s2;
+        g[2] = (a * c.se) * c.inv_s2;
+        g[3] = 0.0;
     }
 };
 

@@ -484,8 +484,10 @@ __global__ void __launch_bounds__(kCT, 1) sv_chain_kernel(SvArgs a) {
                 // pairing of the fixed-lag terms (pf_model.cuh): the reference's (Q5 / Q6) or the exact one, whose main
                 // loop starts one step earlier (the pair (x_0, x_1) at step LAG - 1) and whose tail starts one step later
                 const bool lagged = SMO && inext >= (M::kReferenceIndexing ? LAG : LAG - 1);
-                // the pair (x_tt, x_tt+1), tt = inext - LAG + 1: y = obs[tt - 1] (Q5) or obs[tt + 1]
-                const double yl = lagged ? obs[M::kReferenceIndexing ? inext - LAG : inext - LAG + 2] : 0.0;
+                // the pair (x_tt, x_tt+1), tt = inext - LAG + 1: y = obs[tt - 1] (Q5), obs[tt + 1], or obs[tt] (predictive)
+                const double yl = lagged ? obs[M::kReferenceIndexing ? inext - LAG
+                                                                     : (M::kPredictiveScore ? inext - LAG + 1 : inext - LAG + 2)]
+                                         : 0.0;
                 const int hop0 = (K >= 1) ? ((K - 1) & 3) : 0;
                 const int nh = (K >= 1) ? ((K - 1) >> 2) : 0;        // 0 or 1 (LAG <= 10)
                 const int g1 = inext - (hop0 + 1);
@@ -550,7 +552,8 @@ __global__ void __launch_bounds__(kCT, 1) sv_chain_kernel(SvArgs a) {
                 o_traj[inext] = s_x[0];   // Q11: traj[i] = X_i[0]
                 if constexpr (SMO) if (inext >= (M::kReferenceIndexing ? LAG : LAG - 1)) {
                     const int tt = inext - LAG + 1;
-                    const int gs = M::kReferenceIndexing ? tt : tt + 1;   // gradient slot: tt (Q5) or the pair's second step
+                    // gradient slot: tt (Q5, predictive) or the pair's second step
+                    const int gs = (M::kReferenceIndexing || M::kPredictiveScore) ? tt : tt + 1;
                     o_smo[tt] = acc[1] / S_i;
                     o_grad[gs] = acc[2] / S_i;
                     o_grad[NOBS + gs] = acc[3] / S_i;
@@ -563,7 +566,8 @@ __global__ void __launch_bounds__(kCT, 1) sv_chain_kernel(SvArgs a) {
             CPROF(4);   // cumulative weights, sums, fixed-lag terms, outputs
         }   // time loop
 
-        // ---------------- tail (:540-562, Q6; exact pairing: slots NOBS-LAG+1 .. NOBS-1, pairs under the final weights)
+        // ---------------- tail (:540-562, Q6; exact pairing: slots NOBS-LAG+1 .. NOBS-1, pairs under the final weights;
+        // predictive: the same slots, k = 0 adds the final generation's term into slot T)
         if (SMO && status == 0) {
             const int T = NOBS - 1;
             const double S_T = s_S[T % kMaxLagC];
@@ -576,7 +580,8 @@ __global__ void __launch_bounds__(kCT, 1) sv_chain_kernel(SvArgs a) {
                 for (int q = 0; q < NT; ++q) tacc[q] = 0.0;
                 const double ylag = obs_wrap(obs, ip - LAG, NOBS);
                 const double S_ip = s_S[ip % kMaxLagC];
-                const double y1 = M::kReferenceIndexing ? obs_wrap(obs, ip - 1, NOBS) : (k >= 1 ? obs[ip + 1] : 0.0);
+                const double y1 = M::kReferenceIndexing ? obs_wrap(obs, ip - 1, NOBS)
+                                                        : (M::kPredictiveScore ? obs[ip] : (k >= 1 ? obs[ip + 1] : 0.0));
                 const double* shI = SHG(ip);
                 for (int j = tid; j < N; j += kCT) {
                     int b = j, bprev = j;
@@ -614,13 +619,21 @@ __global__ void __launch_bounds__(kCT, 1) sv_chain_kernel(SvArgs a) {
                         tacc[2] += g[1] * wi;
                         tacc[3] += g[2] * wi;
                         tacc[4] += g[3] * wi;
+                    } else if constexpr (M::kPredictiveScore) {   // the final generation's term
+                        const double wi = sT / S_T;
+                        double g[4];
+                        M::score_last(c, curr, y1, g);
+                        tacc[1] += g[0] * wi;
+                        tacc[2] += g[1] * wi;
+                        tacc[3] += g[2] * wi;
+                        tacc[4] += g[3] * wi;
                     }
                 }
                 block_sum<NT>(tacc, s_red);
                 if (tid == 0) {
                     o_smo[ip] += tacc[0];
-                    if (k >= 1) {
-                        const int tt = M::kReferenceIndexing ? ip - LAG + 1 : ip + 1;
+                    if (k >= 1 || M::kPredictiveScore) {
+                        const int tt = M::kReferenceIndexing ? ip - LAG + 1 : (M::kPredictiveScore ? ip : ip + 1);
                         if (tt >= 0) {
                             o_grad[tt] += tacc[1];
                             o_grad[NOBS + tt] += tacc[2];
@@ -710,6 +723,7 @@ cudaError_t sv_chain_launch(const SvArgs& a, int grid, int filter, cudaStream_t 
                                        : chain_launch_one<SvLeverageModel, false, true>(a, grid, smem, stream);
     if (a.model_id == 1 && !a.hess) return chain_launch_one<LinearGaussianModel, false, true>(a, grid, smem, stream);
     if (a.model_id == 2 && !a.hess) return chain_launch_one<LinearGaussianFullyAdapted, false, true>(a, grid, smem, stream);
+    if (a.model_id == 4 && !a.hess) return chain_launch_one<LinearGaussianFullyAdaptedGrad, false, true>(a, grid, smem, stream);
     return cudaErrorInvalidValue;
 }
 

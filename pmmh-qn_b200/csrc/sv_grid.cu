@@ -1366,8 +1366,8 @@ __global__ void __launch_bounds__(GT, 1) sv_grid_kernel(const GridArgs a_in, con
             if constexpr (GEN) {
                 // generic path: sc[0] = sum sh curr (smoother), sc[1 + k] = sum sh g[k] of M::score_main on the pair
                 // (curr, next) = (parent value, own value) of the ancestor = (x_tt, x_tt+1), tt = t - LAG + 1;
-                // y = obs[t - LAG] (Q5) or obs[tt + 1]
-                const double yl = a.obs[M::kReferenceIndexing ? t - L : t - L + 2];
+                // y = obs[t - LAG] (Q5), obs[tt + 1], or obs[tt] (predictive)
+                const double yl = a.obs[M::kReferenceIndexing ? t - L : (M::kPredictiveScore ? t - L + 1 : t - L + 2)];
 #pragma unroll
                 for (int k0 = 0; k0 < KPT; k0 += 4) {
                     double pc[4], px[4];
@@ -1574,7 +1574,8 @@ __global__ void __launch_bounds__(256) grid_reduce_kernel(const double* __restri
 // part[irel][block][0] = sum_p W_T[p] hist_idx[p];  [1..4] = sum_p W_i[p] g(hist_idx, hist_idx-1)
 // with i = NOBS - L + irel, idx = L - 1 - irel; hist_k[p] = value of the ancestor k steps back of
 // the particle at sorted position p of the final generation.  Exact pairing (pf_model.cuh, !M::kReferenceIndexing):
-// irel = 0 is 0 (the main loop has that slot), the pair is weighted by W_T and takes y = obs[i + 1].
+// irel = 0 is 0 (the main loop has that slot), the pair is weighted by W_T and takes y = obs[i + 1]; predictive pairing
+// (M::kPredictiveScore): y = obs[i], and irel = L - 1 (idx = 0, i = T) adds M::score_last of the final particle.
 // HESS: partH[irel][block][0..19] = the hessian1 / hessian2 terms of :564-626 (alpha of the ancestor LAG-2 steps
 // back of the final particle, weights W_i, obs[i - LAG] with wrap-around, Q8).  M: the model (g = M::score_tail).
 template <bool HESS, class M>
@@ -1588,7 +1589,7 @@ __global__ void __launch_bounds__(256) grid_tail_kernel(GridArgs a, const double
     typename M::Const k;
     M::init(k, a.params);
     constexpr bool REF = M::kReferenceIndexing;
-    const double y1 = REF ? obs_wrap(a.obs, i - 1, a.NOBS) : a.obs[min(i + 1, T)];
+    const double y1 = REF ? obs_wrap(a.obs, i - 1, a.NOBS) : a.obs[M::kPredictiveScore ? i : min(i + 1, T)];
     const double ST = sums[(size_t)T * 8], Si = sums[(size_t)i * 8];
     const double* shT = a.shring + (size_t)(T % L) * N;
     const double* shi = a.shring + (size_t)(i % L) * N;
@@ -1609,6 +1610,12 @@ __global__ void __launch_bounds__(256) grid_tail_kernel(GridArgs a, const double
         if (idx == 0) {
             curr = a.XE[p].x;
             acc[0] += wT * curr;
+            if constexpr (M::kPredictiveScore) {
+                double g[4];
+                M::score_last(k, curr, y1, g);
+#pragma unroll
+                for (int q = 0; q < 4; ++q) acc[1 + q] += g[q] * wT;
+            }
         } else {
             // entry of the ancestor idx-1 steps back holds (next = its value, curr = its parent's value)
             const int m = idx - 1;
@@ -1736,12 +1743,16 @@ __global__ void __launch_bounds__(256) grid_tail_reduce_kernel(const double* __r
 // sums[t][0] = sum sh, [1] = sum sh x, [2] = sum sh c, [3] = sum sh sq, [4] = sum sh sq c, [5] = sum sh sq^2,
 // [6] = sum sh sq ey (c = lagged ancestor value, sq / ey as stored in P);  tail[irel][0..4].
 // GEN (the generic path of a model other than SV): [3..6] = sum sh g[0..3], traj[0] = the initial state, exact pairing of
-// the fixed-lag terms (pf_model.cuh; models 1 and 2 have kReferenceIndexing = false).
+// the fixed-lag terms (pf_model.cuh; models 1, 2 and 4 have kReferenceIndexing = false).  PRED: the predictive pairing
+// (M::kPredictiveScore, model 4).
 // SMO = false (the filter alone): no smo / grad, tail unused.
 static_assert(SvLeverageModel::kReferenceIndexing && !LinearGaussianModel::kReferenceIndexing &&
-                  !LinearGaussianFullyAdapted::kReferenceIndexing,
+                  !LinearGaussianFullyAdapted::kReferenceIndexing && !LinearGaussianFullyAdaptedGrad::kReferenceIndexing,
               "grid_finish_kernel pairs the fixed-lag terms as the reference does for SV (GEN = false), exactly otherwise");
-template <bool GEN, bool SMO>
+static_assert(!SvLeverageModel::kPredictiveScore && !LinearGaussianModel::kPredictiveScore &&
+                  !LinearGaussianFullyAdapted::kPredictiveScore && LinearGaussianFullyAdaptedGrad::kPredictiveScore,
+              "grid_finish_kernel places the predictive pairing's slots for model 4 only (PRED)");
+template <bool GEN, bool SMO, bool PRED = false>
 __global__ void grid_finish_kernel(const GridCtrl* __restrict__ ctrl, const double* __restrict__ sums,
                                    const double* __restrict__ shift, const double* __restrict__ xmin,
                                    const double* __restrict__ tail, const double* __restrict__ params,
@@ -1790,7 +1801,22 @@ __global__ void grid_finish_kernel(const GridCtrl* __restrict__ ctrl, const doub
         traj[t] = (t == 0 && !GEN) ? params[0] : xmin[t];   // Q10/Q11: traj[t] = X_t[0] for t >= 1, X_0 == mu
         if constexpr (!SMO) continue;
         double s = 0.0, g[4] = {0.0, 0.0, 0.0, 0.0};
-        if constexpr (GEN) {
+        if constexpr (PRED) {
+            // predictive pairing (pf_model.cuh): smo[t] and gradient slot t (the pair (x_t, x_t+1) with obs[t]) from step
+            // t + L - 1; every tail block irel >= 1 adds smo[nobs-L+irel] and gradient[.][nobs-L+irel] (irel = L - 1: the
+            // final generation's term); irel = 0 is empty
+            const int ss = t + L - 1;
+            if (ss < nobs) {
+                const double* sm = sums + (size_t)ss * 8;
+                s = sm[2] / sm[0];
+                for (int q = 0; q < 4; ++q) g[q] = sm[3 + q] / sm[0];
+            }
+            const int irel = t - (nobs - L);
+            if (irel >= 1 && irel < L) {
+                s += tail[irel * 8];
+                for (int q = 0; q < 4; ++q) g[q] += tail[irel * 8 + 1 + q];
+            }
+        } else if constexpr (GEN) {
             // exact pairing (pf_model.cuh): smo[t] from step t + L - 1 (t >= 0), gradient slot t = the pair (x_t-1, x_t)
             // from step t + L - 2; the tail (irel >= 1) adds smo[nobs-L+irel] and gradient[.][nobs-L+irel+1]
             const int ss = t + L - 1, sg = t + L - 2;
@@ -1896,6 +1922,7 @@ const void* grid_kernel_for(int model, int hess, int filter, bool team) {
     }
     if (model == PMMH_MODEL_LINEAR_GAUSSIAN) return grid_kernel_of<false, LinearGaussianModel, true>(team);
     if (model == PMMH_MODEL_LINEAR_GAUSSIAN_FA) return grid_kernel_of<false, LinearGaussianFullyAdapted, true>(team);
+    if (model == PMMH_MODEL_LINEAR_GAUSSIAN_FA_GRAD) return grid_kernel_of<false, LinearGaussianFullyAdaptedGrad, true>(team);
     return hess ? grid_kernel_of<true, SvLeverageModel, true>(team) : grid_kernel_of<false, SvLeverageModel, true>(team);
 }
 
@@ -1903,7 +1930,8 @@ int grid_check(const SvCall& c, int nobs, int n, int lag, int G, int hess) {
     if (c.filter ? (hess || !sv_grid_filter_eligible(nobs, n, G)) : !sv_grid_eligible(nobs, n, lag, G))
         return set_error(PMMH_ERR_INVALID, "grid kernel: sizes not eligible");
     const int model = c.model;
-    if (model != PMMH_MODEL_SV_LEVERAGE && model != PMMH_MODEL_LINEAR_GAUSSIAN && model != PMMH_MODEL_LINEAR_GAUSSIAN_FA)
+    if (model != PMMH_MODEL_SV_LEVERAGE && model != PMMH_MODEL_LINEAR_GAUSSIAN && model != PMMH_MODEL_LINEAR_GAUSSIAN_FA &&
+        !(model == PMMH_MODEL_LINEAR_GAUSSIAN_FA_GRAD && !c.filter))   // (the entries run model 4's filter as model 2's)
         return set_error(PMMH_ERR_INVALID, "grid kernel: unknown model id");
     if (hess && model != PMMH_MODEL_SV_LEVERAGE)
         return set_error(PMMH_ERR_INVALID, "grid kernel: the Hessian branch exists for the SV model only");
@@ -1920,9 +1948,10 @@ int grid_set_attributes() {
         // (DESIGN 4.0), and left unset the evaluation at N = 2^20 is ~6 % slower
         GRID_CUDA(cudaDeviceSetLimit(cudaLimitPersistingL2CacheSize, 0));
         for (int team = 0; team < 2; ++team)
-            for (int model = 0; model < 3; ++model)
-                for (int v = 0; v < 3; ++v)   // smoother, smoother with Hessian (SV only), filter
-                    if (v != 1 || model == PMMH_MODEL_SV_LEVERAGE)
+            for (int model = 0; model <= PMMH_MODEL_LINEAR_GAUSSIAN_FA_GRAD; ++model)
+                for (int v = 0; v < 3; ++v)   // smoother, smoother with Hessian (SV only), filter (not model 4: model 2's)
+                    if (model != 3 && (v != 1 || model == PMMH_MODEL_SV_LEVERAGE) &&   // (3 is not a model id)
+                        (v != 2 || model != PMMH_MODEL_LINEAR_GAUSSIAN_FA_GRAD))
                         GRID_CUDA(cudaFuncSetAttribute(grid_kernel_for(model, v == 1, v == 2, team != 0),
                                                        cudaFuncAttributeMaxDynamicSharedMemorySize, kDynSmem));
         attr_set[dev] = true;
@@ -2010,11 +2039,16 @@ int grid_after(const SvCall& c, const GridArgs& a, const GridLayout& L, char* ws
         grid_tail_kernel<false, LinearGaussianModel><<<dim3(L.nblk, lag), 256, 0, st>>>(a, sums, tailpart, nullptr, L.nblk);
     } else if (model == PMMH_MODEL_LINEAR_GAUSSIAN_FA) {
         grid_tail_kernel<false, LinearGaussianFullyAdapted><<<dim3(L.nblk, lag), 256, 0, st>>>(a, sums, tailpart, nullptr, L.nblk);
+    } else if (model == PMMH_MODEL_LINEAR_GAUSSIAN_FA_GRAD) {
+        grid_tail_kernel<false, LinearGaussianFullyAdaptedGrad><<<dim3(L.nblk, lag), 256, 0, st>>>(a, sums, tailpart, nullptr,
+                                                                                                L.nblk);
     } else {
         grid_tail_kernel<false, SvLeverageModel><<<dim3(L.nblk, lag), 256, 0, st>>>(a, sums, tailpart, nullptr, L.nblk);
     }
     grid_tail_reduce_kernel<<<lag, 256, 0, st>>>(tailpart, L.nblk, tail);
-    auto finish = model == PMMH_MODEL_SV_LEVERAGE ? grid_finish_kernel<false, true> : grid_finish_kernel<true, true>;
+    auto finish = model == PMMH_MODEL_SV_LEVERAGE            ? grid_finish_kernel<false, true>
+                  : model == PMMH_MODEL_LINEAR_GAUSSIAN_FA_GRAD ? grid_finish_kernel<true, true, true>
+                                                                : grid_finish_kernel<true, true>;
     finish<<<(nobs + 255) / 256, 256, 0, st>>>(a.ctrl, sums, a.shiftv, a.xminv, tail, c.params, nobs, lag, (double)n, c.ll,
                                                c.filt, c.smo, c.grad, c.traj, c.diag, (long long*)(ws + L.info));
     GRID_CUDA(cudaGetLastError());

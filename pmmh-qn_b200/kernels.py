@@ -137,7 +137,10 @@ def flps_model_corr(model_id, obs, params, rvr, u, lag=10, store_history=False, 
     kernel, diag kernel 3).  Above: B == 1, n_obs >= 2 lag and up to 7168 particles per SM (1,060,864 on
     148 SMs), one persistent launch over the GPU (grid kernel, diag kernel 5).  Other sizes raise PmmhError.
     ``model_id``: _lib.MODEL_SV_LEVERAGE (bit-identical to flps_sv_corr on the same kernel),
-    _lib.MODEL_LINEAR_GAUSSIAN or _lib.MODEL_LINEAR_GAUSSIAN_FA; params [B, 4] (unused slots ignored).
+    _lib.MODEL_LINEAR_GAUSSIAN, _lib.MODEL_LINEAR_GAUSSIAN_FA or _lib.MODEL_LINEAR_GAUSSIAN_FA_GRAD; params [B, 4]
+    (unused slots ignored).  The fully adapted models 2 and 3 take the series shifted by one (obs[1:]) and their
+    log_like lacks log p(y_1); model 4 adds model 2 a gradient whose slot k holds the contribution of obs[1:][k], so
+    that the slots sum to the score of the full log-likelihood (include/pmmh_qn.h).
     No fallback pass: diag[:, PMMH_DIAG_STATUS] == 1 reports an abandoned evaluation."""
     lib = _lib.load()
     obs, obs_stride, params, rvr, u, batch, n_obs, n = _sv_common(obs, params, rvr, u)
@@ -161,7 +164,7 @@ def filter_model_corr(model_id, obs, params, rvr, u, store_history=False, worksp
     diag of [B] problems without the fixed-lag smoother -- bit-identical to those outputs of flps_model_corr
     for any lag.  Up to 4096 particles: any B (chain kernel, diag kernel 3).  Above: B == 1 and up to 7168
     particles per SM (grid kernel, diag kernel 5).  n_obs >= 2; other sizes raise PmmhError.  ``model_id`` and
-    params as for flps_model_corr.  No fallback pass: diag[:, PMMH_DIAG_STATUS] == 1 reports an abandoned
+    params as for flps_model_corr (model 4 runs model 2's filter).  No fallback pass: diag[:, PMMH_DIAG_STATUS] == 1 reports an abandoned
     evaluation."""
     lib = _lib.load()
     obs, obs_stride, params, rvr, u, batch, n_obs, n = _sv_common(obs, params, rvr, u)
@@ -202,7 +205,7 @@ def flps_model_batch_corr(model_id, obs, params, rvr, u, lag=10, compute_hessian
     outputs of problem b are bit-identical to flps_model_corr on that problem alone with B == 1 (and, for
     _lib.MODEL_SV_LEVERAGE, to flps_sv_corr on the grid kernel, also with the Hessian).  Any B on every shape the
     one-problem grid run takes (above 4096 particles: n_obs >= 2 lag, up to 7168 particles per CTA of
-    ceil(N / 2048)); compute_hessian for the SV model only.  Returns the dict of flps_model_corr, plus hess1 /
+    ceil(N / 2048)); model ids as for flps_model_corr; compute_hessian for the SV model only.  Returns the dict of flps_model_corr, plus hess1 /
     hess2 [B, 4, 4] with compute_hessian.  No fallback pass: diag[:, PMMH_DIAG_STATUS] == 1 reports an abandoned
     problem, the others are unaffected."""
     lib = _lib.load()

@@ -1,12 +1,16 @@
 #!/usr/bin/env python
 """pmmh_flps_model_corr on the grid kernel at the headline shape: one problem, N = 2^20, T = 1000 (n_obs = 1001),
-lag 10.  Four cases, each timed with CUDA events over several evaluations after warm-up:
+lag 10.  Five cases, each timed with CUDA events over several evaluations after warm-up:
 
   lg_bootstrap  the linear Gaussian bootstrap filter (LG_PARAM_SETS[0], observations from golden_inputs.lg_obs)
   lg_fa         the same model as a fully adapted filter (observations shifted by one, n_obs - 1 steps)
+  lg_fa_grad    the fully adapted filter with its fixed-lag gradient (model id 4, lg_fa's inputs)
   sv_model      the SV model through pmmh_flps_model_corr (model id 0)
   sv_entry      pmmh_flps_sv_corr on the same SV inputs (algorithm 0: the grid kernel at this N)
 
+--cases picks some of them, --rounds R runs the chosen cases in turn R times (alternating them; ms_per_eval is then the
+list of the rounds, and the rate is of the fastest).  With lg_fa and lg_fa_grad both run, "fa_grad_shares_fa" says
+whether lg_fa_grad's filt, smo, log_like, traj and diag equal lg_fa's bit for bit.
 Prints one JSON line: ms per evaluation, particle-steps/s (N x steps / time), the card's name and power limit.
 Writes nothing unless --out FILE is given (the line is then appended there as well).
 """
@@ -55,6 +59,8 @@ def main():
     ap.add_argument("--lag", type=int, default=10)
     ap.add_argument("--reps", type=int, default=5)
     ap.add_argument("--warmup", type=int, default=2)
+    ap.add_argument("--cases", default="lg_bootstrap,lg_fa,lg_fa_grad,sv_model,sv_entry")
+    ap.add_argument("--rounds", type=int, default=1)
     ap.add_argument("--out", default=None)
     args = ap.parse_args()
     if not torch.cuda.is_available():
@@ -78,6 +84,8 @@ def main():
                                                          workspace=ws)),
         "lg_fa": (nobs - 1, lambda: K.flps_model_corr(_lib.MODEL_LINEAR_GAUSSIAN_FA, fa_obs, lg_par, fa_rvr, fa_u,
                                                       lag=lag, workspace=ws)),
+        "lg_fa_grad": (nobs - 1, lambda: K.flps_model_corr(_lib.MODEL_LINEAR_GAUSSIAN_FA_GRAD, fa_obs, lg_par, fa_rvr,
+                                                           fa_u, lag=lag, workspace=ws)),
         "sv_model": (nobs, lambda: K.flps_model_corr(_lib.MODEL_SV_LEVERAGE, sv_obs, sv_par, rvr, u, lag=lag,
                                                      workspace=ws)),
         "sv_entry": (nobs, lambda: K.flps_sv_corr(sv_obs, sv_par, rvr, u, lag=lag, compute_hessian=False,
@@ -85,12 +93,22 @@ def main():
     }
     res = {"N": n, "n_obs": nobs, "lag": lag, "reps": args.reps, "warmup": args.warmup,
            "gpu": torch.cuda.get_device_name(0), "power_limit": power_limit()}
-    for name, (steps, fn) in cases.items():
-        ms, out = timed(fn, args.reps, args.warmup)
+    names = args.cases.split(",")
+    times, outs = dict((k, []) for k in names), {}
+    for _ in range(args.rounds):
+        for name in names:
+            ms, outs[name] = timed(cases[name][1], args.reps, args.warmup)
+            times[name].append(round(ms, 3))
+    for name in names:
+        steps, out, ms = cases[name][0], outs[name], times[name]
         d = out["diag"][0].cpu().numpy()
-        res[name] = {"ms_per_eval": round(ms, 3), "particle_steps_per_s": float("%.4g" % (n * (steps - 1) / (ms * 1e-3))),
+        res[name] = {"ms_per_eval": ms[0] if len(ms) == 1 else ms,
+                     "particle_steps_per_s": float("%.4g" % (n * (steps - 1) / (min(ms) * 1e-3))),
                      "kernel": int(d[_lib.DIAG_KERNEL]), "status": int(d[_lib.DIAG_STATUS]),
                      "log_like": float(out["log_like"][0])}
+    if "lg_fa" in outs and "lg_fa_grad" in outs:
+        res["fa_grad_shares_fa"] = all(torch.equal(outs["lg_fa"][k], outs["lg_fa_grad"][k])
+                                       for k in ("filt", "smo", "log_like", "traj", "diag"))
     line = json.dumps(res)
     print(line)
     if args.out:
