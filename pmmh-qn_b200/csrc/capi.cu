@@ -12,6 +12,7 @@
 
 #include "../../include/pmmh_qn.h"
 #include "aux_kernels.cuh"
+#include "pf_model.cuh"
 #include "sv_filter.cuh"
 #include "sv_grid.cuh"
 #include "sv_split.cuh"
@@ -666,53 +667,104 @@ int pmmh_flps_sv_corr_streamed(const double* h_rvs, const double* d_obs, const d
 
 // ---- model-generic entry points: the chain or the grid kernel instantiated for a model of pf_model.cuh ----------
 namespace {
-// the model whose filter instantiation a filter entry runs: model 4 adds a gradient to model 2, so its filter is model 2's
-int filter_model(int model_id) {
-    return model_id == PMMH_MODEL_LINEAR_GAUSSIAN_FA_GRAD ? PMMH_MODEL_LINEAR_GAUSSIAN_FA : model_id;
+// The workspace queries take no model id: any model takes their shapes, the Hessian a model that has it.
+constexpr int kQueryModel = PMMH_MODEL_SV_LEVERAGE;
+
+// the four entries: one problem or a batch (`batched`), the smoother or the filter alone (`filter`, lag 2: no lag
+// condition); their names (pmmh_<name>_corr, pmmh_<name>_workspace_bytes) and the shapes they take, for the refusals
+std::string model_entry_name(bool batched, int filter) {
+    return std::string(filter ? "pmmh_filter_model" : "pmmh_flps_model") + (batched ? "_batch" : "");
 }
-// The plan pmmh_flps_model_corr (filter = 0) or pmmh_filter_model_corr (filter = 1, lag 2: no lag condition) runs:
-// the chain kernel wherever it applies (any batch), else the grid kernel for one problem on sv_grid_ctas(N, SMs, 0)
-// CTAs; anything else is refused.  The workspace is the chosen kernel's alone (there is no fallback pass), with
-// history on the grid kernel (the query has no flag).
-int model_choose(int n_obs, int n, int lag, int batch, int filter, DeviceInfo* di, SvPlan* p) {
-    if (n_obs < 2 || batch < 1)
-        return fail(PMMH_ERR_INVALID, filter ? "pmmh_filter_model_corr: bad arguments" : "pmmh_flps_model_corr: bad arguments");
+const char* model_entry_shapes(bool batched, int filter) {
+    if (batched)
+        return filter ? "pmmh_filter_model_batch_corr: batch >= 1, n_obs >= 2, a tile of n_particles / "
+                        "ceil(n_particles / 2048) particles fits one CTA and a known model id"
+                      : "pmmh_flps_model_batch_corr: batch >= 1, 2 <= lag <= 10, n_obs >= 2 lag, a tile of n_particles / "
+                        "ceil(n_particles / 2048) particles fits one CTA, a known model id, compute_hessian only for the "
+                        "SV model";
+    return filter ? "pmmh_filter_model_corr: a known model id, n_obs >= 2 and 2 <= n_particles <= 4096 (any batch), "
+                    "or batch == 1 and n_particles up to 7168 per SM (1,060,864 on 148 SMs)"
+                  : "pmmh_flps_model_corr: a known model id, 2 <= lag <= 10 and 2 <= n_particles <= 4096 (any batch), "
+                    "or batch == 1, n_obs >= 2 lag and n_particles up to 7168 per SM (1,060,864 on 148 SMs)";
+}
+
+// The plan of a model entry: its kernel (c.kernel), CTAs per problem on the grid kernel (c.grid_G), teams (n_teams)
+// and workspace (total: the chosen kernel's alone, there is no fallback pass; with history on the grid kernel).
+// One problem: the chain kernel wherever it applies (any batch; one CTA per problem, at most one problem per SM at a
+// time), else the grid kernel for one problem on sv_grid_ctas(N, SMs, 0) CTAs.  A batch: the grid kernel, one team of
+// that many CTAs per problem.  Anything else is refused.
+int model_plan(bool batched, int filter, int model_id, int n_obs, int n, int lag, int batch, int hess, DeviceInfo* di,
+               SvPlan* p) {
+    const char* shapes = model_entry_shapes(batched, filter);
+    if (!pmmh::model_known(model_id) || (hess && (filter || !pmmh::model_has_hessian(model_id))))
+        return fail(PMMH_ERR_INVALID, shapes);
+    if (batch < 1 || n_obs < 2 || (hess != 0 && hess != 1)) return fail(PMMH_ERR_INVALID, shapes);
     int rc = get_device_info(di);
     if (rc != PMMH_OK) return rc;
     memset(p, 0, sizeof(*p));
-    p->c.grid_G = pmmh::sv_grid_ctas(n, di->sm, 0);
-    // G, n_teams and grid are the chain kernel's launch shape (one CTA per problem, at most one problem per SM at a
-    // time); the grid plan carries them unused (sv_grid_run reads grid_G only)
-    p->G = 1;
-    p->n_teams = p->grid = batch < di->sm ? batch : di->sm;
-    if (pmmh::sv_chain_eligible(n, lag) && pmmh::sv_chain_smem_bytes(n) <= kMaxDynSmem) {
+    const int G = p->c.grid_G = pmmh::sv_grid_ctas(n, di->sm, 0);
+    if (!batched && pmmh::sv_chain_eligible(n, lag) && pmmh::sv_chain_smem_bytes(n) <= kMaxDynSmem) {
         p->c.kernel = SvKernel::Chain;
+        p->G = 1;
+        p->n_teams = p->grid = batch < di->sm ? batch : di->sm;
         p->chain_stride = pmmh::sv_chain_ws_bytes(n, lag, n_obs, 0, filter);
         p->total = (size_t)p->grid * p->chain_stride;
-    } else if (batch == 1 && (filter ? pmmh::sv_grid_filter_eligible(n_obs, n, p->c.grid_G)
-                                     : pmmh::sv_grid_eligible(n_obs, n, lag, p->c.grid_G))) {
+    } else if ((batched || batch == 1) && (filter ? pmmh::sv_grid_filter_eligible(n_obs, n, G)
+                                                  : pmmh::sv_grid_eligible(n_obs, n, lag, G))) {
         p->c.kernel = SvKernel::Grid;
-        p->total = pmmh::sv_grid_ws_bytes(n_obs, n, lag, p->c.grid_G, 1, 0, filter);
-    } else if (filter) {
-        return fail(PMMH_ERR_INVALID, "pmmh_filter_model_corr: n_obs >= 2 and 2 <= n_particles <= 4096 (any batch), "
-                                      "or batch == 1 and n_particles up to 7168 per SM (1,060,864 on 148 SMs)");
+        p->n_teams = pmmh::sv_grid_teams(batch, di->sm, G);
+        p->total = (size_t)p->n_teams * pmmh::sv_grid_ws_bytes(n_obs, n, lag, G, 1, hess, filter);
     } else {
-        return fail(PMMH_ERR_INVALID, "pmmh_flps_model_corr: 2 <= lag <= 10 and 2 <= n_particles <= 4096 (any batch), "
-                                      "or batch == 1, n_obs >= 2 lag and n_particles up to 7168 per SM "
-                                      "(1,060,864 on 148 SMs)");
+        return fail(PMMH_ERR_INVALID, shapes);
     }
     return PMMH_OK;
+}
+
+int model_query(bool batched, int filter, int n_obs, int n, int lag, int batch, int hess, size_t* bytes) {
+    if (!bytes)
+        return fail(PMMH_ERR_INVALID, (model_entry_name(batched, filter) + "_workspace_bytes: bytes is null").c_str());
+    DeviceInfo di;
+    SvPlan p;
+    int rc = model_plan(batched, filter, kQueryModel, n_obs, n, lag, batch, hess, &di, &p);
+    if (rc == PMMH_OK) *bytes = p.total;
+    return rc;
+}
+
+// Checks and runs one model entry (the filter: d_smo, d_grad unused; the Hessian outputs: batched smoother only).
+// No fallback pass: an abandoned evaluation is reported in d_diag[PMMH_DIAG_STATUS].
+int model_run(bool batched, int filter, int model_id, const double* d_obs, long long obs_stride, const double* d_params,
+              const double* d_rvr, const double* d_u, int n_obs, int n, int lag, int batch, int hess, double* d_filt,
+              double* d_smo, double* d_ll, double* d_grad, double* d_traj, double* d_h1, double* d_h2,
+              long long* d_diag, double* d_xh, int* d_ah, void* d_ws, size_t ws_bytes, void* stream) {
+    const std::string name = model_entry_name(batched, filter) + "_corr";
+    if (!d_obs || !d_params || !d_rvr || !d_u || !d_filt || !d_ll || !d_traj || !d_diag ||
+        (!filter && (!d_smo || !d_grad)) || (!d_ws && (batched || !filter)) || (hess && (!d_h1 || !d_h2)))
+        return fail(PMMH_ERR_INVALID, (name + ": null pointer argument").c_str());
+    if ((d_xh == nullptr) != (d_ah == nullptr))
+        return fail(PMMH_ERR_INVALID, "d_x_hist and d_a_hist must be given together");
+    if (!batched && !filter && n_obs < lag + 1) return fail(PMMH_ERR_INVALID, "n_obs must be at least lag + 1");
+    DeviceInfo di;
+    SvPlan p;
+    int rc = model_plan(batched, filter, model_id, n_obs, n, lag, batch, hess, &di, &p);
+    if (rc != PMMH_OK) return rc;
+    if (ws_bytes < p.total) return fail(PMMH_ERR_WORKSPACE, (name + ": workspace too small").c_str());
+    if (p.total && !d_ws) return fail(PMMH_ERR_INVALID, (name + ": null workspace").c_str());
+    rc = check_device(di, p.c.kernel == SvKernel::Grid);
+    if (rc != PMMH_OK) return rc;
+    pmmh::SvCall c = {};
+    c.obs = d_obs; c.obs_stride = obs_stride; c.params = d_params; c.rvr = d_rvr; c.u = d_u;
+    c.filt = d_filt; c.smo = d_smo; c.ll = d_ll; c.grad = d_grad; c.traj = d_traj; c.diag = d_diag;
+    if (hess) { c.hess1 = d_h1; c.hess2 = d_h2; }
+    c.x_hist = d_xh; c.a_hist = d_ah; c.model = model_id; c.filter = filter;
+    c.prof = batched ? nullptr : g_sv_prof;   // (phase clocks: one problem only)
+    c.ws = d_ws; c.ws_bytes = ws_bytes; c.stream = (cudaStream_t)stream;
+    if (p.c.kernel == SvKernel::Grid) return pmmh::sv_grid_run(c, batch, n_obs, n, lag, p.c.grid_G, p.n_teams, hess);
+    return sv_launch_plan(p, {n_obs, n, lag, batch, 0, pmmh::kSvFlps, d_xh != nullptr, 0}, c);
 }
 }  // namespace
 
 int pmmh_flps_model_workspace_bytes(int n_obs, int n_particles, int lag, int batch, size_t* bytes) {
-    if (!bytes) return fail(PMMH_ERR_INVALID, "pmmh_flps_model_workspace_bytes: bad arguments");
-    DeviceInfo di;
-    SvPlan p;
-    int rc = model_choose(n_obs, n_particles, lag, batch, 0, &di, &p);
-    if (rc != PMMH_OK) return rc;
-    *bytes = p.total;
-    return PMMH_OK;
+    return model_query(false, 0, n_obs, n_particles, lag, batch, 0, bytes);
 }
 
 int pmmh_flps_model_corr(int model_id, const double* d_obs, long long obs_stride, const double* d_params,
@@ -720,40 +772,13 @@ int pmmh_flps_model_corr(int model_id, const double* d_obs, long long obs_stride
                          double* d_filt, double* d_smo, double* d_log_like, double* d_gradient, double* d_traj,
                          long long* d_diag, double* d_x_hist, int* d_a_hist, void* d_workspace,
                          size_t workspace_bytes, void* stream) {
-    if (!d_obs || !d_params || !d_rvr || !d_u || !d_filt || !d_smo || !d_log_like || !d_gradient || !d_traj ||
-        !d_diag || !d_workspace)
-        return fail(PMMH_ERR_INVALID, "pmmh_flps_model_corr: null pointer argument");
-    if (model_id != PMMH_MODEL_SV_LEVERAGE && model_id != PMMH_MODEL_LINEAR_GAUSSIAN &&
-        model_id != PMMH_MODEL_LINEAR_GAUSSIAN_FA && model_id != PMMH_MODEL_LINEAR_GAUSSIAN_FA_GRAD)
-        return fail(PMMH_ERR_INVALID, "pmmh_flps_model_corr: unknown model id");
-    if ((d_x_hist == nullptr) != (d_a_hist == nullptr))
-        return fail(PMMH_ERR_INVALID, "d_x_hist and d_a_hist must be given together");
-    if (n_obs < lag + 1) return fail(PMMH_ERR_INVALID, "n_obs must be at least lag + 1");
-    DeviceInfo di;
-    SvPlan p;
-    int rc = model_choose(n_obs, n_particles, lag, batch, 0, &di, &p);
-    if (rc != PMMH_OK) return rc;
-    if (workspace_bytes < p.total) return fail(PMMH_ERR_WORKSPACE, "workspace too small");
-    rc = check_device(di, p.c.kernel == SvKernel::Grid);
-    if (rc != PMMH_OK) return rc;
-    // (no fallback pass: an abandoned evaluation is reported in d_diag[PMMH_DIAG_STATUS])
-    const SvShape s = {n_obs, n_particles, lag, batch, 0, pmmh::kSvFlps, d_x_hist != nullptr, 0};
-    pmmh::SvCall c = {};
-    c.obs = d_obs; c.obs_stride = obs_stride; c.params = d_params; c.rvr = d_rvr; c.u = d_u;
-    c.filt = d_filt; c.smo = d_smo; c.ll = d_log_like; c.grad = d_gradient; c.traj = d_traj; c.diag = d_diag;
-    c.x_hist = d_x_hist; c.a_hist = d_a_hist; c.model = model_id; c.prof = g_sv_prof;
-    c.ws = d_workspace; c.ws_bytes = workspace_bytes; c.stream = (cudaStream_t)stream;
-    return sv_launch_plan(p, s, c);
+    return model_run(false, 0, model_id, d_obs, obs_stride, d_params, d_rvr, d_u, n_obs, n_particles, lag, batch, 0,
+                     d_filt, d_smo, d_log_like, d_gradient, d_traj, nullptr, nullptr, d_diag, d_x_hist, d_a_hist,
+                     d_workspace, workspace_bytes, stream);
 }
 
 int pmmh_filter_model_workspace_bytes(int n_obs, int n_particles, int batch, size_t* bytes) {
-    if (!bytes) return fail(PMMH_ERR_INVALID, "pmmh_filter_model_workspace_bytes: bad arguments");
-    DeviceInfo di;
-    SvPlan p;
-    int rc = model_choose(n_obs, n_particles, 2, batch, 1, &di, &p);
-    if (rc != PMMH_OK) return rc;
-    *bytes = p.total;
-    return PMMH_OK;
+    return model_query(false, 1, n_obs, n_particles, 2, batch, 0, bytes);
 }
 
 int pmmh_filter_model_corr(int model_id, const double* d_obs, long long obs_stride, const double* d_params,
@@ -761,65 +786,14 @@ int pmmh_filter_model_corr(int model_id, const double* d_obs, long long obs_stri
                            double* d_filt, double* d_log_like, double* d_traj, long long* d_diag,
                            double* d_x_hist, int* d_a_hist, void* d_workspace, size_t workspace_bytes,
                            void* stream) {
-    if (!d_obs || !d_params || !d_rvr || !d_u || !d_filt || !d_log_like || !d_traj || !d_diag)
-        return fail(PMMH_ERR_INVALID, "pmmh_filter_model_corr: null pointer argument");
-    if (model_id != PMMH_MODEL_SV_LEVERAGE && model_id != PMMH_MODEL_LINEAR_GAUSSIAN &&
-        model_id != PMMH_MODEL_LINEAR_GAUSSIAN_FA && model_id != PMMH_MODEL_LINEAR_GAUSSIAN_FA_GRAD)
-        return fail(PMMH_ERR_INVALID, "pmmh_filter_model_corr: unknown model id");
-    if ((d_x_hist == nullptr) != (d_a_hist == nullptr))
-        return fail(PMMH_ERR_INVALID, "d_x_hist and d_a_hist must be given together");
-    DeviceInfo di;
-    SvPlan p;
-    int rc = model_choose(n_obs, n_particles, 2, batch, 1, &di, &p);
-    if (rc != PMMH_OK) return rc;
-    if (workspace_bytes < p.total) return fail(PMMH_ERR_WORKSPACE, "workspace too small");
-    if (p.total && !d_workspace) return fail(PMMH_ERR_INVALID, "pmmh_filter_model_corr: null workspace");
-    rc = check_device(di, p.c.kernel == SvKernel::Grid);
-    if (rc != PMMH_OK) return rc;
-    const SvShape s = {n_obs, n_particles, 2, batch, 0, pmmh::kSvFlps, d_x_hist != nullptr, 0};
-    pmmh::SvCall c = {};
-    c.obs = d_obs; c.obs_stride = obs_stride; c.params = d_params; c.rvr = d_rvr; c.u = d_u;
-    c.filt = d_filt; c.ll = d_log_like; c.traj = d_traj; c.diag = d_diag;
-    c.x_hist = d_x_hist; c.a_hist = d_a_hist; c.model = filter_model(model_id); c.filter = 1; c.prof = g_sv_prof;
-    c.ws = d_workspace; c.ws_bytes = workspace_bytes; c.stream = (cudaStream_t)stream;
-    return sv_launch_plan(p, s, c);
+    return model_run(false, 1, model_id, d_obs, obs_stride, d_params, d_rvr, d_u, n_obs, n_particles, 2, batch, 0,
+                     d_filt, nullptr, d_log_like, nullptr, d_traj, nullptr, nullptr, d_diag, d_x_hist, d_a_hist,
+                     d_workspace, workspace_bytes, stream);
 }
-
-// ---- batches on the grid kernel: one team of sv_grid_ctas(N, SMs, 0) CTAs per problem ------------------------------
-namespace {
-// shapes the batch entries take (filter: no lag), team count and workspace; `who` names the entry in errors
-int grid_batch_plan(const char* who, int model_id, int n_obs, int n, int lag, int batch, int hess, int filter,
-                    DeviceInfo* di, int* G, int* nteams, size_t* bytes) {
-    if (model_id != PMMH_MODEL_SV_LEVERAGE && model_id != PMMH_MODEL_LINEAR_GAUSSIAN &&
-        model_id != PMMH_MODEL_LINEAR_GAUSSIAN_FA && model_id != PMMH_MODEL_LINEAR_GAUSSIAN_FA_GRAD)
-        return fail(PMMH_ERR_INVALID, who);
-    if (hess && (filter || model_id != PMMH_MODEL_SV_LEVERAGE)) return fail(PMMH_ERR_INVALID, who);
-    if (batch < 1 || n_obs < 2 || (hess != 0 && hess != 1)) return fail(PMMH_ERR_INVALID, who);
-    int rc = get_device_info(di);
-    if (rc != PMMH_OK) return rc;
-    *G = pmmh::sv_grid_ctas(n, di->sm, 0);
-    if (filter ? !pmmh::sv_grid_filter_eligible(n_obs, n, *G) : !pmmh::sv_grid_eligible(n_obs, n, lag, *G))
-        return fail(PMMH_ERR_INVALID, who);
-    *nteams = pmmh::sv_grid_teams(batch, di->sm, *G);
-    *bytes = (size_t)*nteams * pmmh::sv_grid_ws_bytes(n_obs, n, lag, *G, 1, hess, filter);
-    return PMMH_OK;
-}
-constexpr const char* kFlpsBatchShapes =
-    "pmmh_flps_model_batch_corr: batch >= 1, 2 <= lag <= 10, n_obs >= 2 lag, a tile of n_particles / "
-    "ceil(n_particles / 2048) particles fits one CTA, a known model id, compute_hessian only for the SV model";
-constexpr const char* kFilterBatchShapes =
-    "pmmh_filter_model_batch_corr: batch >= 1, n_obs >= 2, a tile of n_particles / ceil(n_particles / 2048) "
-    "particles fits one CTA and a known model id";
-}  // namespace
 
 int pmmh_flps_model_batch_workspace_bytes(int n_obs, int n_particles, int lag, int batch, int compute_hessian,
                                           size_t* bytes) {
-    if (!bytes) return fail(PMMH_ERR_INVALID, "pmmh_flps_model_batch_workspace_bytes: bytes is null");
-    DeviceInfo di;
-    int G, nteams;
-    // the model is not an argument: any model takes the shape, the Hessian only the SV model
-    return grid_batch_plan(kFlpsBatchShapes, PMMH_MODEL_SV_LEVERAGE, n_obs, n_particles, lag, batch, compute_hessian, 0,
-                           &di, &G, &nteams, bytes);
+    return model_query(true, 0, n_obs, n_particles, lag, batch, compute_hessian, bytes);
 }
 
 int pmmh_flps_model_batch_corr(int model_id, const double* d_obs, long long obs_stride, const double* d_params,
@@ -828,35 +802,13 @@ int pmmh_flps_model_batch_corr(int model_id, const double* d_obs, long long obs_
                                double* d_gradient, double* d_traj, double* d_hess1, double* d_hess2, long long* d_diag,
                                double* d_x_hist, int* d_a_hist, void* d_workspace, size_t workspace_bytes,
                                void* stream) {
-    if (!d_obs || !d_params || !d_rvr || !d_u || !d_filt || !d_smo || !d_log_like || !d_gradient || !d_traj ||
-        !d_diag || !d_workspace || (compute_hessian && (!d_hess1 || !d_hess2)))
-        return fail(PMMH_ERR_INVALID, "pmmh_flps_model_batch_corr: null pointer argument");
-    if ((d_x_hist == nullptr) != (d_a_hist == nullptr))
-        return fail(PMMH_ERR_INVALID, "d_x_hist and d_a_hist must be given together");
-    DeviceInfo di;
-    int G, nteams;
-    size_t bytes;
-    int rc = grid_batch_plan(kFlpsBatchShapes, model_id, n_obs, n_particles, lag, batch, compute_hessian, 0, &di, &G,
-                             &nteams, &bytes);
-    if (rc != PMMH_OK) return rc;
-    if (workspace_bytes < bytes) return fail(PMMH_ERR_WORKSPACE, "pmmh_flps_model_batch_corr: workspace too small");
-    rc = check_device(di, true);
-    if (rc != PMMH_OK) return rc;
-    pmmh::SvCall c = {};
-    c.obs = d_obs; c.obs_stride = obs_stride; c.params = d_params; c.rvr = d_rvr; c.u = d_u;
-    c.filt = d_filt; c.smo = d_smo; c.ll = d_log_like; c.grad = d_gradient; c.traj = d_traj; c.diag = d_diag;
-    if (compute_hessian) { c.hess1 = d_hess1; c.hess2 = d_hess2; }
-    c.x_hist = d_x_hist; c.a_hist = d_a_hist; c.model = model_id;
-    c.ws = d_workspace; c.ws_bytes = workspace_bytes; c.stream = (cudaStream_t)stream;
-    return pmmh::sv_grid_run(c, batch, n_obs, n_particles, lag, G, nteams, compute_hessian);
+    return model_run(true, 0, model_id, d_obs, obs_stride, d_params, d_rvr, d_u, n_obs, n_particles, lag, batch,
+                     compute_hessian, d_filt, d_smo, d_log_like, d_gradient, d_traj, d_hess1, d_hess2, d_diag, d_x_hist,
+                     d_a_hist, d_workspace, workspace_bytes, stream);
 }
 
 int pmmh_filter_model_batch_workspace_bytes(int n_obs, int n_particles, int batch, size_t* bytes) {
-    if (!bytes) return fail(PMMH_ERR_INVALID, "pmmh_filter_model_batch_workspace_bytes: bytes is null");
-    DeviceInfo di;
-    int G, nteams;
-    return grid_batch_plan(kFilterBatchShapes, PMMH_MODEL_SV_LEVERAGE, n_obs, n_particles, 2, batch, 0, 1, &di, &G,
-                           &nteams, bytes);
+    return model_query(true, 1, n_obs, n_particles, 2, batch, 0, bytes);
 }
 
 int pmmh_filter_model_batch_corr(int model_id, const double* d_obs, long long obs_stride, const double* d_params,
@@ -864,24 +816,9 @@ int pmmh_filter_model_batch_corr(int model_id, const double* d_obs, long long ob
                                  double* d_filt, double* d_log_like, double* d_traj, long long* d_diag,
                                  double* d_x_hist, int* d_a_hist, void* d_workspace, size_t workspace_bytes,
                                  void* stream) {
-    if (!d_obs || !d_params || !d_rvr || !d_u || !d_filt || !d_log_like || !d_traj || !d_diag || !d_workspace)
-        return fail(PMMH_ERR_INVALID, "pmmh_filter_model_batch_corr: null pointer argument");
-    if ((d_x_hist == nullptr) != (d_a_hist == nullptr))
-        return fail(PMMH_ERR_INVALID, "d_x_hist and d_a_hist must be given together");
-    DeviceInfo di;
-    int G, nteams;
-    size_t bytes;
-    int rc = grid_batch_plan(kFilterBatchShapes, model_id, n_obs, n_particles, 2, batch, 0, 1, &di, &G, &nteams, &bytes);
-    if (rc != PMMH_OK) return rc;
-    if (workspace_bytes < bytes) return fail(PMMH_ERR_WORKSPACE, "pmmh_filter_model_batch_corr: workspace too small");
-    rc = check_device(di, true);
-    if (rc != PMMH_OK) return rc;
-    pmmh::SvCall c = {};
-    c.obs = d_obs; c.obs_stride = obs_stride; c.params = d_params; c.rvr = d_rvr; c.u = d_u;
-    c.filt = d_filt; c.ll = d_log_like; c.traj = d_traj; c.diag = d_diag;
-    c.x_hist = d_x_hist; c.a_hist = d_a_hist; c.model = filter_model(model_id); c.filter = 1;
-    c.ws = d_workspace; c.ws_bytes = workspace_bytes; c.stream = (cudaStream_t)stream;
-    return pmmh::sv_grid_run(c, batch, n_obs, n_particles, 2, G, nteams, 0);
+    return model_run(true, 1, model_id, d_obs, obs_stride, d_params, d_rvr, d_u, n_obs, n_particles, 2, batch, 0,
+                     d_filt, nullptr, d_log_like, nullptr, d_traj, nullptr, nullptr, d_diag, d_x_hist, d_a_hist,
+                     d_workspace, workspace_bytes, stream);
 }
 
 int pmmh_bpf_sv_corr(const double* d_obs, long long obs_stride, const double* d_params,

@@ -4,10 +4,13 @@
 // "how the propagation and weighting of particles is carried out as well as the gradients of the
 // log joint distribution of states and measurements").  Everything else -- sorted correlated
 // systematic resampling, the counting sort, cumulative weights, fixed-lag bookkeeping, the tail --
-// is model independent and lives in the kernel; kReferenceIndexing picks how the kernel pairs the
-// fixed-lag score terms.
+// is model independent and lives in the kernel; kPairing picks how the kernel pairs the fixed-lag score terms.
 //
 // A model M provides (all __device__, fp64, no contraction):
+//   M::kId                               its model id (PMMH_MODEL_*, include/pmmh_qn.h)
+//   M::Filter                            the model whose filter instantiation the filter entries run (itself, or
+//                                        the model it adds a gradient to)
+//   M::kHessian                          constexpr: the kernels have its Hessian branch (the SV model only)
 //   struct M::Const                      constants derived from the parameter vector (<= 4 doubles)
 //   M::init(Const&, const double* par)
 //   M::initial_state(c)                  value of every particle of generation 0 (the reference's
@@ -29,21 +32,21 @@
 //   M::score_tail(c, curr, next, y, g)   the same in the tail loop
 //   M::kScoreIsZero                      constexpr: score_main / score_tail are identically 0 (the
 //                                        grid kernel then skips the calls; the smoother still runs)
-//   M::kReferenceIndexing                constexpr: how the fixed-lag terms are paired (below)
-//   M::kPredictiveScore                  constexpr: the exact pairing shifted for a fully adapted filter (below)
-//   M::score_last(c, x, y_next, g)       (kPredictiveScore only) the final generation's term
+//   M::kPairing                          constexpr: how the fixed-lag terms are paired (below)
+//   M::score_last(c, x, y_next, g)       (Pairing::Predictive only) the final generation's term
+// A new model is such a struct plus its entry in Models at the end of this file, and its id in include/pmmh_qn.h.
 //
-// kReferenceIndexing = true (the SV model, parity with the reference): the reference's quirks Q5 / Q6.  The main loop
+// Pairing::Reference (the SV model, parity with the reference): the reference's quirks Q5 / Q6.  The main loop
 // at step i >= LAG adds the pair (x_tt, x_tt+1), tt = i - LAG + 1, with y = obs[tt - 1] (score_main, Q5) into slot tt;
 // the tail i = NOBS-LAG .. NOBS-1 adds smo[i] under the final weights and the pair (x_i, x_i+1) with y = obs[i - 1]
 // wrapped (score_tail, Q6, :548-557, another operation order) under the weights of generation i into slot i - LAG + 1.
-// kReferenceIndexing = false (models of no reference: the exact pairing): the pair (x_t, x_t+1), t = 0 .. NOBS-2,
+// Pairing::Exact (models of no reference): the pair (x_t, x_t+1), t = 0 .. NOBS-2,
 // contributes d/dtheta log p(x_t+1 | x_t) + d/dtheta log p(y_t+1 | x_t+1) once, with y = obs[t + 1], weighted by the
 // generation at which it is read: W_{t+LAG-1} in the main loop (steps i >= LAG - 1; the pair t = 0 has curr =
 // initial_state for every particle, Q1), W_{NOBS-1} in the tail (t = NOBS-LAG+1 .. NOBS-2).  Gradient slot s holds
 // step s's contribution (the pair (x_s-1, x_s)); slot 0 is 0.  smo[t] = the weighted mean of x_t under the same
 // weights, every slot written once: the tail starts one step after the last main-loop slot.
-// kPredictiveScore = true (exact pairing on the shifted series of a fully adapted filter, model 4): the same pairs, read
+// Pairing::Predictive (exact pairing on the shifted series of a fully adapted filter, model 4): the same pairs, read
 // under the same weights, but the pair (x_t, x_t+1) takes y = obs[t] (= y_t+1 of the unshifted series) and goes into
 // slot t; the final generation adds score_last(x_NOBS-1, obs[NOBS-1]) under W_{NOBS-1} into slot NOBS-1 (the pair
 // (x_NOBS-1, x_NOBS) with x_NOBS integrated out).  Slot t then holds the contribution of obs[t], and the slots sum
@@ -52,12 +55,30 @@
 #pragma once
 #include <math.h>
 
+#include "../../include/pmmh_qn.h"
 #include "sv_math.cuh"
 
 namespace pmmh {
 
+enum class Pairing { Reference, Exact, Predictive };
+
+// The offsets of the pairings above; the main loop reads the pair (x_t, x_t+1) at step t + LAG - 1.
+// The first step of the main loop that adds a fixed-lag term:
+__host__ __device__ constexpr int pair_first_step(Pairing p, int lag) {
+    return p == Pairing::Reference ? lag : lag - 1;
+}
+// the observation index of the pair (x_t, x_t+1) (Reference: t - 1, wrapped in the tail):
+__host__ __device__ constexpr int pair_obs(Pairing p, int t) {
+    return p == Pairing::Reference ? t - 1 : (p == Pairing::Predictive ? t : t + 1);
+}
+// the gradient slot of the pair (x_t, x_t+1) (Reference: in the main loop; its tail puts it into t - LAG + 1, Q6):
+__host__ __device__ constexpr int pair_slot(Pairing p, int t) { return p == Pairing::Exact ? t + 1 : t; }
+
 // ---- 0: stochastic volatility with leverage (the reference's model; models/stochastic_volatility.py)
 struct SvLeverageModel {
+    static constexpr int kId = PMMH_MODEL_SV_LEVERAGE;
+    typedef SvLeverageModel Filter;
+    static constexpr bool kHessian = true;
     typedef SvConst Const;
     static __device__ __forceinline__ void init(Const& c, const double* par) { sv_const_init(c, par); }
     static __device__ __forceinline__ double initial_state(const Const& c) {
@@ -65,8 +86,7 @@ struct SvLeverageModel {
         return c.mu + stdev0 * 0.0;   // :309 (Q1)
     }
     static constexpr bool kScoreIsZero = false;
-    static constexpr bool kReferenceIndexing = true;
-    static constexpr bool kPredictiveScore = false;
+    static constexpr Pairing kPairing = Pairing::Reference;
     static __device__ __forceinline__ double propagate(const Const& c, double xp, double y1, double u) {
         double mean = c.mu + c.phi * (xp - c.mu);
         mean += c.sr * exp(-0.5 * xp) * y1;
@@ -108,6 +128,9 @@ struct SvLeverageModel {
 // here to show that a second model plugs into the same kernel, and because its exact likelihood is
 // known (Kalman filter), which the tests use.
 struct LinearGaussianModel {
+    static constexpr int kId = PMMH_MODEL_LINEAR_GAUSSIAN;
+    typedef LinearGaussianModel Filter;
+    static constexpr bool kHessian = false;
     struct Const {
         double phi, sv, se, inv_sv2, inv_se2, log_se;
     };
@@ -121,8 +144,7 @@ struct LinearGaussianModel {
     }
     static __device__ __forceinline__ double initial_state(const Const&) { return 0.0; }
     static constexpr bool kScoreIsZero = false;
-    static constexpr bool kReferenceIndexing = false;
-    static constexpr bool kPredictiveScore = false;
+    static constexpr Pairing kPairing = Pairing::Exact;
     static __device__ __forceinline__ double propagate(const Const& c, double xp, double, double u) {
         return c.phi * xp + c.sv * u;
     }
@@ -169,6 +191,9 @@ struct LinearGaussianModel {
 // y_2 .. y_T given y_1 (the caller adds log p(y_1)), and E[x_t | y_1 .. y_{t+1}] in `filt`; the score terms are not
 // defined for this variant (gradient rows 0).
 struct LinearGaussianFullyAdapted {
+    static constexpr int kId = PMMH_MODEL_LINEAR_GAUSSIAN_FA;
+    typedef LinearGaussianFullyAdapted Filter;
+    static constexpr bool kHessian = false;
     struct Const {
         double phi, sv, se, k, sdp, inv_s2, log_s;   // gain, proposal sd, predictive variance
     };
@@ -185,8 +210,7 @@ struct LinearGaussianFullyAdapted {
     static __device__ __forceinline__ double initial_state(const Const&) { return 0.0; }
     // x_t | x_{t-1}, y_t ~ N(phi x + k (y_t - phi x), sv^2 se^2 / (sv^2 + se^2))
     static constexpr bool kScoreIsZero = true;
-    static constexpr bool kReferenceIndexing = false;   // smo: x_t under W_{t+LAG-1}, i.e. given y_1 .. y_{t+LAG}
-    static constexpr bool kPredictiveScore = false;
+    static constexpr Pairing kPairing = Pairing::Exact;   // smo: x_t under W_{t+LAG-1}, i.e. given y_1 .. y_{t+LAG}
     static __device__ __forceinline__ double propagate(const Const& c, double xp, double y_now, double u) {
         const double m = c.phi * xp;
         return (m + c.k * (y_now - m)) + c.sdp * u;
@@ -226,11 +250,13 @@ struct LinearGaussianFullyAdapted {
 
 // ---- 4: model 2's fully adapted filter with a fixed-lag gradient.  Propagation, weights, shift and child range are
 // model 2's (inherited), so every output model 2 has -- filt, smo, log-likelihood, traj, diag, history -- is
-// bit-identical to it.  The gradient pairs the terms predictively (kPredictiveScore above): slot t holds the
+// bit-identical to it, and the filter entries run model 2's instantiation (Filter).  The gradient pairs the terms
+// predictively (Pairing::Predictive above): slot t holds the
 // contribution of obs'[t] = y_t+1, and the slots sum to an estimate of the score of log p(y_1 .. y_T), the first
 // observation's term included (the log-likelihood still lacks log p(y_1)).  Checked against the restatement
 // oracle/generic_pf.py LinearGaussianFullyAdaptedGrad and the exact fixed-lag Kalman targets of oracle/kalman.py.
 struct LinearGaussianFullyAdaptedGrad : LinearGaussianFullyAdapted {
+    static constexpr int kId = PMMH_MODEL_LINEAR_GAUSSIAN_FA_GRAD;
     struct Const : LinearGaussianFullyAdapted::Const {
         double inv_sv2, inv_sv, inv_se2, inv_se;
     };
@@ -242,7 +268,7 @@ struct LinearGaussianFullyAdaptedGrad : LinearGaussianFullyAdapted {
         c.inv_se = 1.0 / c.se;
     }
     static constexpr bool kScoreIsZero = false;
-    static constexpr bool kPredictiveScore = true;
+    static constexpr Pairing kPairing = Pairing::Predictive;
     // d/d(phi, sigma_v, sigma_e) of log N(next; phi curr, sigma_v^2) + log N(y; next, sigma_e^2), y = obs'[time(curr)]
     static __device__ __forceinline__ void score_main(const Const& c, double curr, double next, double y, double g[4]) {
         const double r = next - c.phi * curr;
@@ -266,5 +292,34 @@ struct LinearGaussianFullyAdaptedGrad : LinearGaussianFullyAdapted {
         g[3] = 0.0;
     }
 };
+
+// ---- the model table: every model the kernels are instantiated for.  Models::with(id, f) calls f(ModelTag<M>()) for
+// the model M of that id (false, and no call, for an unknown id); Models::each(f) calls it for every model.
+template <class M>
+struct ModelTag {
+    typedef M type;
+};
+template <class... Ms>
+struct ModelList {
+    template <class F>
+    static bool with(int id, F&& f) { return ((Ms::kId == id ? (f(ModelTag<Ms>()), true) : false) || ...); }
+    template <class F>
+    static void each(F&& f) { (f(ModelTag<Ms>()), ...); }
+    static constexpr bool ids_distinct() {   // (a derived model inherits its base's id unless it states its own)
+        int same = 0;
+        for (int a : {Ms::kId...}) for (int b : {Ms::kId...}) same += a == b;
+        return same == (int)sizeof...(Ms);
+    }
+};
+typedef ModelList<SvLeverageModel, LinearGaussianModel, LinearGaussianFullyAdapted, LinearGaussianFullyAdaptedGrad>
+    Models;
+static_assert(Models::ids_distinct(), "every model states its own id");
+
+inline bool model_known(int id) { return Models::with(id, [](auto) {}); }
+inline bool model_has_hessian(int id) {
+    bool h = false;
+    Models::with(id, [&](auto m) { h = decltype(m)::type::kHessian; });
+    return h;
+}
 
 }  // namespace pmmh

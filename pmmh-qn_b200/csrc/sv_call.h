@@ -24,7 +24,7 @@ struct SvCall {
     long long* diag;
     double* x_hist;          // optional, together with a_hist
     int* a_hist;
-    int model;               // PMMH_MODEL_* (pf_model.cuh)
+    int model;               // model id (the table Models in pf_model.cuh)
     int filter;              // 1: the particle filter alone (chain and grid kernels): smo / grad are not written
     long long* prof;         // optional per-CTA phase clocks (pmmh_sv_debug_profile)
     void* ws;

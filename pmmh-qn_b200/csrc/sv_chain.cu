@@ -22,7 +22,7 @@
 //     comes from a ring in global memory (L2 resident: 64 KB per generation and problem).
 // The tail (:540-562, Q6) chases one-step ancestors through global rings of the last LAG
 // generations.  Quirks reproduced: Q1, Q3 (as in the other kernels: cumulative weights are
-// normalised at look-up), Q5 and Q6 for the SV model (M::kReferenceIndexing; the other models pair the fixed-lag terms
+// normalised at look-up), Q5 and Q6 for the SV model (M::kPairing; the other models pair the fixed-lag terms
 // exactly, pf_model.cuh), Q11.  Sums over particles are fixed-order tree sums.
 // Hessian branch: the cumulative alpha of a particle (4 doubles) lives in a global ring by sorted
 // position next to the (value, parent value) ring; the child adds its own term to its parent's
@@ -483,11 +483,9 @@ __global__ void __launch_bounds__(kCT, 1) sv_chain_kernel(SvArgs a) {
                 double run = chain_scan_d(tsum, s_w, &S_i);
                 // pairing of the fixed-lag terms (pf_model.cuh): the reference's (Q5 / Q6) or the exact one, whose main
                 // loop starts one step earlier (the pair (x_0, x_1) at step LAG - 1) and whose tail starts one step later
-                const bool lagged = SMO && inext >= (M::kReferenceIndexing ? LAG : LAG - 1);
+                const bool lagged = SMO && inext >= pair_first_step(M::kPairing, LAG);
                 // the pair (x_tt, x_tt+1), tt = inext - LAG + 1: y = obs[tt - 1] (Q5), obs[tt + 1], or obs[tt] (predictive)
-                const double yl = lagged ? obs[M::kReferenceIndexing ? inext - LAG
-                                                                     : (M::kPredictiveScore ? inext - LAG + 1 : inext - LAG + 2)]
-                                         : 0.0;
+                const double yl = lagged ? obs[pair_obs(M::kPairing, inext - LAG + 1)] : 0.0;
                 const int hop0 = (K >= 1) ? ((K - 1) & 3) : 0;
                 const int nh = (K >= 1) ? ((K - 1) >> 2) : 0;        // 0 or 1 (LAG <= 10)
                 const int g1 = inext - (hop0 + 1);
@@ -550,10 +548,9 @@ __global__ void __launch_bounds__(kCT, 1) sv_chain_kernel(SvArgs a) {
                 s_S[inext % kMaxLagC] = S_i;
                 o_filt[inext] = acc[0] / S_i;
                 o_traj[inext] = s_x[0];   // Q11: traj[i] = X_i[0]
-                if constexpr (SMO) if (inext >= (M::kReferenceIndexing ? LAG : LAG - 1)) {
+                if constexpr (SMO) if (inext >= pair_first_step(M::kPairing, LAG)) {
                     const int tt = inext - LAG + 1;
-                    // gradient slot: tt (Q5, predictive) or the pair's second step
-                    const int gs = (M::kReferenceIndexing || M::kPredictiveScore) ? tt : tt + 1;
+                    const int gs = pair_slot(M::kPairing, tt);
                     o_smo[tt] = acc[1] / S_i;
                     o_grad[gs] = acc[2] / S_i;
                     o_grad[NOBS + gs] = acc[3] / S_i;
@@ -572,7 +569,8 @@ __global__ void __launch_bounds__(kCT, 1) sv_chain_kernel(SvArgs a) {
             const int T = NOBS - 1;
             const double S_T = s_S[T % kMaxLagC];
             const double* shT = SHG(T);
-            for (int k = 0; k < (M::kReferenceIndexing ? LAG : LAG - 1); ++k) {
+            constexpr Pairing PR = M::kPairing;
+            for (int k = 0; k < (PR == Pairing::Reference ? LAG : LAG - 1); ++k) {
                 const int ip = T - k;
                 constexpr int NT = 5;
                 double tacc[NT];
@@ -580,8 +578,8 @@ __global__ void __launch_bounds__(kCT, 1) sv_chain_kernel(SvArgs a) {
                 for (int q = 0; q < NT; ++q) tacc[q] = 0.0;
                 const double ylag = obs_wrap(obs, ip - LAG, NOBS);
                 const double S_ip = s_S[ip % kMaxLagC];
-                const double y1 = M::kReferenceIndexing ? obs_wrap(obs, ip - 1, NOBS)
-                                                        : (M::kPredictiveScore ? obs[ip] : (k >= 1 ? obs[ip + 1] : 0.0));
+                const double y1 = PR == Pairing::Reference ? obs_wrap(obs, pair_obs(PR, ip), NOBS)
+                                  : (k >= 1 || PR == Pairing::Predictive ? obs[pair_obs(PR, ip)] : 0.0);
                 const double* shI = SHG(ip);
                 for (int j = tid; j < N; j += kCT) {
                     int b = j, bprev = j;
@@ -597,7 +595,7 @@ __global__ void __launch_bounds__(kCT, 1) sv_chain_kernel(SvArgs a) {
                         const double next = __ldcg(&XPG(ip + 1)[bprev]).x;
                         double g[4];
                         double wi;
-                        if constexpr (M::kReferenceIndexing) {
+                        if constexpr (PR == Pairing::Reference) {
                             double si = __ldcg(&shI[j]);
                             if (!isfinite(si)) si = 0.0;
                             wi = si / S_ip;
@@ -619,7 +617,7 @@ __global__ void __launch_bounds__(kCT, 1) sv_chain_kernel(SvArgs a) {
                         tacc[2] += g[1] * wi;
                         tacc[3] += g[2] * wi;
                         tacc[4] += g[3] * wi;
-                    } else if constexpr (M::kPredictiveScore) {   // the final generation's term
+                    } else if constexpr (PR == Pairing::Predictive) {   // the final generation's term
                         const double wi = sT / S_T;
                         double g[4];
                         M::score_last(c, curr, y1, g);
@@ -632,8 +630,8 @@ __global__ void __launch_bounds__(kCT, 1) sv_chain_kernel(SvArgs a) {
                 block_sum<NT>(tacc, s_red);
                 if (tid == 0) {
                     o_smo[ip] += tacc[0];
-                    if (k >= 1 || M::kPredictiveScore) {
-                        const int tt = M::kReferenceIndexing ? ip - LAG + 1 : (M::kPredictiveScore ? ip : ip + 1);
+                    if (k >= 1 || PR == Pairing::Predictive) {
+                        const int tt = PR == Pairing::Reference ? ip - LAG + 1 : pair_slot(PR, ip);
                         if (tt >= 0) {
                             o_grad[tt] += tacc[1];
                             o_grad[NOBS + tt] += tacc[2];
@@ -710,21 +708,21 @@ static cudaError_t chain_launch_one(const SvArgs& a, int grid, int smem, cudaStr
     return cudaGetLastError();
 }
 
+// the filter runs the instantiation of M::Filter; the Hessian branch exists where M::kHessian
 cudaError_t sv_chain_launch(const SvArgs& a, int grid, int filter, cudaStream_t stream) {
     const int smem = sv_chain_smem_bytes(a.N);
-    if (filter) {
-        if (a.hess) return cudaErrorInvalidValue;
-        if (a.model_id == 0) return chain_launch_one<SvLeverageModel, false, false>(a, grid, smem, stream);
-        if (a.model_id == 1) return chain_launch_one<LinearGaussianModel, false, false>(a, grid, smem, stream);
-        if (a.model_id == 2) return chain_launch_one<LinearGaussianFullyAdapted, false, false>(a, grid, smem, stream);
-        return cudaErrorInvalidValue;
-    }
-    if (a.model_id == 0) return a.hess ? chain_launch_one<SvLeverageModel, true, true>(a, grid, smem, stream)
-                                       : chain_launch_one<SvLeverageModel, false, true>(a, grid, smem, stream);
-    if (a.model_id == 1 && !a.hess) return chain_launch_one<LinearGaussianModel, false, true>(a, grid, smem, stream);
-    if (a.model_id == 2 && !a.hess) return chain_launch_one<LinearGaussianFullyAdapted, false, true>(a, grid, smem, stream);
-    if (a.model_id == 4 && !a.hess) return chain_launch_one<LinearGaussianFullyAdaptedGrad, false, true>(a, grid, smem, stream);
-    return cudaErrorInvalidValue;
+    cudaError_t err = cudaErrorInvalidValue;
+    Models::with(a.model_id, [&](auto m) {
+        typedef typename decltype(m)::type M;
+        if (filter) {
+            if (!a.hess) err = chain_launch_one<typename M::Filter, false, false>(a, grid, smem, stream);
+        } else if (!a.hess) {
+            err = chain_launch_one<M, false, true>(a, grid, smem, stream);
+        } else if constexpr (M::kHessian) {
+            err = chain_launch_one<M, true, true>(a, grid, smem, stream);
+        }
+    });
+    return err;
 }
 
 }  // namespace pmmh

@@ -44,7 +44,7 @@ struct SvArgs {
     int only_failed; // general kernel: only run problems whose diag status is 1 (fallback pass)
     int RING;        // ring depth of the X / A / R histories (LAG + 1), or NOBS with full history
     int mode, hess;
-    int model_id;    // chain kernel: 0 = SV with leverage (the reference's model), 1 = linear Gaussian (pf_model.cuh)
+    int model_id;    // chain kernel: the model id (the table Models in pf_model.cuh)
     int SQ;          // low slots of X kept for all times (Q7 / Q11)
     int SQW;         // low slots of W kept for all times (Q10, bpf only)
     const double* obs;

@@ -435,9 +435,6 @@ __global__ void __launch_bounds__(GT, 1) sv_grid_kernel(const GridArgs a_in, con
     if constexpr (TEAM) a_team = team_args(a_in, tm);
     const GridArgs& a = TEAM ? a_team : a_in;   // this CTA's problem
     constexpr bool GEN = !std::is_same<M, SvLeverageModel>::value;
-    // first step with fixed-lag terms: the reference's pairing (Q5) starts at LAG, the exact one (pf_model.cuh) one step
-    // earlier with the pair (x_0, x_1)
-    constexpr int LAG0 = M::kReferenceIndexing ? 0 : 1;
     static_assert(!(GEN && HESS), "the Hessian branch exists for the SV model only");
     static_assert(SMO || !HESS, "the Hessian branch needs the smoother");
     constexpr int KPT = kCap / GT;          // entries per thread (strided assignment)
@@ -1330,7 +1327,8 @@ __global__ void __launch_bounds__(GT, 1) sv_grid_kernel(const GridArgs a_in, con
                     __stcg((double2*)&a.tinfo[c * 4 + 2], make_double2(v[1], v[2]));
                     ps[1] = v[0];
                     ps[7] = 0.0;
-                    if (!SMO || t < L - LAG0 || (a.dbg & 4)) {   // later steps: the score terms below write ps[2..6]
+                    // later steps: the score terms below write ps[2..6]
+                    if (!SMO || t < pair_first_step(M::kPairing, L) || (a.dbg & 4)) {
 #pragma unroll
                         for (int i = 2; i < 7; ++i) ps[i] = 0.0;
                     }
@@ -1346,7 +1344,7 @@ __global__ void __launch_bounds__(GT, 1) sv_grid_kernel(const GridArgs a_in, con
         }
         PROF_MARK(11);   // B scan+publish
         GRID_ARRIVE();   // ---- barrier 3: tile totals published
-        if (SMO && t >= L - LAG0 && !(a.dbg & 4)) {
+        if (SMO && t >= pair_first_step(M::kPairing, L) && !(a.dbg & 4)) {
             // fixed-lag score terms (:445-470): weight x monomials of the payload of the ancestor
             // LAG-2 generations back (one random sector each), fixed summation order
             const PEntry* Pg = a.P + (size_t)((t - (L - 2)) % RP) * N * RS;
@@ -1367,7 +1365,7 @@ __global__ void __launch_bounds__(GT, 1) sv_grid_kernel(const GridArgs a_in, con
                 // generic path: sc[0] = sum sh curr (smoother), sc[1 + k] = sum sh g[k] of M::score_main on the pair
                 // (curr, next) = (parent value, own value) of the ancestor = (x_tt, x_tt+1), tt = t - LAG + 1;
                 // y = obs[t - LAG] (Q5), obs[tt + 1], or obs[tt] (predictive)
-                const double yl = a.obs[M::kReferenceIndexing ? t - L : (M::kPredictiveScore ? t - L + 1 : t - L + 2)];
+                const double yl = a.obs[pair_obs(M::kPairing, t - L + 1)];
 #pragma unroll
                 for (int k0 = 0; k0 < KPT; k0 += 4) {
                     double pc[4], px[4];
@@ -1573,9 +1571,9 @@ __global__ void __launch_bounds__(256) grid_reduce_kernel(const double* __restri
 
 // part[irel][block][0] = sum_p W_T[p] hist_idx[p];  [1..4] = sum_p W_i[p] g(hist_idx, hist_idx-1)
 // with i = NOBS - L + irel, idx = L - 1 - irel; hist_k[p] = value of the ancestor k steps back of
-// the particle at sorted position p of the final generation.  Exact pairing (pf_model.cuh, !M::kReferenceIndexing):
+// the particle at sorted position p of the final generation.  Exact pairing (pf_model.cuh, Pairing::Exact):
 // irel = 0 is 0 (the main loop has that slot), the pair is weighted by W_T and takes y = obs[i + 1]; predictive pairing
-// (M::kPredictiveScore): y = obs[i], and irel = L - 1 (idx = 0, i = T) adds M::score_last of the final particle.
+// (Pairing::Predictive): y = obs[i], and irel = L - 1 (idx = 0, i = T) adds M::score_last of the final particle.
 // HESS: partH[irel][block][0..19] = the hessian1 / hessian2 terms of :564-626 (alpha of the ancestor LAG-2 steps
 // back of the final particle, weights W_i, obs[i - LAG] with wrap-around, Q8).  M: the model (g = M::score_tail).
 template <bool HESS, class M>
@@ -1588,8 +1586,9 @@ __global__ void __launch_bounds__(256) grid_tail_kernel(GridArgs a, const double
     const int irel = blockIdx.y, i = a.NOBS - L + irel, idx = L - 1 - irel;
     typename M::Const k;
     M::init(k, a.params);
-    constexpr bool REF = M::kReferenceIndexing;
-    const double y1 = REF ? obs_wrap(a.obs, i - 1, a.NOBS) : a.obs[M::kPredictiveScore ? i : min(i + 1, T)];
+    constexpr bool REF = M::kPairing == Pairing::Reference;
+    const double y1 = REF ? obs_wrap(a.obs, pair_obs(M::kPairing, i), a.NOBS)
+                          : a.obs[M::kPairing == Pairing::Predictive ? i : min(i + 1, T)];
     const double ST = sums[(size_t)T * 8], Si = sums[(size_t)i * 8];
     const double* shT = a.shring + (size_t)(T % L) * N;
     const double* shi = a.shring + (size_t)(i % L) * N;
@@ -1610,7 +1609,7 @@ __global__ void __launch_bounds__(256) grid_tail_kernel(GridArgs a, const double
         if (idx == 0) {
             curr = a.XE[p].x;
             acc[0] += wT * curr;
-            if constexpr (M::kPredictiveScore) {
+            if constexpr (M::kPairing == Pairing::Predictive) {
                 double g[4];
                 M::score_last(k, curr, y1, g);
 #pragma unroll
@@ -1743,15 +1742,8 @@ __global__ void __launch_bounds__(256) grid_tail_reduce_kernel(const double* __r
 // sums[t][0] = sum sh, [1] = sum sh x, [2] = sum sh c, [3] = sum sh sq, [4] = sum sh sq c, [5] = sum sh sq^2,
 // [6] = sum sh sq ey (c = lagged ancestor value, sq / ey as stored in P);  tail[irel][0..4].
 // GEN (the generic path of a model other than SV): [3..6] = sum sh g[0..3], traj[0] = the initial state, exact pairing of
-// the fixed-lag terms (pf_model.cuh; models 1, 2 and 4 have kReferenceIndexing = false).  PRED: the predictive pairing
-// (M::kPredictiveScore, model 4).
+// the fixed-lag terms (pf_model.cuh).  PRED: the predictive pairing.  Both derive from the model in grid_finish_for.
 // SMO = false (the filter alone): no smo / grad, tail unused.
-static_assert(SvLeverageModel::kReferenceIndexing && !LinearGaussianModel::kReferenceIndexing &&
-                  !LinearGaussianFullyAdapted::kReferenceIndexing && !LinearGaussianFullyAdaptedGrad::kReferenceIndexing,
-              "grid_finish_kernel pairs the fixed-lag terms as the reference does for SV (GEN = false), exactly otherwise");
-static_assert(!SvLeverageModel::kPredictiveScore && !LinearGaussianModel::kPredictiveScore &&
-                  !LinearGaussianFullyAdapted::kPredictiveScore && LinearGaussianFullyAdaptedGrad::kPredictiveScore,
-              "grid_finish_kernel places the predictive pairing's slots for model 4 only (PRED)");
 template <bool GEN, bool SMO, bool PRED = false>
 __global__ void grid_finish_kernel(const GridCtrl* __restrict__ ctrl, const double* __restrict__ sums,
                                    const double* __restrict__ shift, const double* __restrict__ xmin,
@@ -1855,6 +1847,15 @@ __global__ void grid_finish_kernel(const GridCtrl* __restrict__ ctrl, const doub
     }
 }
 
+// the finish kernel of model M: GEN is the grid kernel's (the layout of its sums), which pairs the terms as the
+// reference does on the SV path alone
+template <class M, bool SMO>
+auto grid_finish_for() {
+    constexpr bool GEN = !std::is_same<M, SvLeverageModel>::value;
+    static_assert(GEN == (M::kPairing != Pairing::Reference), "the SV path alone pairs the terms as the reference does");
+    return grid_finish_kernel<GEN, SMO, SMO && M::kPairing == Pairing::Predictive>;
+}
+
 struct GridLayout {
     size_t ctrl, ghist, tilecnt, tinfo, H, XE, perm, R, P, psum, shiftv, xminv, shring, parentpos, sums,
         tailpart, tail, info, ustash, xlow, psumH, sumsH, tailpartH, total;
@@ -1913,27 +1914,28 @@ template <bool HESS, class M, bool SMO>
 const void* grid_kernel_of(bool team) {
     return team ? (const void*)sv_grid_kernel<1024, HESS, M, SMO, true> : (const void*)sv_grid_kernel<1024, HESS, M, SMO, false>;
 }
-// the persistent kernel of (model, hess, filter): one problem, or teams of CTAs
+// the persistent kernel of (model, hess, filter): one problem, or teams of CTAs; the filter runs the model's Filter;
+// nullptr for an unknown model id or a Hessian the model does not have
 const void* grid_kernel_for(int model, int hess, int filter, bool team) {
-    if (filter) {
-        if (model == PMMH_MODEL_LINEAR_GAUSSIAN) return grid_kernel_of<false, LinearGaussianModel, false>(team);
-        if (model == PMMH_MODEL_LINEAR_GAUSSIAN_FA) return grid_kernel_of<false, LinearGaussianFullyAdapted, false>(team);
-        return grid_kernel_of<false, SvLeverageModel, false>(team);
-    }
-    if (model == PMMH_MODEL_LINEAR_GAUSSIAN) return grid_kernel_of<false, LinearGaussianModel, true>(team);
-    if (model == PMMH_MODEL_LINEAR_GAUSSIAN_FA) return grid_kernel_of<false, LinearGaussianFullyAdapted, true>(team);
-    if (model == PMMH_MODEL_LINEAR_GAUSSIAN_FA_GRAD) return grid_kernel_of<false, LinearGaussianFullyAdaptedGrad, true>(team);
-    return hess ? grid_kernel_of<true, SvLeverageModel, true>(team) : grid_kernel_of<false, SvLeverageModel, true>(team);
+    const void* k = nullptr;
+    Models::with(model, [&](auto m) {
+        typedef typename decltype(m)::type M;
+        if (filter) {
+            k = grid_kernel_of<false, typename M::Filter, false>(team);
+        } else if (!hess) {
+            k = grid_kernel_of<false, M, true>(team);
+        } else if constexpr (M::kHessian) {
+            k = grid_kernel_of<true, M, true>(team);
+        }
+    });
+    return k;
 }
 
 int grid_check(const SvCall& c, int nobs, int n, int lag, int G, int hess) {
     if (c.filter ? (hess || !sv_grid_filter_eligible(nobs, n, G)) : !sv_grid_eligible(nobs, n, lag, G))
         return set_error(PMMH_ERR_INVALID, "grid kernel: sizes not eligible");
-    const int model = c.model;
-    if (model != PMMH_MODEL_SV_LEVERAGE && model != PMMH_MODEL_LINEAR_GAUSSIAN && model != PMMH_MODEL_LINEAR_GAUSSIAN_FA &&
-        !(model == PMMH_MODEL_LINEAR_GAUSSIAN_FA_GRAD && !c.filter))   // (the entries run model 4's filter as model 2's)
-        return set_error(PMMH_ERR_INVALID, "grid kernel: unknown model id");
-    if (hess && model != PMMH_MODEL_SV_LEVERAGE)
+    if (!model_known(c.model)) return set_error(PMMH_ERR_INVALID, "grid kernel: unknown model id");
+    if (hess && !model_has_hessian(c.model))
         return set_error(PMMH_ERR_INVALID, "grid kernel: the Hessian branch exists for the SV model only");
     return PMMH_OK;
 }
@@ -1947,13 +1949,15 @@ int grid_set_attributes() {
         // no persisting L2 set-aside for the kernel's evict_last accesses: with one every phase is slower
         // (DESIGN 4.0), and left unset the evaluation at N = 2^20 is ~6 % slower
         GRID_CUDA(cudaDeviceSetLimit(cudaLimitPersistingL2CacheSize, 0));
-        for (int team = 0; team < 2; ++team)
-            for (int model = 0; model <= PMMH_MODEL_LINEAR_GAUSSIAN_FA_GRAD; ++model)
-                for (int v = 0; v < 3; ++v)   // smoother, smoother with Hessian (SV only), filter (not model 4: model 2's)
-                    if (model != 3 && (v != 1 || model == PMMH_MODEL_SV_LEVERAGE) &&   // (3 is not a model id)
-                        (v != 2 || model != PMMH_MODEL_LINEAR_GAUSSIAN_FA_GRAD))
-                        GRID_CUDA(cudaFuncSetAttribute(grid_kernel_for(model, v == 1, v == 2, team != 0),
-                                                       cudaFuncAttributeMaxDynamicSharedMemorySize, kDynSmem));
+        cudaError_t err = cudaSuccess;
+        Models::each([&](auto m) {
+            for (int team = 0; team < 2; ++team)
+                for (int v = 0; v < 3; ++v)   // smoother, smoother with Hessian (where the model has one), filter
+                    if (const void* k = grid_kernel_for(decltype(m)::type::kId, v == 1, v == 2, team != 0))
+                        if (err == cudaSuccess)
+                            err = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, kDynSmem);
+        });
+        GRID_CUDA(err);
         attr_set[dev] = true;
     }
     return PMMH_OK;
@@ -2017,40 +2021,30 @@ GridArgs grid_args(const SvCall& c, const GridLayout& L, char* ws, int nobs, int
 int grid_after(const SvCall& c, const GridArgs& a, const GridLayout& L, char* ws, int nobs, int n, int lag, int G,
                int hess) {
     const cudaStream_t st = c.stream;
-    const int model = c.model;
     double* sums = (double*)(ws + L.sums);
     double* tailpart = (double*)(ws + L.tailpart);
     double* tail = (double*)(ws + L.tail);
     grid_reduce_kernel<<<nobs, 256, 0, st>>>(a.psum, G, sums);
-    if (c.filter) {
-        auto finish = model == PMMH_MODEL_SV_LEVERAGE ? grid_finish_kernel<false, false> : grid_finish_kernel<true, false>;
-        finish<<<(nobs + 255) / 256, 256, 0, st>>>(a.ctrl, sums, a.shiftv, a.xminv, nullptr, c.params, nobs, lag, (double)n,
-                                                   c.ll, c.filt, nullptr, nullptr, c.traj, c.diag, (long long*)(ws + L.info));
-        GRID_CUDA(cudaGetLastError());
-        return PMMH_OK;
-    }
-    if (hess) {
-        double* sumsH = (double*)(ws + L.sumsH);
-        double* tailpartH = (double*)(ws + L.tailpartH);
-        grid_reduceH_kernel<<<nobs, 640, 0, st>>>(a.psumH, G, lag, sumsH);
-        grid_tail_kernel<true, SvLeverageModel><<<dim3(L.nblk, lag), 256, 0, st>>>(a, sums, tailpart, tailpartH, L.nblk);
-        grid_hess_finish_kernel<<<1, 32, 0, st>>>(a.ctrl, sums, sumsH, tailpartH, c.params, L.nblk, nobs, lag, c.hess1, c.hess2);
-    } else if (model == PMMH_MODEL_LINEAR_GAUSSIAN) {
-        grid_tail_kernel<false, LinearGaussianModel><<<dim3(L.nblk, lag), 256, 0, st>>>(a, sums, tailpart, nullptr, L.nblk);
-    } else if (model == PMMH_MODEL_LINEAR_GAUSSIAN_FA) {
-        grid_tail_kernel<false, LinearGaussianFullyAdapted><<<dim3(L.nblk, lag), 256, 0, st>>>(a, sums, tailpart, nullptr, L.nblk);
-    } else if (model == PMMH_MODEL_LINEAR_GAUSSIAN_FA_GRAD) {
-        grid_tail_kernel<false, LinearGaussianFullyAdaptedGrad><<<dim3(L.nblk, lag), 256, 0, st>>>(a, sums, tailpart, nullptr,
-                                                                                                L.nblk);
-    } else {
-        grid_tail_kernel<false, SvLeverageModel><<<dim3(L.nblk, lag), 256, 0, st>>>(a, sums, tailpart, nullptr, L.nblk);
-    }
-    grid_tail_reduce_kernel<<<lag, 256, 0, st>>>(tailpart, L.nblk, tail);
-    auto finish = model == PMMH_MODEL_SV_LEVERAGE            ? grid_finish_kernel<false, true>
-                  : model == PMMH_MODEL_LINEAR_GAUSSIAN_FA_GRAD ? grid_finish_kernel<true, true, true>
-                                                                : grid_finish_kernel<true, true>;
-    finish<<<(nobs + 255) / 256, 256, 0, st>>>(a.ctrl, sums, a.shiftv, a.xminv, tail, c.params, nobs, lag, (double)n, c.ll,
-                                               c.filt, c.smo, c.grad, c.traj, c.diag, (long long*)(ws + L.info));
+    Models::with(c.model, [&](auto m) {   // (grid_check has refused an unknown id and a Hessian the model lacks)
+        typedef typename decltype(m)::type M;
+        const auto finish = c.filter ? grid_finish_for<typename M::Filter, false>() : grid_finish_for<M, true>();
+        if (!c.filter) {
+            if (!hess) {
+                grid_tail_kernel<false, M><<<dim3(L.nblk, lag), 256, 0, st>>>(a, sums, tailpart, nullptr, L.nblk);
+            } else if constexpr (M::kHessian) {
+                double* sumsH = (double*)(ws + L.sumsH);
+                double* tailpartH = (double*)(ws + L.tailpartH);
+                grid_reduceH_kernel<<<nobs, 640, 0, st>>>(a.psumH, G, lag, sumsH);
+                grid_tail_kernel<true, M><<<dim3(L.nblk, lag), 256, 0, st>>>(a, sums, tailpart, tailpartH, L.nblk);
+                grid_hess_finish_kernel<<<1, 32, 0, st>>>(a.ctrl, sums, sumsH, tailpartH, c.params, L.nblk, nobs, lag,
+                                                          c.hess1, c.hess2);
+            }
+            grid_tail_reduce_kernel<<<lag, 256, 0, st>>>(tailpart, L.nblk, tail);
+        }
+        finish<<<(nobs + 255) / 256, 256, 0, st>>>(a.ctrl, sums, a.shiftv, a.xminv, c.filter ? nullptr : tail, c.params,
+                                                   nobs, lag, (double)n, c.ll, c.filt, c.smo, c.grad, c.traj, c.diag,
+                                                   (long long*)(ws + L.info));
+    });
     GRID_CUDA(cudaGetLastError());
     return PMMH_OK;
 }

@@ -15,9 +15,9 @@ size_t sv_grid_ws_bytes(int nobs, int n, int lag, int G, int hist, int hess = 0,
 // `batch` problems of one shape (problem b's inputs and outputs one problem further on), each on its own G CTAs, in
 // waves of nteams = sv_grid_teams(batch, SMs, G) problems: one cooperative launch of (problems in the wave) x G CTAs per
 // wave.  Every problem's outputs are bit-identical to its run alone (batch = nteams = 1).  The workspace is
-// min(batch, nteams) slices of sv_grid_ws_bytes (hist: c.x_hist given).  c.model selects the instantiation (PMMH_MODEL_*, pf_model.cuh); hess:
-// the Hessian branch (SV only); c.filter: the filter alone (lag unused).  Host-streamed u (c.slot > 0) and the phase
-// clocks (c.prof) take batch = 1 only.
+// min(batch, nteams) slices of sv_grid_ws_bytes (hist: c.x_hist given).  c.model selects the instantiation (the table
+// Models in pf_model.cuh; the filter runs the model's Filter); hess: the Hessian branch (SV only); c.filter: the filter
+// alone (lag unused).  Host-streamed u (c.slot > 0) and the phase clocks (c.prof) take batch = 1 only.
 int sv_grid_teams(int batch, int sm_count, int G);
 int sv_grid_run(const SvCall& c, int batch, int nobs, int n, int lag, int G, int nteams, int hess);
 }  // namespace pmmh

@@ -131,6 +131,33 @@ def flps_sv_corr(obs, params, rvr, u, lag=10, compute_hessian=False, store_histo
     return out
 
 
+def _workspace_bytes(query, *sizes):
+    wb = ctypes.c_size_t()
+    _lib.check(getattr(_lib.load(), query)(*sizes, ctypes.byref(wb)), query)
+    return wb.value
+
+
+def _model_corr(name, model_id, obs, params, rvr, u, lag, hess, store_history, workspace):
+    """pmmh_<name>_corr after its workspace query pmmh_<name>_workspace_bytes: the smoother (name flps_model or
+    flps_model_batch) or the filter alone (filter_model or filter_model_batch)"""
+    lib = _lib.load()
+    obs, obs_stride, params, rvr, u, batch, n_obs, n = _sv_common(obs, params, rvr, u)
+    dev = u.device
+    smoother, batched = name.startswith("flps"), name.endswith("batch")
+    out = _sv_outputs(dev, batch, n_obs, n, smoother=smoother, hessian=bool(hess), history=store_history)
+    sizes = [n_obs, n] + ([lag] if smoother else []) + [batch] + ([hess] if smoother and batched else [])
+    ws = (workspace or Workspace()).get(_workspace_bytes("pmmh_%s_workspace_bytes" % name, *sizes), dev)
+    keys = ["filt", "smo", "log_like", "gradient", "traj"] if smoother else ["filt", "log_like", "traj"]
+    if smoother and batched:
+        keys += ["hess1", "hess2"]
+    outs = [_ptr(out.get(k)) for k in keys + ["diag", "X", "A"]]
+    entry = "pmmh_%s_corr" % name
+    _lib.check(getattr(lib, entry)(int(model_id), _ptr(obs), obs_stride, _ptr(params), _ptr(rvr), _ptr(u), *sizes,
+                                   *outs, _ptr(ws), ws.numel(), _stream()), entry)
+    out["_workspace"] = ws
+    return out
+
+
 def flps_model_corr(model_id, obs, params, rvr, u, lag=10, store_history=False, workspace=None):
     """Model-generic fixed-lag smoother (pmmh_flps_model_corr, csrc/pf_model.cuh): log-likelihood +
     gradient of [B] problems.  2 <= lag <= 10.  Up to 4096 particles: any B, one CTA per problem (chain
@@ -138,25 +165,11 @@ def flps_model_corr(model_id, obs, params, rvr, u, lag=10, store_history=False, 
     148 SMs), one persistent launch over the GPU (grid kernel, diag kernel 5).  Other sizes raise PmmhError.
     ``model_id``: _lib.MODEL_SV_LEVERAGE (bit-identical to flps_sv_corr on the same kernel),
     _lib.MODEL_LINEAR_GAUSSIAN, _lib.MODEL_LINEAR_GAUSSIAN_FA or _lib.MODEL_LINEAR_GAUSSIAN_FA_GRAD; params [B, 4]
-    (unused slots ignored).  The fully adapted models 2 and 3 take the series shifted by one (obs[1:]) and their
+    (unused slots ignored).  The fully adapted models 2 and 4 take the series shifted by one (obs[1:]) and their
     log_like lacks log p(y_1); model 4 adds model 2 a gradient whose slot k holds the contribution of obs[1:][k], so
     that the slots sum to the score of the full log-likelihood (include/pmmh_qn.h).
     No fallback pass: diag[:, PMMH_DIAG_STATUS] == 1 reports an abandoned evaluation."""
-    lib = _lib.load()
-    obs, obs_stride, params, rvr, u, batch, n_obs, n = _sv_common(obs, params, rvr, u)
-    dev = u.device
-    out = _sv_outputs(dev, batch, n_obs, n, history=store_history)
-    xh, ah = out.get("X"), out.get("A")
-    wb = ctypes.c_size_t()
-    _lib.check(lib.pmmh_flps_model_workspace_bytes(n_obs, n, lag, batch, ctypes.byref(wb)),
-               "pmmh_flps_model_workspace_bytes")
-    ws = (workspace or Workspace()).get(wb.value, dev)
-    _lib.check(lib.pmmh_flps_model_corr(
-        int(model_id), _ptr(obs), obs_stride, _ptr(params), _ptr(rvr), _ptr(u), n_obs, n, lag, batch,
-        _ptr(out["filt"]), _ptr(out["smo"]), _ptr(out["log_like"]), _ptr(out["gradient"]), _ptr(out["traj"]),
-        _ptr(out["diag"]), _ptr(xh), _ptr(ah), _ptr(ws), ws.numel(), _stream()), "pmmh_flps_model_corr")
-    out["_workspace"] = ws
-    return out
+    return _model_corr("flps_model", model_id, obs, params, rvr, u, lag, 0, store_history, workspace)
 
 
 def filter_model_corr(model_id, obs, params, rvr, u, store_history=False, workspace=None):
@@ -166,37 +179,16 @@ def filter_model_corr(model_id, obs, params, rvr, u, store_history=False, worksp
     particles per SM (grid kernel, diag kernel 5).  n_obs >= 2; other sizes raise PmmhError.  ``model_id`` and
     params as for flps_model_corr (model 4 runs model 2's filter).  No fallback pass: diag[:, PMMH_DIAG_STATUS] == 1 reports an abandoned
     evaluation."""
-    lib = _lib.load()
-    obs, obs_stride, params, rvr, u, batch, n_obs, n = _sv_common(obs, params, rvr, u)
-    dev = u.device
-    out = _sv_outputs(dev, batch, n_obs, n, smoother=False, history=store_history)
-    xh, ah = out.get("X"), out.get("A")
-    wb = ctypes.c_size_t()
-    _lib.check(lib.pmmh_filter_model_workspace_bytes(n_obs, n, batch, ctypes.byref(wb)),
-               "pmmh_filter_model_workspace_bytes")
-    ws = (workspace or Workspace()).get(wb.value, dev)
-    _lib.check(lib.pmmh_filter_model_corr(
-        int(model_id), _ptr(obs), obs_stride, _ptr(params), _ptr(rvr), _ptr(u), n_obs, n, batch,
-        _ptr(out["filt"]), _ptr(out["log_like"]), _ptr(out["traj"]), _ptr(out["diag"]), _ptr(xh), _ptr(ah),
-        _ptr(ws), ws.numel(), _stream()), "pmmh_filter_model_corr")
-    out["_workspace"] = ws
-    return out
+    return _model_corr("filter_model", model_id, obs, params, rvr, u, 2, 0, store_history, workspace)
 
 
 def flps_model_batch_workspace_bytes(n_obs, n_particles, lag, batch, compute_hessian=0):
-    lib = _lib.load()
-    wb = ctypes.c_size_t()
-    _lib.check(lib.pmmh_flps_model_batch_workspace_bytes(n_obs, n_particles, lag, batch, int(bool(compute_hessian)),
-                                                         ctypes.byref(wb)), "pmmh_flps_model_batch_workspace_bytes")
-    return wb.value
+    return _workspace_bytes("pmmh_flps_model_batch_workspace_bytes", n_obs, n_particles, lag, batch,
+                            int(bool(compute_hessian)))
 
 
 def filter_model_batch_workspace_bytes(n_obs, n_particles, batch):
-    lib = _lib.load()
-    wb = ctypes.c_size_t()
-    _lib.check(lib.pmmh_filter_model_batch_workspace_bytes(n_obs, n_particles, batch, ctypes.byref(wb)),
-               "pmmh_filter_model_batch_workspace_bytes")
-    return wb.value
+    return _workspace_bytes("pmmh_filter_model_batch_workspace_bytes", n_obs, n_particles, batch)
 
 
 def flps_model_batch_corr(model_id, obs, params, rvr, u, lag=10, compute_hessian=0, store_history=False,
@@ -208,21 +200,8 @@ def flps_model_batch_corr(model_id, obs, params, rvr, u, lag=10, compute_hessian
     ceil(N / 2048)); model ids as for flps_model_corr; compute_hessian for the SV model only.  Returns the dict of flps_model_corr, plus hess1 /
     hess2 [B, 4, 4] with compute_hessian.  No fallback pass: diag[:, PMMH_DIAG_STATUS] == 1 reports an abandoned
     problem, the others are unaffected."""
-    lib = _lib.load()
-    obs, obs_stride, params, rvr, u, batch, n_obs, n = _sv_common(obs, params, rvr, u)
-    dev = u.device
-    hess = int(bool(compute_hessian))
-    out = _sv_outputs(dev, batch, n_obs, n, hessian=bool(hess), history=store_history)
-    xh, ah = out.get("X"), out.get("A")
-    nbytes = flps_model_batch_workspace_bytes(n_obs, n, lag, batch, hess)
-    ws = (workspace or Workspace()).get(nbytes, dev)
-    _lib.check(lib.pmmh_flps_model_batch_corr(
-        int(model_id), _ptr(obs), obs_stride, _ptr(params), _ptr(rvr), _ptr(u), n_obs, n, lag, batch, hess,
-        _ptr(out["filt"]), _ptr(out["smo"]), _ptr(out["log_like"]), _ptr(out["gradient"]), _ptr(out["traj"]),
-        _ptr(out.get("hess1")), _ptr(out.get("hess2")), _ptr(out["diag"]), _ptr(xh), _ptr(ah), _ptr(ws), ws.numel(),
-        _stream()), "pmmh_flps_model_batch_corr")
-    out["_workspace"] = ws
-    return out
+    return _model_corr("flps_model_batch", model_id, obs, params, rvr, u, lag, int(bool(compute_hessian)),
+                       store_history, workspace)
 
 
 def filter_model_batch_corr(model_id, obs, params, rvr, u, store_history=False, workspace=None):
@@ -230,19 +209,7 @@ def filter_model_batch_corr(model_id, obs, params, rvr, u, store_history=False, 
     (pmmh_filter_model_batch_corr): the outputs of problem b are bit-identical to filter_model_corr on that problem
     alone (and to those outputs of flps_model_batch_corr).  Any B where a tile of the one-problem grid run fits one
     CTA, n_obs >= 2.  Returns the dict of filter_model_corr."""
-    lib = _lib.load()
-    obs, obs_stride, params, rvr, u, batch, n_obs, n = _sv_common(obs, params, rvr, u)
-    dev = u.device
-    out = _sv_outputs(dev, batch, n_obs, n, smoother=False, history=store_history)
-    xh, ah = out.get("X"), out.get("A")
-    nbytes = filter_model_batch_workspace_bytes(n_obs, n, batch)
-    ws = (workspace or Workspace()).get(nbytes, dev)
-    _lib.check(lib.pmmh_filter_model_batch_corr(
-        int(model_id), _ptr(obs), obs_stride, _ptr(params), _ptr(rvr), _ptr(u), n_obs, n, batch,
-        _ptr(out["filt"]), _ptr(out["log_like"]), _ptr(out["traj"]), _ptr(out["diag"]), _ptr(xh), _ptr(ah),
-        _ptr(ws), ws.numel(), _stream()), "pmmh_filter_model_batch_corr")
-    out["_workspace"] = ws
-    return out
+    return _model_corr("filter_model_batch", model_id, obs, params, rvr, u, 2, 0, store_history, workspace)
 
 
 def flps_sv_corr_philox(obs, params, rvr, seed, philox_offset, n_particles, lag=10, workspace=None):
