@@ -44,6 +44,14 @@
 //     threads (DRAM traffic 189 -> 138 MB per step, but the three dependent 4-byte gathers still miss L2:
 //     27 us against 14 us for the records, 118 us per step).  With the hints: 100 us; with the fence-free barrier
 //     (release / acquire on the counter, abandon flag in its bit 31): 94 - 96 us.
+//   * per-thread state off the stack (1024 threads at 64 registers, and 208 KB of shared memory leave ~28 KB of L1:
+//     a stack slot is an L2 round trip): the records pass selects the lagged ancestor by compare-and-select (pick8),
+//     phase C's rare exact search runs after its unrolled loop, the tie counters of phase C are shared-memory
+//     atomics, and the children's values, ancestor rows and mailbox slots of phase A sit in shared memory regions
+//     that are dead from phase C's ancestor fill to phase B (ChildSlots).  ptxas (-Xptxas -v): stack frame / spill
+//     stores / loads of the SV gradient instantiation 144 / 516 / 556 -> 32 / 96 / 112 bytes, team 152 / 544 / 568
+//     -> 80 / 316 / 492 (tools/grid_local_memory.py counts the STL / LDL sites per phase).  Measured (B200, 1000 W):
+//     94 -> 82 us per step, bit-identical outputs.
 //   * second instantiation HESS = true: the Hessian branch (:361-390, :472-534, :564-626), cumulative alpha in the second
 //     sector of 64-byte record / payload entries; 162 us per step (DESIGN 4.0).
 //   * host-resident u: particle-major slots filled by the copy engine, one 32-byte sector (4 steps) per particle re-laid
@@ -158,6 +166,7 @@ struct GridArgs {
 
 struct StepScalars {
     double S, invS, mhat, shat, inv_shat, shift, lo, scale, tot, offk;
+    double tol_soft, tol_near;   // resampling ties: sequential-vs-tree summation bound, 64 ulp of N
     int carry, abort_now, binlo, binhi;
 };
 
@@ -263,17 +272,13 @@ __device__ __forceinline__ int warp_incl_max(int v, int lane) {
     }
     return v;
 }
+// r[min(idx, 7)] for idx >= 0 by compare-and-select over the static indices: a runtime index into r would put the
+// records of the records pass on the stack
 __device__ __forceinline__ int pick8(const int (&r)[8], int idx) {
-    switch (idx) {
-        case 0: return r[0];
-        case 1: return r[1];
-        case 2: return r[2];
-        case 3: return r[3];
-        case 4: return r[4];
-        case 5: return r[5];
-        case 6: return r[6];
-        default: return r[7];
-    }
+    int v = r[0];
+#pragma unroll
+    for (int z = 1; z < 8; ++z) v = idx >= z ? r[z] : v;
+    return v;
 }
 
 // the resampling point of child j, (u + j) / N as the reference computes it (:703)
@@ -281,27 +286,34 @@ __device__ __forceinline__ double cpoint(double u, int j, double dn, double inv_
     const double s = u + (double)j;
     return pow2 ? s * inv_n : s / dn;
 }
-__device__ __noinline__ int count_le_slow(int est, double c, double u, int N, double dn, double inv_n, bool pow2) {
+__device__ __forceinline__ int count_le_slow(int est, double c, double u, int N, double dn, double inv_n, bool pow2) {
     while (est > 0 && cpoint(u, est - 1, dn, inv_n, pow2) > c) --est;
     while (est < N && cpoint(u, est, dn, inv_n, pow2) <= c) ++est;
     return est;
 }
 // #{ j in [0, N) : (u + j) / N <= c }: closed form, then the exact predicate of :703-711 on both
-// neighbours.  frac_out = distance of c*N - u to the nearest integer (how close to a tie).
-__device__ __forceinline__ int count_le(double c, double u, int N, double dn, double inv_n, bool pow2,
-                                        double& frac_out) {
+// neighbours.  false: the closed form missed (a tie within rounding, or the ends of the range: rare), `est` is where
+// the exact search count_le_slow starts.  frac_out = distance of c*N - u to the nearest integer (how close to a tie).
+__device__ __forceinline__ bool count_le_fast(double c, double u, int N, double dn, double inv_n, bool pow2, int& est,
+                                              double& frac_out) {
     const double e = c * dn - u;
-    if (!(e >= 0.0) || e >= dn - 1.0) {   // the ends of the range: rare, exact search
+    if (!(e >= 0.0) || e >= dn - 1.0) {
         frac_out = 1.0;
-        return count_le_slow(e >= 0.0 ? N : 0, c, u, N, dn, inv_n, pow2);
+        est = e >= 0.0 ? N : 0;
+        return false;
     }
     const int fi = (int)e;               // floor(e), 0 <= fi <= N - 2
     const double fl = (double)fi;
     const double fr = e - fl;
     frac_out = fmin(fr, 1.0 - fr);
     const double slo = u + fl, shi = u + (fl + 1.0);   // u + j for j = fi, fi + 1 (both exact conversions)
-    const bool ok = pow2 ? (slo * inv_n <= c && !(shi * inv_n <= c)) : (slo / dn <= c && !(shi / dn <= c));
-    return ok ? fi + 1 : count_le_slow(fi + 1, c, u, N, dn, inv_n, pow2);
+    est = fi + 1;
+    return pow2 ? (slo * inv_n <= c && !(shi * inv_n <= c)) : (slo / dn <= c && !(shi / dn <= c));
+}
+__device__ __forceinline__ int count_le(double c, double u, int N, double dn, double inv_n, bool pow2,
+                                        double& frac_out) {
+    int est;
+    return count_le_fast(c, u, N, dn, inv_n, pow2, est, frac_out) ? est : count_le_slow(est, c, u, N, dn, inv_n, pow2);
 }
 
 __device__ __forceinline__ int fine_bin(double x, double mhat, double inv_shat) {
@@ -420,6 +432,21 @@ __device__ __forceinline__ GridArgs team_args(const GridArgs& a0, const GridTeam
     return a;
 }
 
+// K values per thread, entry kk of thread tid for child kk * GT + tid: in shared memory from `base` on (SH; every
+// slot is read back only by the thread that wrote it, so no synchronisation), or in registers
+template <class T, int K, int GT, bool SH>
+struct ChildSlots {
+    T* p;
+    __device__ __forceinline__ explicit ChildSlots(unsigned char* base) : p((T*)base + threadIdx.x) {}
+    __device__ __forceinline__ T& operator[](int kk) { return p[kk * GT]; }
+};
+template <class T, int K, int GT>
+struct ChildSlots<T, K, GT, false> {
+    T v[K];
+    __device__ __forceinline__ explicit ChildSlots(unsigned char*) {}
+    __device__ __forceinline__ T& operator[](int kk) { return v[kk]; }
+};
+
 // ---------------------------------------------------------------------------------------------
 // the kernel
 // ---------------------------------------------------------------------------------------------
@@ -454,6 +481,11 @@ __global__ void __launch_bounds__(GT, 1) sv_grid_kernel(const GridArgs a_in, con
     double* s_sh = (double*)(smem + 131072);           // [kCap] unnormalised weights, sorted order
     int* s_sub = (int*)(smem + 196608);                // [kNSB] sub-bin counters, then first positions
     int* s_ub = s_jb;                                  // [kCap] child range ends (phase C)
+    // phase A1 -> A2: the children's values, parent / lagged ancestor rows and mailbox slots (xn, bp, kr below) in the
+    // s_jb / s_ab / s_sh regions, dead from the end of phase C's ancestor fill to phase B; the Hessian branch's
+    // s_deflist holds s_jb / s_ab then, so there they stay in registers; so they do in the generic filter, whose
+    // phase A holds them there with less stack and spilling than through shared memory (ptxas -v)
+    constexpr bool SLOTS_SMEM = !HESS && (SMO || !GEN);
     // phase A view (Hessian branch: list of deferred alpha terms = (child, parent row) pairs in the s_jb / s_ab region)
     int2* s_deflist = (int2*)(smem + 65536);         // [kCap]
     int* s_fhist = (int*)smem;                         // [kNF] histogram of this CTA's children
@@ -468,6 +500,7 @@ __global__ void __launch_bounds__(GT, 1) sv_grid_kernel(const GridArgs a_in, con
     __shared__ int s_wi[32];
     __shared__ long long s_prof[kProf];
     __shared__ int s_ndef;   // Hessian branch: length of the list of deferred alpha terms
+    __shared__ unsigned s_ties[2];   // resampling decisions near a tie (diag: near, soft) of this CTA
 
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     const int c = TEAM ? (int)(blockIdx.x % (unsigned)a.G) : blockIdx.x, G = a.G, N = a.N, NOBS = a.NOBS, L = a.LAG, Wc = a.Wc, RP = a.RP;
@@ -482,7 +515,7 @@ __global__ void __launch_bounds__(GT, 1) sv_grid_kernel(const GridArgs a_in, con
     const unsigned long long pol_rld = pol_dead, pol_pld = pol_dead, pol_xld = pol_dead, pol_rst = pol_keep;
     constexpr double kBinW = 2.0 * kZ / (double)kNF;    // width of a histogram bin in predicted sd
     unsigned epoch = 0;                 // arrives done so far
-    unsigned cnt_near = 0, cnt_soft = 0, cnt_key = 0;
+    unsigned cnt_key = 0;
     int my_max_bin = 0;
     long long pclk = 0;
     const bool prof = a.prof != nullptr;
@@ -532,6 +565,9 @@ __global__ void __launch_bounds__(GT, 1) sv_grid_kernel(const GridArgs a_in, con
     if (tid == 0) {
         M::init(s_k, a.params);
         s_sc.abort_now = 0;
+        s_sc.tol_soft = 2.220446049250313e-16 * dn * (4.0 + 2.0 * sqrt(dn));
+        s_sc.tol_near = 64.0 * 2.220446049250313e-16 * dn;
+        s_ties[0] = s_ties[1] = 0;
         for (int i = 0; i < kProf; ++i) s_prof[i] = 0;
     }
     for (int i = tid; i < kMaxTiles; i += GT) s_tcnt[i] = 0;
@@ -658,10 +694,10 @@ __global__ void __launch_bounds__(GT, 1) sv_grid_kernel(const GridArgs a_in, con
         {
             const double invS = s_sc.invS, offk = s_sc.offk;
             const int Lc = ((n + GT - 1) / GT) | 1, q0 = tid * Lc;
-            const double tol_soft = 2.220446049250313e-16 * dn * (4.0 + 2.0 * sqrt(dn));
-            const double tol_near = 64.0 * 2.220446049250313e-16 * dn;
+            const double tol_soft = s_sc.tol_soft, tol_near = s_sc.tol_near;
+            unsigned nsoft = 0, nnear = 0;
             int ubv[KCH];
-            int rmax = 0;
+            unsigned slow = 0;   // bit kk: the closed form missed for parent q0 + kk, exact search below
             double run = 0.0;
 #pragma unroll
             for (int kk = 0; kk < KCH; ++kk) {
@@ -675,13 +711,41 @@ __global__ void __launch_bounds__(GT, 1) sv_grid_kernel(const GridArgs a_in, con
                         ub = N;
                     } else {
                         double fr;
-                        ub = count_le(cN, ur, N, dn, inv_n, pow2, fr);
+                        if (!count_le_fast(cN, ur, N, dn, inv_n, pow2, ub, fr)) {
+                            slow |= 1u << kk;
+                            s_ub[q] = ub;
+                        }
                         if (fr < tol_soft) {
-                            ++cnt_soft;
-                            if (fr < tol_near * fmax(cN, inv_n)) ++cnt_near;
+                            ++nsoft;
+                            if (fr < tol_near * fmax(cN, inv_n)) ++nnear;
                         }
                     }
-                    rmax = max(rmax, ub);
+                    ubv[kk] = ub;
+                }
+            }
+            if (nsoft) {
+                atomicAdd(&s_ties[1], nsoft);
+                if (nnear) atomicAdd(&s_ties[0], nnear);
+            }
+            if (slow) {
+                // the exact search, kept out of the unrolled loop (its live registers would go to the stack): the
+                // same running sum again, the result through this thread's own s_ub slots
+                double rs = 0.0;
+#pragma unroll 1
+                for (int kk = 0; kk < Lc && q0 + kk < n; ++kk) {
+                    const int q = q0 + kk;
+                    rs = rs + s_sh[q];
+                    if ((slow >> kk) & 1u) s_ub[q] = count_le_slow(s_ub[q], (offk + (toff + rs)) * invS, ur, N, dn, inv_n, pow2);
+                }
+#pragma unroll
+                for (int kk = 0; kk < KCH; ++kk)
+                    if ((slow >> kk) & 1u) ubv[kk] = s_ub[q0 + kk];
+            }
+            int rmax = 0;
+#pragma unroll
+            for (int kk = 0; kk < KCH; ++kk) {
+                if (kk < Lc && q0 + kk < n) {
+                    rmax = max(rmax, ubv[kk]);
                     ubv[kk] = rmax;
                 }
             }
@@ -763,14 +827,15 @@ __global__ void __launch_bounds__(GT, 1) sv_grid_kernel(const GridArgs a_in, con
         // --------------------------------------------------------------------------------------
         // phase A1: parents of this CTA's children, propagation (:354-358), value histogram
         // --------------------------------------------------------------------------------------
-        double xn[KPT];
-        int bp[KPT];
+        ChildSlots<double, KPT, GT, SLOTS_SMEM> xn(smem + 131072);   // value
+        ChildSlots<int, KPT, GT, SLOTS_SMEM> bp(smem + 65536);       // birth row of the parent, then lagged ancestor row
         {
+            int hp[KPT];   // sorted position of the parent
 #pragma unroll
             for (int kk = 0; kk < KPT; ++kk) {
                 const int i = kk * GT + tid;
-                bp[kk] = 0;
-                if (i < nc) bp[kk] = ld_hint_b32(&a.H[jb + i], pol_dead);
+                hp[kk] = 0;
+                if (i < nc) hp[kk] = ld_hint_b32(&a.H[jb + i], pol_dead);
             }
             const double y1 = a.obs[t - 1];
             const double ylag = a.obs[t >= 2 ? t - 2 : 0];   // Q5: the score terms of step i use obs[i - LAG]; i = t + LAG - 2
@@ -819,7 +884,7 @@ __global__ void __launch_bounds__(GT, 1) sv_grid_kernel(const GridArgs a_in, con
                     xe[u] = make_double2(0.0, 0.0);
                     uu[u] = 0.0;
                     if (i < nc) {
-                        int p = bp[k0 + u];
+                        int p = hp[k0 + u];
                         if ((unsigned)p >= (unsigned)N) {
                             orphan = true;
                             p = 0;
@@ -1019,7 +1084,7 @@ __global__ void __launch_bounds__(GT, 1) sv_grid_kernel(const GridArgs a_in, con
         }
         __syncthreads();
         PROF_MARK(20);   // A2: histogram scan + tile map
-        int kr[KPT];
+        ChildSlots<int, KPT, GT, SLOTS_SMEM> kr(smem + 98304);   // (tile << 16) | rank in the tile's run
         {
             const double mhat = s_sc.mhat, inv_shat = s_sc.inv_shat;
 #pragma unroll
@@ -1537,14 +1602,14 @@ __global__ void __launch_bounds__(GT, 1) sv_grid_kernel(const GridArgs a_in, con
         if (s_sc.abort_now) break;
     }
 
-    // diagnostics
-    cnt_near = __reduce_add_sync(kFullMask, cnt_near);
-    cnt_soft = __reduce_add_sync(kFullMask, cnt_soft);
+    // diagnostics (every exit from the time loop follows a __syncthreads: s_ties is complete)
+    if (tid == 0) {
+        if (s_ties[0]) atomicAdd(&ctrl->near_ties, (unsigned long long)s_ties[0]);
+        if (s_ties[1]) atomicAdd(&ctrl->soft_ties, (unsigned long long)s_ties[1]);
+    }
     cnt_key = __reduce_add_sync(kFullMask, cnt_key);
     my_max_bin = __reduce_max_sync(kFullMask, my_max_bin);
     if (lane == 0) {
-        if (cnt_near) atomicAdd(&ctrl->near_ties, (unsigned long long)cnt_near);
-        if (cnt_soft) atomicAdd(&ctrl->soft_ties, (unsigned long long)cnt_soft);
         if (cnt_key) atomicAdd(&ctrl->key_ties, (unsigned long long)(cnt_key / 2));
         atomicMax(&ctrl->max_bin, my_max_bin);
     }
