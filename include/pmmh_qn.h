@@ -213,6 +213,17 @@ int pmmh_flps_sv_corr_philox(const double* d_obs, const double* d_params, const 
  * pmmh_flps_model_batch_corr take it on the sizes of model 2 (compute_hessian == 1 is refused); the filter entries run
  * model 2's filter for it. */
 #define PMMH_MODEL_LINEAR_GAUSSIAN_FA_GRAD 4   /* id 3 is unassigned: every entry refuses it as an unknown id */
+/* PMMH_MODEL_LINEAR_GAUSSIAN_FA_HESS: model 4 with a fixed-lag Hessian.  Every output model 4 has is bit-identical to
+ * model 4's on every entry and shape (with compute_hessian 0 or 1); the filter entries run model 2's filter for it.
+ * pmmh_flps_model_batch_corr with compute_hessian == 1 (on the grid kernel: batch 1 and small n_particles included)
+ * writes d_hess1 / d_hess2 [4][4] (rows and columns 0..2 = phi, sigma_v, sigma_e; row and column 3 are 0) by Louis'
+ * identity on the gradient's pairs and weights: with s_k the term of gradient slot k and H_k its matrix of second
+ * derivatives, hess1 = sum_k E[H_k] and hess2 = sum_k E[s_k s_k' + alpha_k s_k' + s_k alpha_k'], where alpha_k is the
+ * sum of the slot terms 0 .. k-1 along the lineage of the particle read (the score accumulated along its genealogy),
+ * each expectation under the weights that read slot k.  hess1 + hess2 - g g', g = the sum of the gradient slots,
+ * estimates the Hessian of the full log-likelihood log p(y_1 .. y_T).  alpha runs along the whole genealogy, so the
+ * estimate's variance grows with n_obs / n_particles. */
+#define PMMH_MODEL_LINEAR_GAUSSIAN_FA_HESS 6   /* id 5 is unassigned */
 int pmmh_flps_model_workspace_bytes(int n_obs, int n_particles, int lag, int batch, size_t* bytes);
 int pmmh_flps_model_corr(int model_id, const double* d_obs, long long obs_stride, const double* d_params,
                          const double* d_rvr, const double* d_u, int n_obs, int n_particles, int lag, int batch,
@@ -255,7 +266,8 @@ int pmmh_filter_model_corr(int model_id, const double* d_obs, long long obs_stri
  * d_diag [PMMH_DIAG_COUNT]; optional d_x_hist / d_a_hist [batch][n_obs][n_particles], given together.
  *   Shapes: any batch >= 1 with a tile of n_particles / G particles that fits one CTA (up to 7168 particles per
  * CTA); the smoother needs 2 <= lag <= 10 and n_obs >= 2 lag, the filter n_obs >= 2.  compute_hessian == 1 (the
- * SV model's Hessian branch; d_hess1 / d_hess2 required) is taken for PMMH_MODEL_SV_LEVERAGE only; with 0 the
+ * Hessian branch; d_hess1 / d_hess2 required) is taken for PMMH_MODEL_SV_LEVERAGE and
+ * PMMH_MODEL_LINEAR_GAUSSIAN_FA_HESS only; with 0 the
  * Hessian outputs may be NULL and are not written.  Anything else is refused with PMMH_ERR_INVALID, by the
  * workspace queries too; a workspace below the query's size gives PMMH_ERR_WORKSPACE.
  *   Workspace: min(batch, nteams) slices of the one-problem grid workspace with history (per slice:

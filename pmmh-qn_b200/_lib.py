@@ -21,6 +21,7 @@ DIAG_NEAR_TIES, DIAG_MAX_BIN, DIAG_STATUS, DIAG_KEY_TIES, DIAG_WAVEFRONT, DIAG_T
 DIAG_SOFT_TIES = 4   # flps on the grid kernel (same slot as the bpf wave-front depth)
 DIAG_COUNT = 8
 MODEL_SV_LEVERAGE, MODEL_LINEAR_GAUSSIAN, MODEL_LINEAR_GAUSSIAN_FA, MODEL_LINEAR_GAUSSIAN_FA_GRAD = 0, 1, 2, 4
+MODEL_LINEAR_GAUSSIAN_FA_HESS = 6
 BPF_PARITY, BPF_INTENDED = 0, 1
 
 # name -> (restype, argtypes); mirrors include/pmmh_qn.h one to one

@@ -10,7 +10,10 @@
 //   M::kId                               its model id (PMMH_MODEL_*, include/pmmh_qn.h)
 //   M::Filter                            the model whose filter instantiation the filter entries run (itself, or
 //                                        the model it adds a gradient to)
-//   M::kHessian                          constexpr: the kernels have its Hessian branch (the SV model only)
+//   M::Gradient                          the model whose smoother instantiation a call without the Hessian runs
+//                                        (itself, or the model it adds a Hessian to)
+//   M::kHessian                          constexpr: the kernels have its Hessian branch (the SV model: the
+//                                        reference's, Pairing::Reference; model 6: the generic one, grid kernel)
 //   struct M::Const                      constants derived from the parameter vector (<= 4 doubles)
 //   M::init(Const&, const double* par)
 //   M::initial_state(c)                  value of every particle of generation 0 (the reference's
@@ -34,6 +37,9 @@
 //                                        grid kernel then skips the calls; the smoother still runs)
 //   M::kPairing                          constexpr: how the fixed-lag terms are paired (below)
 //   M::score_last(c, x, y_next, g)       (Pairing::Predictive only) the final generation's term
+//   M::hess_main(c, curr, next, y, h)    (generic Hessian branch only) the second derivatives of score_main's term:
+//   M::hess_last(c, x, y_next, h)        10 entries, the upper triangle of the 4 x 4 matrix row by row ((0,0), (0,1),
+//                                        (0,2), (0,3), (1,1), .. (3,3)); and of score_last's term
 // A new model is such a struct plus its entry in Models at the end of this file, and its id in include/pmmh_qn.h.
 //
 // Pairing::Reference (the SV model, parity with the reference): the reference's quirks Q5 / Q6.  The main loop
@@ -52,6 +58,14 @@
 // (x_NOBS-1, x_NOBS) with x_NOBS integrated out).  Slot t then holds the contribution of obs[t], and the slots sum
 // to an estimate of the score of the whole series.
 // Unused gradient slots stay 0.  Model ids are part of the C ABI (include/pmmh_qn.h).
+//
+// The generic Hessian branch (Pairing::Predictive, grid kernel): Louis' identity on the gradient's pairs and weights.
+// s_k is gradient slot k's term and H_k = hess_main / hess_last of the same pair; alpha is the score accumulated along
+// a lineage, alpha(x_0) = 0, alpha(child) = alpha(parent) + score_main(parent, child, obs[t - 1]) at the child's birth
+// (generation t).  hess1 = sum_k E[H_k] and hess2 = sum_k E[s_k s_k' + alpha_k s_k' + s_k alpha_k'] under the weights
+// that read slot k, alpha_k = alpha of x_k on the lineage read (the pair's first state).  The estimate of the
+// log-likelihood's Hessian is hess1 + hess2 - g g' with g = the sum of the gradient slots.  alpha runs along the whole
+// genealogy, so its variance grows with T / N as the genealogy degenerates (the reference's estimator for the SV model).
 #pragma once
 #include <math.h>
 
@@ -78,6 +92,7 @@ __host__ __device__ constexpr int pair_slot(Pairing p, int t) { return p == Pair
 struct SvLeverageModel {
     static constexpr int kId = PMMH_MODEL_SV_LEVERAGE;
     typedef SvLeverageModel Filter;
+    typedef SvLeverageModel Gradient;
     static constexpr bool kHessian = true;
     typedef SvConst Const;
     static __device__ __forceinline__ void init(Const& c, const double* par) { sv_const_init(c, par); }
@@ -130,6 +145,7 @@ struct SvLeverageModel {
 struct LinearGaussianModel {
     static constexpr int kId = PMMH_MODEL_LINEAR_GAUSSIAN;
     typedef LinearGaussianModel Filter;
+    typedef LinearGaussianModel Gradient;
     static constexpr bool kHessian = false;
     struct Const {
         double phi, sv, se, inv_sv2, inv_se2, log_se;
@@ -193,6 +209,7 @@ struct LinearGaussianModel {
 struct LinearGaussianFullyAdapted {
     static constexpr int kId = PMMH_MODEL_LINEAR_GAUSSIAN_FA;
     typedef LinearGaussianFullyAdapted Filter;
+    typedef LinearGaussianFullyAdapted Gradient;
     static constexpr bool kHessian = false;
     struct Const {
         double phi, sv, se, k, sdp, inv_s2, log_s;   // gain, proposal sd, predictive variance
@@ -257,6 +274,7 @@ struct LinearGaussianFullyAdapted {
 // oracle/generic_pf.py LinearGaussianFullyAdaptedGrad and the exact fixed-lag Kalman targets of oracle/kalman.py.
 struct LinearGaussianFullyAdaptedGrad : LinearGaussianFullyAdapted {
     static constexpr int kId = PMMH_MODEL_LINEAR_GAUSSIAN_FA_GRAD;
+    typedef LinearGaussianFullyAdaptedGrad Gradient;
     struct Const : LinearGaussianFullyAdapted::Const {
         double inv_sv2, inv_sv, inv_se2, inv_se;
     };
@@ -293,6 +311,37 @@ struct LinearGaussianFullyAdaptedGrad : LinearGaussianFullyAdapted {
     }
 };
 
+// ---- 6: model 4 with the generic Hessian branch (grid kernel; the header comment above).  Every output model 4 has is
+// bit-identical to it: a call without the Hessian runs model 4's instantiation (Gradient), the filter entries model 2's.
+// The Hessian hooks are the second derivatives over (phi, sigma_v, sigma_e) of score_main's and score_last's terms; row
+// and column 3 stay 0.
+struct LinearGaussianFullyAdaptedHess : LinearGaussianFullyAdaptedGrad {
+    static constexpr int kId = PMMH_MODEL_LINEAR_GAUSSIAN_FA_HESS;
+    static constexpr bool kHessian = true;
+    static __device__ __forceinline__ void hess_main(const Const& c, double curr, double next, double y, double h[10]) {
+        const double r = next - c.phi * curr;
+        const double ry = y - next;
+        h[0] = -(curr * curr) * c.inv_sv2;
+        h[1] = -2.0 * (r * curr) * (c.inv_sv2 * c.inv_sv);
+        h[4] = (1.0 - 3.0 * (r * r) * c.inv_sv2) * c.inv_sv2;
+        h[7] = (1.0 - 3.0 * (ry * ry) * c.inv_se2) * c.inv_se2;
+        h[2] = h[3] = h[5] = h[6] = h[8] = h[9] = 0.0;
+    }
+    // s2 = sigma_v^2 + sigma_e^2, r = y_next - phi x, a = r^2 / s2 - 1, b = 2 r^2 / s2 - 1
+    static __device__ __forceinline__ void hess_last(const Const& c, double x, double y_next, double h[10]) {
+        const double r = y_next - c.phi * x;
+        const double a = (r * r) * c.inv_s2 - 1.0, b = 2.0 * (r * r) * c.inv_s2 - 1.0;
+        const double i4 = c.inv_s2 * c.inv_s2;
+        h[0] = -(x * x) * c.inv_s2;
+        h[1] = -2.0 * (r * x) * c.sv * i4;
+        h[2] = -2.0 * (r * x) * c.se * i4;
+        h[4] = (a - 2.0 * (c.sv * c.sv) * c.inv_s2 * b) * c.inv_s2;
+        h[5] = -2.0 * (c.sv * c.se) * i4 * b;
+        h[7] = (a - 2.0 * (c.se * c.se) * c.inv_s2 * b) * c.inv_s2;
+        h[3] = h[6] = h[8] = h[9] = 0.0;
+    }
+};
+
 // ---- the model table: every model the kernels are instantiated for.  Models::with(id, f) calls f(ModelTag<M>()) for
 // the model M of that id (false, and no call, for an unknown id); Models::each(f) calls it for every model.
 template <class M>
@@ -311,7 +360,8 @@ struct ModelList {
         return same == (int)sizeof...(Ms);
     }
 };
-typedef ModelList<SvLeverageModel, LinearGaussianModel, LinearGaussianFullyAdapted, LinearGaussianFullyAdaptedGrad>
+typedef ModelList<SvLeverageModel, LinearGaussianModel, LinearGaussianFullyAdapted, LinearGaussianFullyAdaptedGrad,
+                  LinearGaussianFullyAdaptedHess>
     Models;
 static_assert(Models::ids_distinct(), "every model states its own id");
 

@@ -6,7 +6,7 @@
 // iteration) and, as a second instantiation, the Hessian branch (compute_hessian = 1,
 // :361-390 alpha recursion with Q7 / Q8, :472-534, :564-626: what mh_second_order.py asks for).
 // The kernel is a template over the MODEL (pf_model.cuh: propagation, log-weight, score terms);
-// the Hessian branch exists for the reference's SV model only.
+// its Hessian branch exists for the reference's SV model only.
 //
 // One persistent launch, CTAs loop over the problems of the batch; nothing is exchanged between
 // CTAs.  Per time step (all in shared memory unless noted):
@@ -708,7 +708,8 @@ static cudaError_t chain_launch_one(const SvArgs& a, int grid, int smem, cudaStr
     return cudaGetLastError();
 }
 
-// the filter runs the instantiation of M::Filter; the Hessian branch exists where M::kHessian
+// the filter runs the instantiation of M::Filter, the smoother without the Hessian that of M::Gradient; this kernel has
+// the SV model's Hessian branch only (the generic one is the grid kernel's)
 cudaError_t sv_chain_launch(const SvArgs& a, int grid, int filter, cudaStream_t stream) {
     const int smem = sv_chain_smem_bytes(a.N);
     cudaError_t err = cudaErrorInvalidValue;
@@ -717,8 +718,8 @@ cudaError_t sv_chain_launch(const SvArgs& a, int grid, int filter, cudaStream_t 
         if (filter) {
             if (!a.hess) err = chain_launch_one<typename M::Filter, false, false>(a, grid, smem, stream);
         } else if (!a.hess) {
-            err = chain_launch_one<M, false, true>(a, grid, smem, stream);
-        } else if constexpr (M::kHessian) {
+            err = chain_launch_one<typename M::Gradient, false, true>(a, grid, smem, stream);
+        } else if constexpr (M::kHessian && M::kPairing == Pairing::Reference) {
             err = chain_launch_one<M, true, true>(a, grid, smem, stream);
         }
     });

@@ -390,6 +390,20 @@ __device__ __forceinline__ void deferred_alpha_pass(const GridArgs& a, const SvC
     }
 }
 
+// generic Hessian branch (pf_model.cuh): h1 += w H and h2 += w (g g' + al g' + g al') over the upper triangles (row by
+// row, as M::hess_main writes H)
+__device__ __forceinline__ void louis_add(const double (&hh)[10], const double (&g)[4], const double* al, double w,
+                                          double* h1, double* h2) {
+    int z = 0;
+#pragma unroll
+    for (int r = 0; r < 4; ++r)
+#pragma unroll
+        for (int c = r; c < 4; ++c, ++z) {
+            h1[z] = fma(w, hh[z], h1[z]);
+            h2[z] = fma(w, g[r] * g[c] + al[r] * g[c] + g[r] * al[c], h2[z]);
+        }
+}
+
 // Teams: CTA b runs tile b % G of problem (team) b / G.  a_in addresses team 0; team k's workspace slice starts
 // ws_stride bytes after team k-1's (the one-problem layout, so every team has its own barrier counter, abandon bit
 // and status word), its inputs and history one problem further on (obs by obs_stride doubles)
@@ -462,7 +476,10 @@ __global__ void __launch_bounds__(GT, 1) sv_grid_kernel(const GridArgs a_in, con
     if constexpr (TEAM) a_team = team_args(a_in, tm);
     const GridArgs& a = TEAM ? a_team : a_in;   // this CTA's problem
     constexpr bool GEN = !std::is_same<M, SvLeverageModel>::value;
-    static_assert(!(GEN && HESS), "the Hessian branch exists for the SV model only");
+    // (static: a plain constexpr local changes the register allocation of the SV instantiations)
+    static constexpr bool SVH = HESS && !GEN;   // the SV model's Hessian branch (the reference's, Q7 / Q8)
+    static constexpr bool GENH = HESS && GEN;   // the generic Hessian branch (pf_model.cuh), predictive pairing
+    static_assert(!GENH || M::kPairing == Pairing::Predictive, "the generic Hessian branch pairs the terms predictively");
     static_assert(SMO || !HESS, "the Hessian branch needs the smoother");
     constexpr int KPT = kCap / GT;          // entries per thread (strided assignment)
     constexpr int KCH = KPT | 1;            // longest chunk of the thread-contiguous passes (odd)
@@ -482,10 +499,10 @@ __global__ void __launch_bounds__(GT, 1) sv_grid_kernel(const GridArgs a_in, con
     int* s_sub = (int*)(smem + 196608);                // [kNSB] sub-bin counters, then first positions
     int* s_ub = s_jb;                                  // [kCap] child range ends (phase C)
     // phase A1 -> A2: the children's values, parent / lagged ancestor rows and mailbox slots (xn, bp, kr below) in the
-    // s_jb / s_ab / s_sh regions, dead from the end of phase C's ancestor fill to phase B; the Hessian branch's
+    // s_jb / s_ab / s_sh regions, dead from the end of phase C's ancestor fill to phase B; the SV Hessian branch's
     // s_deflist holds s_jb / s_ab then, so there they stay in registers; so they do in the generic filter, whose
     // phase A holds them there with less stack and spilling than through shared memory (ptxas -v)
-    constexpr bool SLOTS_SMEM = !HESS && (SMO || !GEN);
+    constexpr bool SLOTS_SMEM = !SVH && (SMO || !GEN);
     // phase A view (Hessian branch: list of deferred alpha terms = (child, parent row) pairs in the s_jb / s_ab region)
     int2* s_deflist = (int2*)(smem + 65536);         // [kCap]
     int* s_fhist = (int*)smem;                         // [kNF] histogram of this CTA's children
@@ -598,7 +615,9 @@ __global__ void __launch_bounds__(GT, 1) sv_grid_kernel(const GridArgs a_in, con
             if constexpr (SMO) st_rec(&a.R[(size_t)(pstart + q) * RS], pol_keep, 0, 0, 0, 0, 0, 0, 0, 0);
             if constexpr (HESS) {
                 st_rec(&a.R[(size_t)(pstart + q) * RS + 1], pol_keep, 0, 0, 0, 0, 0, 0, 0, 0);   // alpha = 0
-                if (pstart + q < a.SQ) a.xlow[(size_t)(pstart + q) * NOBS] = mu;
+                if constexpr (SVH) {
+                    if (pstart + q < a.SQ) a.xlow[(size_t)(pstart + q) * NOBS] = mu;
+                }
             }
             if (a.hist) {
                 a.Xhist[pstart + q] = mu;
@@ -933,7 +952,7 @@ __global__ void __launch_bounds__(GT, 1) sv_grid_kernel(const GridArgs a_in, con
             if (orphan) GRID_FLAG(4);
         }
         PROF_MARK(19);   // A1: gathers + propagation + histogram
-        if (HESS && tid == 0) s_ndef = 0;
+        if (SVH && tid == 0) s_ndef = 0;
         __syncthreads();
         {
             int* gh = a.ghist + (size_t)par * kNF;
@@ -955,27 +974,29 @@ __global__ void __launch_bounds__(GT, 1) sv_grid_kernel(const GridArgs a_in, con
             // Q7: the "current" state is particles[t - 1 + ancestor] read through the flat layout = sorted value
             // `sl` of time tq (table of the first SQ sorted values of every generation), or the unsorted new value
             // `sl` of this generation (complete only after barrier 1: deferred), or 0.  Q8: obs[t - LAG] wraps.
-            const double yi = a.obs[t], ylagH = HESS ? obs_wrap(a.obs, t - L, NOBS) : 0.0;
+            // Generic Hessian branch: the child's term is score_main of its own pair (parent value from the payload
+            // this thread wrote in phase A1, y = obs[t - 1]); the record's second sector takes the child's cumulative
+            // alpha, the payload's second sector the parent's (alpha_k of the pair (x_k, x_k+1) the payload holds).
+            const double yi = a.obs[t], ylagH = SVH ? obs_wrap(a.obs, t - L, NOBS) : 0.0;
+            const double ypair = GENH ? a.obs[pair_obs(M::kPairing, t - 1)] : 0.0;
             REntry* Pc = (REntry*)(a.P + (size_t)(t % RP) * N * RS);
 #pragma unroll
             for (int k0 = 0; k0 < KPT; k0 += RB) {
                 int r[RB][8];
                 double2 pa0[HESS ? RB : 1], pa1[HESS ? RB : 1];
-                double cur[HESS ? RB : 1];
+                double cur[SVH ? RB : 1];
 #pragma unroll
                 for (int u = 0; u < RB; ++u) {
                     const int i = (k0 + u) * GT + tid;
 #pragma unroll
                     for (int z = 0; z < 8; ++z) r[u][z] = 0;
-                    if constexpr (HESS) {
-                        pa0[u] = pa1[u] = make_double2(0.0, 0.0);
-                        cur[u] = 0.0;
-                    }
+                    if constexpr (HESS) pa0[u] = pa1[u] = make_double2(0.0, 0.0);
+                    if constexpr (SVH) cur[u] = 0.0;
                     if (i < nc) {
                         const REntry* src = &Rp[(size_t)((a.dbg & 8) ? jb + i : bp[k0 + u]) * RS];
                         ld_rec(src, pol_rld, r[u]);
-                        if constexpr (HESS) {
-                            ld_f64x4(src + 1, pol_rld, pa0[u].x, pa0[u].y, pa1[u].x, pa1[u].y);
+                        if constexpr (HESS) ld_f64x4(src + 1, pol_rld, pa0[u].x, pa0[u].y, pa1[u].x, pa1[u].y);
+                        if constexpr (SVH) {
                             const unsigned qq = (unsigned)(t - 1) + (unsigned)__ldcg(&a.H[jb + i]);
                             const unsigned sl = qq / (unsigned)NOBS, tq = qq - sl * (unsigned)NOBS;
                             if ((int)tq < t) cur[u] = ((int)sl < a.SQ) ? __ldcg(&a.xlow[(size_t)sl * NOBS + tq]) : 0.0;
@@ -995,13 +1016,19 @@ __global__ void __launch_bounds__(GT, 1) sv_grid_kernel(const GridArgs a_in, con
                         if (L == 3) anc = b;
                         else if (L > 3) anc = pick8(r[u], L - 4);
                         bp[k0 + u] = anc;
-                        if constexpr (HESS) {
+                        if constexpr (SVH) {
                             double al[4];
                             sv_alpha_terms(s_k, xn[k0 + u], cur[u], yi, ylagH, al);
                             const double c0 = al[0] + pa0[u].x, c1 = al[1] + pa0[u].y;
                             const double c2 = al[2] + pa1[u].x, c3 = al[3] + pa1[u].y;
                             st_keep_f64x4(&Rc[(size_t)j * RS + 1], pol_rst, c0, c1, c2, c3);
                             st_stream_f64x4(&Pc[(size_t)j * RS + 1], pol_stream, c0, c1, c2, c3);
+                        } else if constexpr (GENH) {
+                            double g[4];
+                            M::score_main(s_k, __ldcg(&((const PEntry*)Pc)[(size_t)j * RS].c), xn[k0 + u], ypair, g);
+                            st_keep_f64x4(&Rc[(size_t)j * RS + 1], pol_rst, pa0[u].x + g[0], pa0[u].y + g[1],
+                                          pa1[u].x + g[2], pa1[u].y + g[3]);
+                            st_stream_f64x4(&Pc[(size_t)j * RS + 1], pol_stream, pa0[u].x, pa0[u].y, pa1[u].x, pa1[u].y);
                         }
                     }
                 }
@@ -1022,7 +1049,7 @@ __global__ void __launch_bounds__(GT, 1) sv_grid_kernel(const GridArgs a_in, con
         // the unsorted new value `sl` (complete since barrier 1) if sl <= j, else 0.  The records pass listed these
         // children; one thread per entry redoes the term after the arrive of barrier 2 (outputs only: read by the
         // children of the next step and by the score terms LAG-2 steps later; LAG = 2: before the arrive)
-        if constexpr (HESS) {
+        if constexpr (SVH) {
             if (L == 2) {
                 __syncthreads();
                 deferred_alpha_pass(a, s_k, s_deflist, min(s_ndef, kCap), t, jb, tid, GT, pol_rld, pol_rst, pol_stream);
@@ -1155,7 +1182,7 @@ __global__ void __launch_bounds__(GT, 1) sv_grid_kernel(const GridArgs a_in, con
         }
         PROF_MARK(6);   // A2 scan+scatter
         GRID_ARRIVE();   // ---- barrier 2: mailboxes complete
-        if constexpr (HESS) {
+        if constexpr (SVH) {
             if (L != 2) deferred_alpha_pass(a, s_k, s_deflist, min(s_ndef, kCap), t, jb, tid, GT, pol_rld, pol_rst, pol_stream);
             PROF_MARK(14);   // deferred alpha terms (Hessian branch)
         }
@@ -1329,7 +1356,7 @@ __global__ void __launch_bounds__(GT, 1) sv_grid_kernel(const GridArgs a_in, con
                                      make_int4((int)(xb & 0xffffffffll), (int)(xb >> 32), (int)(eb & 0xffffffffll), (int)(eb >> 32)));
                     }
                     st_hint_b32(&a.perm[pstart + q], pol_keep, j);
-                    if constexpr (HESS) {
+                    if constexpr (SVH) {
                         if (pstart + q < a.SQ) a.xlow[(size_t)(pstart + q) * NOBS + t] = x;
                     }
                     s_sh[q] = sh;
@@ -1421,8 +1448,8 @@ __global__ void __launch_bounds__(GT, 1) sv_grid_kernel(const GridArgs a_in, con
             // pass (hacc[10..19]; the payloads come from L2 there).  Weights are the unnormalised ones (divided by S
             // afterwards).  The isfinite guards of :521-534 are kept for hessian2; a non-finite particle value
             // abandons the evaluation (phase A1), so hessian1 needs none.
-            double hm[HESS ? 4 : 1];
-            if constexpr (HESS) {
+            double hm[SVH ? 4 : 1];
+            if constexpr (SVH) {
 #pragma unroll
                 for (int i = 0; i < 4; ++i) hm[i] = 0.0;
             }
@@ -1443,7 +1470,7 @@ __global__ void __launch_bounds__(GT, 1) sv_grid_kernel(const GridArgs a_in, con
                             double d1, d2;
                             asm volatile("ld.global.cg.L2::cache_hint.v4.f64 {%0,%1,%2,%3}, [%4], %5;"
                                          : "=d"(pc[u]), "=d"(d1), "=d"(d2), "=d"(px[u])
-                                         : "l"(pp), "l"(pol_pld));
+                                         : "l"(pp), "l"(HESS ? pol_keep : pol_pld));
                         }
                     }
 #pragma unroll
@@ -1502,19 +1529,19 @@ __global__ void __launch_bounds__(GT, 1) sv_grid_kernel(const GridArgs a_in, con
 #pragma unroll
             for (int i = 0; i < 5; ++i) sc[i] = warp_sum(sc[i]);
             __syncthreads();
-            if constexpr (HESS) {
+            if constexpr (SVH) {
 #pragma unroll
                 for (int i = 0; i < 4; ++i) hm[i] = warp_sum(hm[i]);
             }
             if (lane == 0) {
 #pragma unroll
                 for (int i = 0; i < 5; ++i) s_red[32 * i + warp] = sc[i];
-                if constexpr (HESS) {
+                if constexpr (SVH) {
 #pragma unroll
                     for (int i = 0; i < 4; ++i) s_redH[32 * i + warp] = hm[i];
                 }
             }
-            if constexpr (HESS) {
+            if constexpr (SVH) {
                 constexpr int SB = 1;   // 64-byte entries in flight per thread
                 double h2[10];
 #pragma unroll
@@ -1579,11 +1606,45 @@ __global__ void __launch_bounds__(GT, 1) sv_grid_kernel(const GridArgs a_in, con
 #pragma unroll
                     for (int i = 0; i < 10; ++i) s_redH[32 * (10 + i) + warp] = h2[i];
                 }
+            } else if constexpr (GENH) {
+                // generic Hessian branch: a second pass over the same payloads (from L2) with their second sector,
+                // alpha_k; the ten entries of hessian1 and of hessian2 under the unnormalised weights (divided by S
+                // afterwards)
+                double h1[10], h2[10];
+#pragma unroll
+                for (int i = 0; i < 10; ++i) h1[i] = h2[i] = 0.0;
+                const double yl = a.obs[pair_obs(M::kPairing, t - L + 1)];
+#pragma unroll 1
+                for (int kk = 0; kk < KPT; ++kk) {
+                    const int q = kk * GT + tid;
+                    if (q < n) {
+                        const PEntry* pp = &Pg[(size_t)min(max(s_ab[q], 0), N - 1) * RS];
+                        double pc, d1, d2, px, al[4];
+                        ld_f64x4(pp, pol_pld, pc, d1, d2, px);
+                        ld_f64x4(pp + 1, pol_pld, al[0], al[1], al[2], al[3]);
+                        double g[4], hh[10];
+                        M::score_main(s_k, pc, px, yl, g);
+                        M::hess_main(s_k, pc, px, yl, hh);
+                        louis_add(hh, g, al, s_sh[q], h1, h2);
+                    }
+                }
+#pragma unroll
+                for (int i = 0; i < 10; ++i) {
+                    h1[i] = warp_sum(h1[i]);
+                    h2[i] = warp_sum(h2[i]);
+                }
+                if (lane == 0) {
+#pragma unroll
+                    for (int i = 0; i < 10; ++i) {
+                        s_redH[32 * i + warp] = h1[i];
+                        s_redH[32 * (10 + i) + warp] = h2[i];
+                    }
+                }
             }
             __syncthreads();
             if constexpr (HESS) {
                 for (int k = warp; k < 20; k += NW) {   // a warp sums component k over the warps (fixed order)
-                    const double v = (k < 4 || k >= 10) ? warp_sum((lane < NW) ? s_redH[32 * k + lane] : 0.0) : 0.0;
+                    const double v = (GEN || k < 4 || k >= 10) ? warp_sum((lane < NW) ? s_redH[32 * k + lane] : 0.0) : 0.0;
                     if (lane == 0) a.psumH[((size_t)t * G + c) * 20 + k] = v;
                 }
             }
@@ -1640,7 +1701,9 @@ __global__ void __launch_bounds__(256) grid_reduce_kernel(const double* __restri
 // irel = 0 is 0 (the main loop has that slot), the pair is weighted by W_T and takes y = obs[i + 1]; predictive pairing
 // (Pairing::Predictive): y = obs[i], and irel = L - 1 (idx = 0, i = T) adds M::score_last of the final particle.
 // HESS: partH[irel][block][0..19] = the hessian1 / hessian2 terms of :564-626 (alpha of the ancestor LAG-2 steps
-// back of the final particle, weights W_i, obs[i - LAG] with wrap-around, Q8).  M: the model (g = M::score_tail).
+// back of the final particle, weights W_i, obs[i - LAG] with wrap-around, Q8); for a generic model the upper triangles
+// of hessian1 / hessian2 of the same pairs as the gradient (M::hess_main, and M::hess_last with the final particle's own
+// alpha for irel = L - 1).  M: the model (g = M::score_tail).
 template <bool HESS, class M>
 __global__ void __launch_bounds__(256) grid_tail_kernel(GridArgs a, const double* __restrict__ sums,
                                                         double* __restrict__ part, double* __restrict__ partH,
@@ -1679,6 +1742,11 @@ __global__ void __launch_bounds__(256) grid_tail_kernel(GridArgs a, const double
                 M::score_last(k, curr, y1, g);
 #pragma unroll
                 for (int q = 0; q < 4; ++q) acc[1 + q] += g[q] * wT;
+                if constexpr (HESS) {
+                    double hh[10];
+                    M::hess_last(k, curr, y1, hh);
+                    louis_add(hh, g, (const double*)&Rt[(size_t)b * RS + 1], wT, hacc, hacc + 10);
+                }
             }
         } else {
             // entry of the ancestor idx-1 steps back holds (next = its value, curr = its parent's value)
@@ -1698,7 +1766,11 @@ __global__ void __launch_bounds__(256) grid_tail_kernel(GridArgs a, const double
             }
 #pragma unroll
             for (int q = 0; q < 4; ++q) acc[1 + q] += g[q] * wi;
-            if constexpr (HESS) {
+            if constexpr (HESS && !REF) {
+                double hh[10];
+                M::hess_main(k, curr, pe_n, y1, hh);
+                louis_add(hh, g, (const double*)&a.P[((size_t)((T - m) % RP) * N + row) * RS + 1], wT, hacc, hacc + 10);
+            } else if constexpr (HESS) {
                 const int m2 = L - 2;
                 const int row2 = (m2 == 0) ? b : min(max(Rt[(size_t)b * RS].a[m2 - 1], 0), N - 1);
                 const double* a4 = (const double*)&a.P[((size_t)((T - m2) % RP) * N + row2) * RS + 1];
@@ -1716,12 +1788,13 @@ __global__ void __launch_bounds__(256) grid_tail_kernel(GridArgs a, const double
     }
 }
 
-// Hessian branch: sumsH[t][k] = sum over the tiles of psumH[t][.][k] (t >= lag; 0 before)
-__global__ void __launch_bounds__(640) grid_reduceH_kernel(const double* __restrict__ psumH, int G, int lag,
+// Hessian branch: sumsH[t][k] = sum over the tiles of psumH[t][.][k] (t >= first, the first step with fixed-lag terms;
+// 0 before)
+__global__ void __launch_bounds__(640) grid_reduceH_kernel(const double* __restrict__ psumH, int G, int first,
                                                            double* __restrict__ sumsH) {
     const int t = blockIdx.x, k = threadIdx.x >> 5, lane = threadIdx.x & 31;   // 20 warps = 20 components
     double s = 0.0;
-    if (t >= lag)
+    if (t >= first)
         for (int c = lane; c < G; c += 32) s = s + psumH[((size_t)t * G + c) * 20 + k];
     s = warp_sum(s);
     if (lane == 0) sumsH[(size_t)t * 20 + k] = s;
@@ -1779,6 +1852,35 @@ __global__ void __launch_bounds__(32) grid_hess_finish_kernel(const GridCtrl* __
             h += v / S;
         }
         for (int irel = 0; irel < lag - 1; ++irel)
+            for (int q = 0; q < nblk; ++q) h += partH[((size_t)irel * nblk + q) * 20 + k];
+        tri[k] = h;
+    }
+    __syncwarp();
+    if (k < 16) {
+        const int r = k >> 2, cidx = k & 3;
+        const int lo = min(r, cidx), hi = max(r, cidx);
+        const int ti = lo * 4 - (lo * (lo - 1)) / 2 + (hi - lo);
+        hess1[k] = tri[ti];
+        hess2[k] = tri[10 + ti];
+    }
+}
+
+// generic Hessian branch: hessian1 / hessian2 = the main-loop sums of steps first .. nobs-1 divided by the weight sum
+// of their step, plus the tail blocks irel = 1 .. lag-1, in that order; upper triangles expanded into the symmetric
+// 4 x 4 outputs
+__global__ void __launch_bounds__(32) grid_hess_finish_gen_kernel(const GridCtrl* __restrict__ ctrl,
+                                                                  const double* __restrict__ sums,
+                                                                  const double* __restrict__ sumsH,
+                                                                  const double* __restrict__ partH, int nblk, int nobs,
+                                                                  int first, int lag, double* __restrict__ hess1,
+                                                                  double* __restrict__ hess2) {
+    __shared__ double tri[20];
+    const int k = threadIdx.x;
+    if (ctrl->status != 0) return;   // abandoned: diag reports it
+    if (k < 20) {
+        double h = 0.0;
+        for (int t = first; t < nobs; ++t) h += sumsH[(size_t)t * 20 + k] / sums[(size_t)t * 8];
+        for (int irel = 1; irel < lag; ++irel)
             for (int q = 0; q < nblk; ++q) h += partH[((size_t)irel * nblk + q) * 20 + k];
         tri[k] = h;
     }
@@ -1979,8 +2081,8 @@ template <bool HESS, class M, bool SMO>
 const void* grid_kernel_of(bool team) {
     return team ? (const void*)sv_grid_kernel<1024, HESS, M, SMO, true> : (const void*)sv_grid_kernel<1024, HESS, M, SMO, false>;
 }
-// the persistent kernel of (model, hess, filter): one problem, or teams of CTAs; the filter runs the model's Filter;
-// nullptr for an unknown model id or a Hessian the model does not have
+// the persistent kernel of (model, hess, filter): one problem, or teams of CTAs; the filter runs the model's Filter,
+// the smoother without the Hessian its Gradient; nullptr for an unknown model id or a Hessian the model does not have
 const void* grid_kernel_for(int model, int hess, int filter, bool team) {
     const void* k = nullptr;
     Models::with(model, [&](auto m) {
@@ -1988,7 +2090,7 @@ const void* grid_kernel_for(int model, int hess, int filter, bool team) {
         if (filter) {
             k = grid_kernel_of<false, typename M::Filter, false>(team);
         } else if (!hess) {
-            k = grid_kernel_of<false, M, true>(team);
+            k = grid_kernel_of<false, typename M::Gradient, true>(team);
         } else if constexpr (M::kHessian) {
             k = grid_kernel_of<true, M, true>(team);
         }
@@ -2001,7 +2103,7 @@ int grid_check(const SvCall& c, int nobs, int n, int lag, int G, int hess) {
         return set_error(PMMH_ERR_INVALID, "grid kernel: sizes not eligible");
     if (!model_known(c.model)) return set_error(PMMH_ERR_INVALID, "grid kernel: unknown model id");
     if (hess && !model_has_hessian(c.model))
-        return set_error(PMMH_ERR_INVALID, "grid kernel: the Hessian branch exists for the SV model only");
+        return set_error(PMMH_ERR_INVALID, "grid kernel: compute_hessian for a model without a Hessian branch");
     return PMMH_OK;
 }
 
@@ -2095,14 +2197,20 @@ int grid_after(const SvCall& c, const GridArgs& a, const GridLayout& L, char* ws
         const auto finish = c.filter ? grid_finish_for<typename M::Filter, false>() : grid_finish_for<M, true>();
         if (!c.filter) {
             if (!hess) {
-                grid_tail_kernel<false, M><<<dim3(L.nblk, lag), 256, 0, st>>>(a, sums, tailpart, nullptr, L.nblk);
+                grid_tail_kernel<false, typename M::Gradient><<<dim3(L.nblk, lag), 256, 0, st>>>(a, sums, tailpart,
+                                                                                                nullptr, L.nblk);
             } else if constexpr (M::kHessian) {
                 double* sumsH = (double*)(ws + L.sumsH);
                 double* tailpartH = (double*)(ws + L.tailpartH);
-                grid_reduceH_kernel<<<nobs, 640, 0, st>>>(a.psumH, G, lag, sumsH);
+                grid_reduceH_kernel<<<nobs, 640, 0, st>>>(a.psumH, G, pair_first_step(M::kPairing, lag), sumsH);
                 grid_tail_kernel<true, M><<<dim3(L.nblk, lag), 256, 0, st>>>(a, sums, tailpart, tailpartH, L.nblk);
-                grid_hess_finish_kernel<<<1, 32, 0, st>>>(a.ctrl, sums, sumsH, tailpartH, c.params, L.nblk, nobs, lag,
-                                                          c.hess1, c.hess2);
+                if constexpr (M::kPairing == Pairing::Reference)
+                    grid_hess_finish_kernel<<<1, 32, 0, st>>>(a.ctrl, sums, sumsH, tailpartH, c.params, L.nblk, nobs,
+                                                              lag, c.hess1, c.hess2);
+                else
+                    grid_hess_finish_gen_kernel<<<1, 32, 0, st>>>(a.ctrl, sums, sumsH, tailpartH, L.nblk, nobs,
+                                                                  pair_first_step(M::kPairing, lag), lag, c.hess1,
+                                                                  c.hess2);
             }
             grid_tail_reduce_kernel<<<lag, 256, 0, st>>>(tailpart, L.nblk, tail);
         }

@@ -164,10 +164,11 @@ def flps_model_corr(model_id, obs, params, rvr, u, lag=10, store_history=False, 
     kernel, diag kernel 3).  Above: B == 1, n_obs >= 2 lag and up to 7168 particles per SM (1,060,864 on
     148 SMs), one persistent launch over the GPU (grid kernel, diag kernel 5).  Other sizes raise PmmhError.
     ``model_id``: _lib.MODEL_SV_LEVERAGE (bit-identical to flps_sv_corr on the same kernel),
-    _lib.MODEL_LINEAR_GAUSSIAN, _lib.MODEL_LINEAR_GAUSSIAN_FA or _lib.MODEL_LINEAR_GAUSSIAN_FA_GRAD; params [B, 4]
-    (unused slots ignored).  The fully adapted models 2 and 4 take the series shifted by one (obs[1:]) and their
-    log_like lacks log p(y_1); model 4 adds model 2 a gradient whose slot k holds the contribution of obs[1:][k], so
-    that the slots sum to the score of the full log-likelihood (include/pmmh_qn.h).
+    _lib.MODEL_LINEAR_GAUSSIAN, _lib.MODEL_LINEAR_GAUSSIAN_FA, _lib.MODEL_LINEAR_GAUSSIAN_FA_GRAD or
+    _lib.MODEL_LINEAR_GAUSSIAN_FA_HESS; params [B, 4] (unused slots ignored).  The fully adapted models 2, 4 and 6 take
+    the series shifted by one (obs[1:]) and their log_like lacks log p(y_1); model 4 adds model 2 a gradient whose slot
+    k holds the contribution of obs[1:][k], so that the slots sum to the score of the full log-likelihood
+    (include/pmmh_qn.h).  Model 6 is model 4 here, bit for bit (its Hessian: flps_model_batch_corr).
     No fallback pass: diag[:, PMMH_DIAG_STATUS] == 1 reports an abandoned evaluation."""
     return _model_corr("flps_model", model_id, obs, params, rvr, u, lag, 0, store_history, workspace)
 
@@ -177,7 +178,7 @@ def filter_model_corr(model_id, obs, params, rvr, u, store_history=False, worksp
     diag of [B] problems without the fixed-lag smoother -- bit-identical to those outputs of flps_model_corr
     for any lag.  Up to 4096 particles: any B (chain kernel, diag kernel 3).  Above: B == 1 and up to 7168
     particles per SM (grid kernel, diag kernel 5).  n_obs >= 2; other sizes raise PmmhError.  ``model_id`` and
-    params as for flps_model_corr (model 4 runs model 2's filter).  No fallback pass: diag[:, PMMH_DIAG_STATUS] == 1 reports an abandoned
+    params as for flps_model_corr (models 4 and 6 run model 2's filter).  No fallback pass: diag[:, PMMH_DIAG_STATUS] == 1 reports an abandoned
     evaluation."""
     return _model_corr("filter_model", model_id, obs, params, rvr, u, 2, 0, store_history, workspace)
 
@@ -197,8 +198,11 @@ def flps_model_batch_corr(model_id, obs, params, rvr, u, lag=10, compute_hessian
     outputs of problem b are bit-identical to flps_model_corr on that problem alone with B == 1 (and, for
     _lib.MODEL_SV_LEVERAGE, to flps_sv_corr on the grid kernel, also with the Hessian).  Any B on every shape the
     one-problem grid run takes (above 4096 particles: n_obs >= 2 lag, up to 7168 particles per CTA of
-    ceil(N / 2048)); model ids as for flps_model_corr; compute_hessian for the SV model only.  Returns the dict of flps_model_corr, plus hess1 /
-    hess2 [B, 4, 4] with compute_hessian.  No fallback pass: diag[:, PMMH_DIAG_STATUS] == 1 reports an abandoned
+    ceil(N / 2048)); model ids as for flps_model_corr; compute_hessian for _lib.MODEL_SV_LEVERAGE (the reference's
+    Hessian branch) and _lib.MODEL_LINEAR_GAUSSIAN_FA_HESS (Louis' identity on model 4's pairs and weights:
+    hess1 + hess2 - g g', g = the summed gradient slots, estimates the Hessian of the full log-likelihood over
+    (phi, sigma_v, sigma_e); row and column 3 are 0).  Every other output of model 6 is model 4's, bit for bit, with
+    compute_hessian 0 or 1.  Returns the dict of flps_model_corr, plus hess1 / hess2 [B, 4, 4] with compute_hessian.  No fallback pass: diag[:, PMMH_DIAG_STATUS] == 1 reports an abandoned
     problem, the others are unaffected."""
     return _model_corr("flps_model_batch", model_id, obs, params, rvr, u, lag, int(bool(compute_hessian)),
                        store_history, workspace)

@@ -10,14 +10,22 @@ the likelihood estimate with the lowest variance of the filters here.  The kerne
 log-likelihood.  ``fully_adapted=False`` runs the bootstrap filter (model id 1) on the whole series.
 
 ``dim_rvs`` = (length of the series the kernel sees, N + 1): T - 1 rows when fully adapted, T otherwise.  ``rvs``
-is that host array or a ``DeviceRVS`` of that shape, as for ``ParticleMethodsCUDA``.  Hessians are not available
-for this model: a call with ``model.using_hessians`` returns False.
+is that host array or a ``DeviceRVS`` of that shape, as for ``ParticleMethodsCUDA``.
+
+``hessian=True`` (fully adapted only) lets the estimator serve second-order samplers: ``smoother`` with
+``model.using_hessians`` runs model id 6 (pmmh_flps_model_batch_corr with compute_hessian, batch 1, on the grid
+kernel) and publishes ``log_joint_hessian_estimate`` = hess1 + hess2 - g g' over (phi, sigma_v, sigma_e), g the summed
+gradient slots (Louis' identity along the particles' genealogy; its variance grows with T / N).  Every other output is
+model 4's.  Below 4097 particles a Hessian call runs on the grid kernel and a gradient-only call on the chain kernel,
+so their log-likelihoods differ in the last bits.  With ``hessian=False`` (default) a call with ``model.using_hessians``
+returns False.
 """
 import numpy as np
 import torch
 
 from ... import kernels as K
-from ..._lib import (DIAG_NEAR_TIES, DIAG_STATUS, MODEL_LINEAR_GAUSSIAN, MODEL_LINEAR_GAUSSIAN_FA_GRAD)
+from ..._lib import (DIAG_NEAR_TIES, DIAG_STATUS, MODEL_LINEAR_GAUSSIAN, MODEL_LINEAR_GAUSSIAN_FA_GRAD,
+                     MODEL_LINEAR_GAUSSIAN_FA_HESS)
 from ..base_state_inference import BaseStateInference
 from .cuda import ParticleMethodsCUDA
 
@@ -36,13 +44,16 @@ class LinearGaussianParticleMethodsCUDA(BaseStateInference):
     _rvs_device = ParticleMethodsCUDA._rvs_device
     _to_host = staticmethod(ParticleMethodsCUDA._to_host)
 
-    def __init__(self, model, no_particles, fixed_lag=10, fully_adapted=True, device=None):
+    def __init__(self, model, no_particles, fixed_lag=10, fully_adapted=True, device=None, hessian=False):
         if model.short_name != 'lgss':
             raise NameError("LinearGaussianParticleMethodsCUDA needs a linear Gaussian model ('lgss').")
+        if hessian and not fully_adapted:
+            raise ValueError("LinearGaussianParticleMethodsCUDA: the Hessian needs the fully adapted filter.")
         if not torch.cuda.is_available():
             raise RuntimeError("LinearGaussianParticleMethodsCUDA needs a CUDA device; there is no CPU fallback.")
         self.device = torch.device(device) if device is not None else torch.device('cuda', torch.cuda.current_device())
         self.fully_adapted = bool(fully_adapted)
+        self.hessian = bool(hessian)
         self.model_id = MODEL_LINEAR_GAUSSIAN_FA_GRAD if self.fully_adapted else MODEL_LINEAR_GAUSSIAN
         self._workspace = K.Workspace()
         self._obs_cache = None
@@ -100,25 +111,39 @@ class LinearGaussianParticleMethodsCUDA(BaseStateInference):
 
     def smoother(self, model, **kwargs):
         """Fixed-lag smoother (pmmh_flps_model_corr): log_like, filtered / smoothed states, trajectory and the
-        gradient estimate (the sum of gradient rows 0..2 over the slots, non-finite entries taken as 0)."""
-        if model.using_hessians:
-            print("LinearGaussianParticleMethodsCUDA: no Hessian estimate for the linear Gaussian model.")
+        gradient estimate (the sum of gradient rows 0..2 over the slots, non-finite entries taken as 0).  With
+        ``model.using_hessians`` (``hessian=True`` only) pmmh_flps_model_batch_corr with the Hessian branch, and the
+        Hessian estimate hess1 + hess2 - g g'."""
+        if model.using_hessians and not self.hessian:
+            print("LinearGaussianParticleMethodsCUDA: no Hessian estimate (construct it with hessian=True).")
             return False
         try:
             obs_d, par_d, rvr, u, extra = self._inputs(model, kwargs)
-            out = K.flps_model_corr(self.model_id, obs_d, par_d, rvr, u, lag=self.settings['fixed_lag'],
-                                    workspace=self._workspace)
-            xf, xs, ll, grad, xtraj, diag = self._to_host(
-                [out['filt'][0], out['smo'][0], out['log_like'], out['gradient'][0], out['traj'][0], out['diag'][0]])
+            hess = bool(model.using_hessians)
+            self.settings['estimate_hessian'] = hess
+            if hess:
+                out = K.flps_model_batch_corr(MODEL_LINEAR_GAUSSIAN_FA_HESS, obs_d, par_d, rvr, u,
+                                              lag=self.settings['fixed_lag'], compute_hessian=1,
+                                              workspace=self._workspace)
+            else:
+                out = K.flps_model_corr(self.model_id, obs_d, par_d, rvr, u, lag=self.settings['fixed_lag'],
+                                        workspace=self._workspace)
+            tensors = [out['filt'][0], out['smo'][0], out['log_like'], out['gradient'][0], out['traj'][0], out['diag'][0]]
+            if hess:
+                tensors += [out['hess1'][0], out['hess2'][0]]
+            xf, xs, ll, grad, xtraj, diag, *h12 = self._to_host(tensors)
             self._check_status(diag)
             self.results.update({'filt_state_est': np.array(xf).flatten()})
             self.results.update({'state_trajectory': np.array(xtraj).flatten()})
             self.results.update({'smo_state_est': np.array(xs).flatten()})
             self.results.update({'log_like': float(ll[0]) + extra})
-            if model.using_gradients:
+            if model.using_gradients or hess:
                 g = np.array(grad[:3], dtype=np.float64)
                 g[~np.isfinite(g)] = 0.0
                 self.results.update({'log_joint_gradient_estimate': g.sum(axis=1)})
+            if hess:
+                g = self.results['log_joint_gradient_estimate']
+                self.results.update({'log_joint_hessian_estimate': (h12[0] + h12[1])[:3, :3] - np.outer(g, g)})
             return self._estimate_gradient_and_hessian(model)
         except Exception as e:
             print("Error in CUDA code for particle smoother.")
