@@ -224,6 +224,19 @@ int pmmh_flps_sv_corr_philox(const double* d_obs, const double* d_params, const 
  * estimates the Hessian of the full log-likelihood log p(y_1 .. y_T).  alpha runs along the whole genealogy, so the
  * estimate's variance grows with n_obs / n_particles. */
 #define PMMH_MODEL_LINEAR_GAUSSIAN_FA_HESS 6   /* id 5 is unassigned */
+/* PMMH_MODEL_SV_LEVERAGE_EXACT: the SV model with the exact fixed-lag score and a fixed-lag Hessian.  Same inputs as
+ * PMMH_MODEL_SV_LEVERAGE (the unshifted series, params mu, phi, sigma_v, rho); d_filt, d_log_like, d_traj, d_diag and the
+ * history are bit-identical to model 0's on the same kernel, and the filter entries run model 0's filter for it.  The
+ * gradient is over the reference's free parameters (mu, atanh phi, log sigma_v, atanh rho), and slot k holds the
+ * expectation of d/dtheta log p(x_{k+1} | x_k, obs[k]) -- the transition scored with the leverage observation its
+ * propagation read -- under the weights of generation c(k) = min(k + lag - 1, n_obs - 1); slot n_obs - 1 is 0.  The
+ * pair (x_0, x_1) takes the total derivative through x_0 = mu.  The slots sum to an estimate of the score of log_like
+ * (model 0 pairs the terms as the reference does, obs[k - 1] and tail pairs re-added: a biased estimate when rho != 0).
+ * d_smo[k] is the mean of x_k under the same weights.  pmmh_flps_model_batch_corr with compute_hessian == 1 (grid kernel)
+ * writes d_hess1 / d_hess2 [4][4] over the same parameters by Louis' identity as for
+ * PMMH_MODEL_LINEAR_GAUSSIAN_FA_HESS; hess1 + hess2 - g g' estimates the Hessian of log_like.  Sizes as for model 0 on
+ * the model entries. */
+#define PMMH_MODEL_SV_LEVERAGE_EXACT 8   /* id 7 is unassigned: every entry refuses it as an unknown id */
 int pmmh_flps_model_workspace_bytes(int n_obs, int n_particles, int lag, int batch, size_t* bytes);
 int pmmh_flps_model_corr(int model_id, const double* d_obs, long long obs_stride, const double* d_params,
                          const double* d_rvr, const double* d_u, int n_obs, int n_particles, int lag, int batch,
@@ -266,8 +279,8 @@ int pmmh_filter_model_corr(int model_id, const double* d_obs, long long obs_stri
  * d_diag [PMMH_DIAG_COUNT]; optional d_x_hist / d_a_hist [batch][n_obs][n_particles], given together.
  *   Shapes: any batch >= 1 with a tile of n_particles / G particles that fits one CTA (up to 7168 particles per
  * CTA); the smoother needs 2 <= lag <= 10 and n_obs >= 2 lag, the filter n_obs >= 2.  compute_hessian == 1 (the
- * Hessian branch; d_hess1 / d_hess2 required) is taken for PMMH_MODEL_SV_LEVERAGE and
- * PMMH_MODEL_LINEAR_GAUSSIAN_FA_HESS only; with 0 the
+ * Hessian branch; d_hess1 / d_hess2 required) is taken for PMMH_MODEL_SV_LEVERAGE,
+ * PMMH_MODEL_LINEAR_GAUSSIAN_FA_HESS and PMMH_MODEL_SV_LEVERAGE_EXACT only; with 0 the
  * Hessian outputs may be NULL and are not written.  Anything else is refused with PMMH_ERR_INVALID, by the
  * workspace queries too; a workspace below the query's size gives PMMH_ERR_WORKSPACE.
  *   Workspace: min(batch, nteams) slices of the one-problem grid workspace with history (per slice:

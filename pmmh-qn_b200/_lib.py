@@ -22,6 +22,7 @@ DIAG_SOFT_TIES = 4   # flps on the grid kernel (same slot as the bpf wave-front 
 DIAG_COUNT = 8
 MODEL_SV_LEVERAGE, MODEL_LINEAR_GAUSSIAN, MODEL_LINEAR_GAUSSIAN_FA, MODEL_LINEAR_GAUSSIAN_FA_GRAD = 0, 1, 2, 4
 MODEL_LINEAR_GAUSSIAN_FA_HESS = 6
+MODEL_SV_LEVERAGE_EXACT = 8
 BPF_PARITY, BPF_INTENDED = 0, 1
 
 # name -> (restype, argtypes); mirrors include/pmmh_qn.h one to one

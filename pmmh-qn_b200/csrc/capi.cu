@@ -681,7 +681,7 @@ const char* model_entry_shapes(bool batched, int filter) {
                         "ceil(n_particles / 2048) particles fits one CTA and a known model id"
                       : "pmmh_flps_model_batch_corr: batch >= 1, 2 <= lag <= 10, n_obs >= 2 lag, a tile of n_particles / "
                         "ceil(n_particles / 2048) particles fits one CTA, a known model id, compute_hessian only for the "
-                        "SV model (0) and the fully adapted linear Gaussian model with a Hessian (6)";
+                        "SV models (0, 8) and the fully adapted linear Gaussian model with a Hessian (6)";
     return filter ? "pmmh_filter_model_corr: a known model id, n_obs >= 2 and 2 <= n_particles <= 4096 (any batch), "
                     "or batch == 1 and n_particles up to 7168 per SM (1,060,864 on 148 SMs)"
                   : "pmmh_flps_model_corr: a known model id, 2 <= lag <= 10 and 2 <= n_particles <= 4096 (any batch), "

@@ -13,7 +13,7 @@
 //   M::Gradient                          the model whose smoother instantiation a call without the Hessian runs
 //                                        (itself, or the model it adds a Hessian to)
 //   M::kHessian                          constexpr: the kernels have its Hessian branch (the SV model: the
-//                                        reference's, Pairing::Reference; model 6: the generic one, grid kernel)
+//                                        reference's, Pairing::Reference; models 6 and 8: the generic one, grid kernel)
 //   struct M::Const                      constants derived from the parameter vector (<= 4 doubles)
 //   M::init(Const&, const double* par)
 //   M::initial_state(c)                  value of every particle of generation 0 (the reference's
@@ -40,6 +40,9 @@
 //   M::hess_main(c, curr, next, y, h)    (generic Hessian branch only) the second derivatives of score_main's term:
 //   M::hess_last(c, x, y_next, h)        10 entries, the upper triangle of the 4 x 4 matrix row by row ((0,0), (0,1),
 //                                        (0,2), (0,3), (1,1), .. (3,3)); and of score_last's term
+//   M::score_first(c, x1, y0, g)         (optional, Pairing::Predictive) the term of the pair (x_0, x_1) in place of
+//   M::hess_first(c, x1, y0, h)          score_main / hess_main: for a model whose initial state depends on the
+//                                        parameters, the total derivative through x_0 = initial_state (pair_score)
 // A new model is such a struct plus its entry in Models at the end of this file, and its id in include/pmmh_qn.h.
 //
 // Pairing::Reference (the SV model, parity with the reference): the reference's quirks Q5 / Q6.  The main loop
@@ -52,11 +55,12 @@
 // initial_state for every particle, Q1), W_{NOBS-1} in the tail (t = NOBS-LAG+1 .. NOBS-2).  Gradient slot s holds
 // step s's contribution (the pair (x_s-1, x_s)); slot 0 is 0.  smo[t] = the weighted mean of x_t under the same
 // weights, every slot written once: the tail starts one step after the last main-loop slot.
-// Pairing::Predictive (exact pairing on the shifted series of a fully adapted filter, model 4): the same pairs, read
-// under the same weights, but the pair (x_t, x_t+1) takes y = obs[t] (= y_t+1 of the unshifted series) and goes into
-// slot t; the final generation adds score_last(x_NOBS-1, obs[NOBS-1]) under W_{NOBS-1} into slot NOBS-1 (the pair
-// (x_NOBS-1, x_NOBS) with x_NOBS integrated out).  Slot t then holds the contribution of obs[t], and the slots sum
-// to an estimate of the score of the whole series.
+// Pairing::Predictive: the same pairs, read under the same weights, but the pair (x_t, x_t+1) reads y = obs[t] and
+// fills slot t; the final generation adds score_last(x_NOBS-1, obs[NOBS-1]) under W_{NOBS-1} into slot NOBS-1.  obs[t]
+// is the observation the transition x_t -> x_t+1 is conditioned on: the leverage observation of a bootstrap filter
+// whose propagation reads obs[t] (model 8, score_last = 0: its observation density has no parameters), or, on the
+// shifted series of a fully adapted filter (model 4), y_t+1, with score_last the pair (x_NOBS-1, x_NOBS) with x_NOBS
+// integrated out.  Either way the slots sum to an estimate of the score of the whole series.
 // Unused gradient slots stay 0.  Model ids are part of the C ABI (include/pmmh_qn.h).
 //
 // The generic Hessian branch (Pairing::Predictive, grid kernel): Louis' identity on the gradient's pairs and weights.
@@ -137,6 +141,112 @@ struct SvLeverageModel {
         sv_score_tail(c, curr, next, y, sq, g);
     }
 };
+
+// ---- 8: the SV model with the exact fixed-lag score and a Hessian.  Its particle system is model 0's (inherited:
+// initial state, propagation, weights, shift, child range), so filt, log_like, traj, diag and the history are model 0's
+// bit for bit and the filter entries run model 0's filter (Filter).  The fixed-lag terms pair the states predictively
+// (Pairing::Predictive): the pair (x_t, x_t+1) is scored with its own leverage observation obs[t] -- the one the
+// propagation x_t -> x_t+1 read -- into slot t (model 0 gives it obs[t - 1], Q5, and re-adds tail pairs, Q6).  Free
+// parameters as the reference's: theta = (mu, atanh phi, log sigma_v, atanh rho).  One id for the gradient and the
+// Hessian: a call without the Hessian runs this instantiation (Gradient), the Hessian the generic branch of the grid
+// kernel.  The transition density is N(x'; m, sigma_v^2 (1 - rho^2)), m = mu + phi (x - mu) + sigma_v rho e^{-x/2} y;
+// with s = x' - m and q = 1 / (sigma_v^2 (1 - rho^2)), log p = 1/2 log q - q s^2 / 2 + const, so
+//   d log p = 1/2 dlog q (1 - q s^2) - q s ds,
+//   d2 log p = 1/2 d2log q (1 - q s^2) - 1/2 q s^2 dlog q dlog q' - q s (dlog q ds' + ds dlog q') - q ds ds' - q s d2s,
+// with dlog q = (0, 0, -2, 2 rho), d2log q nonzero only at (3,3): 2 (1 - rho^2).  The pair (x_0, x_1) has x_0 = mu
+// (Q1), so its s depends on mu through x_0 too (score_first / hess_first).  The observation density has no parameters.
+struct SvLeverageExact : SvLeverageModel {
+    static constexpr int kId = PMMH_MODEL_SV_LEVERAGE_EXACT;
+    typedef SvLeverageExact Gradient;
+    static constexpr Pairing kPairing = Pairing::Predictive;
+    // score_main: model 0's (sv_score_main, the derivative of log N(next; m, sigma_v^2 (1 - rho^2)) in theta)
+    static __device__ __forceinline__ void score_tail(const Const& c, double curr, double next, double y, double g[4]) {
+        score_main(c, curr, next, y, g);
+    }
+    static __device__ __forceinline__ void score_last(const Const&, double, double, double g[4]) {
+        g[0] = g[1] = g[2] = g[3] = 0.0;
+    }
+    // the pair (x_0 = mu, x_1): ds/dmu = -(1 - sigma_v rho e^{-mu/2} y0 / 2), ds/d atanh phi = 0
+    static __device__ __forceinline__ void score_first(const Const& c, double x1, double y0, double g[4]) {
+        double sq;
+        sv_score_main(c, c.mu, x1, y0, sq, g);
+        g[0] = c.q * sq * (1.0 - 0.5 * c.sr * exp(-0.5 * c.mu) * y0);
+        g[1] = 0.0;
+    }
+    static __device__ __forceinline__ void hess_main(const Const& c, double curr, double next, double y, double h[10]) {
+        const double d = curr - c.mu, ey = exp(-0.5 * curr) * y;
+        const double s = (next - c.mu - c.phi * d) - c.sr * ey;
+        // ds and the second derivatives of s: (mu, a) entries from m's mu + phi (x - mu), (b, c) from sigma_v rho ey
+        const double ds[4] = {-c.one_m_phi, -d * c.one_m_phi2, -c.sr * ey, -c.sigmav * ey * c.rho_term};
+        const double d2s[10] = {0.0, c.one_m_phi2, 0.0, 0.0, 2.0 * c.phi * c.one_m_phi2 * d, 0.0, 0.0, -c.sr * ey,
+                                -c.sigmav * ey * c.rho_term, 2.0 * c.sr * ey * c.rho_term};
+        sv_exact_hess(c, s, ds, d2s, h);
+    }
+    // the pair (x_0 = mu, x_1): s = x1 - mu - sigma_v rho e^{-mu/2} y0
+    static __device__ __forceinline__ void hess_first(const Const& c, double x1, double y0, double h[10]) {
+        const double ey = exp(-0.5 * c.mu) * y0;
+        const double s = (x1 - c.mu) - c.sr * ey;
+        const double ds[4] = {-(1.0 - 0.5 * c.sr * ey), 0.0, -c.sr * ey, -c.sigmav * ey * c.rho_term};
+        const double d2s[10] = {-0.25 * c.sr * ey, 0.0, 0.5 * c.sr * ey, 0.5 * c.sigmav * ey * c.rho_term, 0.0, 0.0, 0.0,
+                                -c.sr * ey, -c.sigmav * ey * c.rho_term, 2.0 * c.sr * ey * c.rho_term};
+        sv_exact_hess(c, s, ds, d2s, h);
+    }
+    static __device__ __forceinline__ void hess_last(const Const&, double, double, double h[10]) {
+#pragma unroll
+        for (int i = 0; i < 10; ++i) h[i] = 0.0;
+    }
+
+  private:
+    // the second derivatives of 1/2 log q - q s^2 / 2 (the formula above) from s, ds and d2s (upper triangle)
+    static __device__ __forceinline__ void sv_exact_hess(const Const& c, double s, const double ds[4],
+                                                         const double d2s[10], double h[10]) {
+        const double dlq[4] = {0.0, 0.0, -2.0, 2.0 * c.rho};
+        const double qs = c.q * s, hq = 0.5 * c.q * (s * s);
+        int z = 0;
+#pragma unroll
+        for (int i = 0; i < 4; ++i)
+#pragma unroll
+            for (int j = i; j < 4; ++j, ++z) {
+                double v = -hq * (dlq[i] * dlq[j]) - qs * (dlq[i] * ds[j] + ds[i] * dlq[j]) - c.q * (ds[i] * ds[j]) -
+                           qs * d2s[z];
+                if (i == 3 && j == 3) v += c.rho_term * (1.0 - 2.0 * hq);
+                h[z] = v;
+            }
+    }
+};
+
+// the score (pair_score) and second derivatives (pair_hess) of the pair (x_t, x_t+1), first = (t == 0): M::score_first /
+// M::hess_first for the first pair where the model has them, M::score_main / M::hess_main otherwise
+template <class M, class = void>
+struct HasFirstPair {
+    static constexpr bool value = false;
+};
+template <class M>
+struct HasFirstPair<M, decltype((void)&M::score_first)> {
+    static constexpr bool value = true;
+};
+template <class M>
+__device__ __forceinline__ void pair_score(const typename M::Const& c, bool first, double curr, double next, double y,
+                                           double g[4]) {
+    if constexpr (HasFirstPair<M>::value) {
+        if (first) {
+            M::score_first(c, next, y, g);
+            return;
+        }
+    }
+    M::score_main(c, curr, next, y, g);
+}
+template <class M>
+__device__ __forceinline__ void pair_hess(const typename M::Const& c, bool first, double curr, double next, double y,
+                                          double h[10]) {
+    if constexpr (HasFirstPair<M>::value) {
+        if (first) {
+            M::hess_first(c, next, y, h);
+            return;
+        }
+    }
+    M::hess_main(c, curr, next, y, h);
+}
 
 // ---- 1: linear Gaussian state space model  x_t = phi x_{t-1} + sigma_v v_t,  y_t = x_t + sigma_e e_t
 // (parameters phi, sigma_v, sigma_e; the fourth slot is unused).  Not a model of the reference: it is
@@ -361,7 +471,7 @@ struct ModelList {
     }
 };
 typedef ModelList<SvLeverageModel, LinearGaussianModel, LinearGaussianFullyAdapted, LinearGaussianFullyAdaptedGrad,
-                  LinearGaussianFullyAdaptedHess>
+                  LinearGaussianFullyAdaptedHess, SvLeverageExact>
     Models;
 static_assert(Models::ids_distinct(), "every model states its own id");
 

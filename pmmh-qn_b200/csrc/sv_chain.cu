@@ -527,7 +527,7 @@ __global__ void __launch_bounds__(kCT, 1) sv_chain_kernel(SvArgs a) {
                                 // whole series and are reduced once at the end)
                                 sv_hessian_terms_e(c, pv[q].y, ec, ec * ec, sq, yl, g, al, v[q] / S_i, hacc);
                             } else {
-                                M::score_main(c, pv[q].y, pv[q].x, yl, g);
+                                pair_score<M>(c, inext == LAG - 1, pv[q].y, pv[q].x, yl, g);
                             }
                             acc[1] += v[q] * pv[q].y;
                             acc[2] += g[0] * v[q];
@@ -564,7 +564,8 @@ __global__ void __launch_bounds__(kCT, 1) sv_chain_kernel(SvArgs a) {
         }   // time loop
 
         // ---------------- tail (:540-562, Q6; exact pairing: slots NOBS-LAG+1 .. NOBS-1, pairs under the final weights;
-        // predictive: the same slots, k = 0 adds the final generation's term into slot T)
+        // predictive: the same slots, k = 0 adds the final generation's term into slot T).  n_obs >= LAG + 1, so the
+        // tail's pairs start at x_2 and the pair (x_0, x_1) is the main loop's)
         if (SMO && status == 0) {
             const int T = NOBS - 1;
             const double S_T = s_S[T % kMaxLagC];

@@ -974,7 +974,7 @@ __global__ void __launch_bounds__(GT, 1) sv_grid_kernel(const GridArgs a_in, con
             // Q7: the "current" state is particles[t - 1 + ancestor] read through the flat layout = sorted value
             // `sl` of time tq (table of the first SQ sorted values of every generation), or the unsorted new value
             // `sl` of this generation (complete only after barrier 1: deferred), or 0.  Q8: obs[t - LAG] wraps.
-            // Generic Hessian branch: the child's term is score_main of its own pair (parent value from the payload
+            // Generic Hessian branch: the child's term is pair_score of its own pair (parent value from the payload
             // this thread wrote in phase A1, y = obs[t - 1]); the record's second sector takes the child's cumulative
             // alpha, the payload's second sector the parent's (alpha_k of the pair (x_k, x_k+1) the payload holds).
             const double yi = a.obs[t], ylagH = SVH ? obs_wrap(a.obs, t - L, NOBS) : 0.0;
@@ -1025,7 +1025,8 @@ __global__ void __launch_bounds__(GT, 1) sv_grid_kernel(const GridArgs a_in, con
                             st_stream_f64x4(&Pc[(size_t)j * RS + 1], pol_stream, c0, c1, c2, c3);
                         } else if constexpr (GENH) {
                             double g[4];
-                            M::score_main(s_k, __ldcg(&((const PEntry*)Pc)[(size_t)j * RS].c), xn[k0 + u], ypair, g);
+                            pair_score<M>(s_k, t == 1, __ldcg(&((const PEntry*)Pc)[(size_t)j * RS].c), xn[k0 + u],
+                                          ypair, g);
                             st_keep_f64x4(&Rc[(size_t)j * RS + 1], pol_rst, pa0[u].x + g[0], pa0[u].y + g[1],
                                           pa1[u].x + g[2], pa1[u].y + g[3]);
                             st_stream_f64x4(&Pc[(size_t)j * RS + 1], pol_stream, pa0[u].x, pa0[u].y, pa1[u].x, pa1[u].y);
@@ -1454,7 +1455,7 @@ __global__ void __launch_bounds__(GT, 1) sv_grid_kernel(const GridArgs a_in, con
                 for (int i = 0; i < 4; ++i) hm[i] = 0.0;
             }
             if constexpr (GEN) {
-                // generic path: sc[0] = sum sh curr (smoother), sc[1 + k] = sum sh g[k] of M::score_main on the pair
+                // generic path: sc[0] = sum sh curr (smoother), sc[1 + k] = sum sh g[k] of pair_score on the pair
                 // (curr, next) = (parent value, own value) of the ancestor = (x_tt, x_tt+1), tt = t - LAG + 1;
                 // y = obs[t - LAG] (Q5), obs[tt + 1], or obs[tt] (predictive)
                 const double yl = a.obs[pair_obs(M::kPairing, t - L + 1)];
@@ -1481,7 +1482,7 @@ __global__ void __launch_bounds__(GT, 1) sv_grid_kernel(const GridArgs a_in, con
                             sc[0] = fma(wd, pc[u], sc[0]);
                             if constexpr (!M::kScoreIsZero) {
                                 double g[4];
-                                M::score_main(s_k, pc[u], px[u], yl, g);
+                                pair_score<M>(s_k, t == L - 1, pc[u], px[u], yl, g);
 #pragma unroll
                                 for (int i = 0; i < 4; ++i) sc[1 + i] = fma(wd, g[i], sc[1 + i]);
                             }
@@ -1623,8 +1624,8 @@ __global__ void __launch_bounds__(GT, 1) sv_grid_kernel(const GridArgs a_in, con
                         ld_f64x4(pp, pol_pld, pc, d1, d2, px);
                         ld_f64x4(pp + 1, pol_pld, al[0], al[1], al[2], al[3]);
                         double g[4], hh[10];
-                        M::score_main(s_k, pc, px, yl, g);
-                        M::hess_main(s_k, pc, px, yl, hh);
+                        pair_score<M>(s_k, t == L - 1, pc, px, yl, g);
+                        pair_hess<M>(s_k, t == L - 1, pc, px, yl, hh);
                         louis_add(hh, g, al, s_sh[q], h1, h2);
                     }
                 }
@@ -1703,7 +1704,8 @@ __global__ void __launch_bounds__(256) grid_reduce_kernel(const double* __restri
 // HESS: partH[irel][block][0..19] = the hessian1 / hessian2 terms of :564-626 (alpha of the ancestor LAG-2 steps
 // back of the final particle, weights W_i, obs[i - LAG] with wrap-around, Q8); for a generic model the upper triangles
 // of hessian1 / hessian2 of the same pairs as the gradient (M::hess_main, and M::hess_last with the final particle's own
-// alpha for irel = L - 1).  M: the model (g = M::score_tail).
+// alpha for irel = L - 1).  M: the model (g = M::score_tail).  n_obs >= 2 LAG, so the pairs start at x_LAG+1 here: the
+// pair (x_0, x_1) (pair_score) is the persistent kernel's.
 template <bool HESS, class M>
 __global__ void __launch_bounds__(256) grid_tail_kernel(GridArgs a, const double* __restrict__ sums,
                                                         double* __restrict__ part, double* __restrict__ partH,

@@ -169,6 +169,9 @@ def flps_model_corr(model_id, obs, params, rvr, u, lag=10, store_history=False, 
     the series shifted by one (obs[1:]) and their log_like lacks log p(y_1); model 4 adds model 2 a gradient whose slot
     k holds the contribution of obs[1:][k], so that the slots sum to the score of the full log-likelihood
     (include/pmmh_qn.h).  Model 6 is model 4 here, bit for bit (its Hessian: flps_model_batch_corr).
+    _lib.MODEL_SV_LEVERAGE_EXACT (8) runs model 0's particle system on the same inputs (filt, log_like, traj, diag and
+    history bit-identical) with the exact fixed-lag score: slot k holds the transition (x_k, x_k+1) scored with obs[k],
+    the slots sum to an estimate of the score of log_like (its Hessian: flps_model_batch_corr).
     No fallback pass: diag[:, PMMH_DIAG_STATUS] == 1 reports an abandoned evaluation."""
     return _model_corr("flps_model", model_id, obs, params, rvr, u, lag, 0, store_history, workspace)
 
@@ -178,7 +181,7 @@ def filter_model_corr(model_id, obs, params, rvr, u, store_history=False, worksp
     diag of [B] problems without the fixed-lag smoother -- bit-identical to those outputs of flps_model_corr
     for any lag.  Up to 4096 particles: any B (chain kernel, diag kernel 3).  Above: B == 1 and up to 7168
     particles per SM (grid kernel, diag kernel 5).  n_obs >= 2; other sizes raise PmmhError.  ``model_id`` and
-    params as for flps_model_corr (models 4 and 6 run model 2's filter).  No fallback pass: diag[:, PMMH_DIAG_STATUS] == 1 reports an abandoned
+    params as for flps_model_corr (models 4 and 6 run model 2's filter, model 8 model 0's).  No fallback pass: diag[:, PMMH_DIAG_STATUS] == 1 reports an abandoned
     evaluation."""
     return _model_corr("filter_model", model_id, obs, params, rvr, u, 2, 0, store_history, workspace)
 
@@ -201,7 +204,8 @@ def flps_model_batch_corr(model_id, obs, params, rvr, u, lag=10, compute_hessian
     ceil(N / 2048)); model ids as for flps_model_corr; compute_hessian for _lib.MODEL_SV_LEVERAGE (the reference's
     Hessian branch) and _lib.MODEL_LINEAR_GAUSSIAN_FA_HESS (Louis' identity on model 4's pairs and weights:
     hess1 + hess2 - g g', g = the summed gradient slots, estimates the Hessian of the full log-likelihood over
-    (phi, sigma_v, sigma_e); row and column 3 are 0).  Every other output of model 6 is model 4's, bit for bit, with
+    (phi, sigma_v, sigma_e); row and column 3 are 0), and _lib.MODEL_SV_LEVERAGE_EXACT (the same identity on model 8's
+    pairs, over (mu, atanh phi, log sigma_v, atanh rho)).  Every other output of model 6 is model 4's, bit for bit, with
     compute_hessian 0 or 1.  Returns the dict of flps_model_corr, plus hess1 / hess2 [B, 4, 4] with compute_hessian.  No fallback pass: diag[:, PMMH_DIAG_STATUS] == 1 reports an abandoned
     problem, the others are unaffected."""
     return _model_corr("flps_model_batch", model_id, obs, params, rvr, u, lag, int(bool(compute_hessian)),

@@ -7,20 +7,27 @@ then published chain by chain with the host logic of `ParticleMethodsCUDA` (same
 rvs per chain: a NumPy array in the reference's (NOBS, N+1) layout (stacked, uploaded, split on the device)
 or a `DeviceRVS` handle.  Handles that are rows b = 0..B-1 of one [B, NOBS, N] tensor (as `BatchedRVSState`
 hands them out) are used in place; others are stacked (one device copy).
+
+pairing='exact' evaluates the batch with the SV model's exact fixed-lag smoother (model id 8, as
+ParticleMethodsCUDA(pairing='exact')): one `pmmh_flps_model_corr` launch (chain kernel; the grid kernel for a
+batch of one above 4096 particles), or one `pmmh_flps_model_batch_corr` launch (grid kernel, one team per chain)
+when a chain wants the Hessian or a batch exceeds 4096 particles.
 """
 import numpy as np
 import torch
 from scipy.stats import norm
 
 from ... import kernels as K
+from ..._lib import MODEL_SV_LEVERAGE_EXACT
 from ...parameter.rvs import DeviceRVS
 from .cuda import ParticleMethodsCUDA
 
 
 class BatchedParticleMethodsCUDA(object):
-    def __init__(self, model, no_particles=75, fixed_lag=10, device=None, verbose=False):
+    def __init__(self, model, no_particles=75, fixed_lag=10, device=None, verbose=False, pairing='reference'):
         self._one = ParticleMethodsCUDA(model, no_particles=no_particles, fixed_lag=fixed_lag, device=device,
-                                        verbose=verbose)
+                                        verbose=verbose, pairing=pairing)
+        self.pairing = pairing
         self.template = self._one
         self.device = self._one.device
         self.alg_type = self._one.alg_type
@@ -56,6 +63,17 @@ class BatchedParticleMethodsCUDA(object):
         _, u = K.split_rvs(d, n_obs, n)
         return torch.from_numpy(np.ascontiguousarray(rv_r)).to(self.device), u
 
+    def _evaluate_exact(self, obs_d, par, rvr, u, lag, hess):
+        batch, n = u.shape[0], u.shape[2]
+        if hess or (batch > 1 and n > 4096):
+            out = K.flps_model_batch_corr(MODEL_SV_LEVERAGE_EXACT, obs_d, par, rvr, u, lag=lag, compute_hessian=hess,
+                                          workspace=self._workspace)
+        else:
+            out = K.flps_model_corr(MODEL_SV_LEVERAGE_EXACT, obs_d, par, rvr, u, lag=lag, workspace=self._workspace)
+        if not hess:
+            out['hess1'] = out['hess2'] = torch.zeros((batch, 4, 4), dtype=torch.float64, device=self.device)
+        return out
+
     # ------------------------------------------------------------------ the batch
     def evaluate_batch(self, requests):
         if not requests:
@@ -75,8 +93,11 @@ class BatchedParticleMethodsCUDA(object):
                 else:
                     rvs_list.append(np.random.normal(size=self.dim_rvs))
             rvr, u = self._stack_rvs(rvs_list)
-            out = K.flps_sv_corr(obs_d, torch.from_numpy(params).to(self.device), rvr, u,
-                                 lag=self.settings['fixed_lag'], compute_hessian=hess, workspace=self._workspace)
+            par, lag = torch.from_numpy(params).to(self.device), self.settings['fixed_lag']
+            if self.pairing == 'exact':
+                out = self._evaluate_exact(obs_d, par, rvr, u, lag, hess)
+            else:
+                out = K.flps_sv_corr(obs_d, par, rvr, u, lag=lag, compute_hessian=hess, workspace=self._workspace)
             self.no_launches += 1
             host = {k: out[k].cpu().numpy() for k in ("filt", "smo", "log_like", "gradient", "traj", "hess1", "hess2", "diag")}
         except Exception as e:      # the whole batch failed: every chain rejects (cython.py:133-137 per chain)

@@ -7,6 +7,12 @@ samplers read them (parameter/mcmc/base_class.py:100-101,169-183).  The referenc
 NPART / NOBS / LAG into its Cython module at compile time
 (stochastic_volatility.pyx:17-19); here they are constructor arguments.
 
+``pairing='exact'`` runs the SV model's exact fixed-lag smoother instead (model id 8,
+include/pmmh_qn.h PMMH_MODEL_SV_LEVERAGE_EXACT): the same particle system, with every transition
+scored against its own leverage observation, and a Hessian by Louis' identity published as
+hess1 + hess2 - g g'.  The default ``'reference'`` reproduces the reference, quirks Q5 / Q6 / Q9
+included.
+
 ``rvs={'rvs': x}`` accepts either the reference's (n_obs, N+1) NumPy array or a device-resident
 ``DeviceRVS`` handle (pmmh-qn_b200/parameter/rvs.py).  Without ``rvs`` fresh normals are drawn
 as the reference does (cython.py:60,93).
@@ -16,7 +22,7 @@ import torch
 from scipy.stats import norm
 
 from ... import kernels as K
-from ..._lib import BPF_INTENDED, BPF_PARITY, DIAG_NEAR_TIES, DIAG_STATUS, PmmhError
+from ..._lib import BPF_INTENDED, BPF_PARITY, DIAG_NEAR_TIES, DIAG_STATUS, MODEL_SV_LEVERAGE_EXACT, PmmhError
 from ...parameter.rvs import DeviceRVS
 from ..base_state_inference import BaseStateInference
 
@@ -25,12 +31,15 @@ class ParticleMethodsCUDA(BaseStateInference):
     """Bootstrap particle filter and fixed-lag particle smoother (CUDA, sm_100a)."""
 
     def __init__(self, model, no_particles=75, fixed_lag=10, device=None,
-                 bpf_read_mode='parity', ctas_per_problem=0, verbose=False):
+                 bpf_read_mode='parity', ctas_per_problem=0, verbose=False, pairing='reference'):
         self.alg_type = 'particle'
         if model.short_name != 'sv':
             raise NameError("CUDA implementation for model missing.")
+        if pairing not in ('reference', 'exact'):
+            raise ValueError("pairing must be 'reference' or 'exact'")
         if not torch.cuda.is_available():
             raise RuntimeError("ParticleMethodsCUDA needs a CUDA device; there is no CPU fallback.")
+        self.pairing = pairing
         self.device = torch.device(device) if device is not None else torch.device('cuda', torch.cuda.current_device())
         self.bpf_read_mode = {'parity': BPF_PARITY, 'intended': BPF_INTENDED}[bpf_read_mode]
         self.ctas_per_problem = int(ctas_per_problem)
@@ -39,6 +48,8 @@ class ParticleMethodsCUDA(BaseStateInference):
         self.stream_min_particles = 1 << 15   # below this the upload is too small to be worth overlapping
         self._obs_cache = None
         self._init_particle_method(model, int(no_particles), int(fixed_lag), verbose)
+        if pairing == 'exact':
+            self._check_exact_sizes(model)
         self.results = {}
         self.diagnostics = {}
 
@@ -95,6 +106,28 @@ class ParticleMethodsCUDA(BaseStateInference):
             return None
         return out
 
+    def _check_exact_sizes(self, model):
+        """raises PmmhError on the sizes the model entries refuse (the smoother's; the Hessian's when the model asks
+        for it)"""
+        n_obs, n, lag = self.no_obs, self.no_particles, self.settings['fixed_lag']
+        if n_obs < lag + 1:
+            raise PmmhError("pairing='exact' needs n_obs >= lag + 1")
+        K._workspace_bytes("pmmh_flps_model_workspace_bytes", n_obs, n, lag, 1)
+        if model.using_hessians:
+            K._workspace_bytes("pmmh_flps_model_batch_workspace_bytes", n_obs, n, lag, 1, 1)
+
+    def _smoother_exact(self, obs_d, params, hessian_flag, kwargs):
+        """model 8 on the uploaded rvs: flps_model_corr, or flps_model_batch_corr with the Hessian"""
+        rvr, u = self._rvs_device(kwargs)
+        par = torch.from_numpy(params).to(self.device)
+        lag = self.settings['fixed_lag']
+        if hessian_flag:
+            return K.flps_model_batch_corr(MODEL_SV_LEVERAGE_EXACT, obs_d, par, rvr, u, lag=lag, compute_hessian=1,
+                                           workspace=self._workspace)
+        out = K.flps_model_corr(MODEL_SV_LEVERAGE_EXACT, obs_d, par, rvr, u, lag=lag, workspace=self._workspace)
+        out['hess1'] = out['hess2'] = torch.zeros((1, 4, 4), dtype=torch.float64, device=self.device)
+        return out
+
     @staticmethod
     def _to_host(tensors):
         flat = torch.cat([t.reshape(-1).to(torch.float64) for t in tensors]).cpu().numpy()
@@ -136,7 +169,9 @@ class ParticleMethodsCUDA(BaseStateInference):
             _, obs_d = self._obs_device(model)
             params = np.asarray(model.get_all_params(), dtype=np.float64)
             out = None
-            if not hessian_flag and 'rvs' in kwargs:
+            if self.pairing == 'exact':
+                out = self._smoother_exact(obs_d, params, hessian_flag, kwargs)
+            elif not hessian_flag and 'rvs' in kwargs:
                 out = self._smoother_streamed(kwargs['rvs']['rvs'], obs_d, params)
             if out is None:
                 rvr, u = self._rvs_device(kwargs)
@@ -164,7 +199,10 @@ class ParticleMethodsCUDA(BaseStateInference):
             grad[np.isinf(grad)] = 0.0
             grad[np.isnan(grad)] = 0.0
             grad_est = np.nansum(grad, axis=1)
-        if model.using_hessians:
+        if model.using_hessians and self.pairing == 'exact':
+            hessian_est = np.outer(grad_est, grad_est) - (np.array(hess1).reshape((model.no_params, model.no_params)) +
+                                                          np.array(hess2).reshape((model.no_params, model.no_params)))
+        elif model.using_hessians:
             part1 = np.inner(grad_est, grad_est)
             part2 = np.array(hess1).reshape((model.no_params, model.no_params))
             part2 += np.array(hess2).reshape((model.no_params, model.no_params))
@@ -194,7 +232,8 @@ class ParticleMethodsCUDA(BaseStateInference):
                          'initial_state': 0.0,
                          'generate_initial_state': True,
                          'estimate_gradient': True,
-                         'estimate_hessian': True
+                         'estimate_hessian': True,
+                         'pairing': self.pairing
                          }
         self.no_obs = no_obs
         self.no_particles = no_particles
