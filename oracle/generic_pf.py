@@ -201,7 +201,8 @@ def flps_generic(model, obs, rvr, rvp, n_particles, lag=10, dumps=False):
             if idx - 1 >= 0:
                 nxt = ph[idx - 1]
                 y1 = obs[i - 1] if i - 1 >= 0 else obs[i - 1 + nobs]
-                grad[:, i - L + 1] += np.sum(model.score_tail(curr, nxt, y1) * W[i], axis=1)
+                if i - L + 1 >= 0:                                 # slot < 0 (nobs <= 2L - 2): dropped, not wrapped (DESIGN §2)
+                    grad[:, i - L + 1] += np.sum(model.score_tail(curr, nxt, y1) * W[i], axis=1)
     else:
         for t in range(nobs - L + 1, nobs):                        # tail: final weights, one step after the main loop
             k = nobs - 1 - t

@@ -429,11 +429,16 @@ int oracle_flps_sv_corr(const double *obs, const double *params, const double *r
                 g[3] = rho;
                 g[3] -= q_matrix * rho * sq * sq;
                 g[3] += q_matrix * sq * sigmav * exp(-0.5 * curr) * y1 * rho_term;
+                /* Short series (DESIGN.md §2): for NOBS <= 2 LAG - 2 the first tail steps index slot tt < 0,
+                 * outside the reference's C array (undefined there).  Rule: that gradient term is dropped, as
+                 * every kernel drops it; the Hessian sums, which have no slot, keep it. */
                 const int tt = i - LAG + 1;
-                gradient[0 * (size_t)NOBS + tt] += g[0] * Wi[j];
-                gradient[1 * (size_t)NOBS + tt] += g[1] * Wi[j];
-                gradient[2 * (size_t)NOBS + tt] += g[2] * Wi[j];
-                gradient[3 * (size_t)NOBS + tt] += g[3] * Wi[j];
+                if (tt >= 0) {
+                    gradient[0 * (size_t)NOBS + tt] += g[0] * Wi[j];
+                    gradient[1 * (size_t)NOBS + tt] += g[1] * Wi[j];
+                    gradient[2 * (size_t)NOBS + tt] += g[2] * Wi[j];
+                    gradient[3 * (size_t)NOBS + tt] += g[3] * Wi[j];
+                }
                 if (compute_hessian == 1) {
                     double al[NPARAMS];
                     for (int c = 0; c < NPARAMS; c++) al[c] = ah[c][(size_t)(LAG - 2) * N + j];
